@@ -2,6 +2,7 @@
 """Benchmark of the SplitP hot path on B200 (contract: the task statement; metric: BASELINE.json).
 
     python bench.py --gpus N --steps K --warmup W [--workload c2|c3|c4|c5] [--extras c3,c5,c4|none] [--impl reference]
+                    [--dump-outputs DIR]
 
 Headline workload c2 (BASELINE.json configs[1]): balanced 12-taxon Jukes-Cantor tree, branch length 0.05, 1,000,000
 sites (seeded synthetic alignment from bench_inputs.py, identical in both arms), ALL 2,035 splits scored from dense count
@@ -9,10 +10,14 @@ flattenings (4^a x 4^b, 4096 x 4096 for the 462 6|6 splits) through the exact-in
 One step = one pass of the whole path: pack -> pattern count -> (count allreduce) -> per split flatten + Gram +
 high-part correction + score -> (score all-gather).
 
-The same JSON line carries a `workloads` object with the other BASELINE configs, each measured the same way (fewer
-steps): c3 (configs[2], the north-star target: 20-taxon GTR tree, 10M sites, subflattening scores of all 524,267 splits),
+The same JSON line carries a `workloads` object with the other BASELINE configs, each measured the same way (same number of
+timed steps): c3 (configs[2], the north-star target: 20-taxon GTR tree, 10M sites, subflattening scores of all 524,267 splits),
 c5 (configs[4]: 10^5 random splits of a 32-taxon tree) and c4 (configs[3] scaled to 10M sites: 64 taxa, 128-bit pattern
 compression + thin reduced-flattening scores).
+
+`--dump-outputs DIR` writes the scores that each GPU workload's last timed step returned, DIR/<workload>_scores.npy (float64,
+split-list order), and names the file under `dumped` in that workload's result (null when the workload failed).  Every input
+is generated from a fixed seed, so two builds of the project can be compared output for output.
 
 N > 1 (torchrun): splits are sharded for scoring; sites are sharded for counting (exchange of the compacted pattern lists /
 integer allreduce of the pair statistics) unless counting the whole alignment on every rank is cheaper than that exchange
@@ -85,7 +90,15 @@ def parse():
     ap.add_argument("--sites", type=int, default=None, help="override the number of sites of the headline workload")
     ap.add_argument("--max-splits", type=int, default=None, help="score only the first M splits (debug runs)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the scores of every GPU workload's last timed step to DIR/<workload>_scores.npy (float64, one "
+                         "per split in split-list order; under 4.2 MB per workload), to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
+    return args
 
 
 def split_list(wl, max_splits=None):
@@ -226,6 +239,8 @@ def load_reference():
     """The pip-installed, unmodified js51/SplitP from the git-ignored baseline/_ref (None when it did not travel)."""
     ref_dir = os.path.join(ROOT, "baseline", "_ref")
     if not os.path.isdir(os.path.join(ref_dir, "splitp")):
+        print("[bench] baseline/_ref not installed (build() with SPLITP_REFERENCE set installs it): the CPU baseline is the "
+              "oracle port", file=sys.stderr)
         return None
     if ref_dir not in sys.path:
         sys.path.insert(0, ref_dir)
@@ -416,7 +431,7 @@ def reference_arm(args):
     sites = wl["sites"] if wl["method"] == "flattening" else min(wl["sites"], 1_000_000)
     codes = BI.simulate_codes(wl["n"], wl["bl"], wl["model"], sites, wl["seed"])
     vals, cb = [], None
-    steps = max(args.steps, 1)
+    steps = args.steps
     for _ in range(args.warmup):  # warm-up: page in LAPACK / the reference, smallest size class only
         if wl["method"] == "flattening":
             cpu_flattening_sample(name, wl, codes[:, : min(sites, 100_000)], idx_all, sizes={2})
@@ -573,6 +588,7 @@ def gpu_workload(name, wl, args, ctx, steps, warmup, max_splits=None, cpu_baseli
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = int(eng.lib.spb_launch_count()) - launches0
+    sc = scores.cpu().numpy()  # the last timed step's scores, taken before the passes below run the path again
     clocks = sampler.stop()
     step_ms = [a.elapsed_time(b) for a, b in evs]
     t = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
@@ -712,7 +728,9 @@ def gpu_workload(name, wl, args, ctx, steps, warmup, max_splits=None, cpu_baseli
            "clocks": clocks, "e2e": e2e, "gpu_launches": launches, "roofline": roof}
     if count_roof:
         out["roofline_count"] = count_roof
-    sc = scores.cpu().numpy()
+    if args.dump_outputs:
+        np.save(os.path.join(args.dump_outputs, f"{name}_scores.npy"), sc.astype(np.float64, copy=False))
+        out["dumped"] = f"{name}_scores.npy"
     checks = {"finite": bool(np.isfinite(sc).all()), "host_equals_device": bool(np.array_equal(sc, host_scores.numpy()))}
     if partition is not None:
         out["partition"] = partition
@@ -750,6 +768,8 @@ def main():
     from splitp_b200 import distributed as spd
     eng = sp.engine
     rank, local, world = spd.init_from_env()
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
     dev = eng.device()
     peaks = {}
     try:
@@ -777,10 +797,12 @@ def main():
         wl_x = dict(WORKLOADS[ex])
         t0 = time.perf_counter()
         try:
-            r = gpu_workload(ex, wl_x, args, ctx, steps=max(1, min(args.steps, 2)), warmup=3, max_splits=EXTRA_SPLIT_CAP.get(ex),
+            r = gpu_workload(ex, wl_x, args, ctx, steps=args.steps, warmup=3, max_splits=EXTRA_SPLIT_CAP.get(ex),
                              cpu_baseline=(ex != "c4"))
         except Exception as exc:  # noqa: BLE001  (an extra workload must never take the headline line down with it)
             r = {"error": f"{type(exc).__name__}: {exc}"} if rank == 0 else None
+            if r is not None and args.dump_outputs:
+                r["dumped"] = None  # no DIR/<name>_scores.npy for a workload that failed
         torch.cuda.empty_cache()
         if rank == 0 and r is not None:
             r["bench_wall_s"] = round(time.perf_counter() - t0, 2)

@@ -457,3 +457,34 @@ def test_solver_compacts_stragglers_in_a_large_batch(sp, eng, oracle):
     for t in (0, 3, 20):
         one = float(eng.score_gram(G[t:t + 1])[0].item())
         assert_score(one, scores[t])
+
+
+# ---------------------------------------------------------------------------------------------
+# bench.py --dump-outputs: the scores of the last timed step
+# ---------------------------------------------------------------------------------------------
+def test_bench_dump_outputs_holds_the_workload_scores(sp, oracle, tmp_path):
+    """bench.py --steps 2 --dump-outputs DIR on c2 at 20,000 sites (all 2,035 splits): the JSON line reports two timed steps and
+    names the dump, and DIR/c2_scores.npy holds one float64 score per split.  Every 32nd split (64 of them, every side size
+    2 .. 6, so the 6|6 tensor-core Gram path too) is within the score tolerance of the oracle's score of the same seeded
+    alignment."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    import bench_inputs as BI
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "0", "--sites", "20000",
+                        "--extras", "none", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout)
+    assert line["steps"] == 2 and len(line["ms_steps_rank0"]) == 2 and line["dumped"] == "c2_scores.npy"
+    got = np.load(tmp_path / "c2_scores.npy")
+    idx = BI.all_splits_idx(12)
+    assert got.dtype == np.float64 and got.shape == (len(idx),) == (2035,)
+    keys, counts, usable = oracle.get_pattern_counts_arrays(BI.simulate_codes(12, 0.05, "JC", 20_000, 2))
+    picks = range(0, len(idx), 32)
+    assert {min(len(idx[s][0]), len(idx[s][1])) for s in picks} == {2, 3, 4, 5, 6}
+    for s in picks:
+        ia, ib = idx[s]
+        assert_score(got[s], oracle.split_score(oracle.flattening_reduced(keys, counts / usable, 12, ia, ib)))

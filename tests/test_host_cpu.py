@@ -2,6 +2,7 @@
 host logic (split enumeration, tree topology, pattern encoding, sharding) and the N>1 plumbing over gloo.
 No compute calls are made here (there is no GPU in the build container)."""
 import ctypes
+import json
 import os
 import re
 import subprocess
@@ -396,12 +397,57 @@ def test_simulate_codes_accepts_reference_phylogeny_like_tree():
     assert p > 1e-4, (p, stat, dof)
 
 
-def test_as_tree_on_the_real_reference_phylogeny():
-    """With the unmodified reference installed in baseline/_ref: splitp.trees.balanced_newick_tree -> trees.as_tree gives
-    the topology, leaf names, taxa order and branch lengths of trees.balanced_tree (same true splits)."""
+def _phylogeny_from_splits(taxa, splits, branch_length):
+    """A Phylogeny-shaped object (the attributes trees.as_tree reads: .networkx_graph, a DiGraph parent -> child with the
+    branch above each node in its `branch_length` attribute, leaves named by taxon; .taxa) of the rooted binary tree with
+    these true splits, rooted on its one split into equal halves (the root of a balanced tree)."""
+    import networkx as nx
+    everyone = frozenset(taxa)
+    halves = [frozenset(a) for a, b in splits if len(a) == len(b)]
+    assert len(halves) == 1
+    x, y = halves[0], everyone - halves[0]
+    clades = {x, y} | {frozenset([t]) for t in taxa}
+    for a, b in splits:
+        a = frozenset(a)
+        clades.add(a if a <= x or a <= y else everyone - a)  # the side that lies within one half hangs below the root
+    label = {c: next(iter(c)) if len(c) == 1 else "(" + ",".join(sorted(c)) + ")" for c in clades}
+    label[everyone] = "root"
+    g = nx.DiGraph()
+    g.add_node("root", branch_length=None)
+    for c in clades:
+        g.add_node(label[c], branch_length=branch_length)
+    for c in clades:
+        g.add_edge(label[min((p for p in clades | {everyone} if c < p), key=len)], label[c])
+
+    class Phylogeny:
+        networkx_graph = g
+    Phylogeny.taxa = list(taxa)
+    return Phylogeny()
+
+
+def test_as_tree_on_the_real_reference_phylogeny(golden_readme):
+    """The trees the unmodified reference's splitp.trees.balanced_newick_tree returned, as recorded in tests/golden by
+    make_golden.py (taxa and true splits: n = 6 and 8 at branch length 0.1 in golden_erickson.json, n = 10 at 0.05 in
+    golden_readme.npz), rebuilt as Phylogeny-shaped objects: trees.as_tree gives the reference's taxa, taxa order and splits
+    and the branch lengths of the graph, and trees.balanced_tree gives the same taxa, splits and branch lengths.
+    With the reference itself installed in baseline/_ref, its own Phylogeny objects for n = 4 .. 20 are converted too."""
+    from splitp_b200 import trees
+    with open(os.path.join(ROOT, "tests", "golden", "golden_erickson.json")) as f:
+        cases = [(rec["n"], 0.1, [[list(a), list(b)] for a, b in rec["true_splits"]]) for rec in json.load(f)]
+    cases.append((10, 0.05, [[list(a), list(b)] for a, b in (s.split("|") for s in golden_readme["true_splits"].tolist())]))
+    for n, bl, splits in cases:
+        taxa = sorted({t for s in splits for side in s for t in side})
+        if n == 10:
+            assert taxa == [str(t) for t in golden_readme["taxa"]]
+        assert len(taxa) == n and len(splits) == n - 3
+        conv, own = trees.as_tree(_phylogeny_from_splits(taxa, splits, bl)), trees.balanced_tree(n, bl)
+        want = {(tuple(a), tuple(b)) for a, b in splits}
+        assert list(conv.taxa) == list(own.taxa) == taxa
+        assert set(conv.splits()) == set(own.splits()) == want
+        assert sorted(conv.branch_length) == sorted(own.branch_length) == [0.0] + [bl] * (2 * n - 2)
     ref_dir = os.path.join(ROOT, "baseline", "_ref")
     if not os.path.isdir(os.path.join(ref_dir, "splitp")):
-        pytest.skip("baseline/_ref not installed")
+        return
     code = (
         "import sys; sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
         "import warnings; warnings.simplefilter('ignore')\n"
@@ -416,6 +462,30 @@ def test_as_tree_on_the_real_reference_phylogeny():
         "print('ok')\n" % (ref_dir, ROOT))
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-2000:]
+
+
+def test_install_reference_is_offline_and_leaves_the_source_alone(tmp_path):
+    """__graft_entry__.install_reference (what build() runs when SPLITP_REFERENCE names the reference's source tree) installs
+    a pure-Python package without an index into the target, builds from a copy (the source tree stays untouched and may be
+    read-only), and refuses a directory that holds no splitp/ package."""
+    import __graft_entry__
+    src = tmp_path / "SplitP"
+    (src / "splitp").mkdir(parents=True)
+    (src / "splitp" / "__init__.py").write_text("VERSION = '0.3.2'\n")
+    (src / "setup.py").write_text("from setuptools import setup\nsetup(name='splitp', version='0.3.2', packages=['splitp'])\n")
+    before = sorted(p.relative_to(src) for p in src.rglob("*"))
+    for p in src.rglob("*"):
+        p.chmod(p.stat().st_mode & ~0o222)
+    src.chmod(src.stat().st_mode & ~0o222)
+    try:
+        __graft_entry__.install_reference(str(src), str(tmp_path / "_ref"))
+    finally:
+        for p in [src, *src.rglob("*")]:
+            p.chmod(p.stat().st_mode | 0o200)
+    assert (tmp_path / "_ref" / "splitp" / "__init__.py").read_text() == "VERSION = '0.3.2'\n"
+    assert sorted(p.relative_to(src) for p in src.rglob("*")) == before
+    with pytest.raises(FileNotFoundError):
+        __graft_entry__.install_reference(str(tmp_path / "_ref" / "splitp"), str(tmp_path / "other"))
 
 
 def test_warp2_scorer_model_against_lapack(oracle):
