@@ -127,6 +127,18 @@ int64_t spb_thin_filter_words(int64_t cap);
 int spb_thin_gram_wide_filtered(const uint64_t* d_hkeys, const uint32_t* d_hcounts, int64_t cap, const uint64_t* d_special,
                                 int n_taxa, const uint8_t* h_idx_a, int a, uint32_t* d_filter, int64_t filter_words,
                                 double* d_G, void* stream);
+/* Pattern LISTS with 128-bit keys (d_keys uint64 [num][2] = {lo, hi}, 16-byte aligned), e.g. a {pattern: value} mapping of
+ * 32..64 taxa.  Projection: the digits of the m <= n_taxa positions h_pos (HOST array, most significant first) of every key,
+ * as a base-4 number: d_out uint64 [num] for m <= 31 (flattening row / column indices), uint64 [num][2] {lo, hi} (16-byte
+ * aligned) for m >= 32 (keys of a sub-alignment). */
+int spb_project_wide(const uint64_t* d_keys, int64_t num, int n_taxa, const uint8_t* h_pos, int m, uint64_t* d_out, void* stream);
+/* Joint tables N double [n][n][4][4] (N[i][j][x][y] = sum of the values d_vals[p] of the patterns with taxon i in state x
+ * and taxon j in state y; written in full) of a weighted pattern list, for spb_pair_transform.  Computed as E^T diag(v) E
+ * (E = one-hot digits) on the fp64 tensor cores with a fixed summation order: bitwise reproducible, exact for
+ * integer values below 2^53.  Values must be finite.  d_ws: double [spb_pair_tables_wide_ws(num, n_taxa)]. */
+int64_t spb_pair_tables_wide_ws(int64_t num, int n_taxa);
+int spb_pair_tables_wide(const uint64_t* d_keys, const double* d_vals, int64_t num, int n_taxa, double* d_N, double* d_ws,
+                         void* stream);
 
 /* ---- a7-a10: flattening (constructions.py:7-102) ---- */
 /* value kinds for the pattern table handed to the flattening kernels */

@@ -94,6 +94,9 @@ PROTOTYPES = {
     "spb_thin_gram_wide": (_i, [_p, _p, _l, _p, _i, C.c_char_p, _i, _p, _p]),
     "spb_thin_filter_words": (_l, [_l]),
     "spb_thin_gram_wide_filtered": (_i, [_p, _p, _l, _p, _i, C.c_char_p, _i, _p, _l, _p, _p]),
+    "spb_project_wide": (_i, [_p, _l, _i, C.c_char_p, _i, _p, _p]),
+    "spb_pair_tables_wide_ws": (_l, [_l, _i]),
+    "spb_pair_tables_wide": (_i, [_p, _p, _l, _i, _p, _p, _p]),
     "spb_flatten_coo": (_i, [_p, _l, _sp, _p, _p, _p]),
     "spb_flatten_dense": (_i, [_p, _p, _i, _d, _l, _sp, _p, _p]),
     "spb_flatten_dense_w": (_i, [_p, _p, _i, _d, _l, _sp, _p, _p, _p]),

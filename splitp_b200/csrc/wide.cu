@@ -14,6 +14,10 @@
 //                        distinct patterns of the other taxa; G[r1][r2] = sum over patterns p with row part r1 of
 //                        count(p) * count(p with its row part replaced by r2) -- one hash lookup per (p, r2), no
 //                        sort and no 4^b-sized index.  All-zero rows drop out of the score by themselves.
+//   spb_project_wide     digits of an ordered list of taxon positions of every key of a pattern list: flattening row /
+//                        column indices (sides of <= 31 taxa) and the keys of a sub-alignment
+//   spb_pair_tables_wide joint 4x4 tables of every taxon pair of a weighted pattern list ({pattern: value} mappings),
+//                        N = E^T diag(v) E on the fp64 tensor cores; deterministic, exact for integer values
 #include "common.cuh"
 
 using namespace spb;
@@ -295,6 +299,151 @@ __global__ void __launch_bounds__(256) thin_gram_wide_kernel(const unsigned long
   }
 }
 
+// ---- pattern lists with 128-bit keys ({pattern: value} mappings of 32..64 taxa) ----
+
+struct Projection {
+  int m;                      // positions read, most significant first
+  uint8_t shift[SPB_MAX_TAXA];  // bit position of each position's digit inside the 128-bit key
+};
+
+// digits of `pr` positions of every key, packed base 4: a uint64 word per key for m <= 31, a {lo, hi} key for more
+__global__ void __launch_bounds__(256) project_wide_kernel(const unsigned long long* __restrict__ keys, int64_t num, Projection pr,
+                                                           unsigned long long* __restrict__ out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= num) return;
+  const ulonglong2 v = __ldg(reinterpret_cast<const ulonglong2*>(keys + 2 * i));
+  const Key128 k{v.x, v.y};
+  unsigned long long lo = 0, hi = 0;
+  for (int t = 0; t < pr.m; ++t) {
+    hi = (hi << 2) | (lo >> 62);
+    lo = (lo << 2) | get_digit(k, pr.shift[t]);
+  }
+  if (pr.m <= 31) {
+    out[i] = lo;
+  } else {
+    *reinterpret_cast<ulonglong2*>(out + 2 * i) = make_ulonglong2(lo, hi);
+  }
+}
+
+// Joint tables of every taxon pair from a weighted pattern list: with E the P x 4n one-hot matrix of the digits (column
+// 4 t + x = [taxon t of the pattern is in state x]), N = E^T diag(v) E, i.e. N[4i + x][4j + y] = sum_p v_p [p_i = x][p_j = y].
+// The 4n x 4n product runs on the fp64 tensor cores (DMMA m8n8k4) with the fragments generated from the keys: lane l
+// holds A[l / 4][l % 4] = v_p [digit of row l / 4], B[l % 4][l / 4] = [digit of column l / 4] of pattern p = base + l % 4.
+// Grid: x = pattern chunk, y = 32 x 32 output block of the upper block triangle.  A warp keeps the 4 x 4 tiles of its
+// block in registers over every 4th step of its chunk; the 4 warps are added in warp order and the chunk partials by
+// pair_wide_reduce_kernel in chunk order, so the result does not depend on scheduling.  Products are v * 1 or v * 0:
+// integer-valued tables are summed exactly (below 2^53).  Values must be finite (inf * 0 would spread NaN to the
+// other cells of a row).
+constexpr int kPairWarps = 4;
+constexpr int kPairBlock = 32;                  // output rows / columns per block
+constexpr int64_t kPairChunkMin = 4096;         // patterns per chunk at least ...
+constexpr int64_t kPairChunksMax = 64;          // ... and at most this many chunks (the workspace is chunks x blocks x 8 KB)
+
+__device__ __forceinline__ double one_hot(unsigned long long lo, unsigned long long hi, int shift, uint32_t state, double v) {
+  const uint32_t d = shift < 64 ? (uint32_t)((lo >> shift) & 3ull) : (uint32_t)((hi >> (shift - 64)) & 3ull);
+  return d == state ? v : 0.0;
+}
+
+__device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double b) {
+  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};" : "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
+}
+
+__global__ void __launch_bounds__(32 * kPairWarps) pair_wide_kernel(const unsigned long long* __restrict__ keys, const double* __restrict__ vals,
+                                                                    int64_t num, int n, int nblocks, int64_t chunk, double* __restrict__ ws) {
+  __shared__ double red[kPairWarps][kPairBlock][kPairBlock];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, kq = lane & 3, grp = lane >> 2;
+  int bi = 0, rem = blockIdx.y;
+  while (rem >= nblocks - bi) { rem -= nblocks - bi; ++bi; }
+  const int bj = bi + rem;
+  // row / column 32 b + 8 t + grp of the product = taxon 8 b + 2 t + grp / 4 in state grp % 4; -1 = padding past 4n
+  const uint32_t state = (uint32_t)(grp & 3);
+  int sa[4], sb[4];
+#pragma unroll
+  for (int t = 0; t < 4; ++t) {
+    const int ta = 8 * bi + 2 * t + (grp >> 2), tb = 8 * bj + 2 * t + (grp >> 2);
+    sa[t] = ta < n ? 2 * (n - 1 - ta) : -1;
+    sb[t] = tb < n ? 2 * (n - 1 - tb) : -1;
+  }
+  double acc[4][4][2];
+#pragma unroll
+  for (int a = 0; a < 4; ++a)
+#pragma unroll
+    for (int b = 0; b < 4; ++b) acc[a][b][0] = acc[a][b][1] = 0.0;
+  const int64_t p_begin = (int64_t)blockIdx.x * chunk;
+  const int64_t p_end = min(num, p_begin + chunk);
+  for (int64_t p0 = p_begin + 4 * warp; p0 < p_end; p0 += 4 * kPairWarps) {
+    const int64_t p = p0 + kq;
+    unsigned long long lo = 0, hi = 0;
+    double v = 0.0;
+    if (p < p_end) {
+      const ulonglong2 k = __ldg(reinterpret_cast<const ulonglong2*>(keys + 2 * p));
+      lo = k.x;
+      hi = k.y;
+      v = __ldg(vals + p);
+    }
+    double fa[4], fb[4];
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+      fa[t] = sa[t] >= 0 ? one_hot(lo, hi, sa[t], state, v) : 0.0;
+      fb[t] = sb[t] >= 0 ? one_hot(lo, hi, sb[t], state, 1.0) : 0.0;
+    }
+#pragma unroll
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+      for (int b = 0; b < 4; ++b) dmma884(acc[a][b][0], acc[a][b][1], fa[a], fb[b]);
+  }
+#pragma unroll
+  for (int a = 0; a < 4; ++a)
+#pragma unroll
+    for (int b = 0; b < 4; ++b) {
+      red[warp][8 * a + grp][8 * b + 2 * kq] = acc[a][b][0];
+      red[warp][8 * a + grp][8 * b + 2 * kq + 1] = acc[a][b][1];
+    }
+  __syncthreads();
+  double* out = ws + ((int64_t)blockIdx.x * gridDim.y + blockIdx.y) * (kPairBlock * kPairBlock);
+  for (int e = threadIdx.x; e < kPairBlock * kPairBlock; e += 32 * kPairWarps) {
+    const int r = e / kPairBlock, c = e - r * kPairBlock;
+    double s = red[0][r][c];
+#pragma unroll
+    for (int w = 1; w < kPairWarps; ++w) s += red[w][r][c];
+    out[e] = s;
+  }
+}
+
+// chunk partials -> N double [n][n][4][4]; entries below the block diagonal (and below the diagonal of a diagonal block)
+// are read from their mirror image, so N[j][i] is exactly N[i][j]^T
+__global__ void pair_wide_reduce_kernel(const double* __restrict__ ws, int64_t nchunks, int nblocks, int n, double* __restrict__ N) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (int64_t)n * n * 16) return;
+  const int ij = (int)(idx >> 4), cell = (int)(idx & 15);
+  const int i = ij / n, j = ij - i * n;
+  int r = 4 * i + (cell >> 2), c = 4 * j + (cell & 3);
+  if (r > c) { const int t = r; r = c; c = t; }
+  const int rb = r / kPairBlock, cb = c / kPairBlock;
+  const int blk = rb * nblocks - rb * (rb - 1) / 2 + (cb - rb);
+  const int64_t nbp = (int64_t)nblocks * (nblocks + 1) / 2;
+  const double* src = ws + (int64_t)blk * (kPairBlock * kPairBlock) + (r % kPairBlock) * kPairBlock + (c % kPairBlock);
+  double s = 0.0;
+  for (int64_t q = 0; q < nchunks; ++q) s += src[q * nbp * (kPairBlock * kPairBlock)];
+  N[idx] = s;
+}
+
+// chunk length (a multiple of 16 patterns) and number of chunks of a pattern list: a function of `num` only, so that the
+// summation order -- and with it every bit of the result -- is the same on every device
+void pair_wide_plan(int64_t num, int64_t* chunk, int64_t* nchunks) {
+  int64_t c = (num + kPairChunkMin - 1) / kPairChunkMin;
+  if (c > kPairChunksMax) c = kPairChunksMax;
+  if (c < 1) c = 1;
+  int64_t len = (num + c - 1) / c;
+  len = (len + 15) / 16 * 16;
+  if (len < 16) len = 16;
+  *chunk = len;
+  *nchunks = (num + len - 1) / len;
+  if (*nchunks < 1) *nchunks = 1;
+}
+
+int pair_wide_blocks(int n) { return (4 * n + kPairBlock - 1) / kPairBlock; }
+
 int check_table(const uint64_t* d_hkeys, const uint32_t* d_hcounts, int64_t cap, const char* who) {
   SPB_REQUIRE(d_hkeys && d_hcounts, "%s: NULL table", who);
   SPB_REQUIRE(cap >= 2 && (cap & (cap - 1)) == 0, "%s: capacity must be a power of two", who);
@@ -420,4 +569,55 @@ extern "C" int64_t spb_thin_filter_words(int64_t cap) {
 extern "C" int spb_thin_gram_wide(const uint64_t* d_hkeys, const uint32_t* d_hcounts, int64_t cap, const uint64_t* d_special, int n_taxa,
                                   const uint8_t* h_idx_a, int a, double* d_G, void* stream) {
   return spb_thin_gram_wide_filtered(d_hkeys, d_hcounts, cap, d_special, n_taxa, h_idx_a, a, nullptr, 0, d_G, stream);
+}
+
+extern "C" int spb_project_wide(const uint64_t* d_keys, int64_t num, int n_taxa, const uint8_t* h_pos, int m, uint64_t* d_out,
+                                void* stream) {
+  SPB_REQUIRE(n_taxa >= 1 && n_taxa <= SPB_MAX_TAXA && m >= 0 && m <= n_taxa && num >= 0,
+              "spb_project_wide: bad arguments (n_taxa=%d m=%d)", n_taxa, m);
+  SPB_REQUIRE(m == 0 || h_pos, "spb_project_wide: NULL position list");
+  Projection pr;
+  pr.m = m;
+  for (int t = 0; t < m; ++t) {
+    SPB_REQUIRE(h_pos[t] < n_taxa, "spb_project_wide: position %d out of range (n_taxa=%d)", (int)h_pos[t], n_taxa);
+    pr.shift[t] = (uint8_t)(2 * (n_taxa - 1 - h_pos[t]));
+  }
+  if (num == 0) return SPB_OK;
+  SPB_REQUIRE(d_keys && d_out, "spb_project_wide: NULL buffer");
+  SPB_REQUIRE((reinterpret_cast<uintptr_t>(d_keys) & 15) == 0 && (m <= 31 || (reinterpret_cast<uintptr_t>(d_out) & 15) == 0),
+              "spb_project_wide: 128-bit key arrays must be 16-byte aligned");
+  project_wide_kernel<<<(unsigned)((num + 255) / 256), 256, 0, (cudaStream_t)stream>>>((const unsigned long long*)d_keys, num, pr,
+                                                                                     (unsigned long long*)d_out);
+  SPB_LAUNCH_CHECK();
+  return SPB_OK;
+}
+
+extern "C" int64_t spb_pair_tables_wide_ws(int64_t num, int n_taxa) {
+  if (n_taxa < 1 || n_taxa > SPB_MAX_TAXA || num < 0) return 0;
+  int64_t chunk, nchunks;
+  pair_wide_plan(num, &chunk, &nchunks);
+  const int64_t nb = pair_wide_blocks(n_taxa);
+  return nchunks * (nb * (nb + 1) / 2) * (kPairBlock * kPairBlock);
+}
+
+extern "C" int spb_pair_tables_wide(const uint64_t* d_keys, const double* d_vals, int64_t num, int n_taxa, double* d_N, double* d_ws,
+                                    void* stream) {
+  SPB_REQUIRE(d_N && n_taxa >= 1 && n_taxa <= SPB_MAX_TAXA && num >= 0, "spb_pair_tables_wide: bad arguments (n_taxa=%d)", n_taxa);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t cells = (int64_t)n_taxa * n_taxa * 16;
+  if (num == 0) {
+    SPB_CUDA(cudaMemsetAsync(d_N, 0, (size_t)cells * sizeof(double), st));
+    return SPB_OK;
+  }
+  SPB_REQUIRE(d_keys && d_vals && d_ws, "spb_pair_tables_wide: NULL buffer");
+  SPB_REQUIRE((reinterpret_cast<uintptr_t>(d_keys) & 15) == 0, "spb_pair_tables_wide: the key array must be 16-byte aligned");
+  int64_t chunk, nchunks;
+  pair_wide_plan(num, &chunk, &nchunks);
+  const int nb = pair_wide_blocks(n_taxa);
+  const dim3 grid((unsigned)nchunks, (unsigned)(nb * (nb + 1) / 2));
+  pair_wide_kernel<<<grid, 32 * kPairWarps, 0, st>>>((const unsigned long long*)d_keys, d_vals, num, n_taxa, nb, chunk, d_ws);
+  SPB_LAUNCH_CHECK();
+  pair_wide_reduce_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(d_ws, nchunks, nb, n_taxa, d_N);
+  SPB_LAUNCH_CHECK();
+  return SPB_OK;
 }

@@ -289,9 +289,21 @@ def merge_tables(n, keys, counts, first=None, sort=True):
     return PatternTable(n, ok, counts=oc, first=of)
 
 
+NARROW_MAX_TAXA = 31  # uint64 pattern keys
+WIDE_MAX_TAXA = 64    # 128-bit pattern keys {lo, hi}
+
+
+def _base4(codes):
+    """uint8 codes [P, m], m <= 32 -> uint64 base-4 numbers, first column most significant."""
+    m = codes.shape[1]
+    weights = np.uint64(4) ** np.arange(m - 1, -1, -1, dtype=np.uint64)
+    return (codes.astype(np.uint64) * weights).sum(axis=1, dtype=np.uint64)
+
+
 def encode_patterns(patterns):
-    """list of equal-length ACGT strings -> (uint64 keys, n).  Any other character raises KeyError
-    exactly like `__index_of` (constructions.py:166-171) does."""
+    """list of equal-length ACGT strings -> (keys, n): uint64 [P] up to 31 taxa, uint64 [P, 2] = {lo, hi} for 32..64 taxa
+    (the 128-bit key of csrc/wide.cu: lo holds the last 32 digits).  Any other character raises KeyError exactly like
+    `__index_of` (constructions.py:166-171) does."""
     P = len(patterns)
     if P == 0:
         return np.zeros(0, dtype=np.uint64), 0
@@ -299,37 +311,71 @@ def encode_patterns(patterns):
     joined = "".join(patterns)
     if len(joined) != P * n:
         raise KeyError("patterns of unequal length")
-    if n > 31:
-        raise NotImplementedError("pattern keys are uint64: at most 31 taxa")
+    if n > WIDE_MAX_TAXA:
+        raise NotImplementedError(f"pattern keys are at most 128 bits: at most {WIDE_MAX_TAXA} taxa (got {n})")
     raw = np.frombuffer(joined.encode("latin-1", errors="replace"), dtype=np.uint8).reshape(P, n)
     codes = _UPPER_LUT[raw]
     bad = np.argwhere(codes > 3)
     if len(bad):
         raise KeyError(chr(raw[bad[0][0], bad[0][1]]))
-    weights = (np.uint64(4) ** np.arange(n - 1, -1, -1, dtype=np.uint64)) if n else np.zeros(0, np.uint64)
-    return (codes.astype(np.uint64) * weights).sum(axis=1, dtype=np.uint64), n
+    if n <= NARROW_MAX_TAXA:
+        return _base4(codes), n
+    keys = np.empty((P, 2), dtype=np.uint64)
+    keys[:, 0] = _base4(codes[:, n - 32:])
+    keys[:, 1] = _base4(codes[:, :n - 32])
+    return keys, n
 
 
 def decode_keys(keys, n):
-    """uint64 keys -> list of pattern strings."""
+    """uint64 keys [P] (or 128-bit keys [P, 2] = {lo, hi}) -> list of pattern strings."""
     keys = np.asarray(keys, dtype=np.uint64)
     if len(keys) == 0:
         return []
     shifts = (2 * np.arange(n - 1, -1, -1)).astype(np.uint64)
-    codes = ((keys[:, None] >> shifts[None, :]) & np.uint64(3)).astype(np.uint8)
+    if keys.ndim == 2:  # digit j sits in lo (keys[:, 0]) for the last 32 positions, in hi above
+        word = np.where(shifts >= 64, 1, 0)
+        codes = ((keys[:, word] >> (shifts % np.uint64(64))[None, :]) & np.uint64(3)).astype(np.uint8)
+    else:
+        codes = ((keys[:, None] >> shifts[None, :]) & np.uint64(3)).astype(np.uint8)
     chars = np.frombuffer(STATES.encode(), dtype=np.uint8)[codes]
     flat = chars.tobytes().decode("ascii")
     return [flat[i * n:(i + 1) * n] for i in range(len(keys))]
+
+
+class WidePatternTable:
+    """A {pattern: value} mapping of 32..64 taxa on the device: keys int64 [P, 2] = {lo, hi} (the 128-bit key of
+    csrc/wide.cu and `WideTable.compact`), values float64 [P], both in mapping order."""
+
+    counts = None
+    divisor = 0.0
+
+    def __init__(self, n, keys, values, taxa=None):
+        self.n, self.keys, self.values = n, keys, values
+        self.taxa = tuple(taxa) if taxa is not None else None
+        self.integral = False  # as PatternTable.integral
+
+    @property
+    def num(self):
+        return int(self.keys.shape[0])
+
+    def values_f64(self):
+        return self.values
+
+
+def _narrow_only(table, what):
+    """The kernels behind `what` read uint64 pattern keys."""
+    if isinstance(table, WidePatternTable):
+        raise NotImplementedError(f"{what} is limited to {NARROW_MAX_TAXA} taxa (uint64 pattern keys); this table has {table.n}")
 
 
 _TABLE_CACHE = {}
 
 
 def table_from_mapping(mapping):
-    """{pattern: value} mapping (plain dict or Alignment) -> PatternTable with float64 values, in the
-    mapping's iteration order.  A one-entry-per-object cache avoids re-uploading an unchanged mapping
-    (validated against the joined keys and the values, so a mutated mapping is re-encoded)."""
-    if isinstance(mapping, PatternTable):
+    """{pattern: value} mapping (plain dict or Alignment) -> PatternTable (up to 31 taxa) or WidePatternTable (32..64 taxa)
+    with float64 values, in the mapping's iteration order.  A one-entry-per-object cache avoids re-uploading an unchanged
+    mapping (validated against the joined keys and the values, so a mutated mapping is re-encoded)."""
+    if isinstance(mapping, (PatternTable, WidePatternTable)):
         return mapping
     pats = list(mapping.keys())
     raw = list(mapping.values())
@@ -345,7 +391,8 @@ def table_from_mapping(mapping):
     else:
         keys, n = encode_patterns(pats)
         dev = device()
-        table = PatternTable(n, torch.from_numpy(keys.view(np.int64)).to(dev), values=torch.from_numpy(vals).to(dev))
+        keys_d, vals_d = torch.from_numpy(keys.view(np.int64)).to(dev), torch.from_numpy(vals).to(dev)
+        table = WidePatternTable(n, keys_d, vals_d) if keys.ndim == 2 else PatternTable(n, keys_d, values=vals_d)
         if len(_TABLE_CACHE) > 16:
             _TABLE_CACHE.clear()
         _TABLE_CACHE[id(mapping)] = (joined, vals, table)
@@ -371,8 +418,22 @@ def table_to_dict(table, as_counts=False):
 # --------------------------------------------------------------------------------------------
 # flattenings (kernel 2)
 # --------------------------------------------------------------------------------------------
+def project_keys(table, idx):
+    """Digits of the taxon positions `idx` (in that order, first most significant) of every key of a WidePatternTable:
+    int64 [P] for up to 31 positions, 128-bit keys int64 [P, 2] = {lo, hi} for more."""
+    m = len(idx)
+    out = _empty((table.num, 2) if m > NARROW_MAX_TAXA else table.num, torch.int64)
+    call("spb_project_wide", _p(table.keys), table.num, table.n, bytes(idx), m, _p(out), _st())
+    return out
+
+
 def flatten_coo(table, idx_a, idx_b):
     """(rows, cols) int64 of every pattern: the triplets behind FlatFormat.sparse (constructions.py:86-102)."""
+    if isinstance(table, WidePatternTable):
+        if max(len(idx_a), len(idx_b)) > NARROW_MAX_TAXA:
+            raise NotImplementedError(f"flattening: a side of {max(len(idx_a), len(idx_b))} taxa has 4^side row or column indices, "
+                                      f"which do not fit in 64 bits (sides are limited to {NARROW_MAX_TAXA} taxa)")
+        return project_keys(table, idx_a), project_keys(table, idx_b)
     sp = make_split(table.n, idx_a, idx_b)
     rows, cols = _empty(table.num, torch.int64), _empty(table.num, torch.int64)
     call("spb_flatten_coo", _p(table.keys), table.num, C.byref(sp), _p(rows), _p(cols), _st())
@@ -381,6 +442,11 @@ def flatten_coo(table, idx_a, idx_b):
 
 def flatten_dense(table, idx_a, idx_b, as_counts=False):
     a, b = len(idx_a), len(idx_b)
+    if isinstance(table, WidePatternTable):  # rows / columns from the projection kernel, placed as in _flatten_reduced_large
+        rows, cols = flatten_coo(table, idx_a, idx_b)
+        out = _zeros((4 ** a, 4 ** b), torch.float64)
+        _place(out, rows, cols, table.values, covers_all(table.n, idx_a, idx_b))
+        return out
     sp = make_split(table.n, idx_a, idx_b)
     out = _empty((4 ** a, 4 ** b), torch.float64)
     win = None if covers_all(table.n, idx_a, idx_b) else _empty(4 ** (a + b), torch.int32)
@@ -390,6 +456,7 @@ def flatten_dense(table, idx_a, idx_b, as_counts=False):
 
 
 def reduced_plan(table, idx_a, idx_b):
+    _narrow_only(table, "the reduced-flattening plan")
     a, b = len(idx_a), len(idx_b)
     sp = make_split(table.n, idx_a, idx_b)
     rank_r, rank_c = _empty(4 ** a + 1, torch.int32), _empty(4 ** b + 1, torch.int32)
@@ -401,7 +468,7 @@ def reduced_plan(table, idx_a, idx_b):
 
 def flatten_reduced(table, idx_a, idx_b, as_counts=False):
     """constructions.py:31-55: all-zero rows / columns dropped, rows and columns in ascending index order."""
-    if max(len(idx_a), len(idx_b)) > 13:
+    if max(len(idx_a), len(idx_b)) > 13 or isinstance(table, WidePatternTable):
         return _flatten_reduced_large(table, idx_a, idx_b, as_counts)
     sp, rank_r, rank_c, R, Cc = reduced_plan(table, idx_a, idx_b)
     out = _empty((R, Cc), torch.float64)
@@ -415,23 +482,30 @@ def flatten_reduced(table, idx_a, idx_b, as_counts=False):
 
 
 def _flatten_reduced_large(table, idx_a, idx_b, as_counts):
-    # sides above 13 taxa: the used-index flag arrays (4^side cells) no longer fit, so the ranks come from a
-    # sort-unique of the per-pattern indices (torch.unique: library sort, documented in DESIGN.md)
-    if max(len(idx_a), len(idx_b)) > 31:
+    # sides above 13 taxa (and tables with 128-bit keys): the used-index flag arrays (4^side cells) no longer fit, so the
+    # ranks come from a sort-unique of the per-pattern indices (torch.unique: library sort, documented in DESIGN.md)
+    if max(len(idx_a), len(idx_b)) > 31 and not isinstance(table, WidePatternTable):
         raise NotImplementedError("reduced flattening: sides are limited to 31 taxa (int64 indices)")
     rows, cols = flatten_coo(table, idx_a, idx_b)
     ur, ri = torch.unique(rows, return_inverse=True)
     uc, ci = torch.unique(cols, return_inverse=True)
     out = _zeros((len(ur), len(uc)), torch.float64)
     vals = table.counts.to(torch.float64) if (as_counts and table.counts is not None) else table.values_f64()
-    if not covers_all(table.n, idx_a, idx_b):
-        cell = ri * len(uc) + ci
-        order = torch.arange(table.num, device=cell.device)
-        last = torch.zeros(len(ur) * len(uc), dtype=torch.int64, device=cell.device).scatter_reduce_(0, cell, order, "amax")
+    _place(out, ri, ci, vals, covers_all(table.n, idx_a, idx_b))
+    return out
+
+
+def _place(out, ri, ci, vals, covering):
+    """out[ri, ci] = vals; where the split leaves taxa out several patterns share a cell and the last one in table order
+    wins it (the reference's assignment, constructions.py:43,101)."""
+    if not covering:
+        cols = out.shape[1]
+        cell = ri * cols + ci
+        order = torch.arange(cell.shape[0], device=cell.device)
+        last = torch.zeros(out.shape[0] * cols, dtype=torch.int64, device=cell.device).scatter_reduce_(0, cell, order, "amax")
         keep = last[cell] == order
         ri, ci, vals = ri[keep], ci[keep], vals[keep]
     out[ri, ci] = vals
-    return out
 
 
 # --------------------------------------------------------------------------------------------
@@ -969,9 +1043,14 @@ def pair_tables_from_alignment(aln, as_counts=False):
 
 def pair_tables_from_table(table, as_counts=False):
     n = table.n
-    N_tab = _zeros((n, n, 4, 4), torch.float64)
     vals = table.counts.to(torch.float64) if (as_counts and table.counts is not None) else table.values_f64()
-    call("spb_pair_tables_weighted", _p(table.keys), _p(vals.contiguous()), table.num, n, _p(N_tab), _st())
+    if isinstance(table, WidePatternTable):  # deterministic fp64 tensor-core product (csrc/wide.cu)
+        N_tab = _empty((n, n, 4, 4), torch.float64)
+        ws = _empty(max(int(lib.spb_pair_tables_wide_ws(table.num, n)), 1), torch.float64)
+        call("spb_pair_tables_wide", _p(table.keys), _p(vals.contiguous()), table.num, n, _p(N_tab), _p(ws), _st())
+    else:
+        N_tab = _zeros((n, n, 4, 4), torch.float64)
+        call("spb_pair_tables_weighted", _p(table.keys), _p(vals.contiguous()), table.num, n, _p(N_tab), _st())
     T, total = _empty((n, n, 4, 4), torch.float64), _empty(1, torch.float64)
     call("spb_pair_transform", _p(N_tab), n, _p(T), _p(total), _st())
     return PairTables(n, N_tab, T, total)
@@ -1017,9 +1096,23 @@ def subflatten_scores(pt, masks_a, masks_b=None):
 # Alignment.sub_alignment support (splitp/alignment.py:10-31)
 # --------------------------------------------------------------------------------------------
 def marginalise(table, idx):
-    """Pattern table over the taxa positions `idx` (ascending): values of collapsing patterns are added."""
+    """Pattern table over the taxa positions `idx` (ascending): values of collapsing patterns are added.  Keys come back
+    ascending.  A WidePatternTable gives a PatternTable when at most 31 taxa are kept, else a WidePatternTable."""
     idx = sorted(idx)
-    rows, _ = flatten_coo(table, idx, [])
+    if isinstance(table, WidePatternTable) and len(idx) > NARROW_MAX_TAXA:
+        # 128-bit sub-keys: stable two-pass sort (as WideTable.compact), then one sum per run of equal keys
+        keys = project_keys(table, idx)
+        order = _wide_order(keys)
+        keys, vals = keys[order], table.values[order]
+        new = torch.ones(keys.shape[0], dtype=torch.bool, device=keys.device)
+        new[1:] = (keys[1:] != keys[:-1]).any(dim=1)
+        seg = torch.cumsum(new, 0) - 1
+        keys = keys[new].contiguous()
+        acc = torch.zeros(keys.shape[0], dtype=torch.float64, device=keys.device).index_add_(0, seg, vals)
+        out = WidePatternTable(len(idx), keys, acc)
+        out.integral = table.integral
+        return out
+    rows = project_keys(table, idx) if isinstance(table, WidePatternTable) else flatten_coo(table, idx, [])[0]
     if table.counts is not None and len(idx) <= DIRECT_MAX_TAXA:
         # integer counts, at most 12 taxa: add into the direct-indexed table and compact it (the library's own kernels; the
         # compaction returns the keys in ascending order, as torch.unique did)
@@ -1074,6 +1167,7 @@ def table_marginals(table, idx_a, idx_b, ban_row=-1, ban_col=-1):
     """(row sums, column sums) of the flattening of a split that places every taxon on one side, as SideSums of the RAW
     table values (counts stay integers).  ban_row / ban_col: state code 0..3 whose repeated occurrence in the row /
     column pattern zeroes the entry (constructions.py:94-99), -1 = none."""
+    _narrow_only(table, "table marginals")
     sp = make_split(table.n, idx_a, idx_b)
     rs, cs = SideSums(len(idx_a), table.num), SideSums(len(idx_b), table.num)
     ovf = _zeros(1, torch.int32)
@@ -1092,6 +1186,7 @@ def _partials():
 def rank1_divergence_table(table, idx_a, idx_b):
     """sum over patterns of v log(v / (r c)) without materialising the flattening (phylogenetics.py:364-373);
     float64 tensor [1].  NotImplementedError (from the library) for a split that does not cover all taxa."""
+    _narrow_only(table, "the rank-1 divergence")
     rs, cs = table_marginals(table, idx_a, idx_b)
     sp = make_split(table.n, idx_a, idx_b)
     vp, kind, div = table.val_args()
@@ -1139,6 +1234,7 @@ def outer(x, y, out=None, accumulate=False):
 
 def flatten_coo_banned(table, idx_a, idx_b, ban_row=-1, ban_col=-1):
     """(rows, cols, banned) of every pattern; banned[i] = 1 where the banned-state rule assigns 0."""
+    _narrow_only(table, "flattening with banned patterns")
     sp = make_split(table.n, idx_a, idx_b)
     rows, cols = _empty(table.num, torch.int64), _empty(table.num, torch.int64)
     banned = _empty(table.num, torch.uint8)
@@ -1183,10 +1279,7 @@ class WideTable:
             if want_first:
                 first = torch.cat([first, self.hfirst[self.cap:self.cap + 1]])
         if sort and keys.shape[0] > 1:
-            flip = torch.tensor(-(1 << 63), dtype=torch.int64, device=keys.device)  # unsigned order through signed sorts
-            o1 = torch.sort(keys[:, 0] ^ flip, stable=True).indices
-            o2 = torch.sort((keys[:, 1] ^ flip)[o1], stable=True).indices
-            order = o1[o2]
+            order = _wide_order(keys)
             keys, counts = keys[order], counts[order]
             first = first[order] if want_first else None
         return (keys, counts, first) if want_first else (keys, counts)
@@ -1210,6 +1303,15 @@ class WideTable:
             keys, counts = self.compact()
         c = counts.cpu().numpy().view(np.uint32)
         return {p: (int(x) if as_counts or self.divisor <= 0 else int(x) / self.divisor) for p, x in zip(self._patterns(keys), c)}
+
+
+def _wide_order(keys):
+    """Permutation that sorts 128-bit keys int64 [P, 2] = {lo, hi} ascending as unsigned numbers: stable sort by lo, then
+    by hi (torch.sort: library sort, DESIGN.md section 7)."""
+    flip = torch.tensor(-(1 << 63), dtype=torch.int64, device=keys.device)  # unsigned order through signed sorts
+    o1 = torch.sort(keys[:, 0] ^ flip, stable=True).indices
+    o2 = torch.sort((keys[:, 1] ^ flip)[o1], stable=True).indices
+    return o1[o2]
 
 
 def pack_wide(chars, is_ascii=False):

@@ -79,6 +79,9 @@ def flattening_rank_k_approximation(split, alignment):
     taxa = sorted(set(split[0]) | set(split[1]))
     idx_a, idx_b = engine.split_positions(split, taxa)
     table = engine.table_from_mapping(alignment)
+    if isinstance(table, engine.WidePatternTable):
+        raise NotImplementedError(f"flattening_rank_k_approximation: at most {engine.NARROW_MAX_TAXA} taxa (the banned-state "
+                                  f"marginals read uint64 pattern keys); this alignment has {table.n}")
     R, Cn = 4 ** len(idx_a), 4 ** len(idx_b)
     if R * Cn > 1 << 28 or R > engine.MI_DIRECT_CELLS or Cn > engine.MI_DIRECT_CELLS:
         raise MemoryError(f"flattening_rank_k_approximation: a dense {Cn} x {R} result does not fit")
@@ -158,6 +161,10 @@ def erickson_SVD(alignment, taxa=None, method=Method.flattening, show_work=False
     """
     table = engine.table_from_mapping(alignment)
     num_taxa = table.n
+    if isinstance(table, engine.WidePatternTable) and method in (Method.flattening, Method.mutual_information):
+        # every candidate split joins a few taxa against all others: above 31 taxa its long side has more than 4^31 indices
+        raise NotImplementedError(f"erickson_SVD({method}): at most {engine.NARROW_MAX_TAXA} taxa; above that use "
+                                  f"Method.subflattening (this alignment has {num_taxa} taxa)")
     if taxa is None:
         taxa = [str(np.base_repr(i, base=max(i + 1, 2))) if num_taxa <= 36 else f"t{i}" for i in range(num_taxa)]
     known = {}
