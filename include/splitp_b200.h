@@ -327,6 +327,32 @@ int64_t spb_symv_i32_ws(int64_t k, int64_t batch);
 int spb_symv_i32(const int32_t* d_Gi, int64_t k, int64_t ld, int64_t batch, const double* d_Q, double* d_AQ, double* d_Qt, int variant,
                  void* stream);
 
+/* ---- sparse flattenings: scores from the pattern list of a split, without materialising the flattening ----
+ * A batch of `batch` flattenings F_b (at most k rows on the Gram side, C_b columns) is passed over GLOBAL indices:
+ * row b * k + r (rows past a matrix's own row count stay empty and add zero eigenvalues only) and column base_b + c
+ * (the columns of all matrices concatenated, ncols in all), once grouped by row (CSR: d_row_off [batch * k + 1] entry
+ * offsets, d_row_col [nnz] global columns, d_row_val [nnz]) and once by column (CSC: d_col_off [ncols + 1], d_col_row
+ * [nnz] global rows, d_col_val [nnz]).  batch * k and ncols stay below 2^31.  Every sum has a fixed order: results are
+ * bitwise reproducible and exact for integer values and vectors whose sums stay below 2^53.
+ * spb_sparse_gram_small: G [batch][k][k] = F_b F_b^T for k <= 128 from the CSC; d_colbase [batch + 1] = first global column
+ * of every matrix, max_cols = the largest C_b, d_ws: spb_sparse_gram_small_ws(k, batch, max_cols) doubles.  Score G with
+ * spb_score_gram_small.
+ * spb_score_sparse_large_n: spb_score_gram_large_n (same d_info, same cycle budget, same acceptance) with the product
+ * G Q = F (F^T Q) for k > 128; d_ws: spb_score_sparse_large_ws(k, batch, ncols, nnz) doubles.
+ * spb_sparse_product (diagnostic): d_AQ = F (F^T d_Q), d_Q / d_AQ [batch][8][k], through the kernels the solver launches;
+ * d_ws: spb_sparse_product_ws(k, batch, ncols, nnz) doubles.  For tests and scripts/sparse_flattening_timing.py. */
+int64_t spb_sparse_gram_small_ws(int64_t k, int64_t batch, int64_t max_cols);
+int spb_sparse_gram_small(const int64_t* d_col_off, const int32_t* d_col_row, const double* d_col_val, const int64_t* d_colbase,
+                          int64_t k, int64_t batch, int64_t max_cols, double* d_G, double* d_ws, void* stream);
+int64_t spb_score_sparse_large_ws(int64_t k, int64_t batch, int64_t ncols, int64_t nnz);
+int spb_score_sparse_large_n(const int64_t* d_row_off, const int32_t* d_row_col, const double* d_row_val, const int64_t* d_col_off,
+                             const int32_t* d_col_row, const double* d_col_val, int64_t ncols, int64_t nnz, int64_t k, int64_t batch,
+                             double* d_scores, double* d_info, double* d_ws, int max_cycles, void* stream);
+int64_t spb_sparse_product_ws(int64_t k, int64_t batch, int64_t ncols, int64_t nnz);
+int spb_sparse_product(const int64_t* d_row_off, const int32_t* d_row_col, const double* d_row_val, const int64_t* d_col_off,
+                       const int32_t* d_col_row, const double* d_col_val, int64_t ncols, int64_t nnz, int64_t k, int64_t batch,
+                       const double* d_Q, double* d_AQ, double* d_ws, void* stream);
+
 /* ---- marginals, rank-1 approximation and rank-1 divergence of a flattening ----
  * reference: phylogenetics.py:331-341 (r = column sums, c = row sums, approximation = r^T c),
  * phylogenetics.py:364-373 (divergence = sum over non-zero cells of F[x,y] log(F[x,y] / (r[y] c[x]))),

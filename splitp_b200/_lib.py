@@ -138,6 +138,12 @@ PROTOTYPES = {
     "spb_score_gram_large_i32_n": (_i, [_p, _l, _l, _l, _p, _l, _p, _p, _p, _p, _p, _p, _i, _p]),
     "spb_symv_i32_ws": (_l, [_l, _l]),
     "spb_symv_i32": (_i, [_p, _l, _l, _l, _p, _p, _p, _i, _p]),
+    "spb_sparse_gram_small_ws": (_l, [_l, _l, _l]),
+    "spb_sparse_gram_small": (_i, [_p, _p, _p, _p, _l, _l, _l, _p, _p, _p]),
+    "spb_score_sparse_large_ws": (_l, [_l, _l, _l, _l]),
+    "spb_score_sparse_large_n": (_i, [_p, _p, _p, _p, _p, _p, _l, _l, _l, _l, _p, _p, _p, _i, _p]),
+    "spb_sparse_product_ws": (_l, [_l, _l, _l, _l]),
+    "spb_sparse_product": (_i, [_p, _p, _p, _p, _p, _p, _l, _l, _l, _l, _p, _p, _p, _p]),
     "spb_mi_partials": (_l, []),
     "spb_marginals_dense": (_i, [_p, _l, _l, _l, _p, _p, _p]),
     "spb_mi_dense": (_i, [_p, _l, _l, _l, _p, _p, _p, _p, _p]),

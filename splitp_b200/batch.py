@@ -12,6 +12,7 @@ and the inner loop of `erickson_SVD` (phylogenetics.py:126-140).  `score_splits`
     Method.flattening     pack -> pattern count (kernel 1) -> per split: u8 scatter (kernel 2) -> exact integer Gram on the
                           tensor cores (kernel 4) -> eigen-solver (kernel 5); scores equal those of the reduced / dense /
                           sparse flattening (dropping all-zero rows and columns does not change the singular values)
+                          (up to 16 taxa; 17..64 taxa: pattern count -> engine.sparse_flattening_scores, csrc/sparse.cu)
     Method.subflattening  pack -> pair tables -> H N H^T -> per split: gather + Gram + eigenvalues (kernel 3)
 
 Under `torch.distributed` (one process per GPU) the splits are dealt to the ranks for scoring (flattening scores: contiguous
@@ -78,22 +79,57 @@ class HostPlanes:
 
 
 # --------------------------------------------------------------------------------------------
+def _chars(alignment):
+    """(uint8 [n, N] characters, is_ascii, taxa or None) of a dict, tensor or array alignment."""
+    if isinstance(alignment, dict):  # {taxon: sequence string}: parsers.fasta.read_alignment_from_file
+        from .parsers.fasta import _to_bytes_matrix
+        return _to_bytes_matrix(list(alignment.values())), True, list(alignment.keys())
+    if isinstance(alignment, torch.Tensor):
+        return (alignment if alignment.is_cuda else alignment.to(engine.device(), non_blocking=True)), False, None
+    arr = np.asarray(alignment)
+    is_ascii = arr.dtype.kind in "SU" or (arr.dtype == np.uint8 and arr.size and arr.max() > 3 and arr.max() != 255)
+    return arr.astype(np.uint8, copy=False), bool(is_ascii), None
+
+
 def _as_alignment(alignment, want_sm, want_planes):
     """Anything the caller may hold -> engine.DeviceAlignment (+ taxa if known)."""
     if isinstance(alignment, engine.DeviceAlignment):
         return alignment
     if isinstance(alignment, HostPlanes):
         return alignment.to_device()
-    if isinstance(alignment, dict):  # {taxon: sequence string}: parsers.fasta.read_alignment_from_file
-        from .parsers.fasta import _to_bytes_matrix
-        return engine.pack(_to_bytes_matrix(list(alignment.values())), is_ascii=True, taxa=list(alignment.keys()),
-                           want_sm=want_sm, want_planes=want_planes)
-    if isinstance(alignment, torch.Tensor):
-        chars = alignment if alignment.is_cuda else alignment.to(engine.device(), non_blocking=True)
-        return engine.pack(chars, want_sm=want_sm, want_planes=want_planes)
-    arr = np.asarray(alignment)
-    is_ascii = arr.dtype.kind in "SU" or (arr.dtype == np.uint8 and arr.size and arr.max() > 3 and arr.max() != 255)
-    return engine.pack(arr.astype(np.uint8, copy=False), is_ascii=bool(is_ascii), want_sm=want_sm, want_planes=want_planes)
+    chars, is_ascii, taxa = _chars(alignment)
+    return engine.pack(chars, is_ascii=is_ascii, taxa=taxa, want_sm=want_sm, want_planes=want_planes)
+
+
+def _num_taxa(alignment):
+    if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
+        return alignment.n
+    if isinstance(alignment, dict):
+        return len(alignment)
+    return int(alignment.shape[0]) if hasattr(alignment, "shape") else len(alignment)
+
+
+# Flattening scores of alignments with more taxa than this go through engine.sparse_flattening_scores: the dense count
+# flattenings of CountScorer (4^a x 4^b bytes per split, at least 16 per launch) stop fitting in memory at 17 taxa.
+DENSE_FLATTENING_MAX_TAXA = 16
+
+
+def uses_sparse_flattening(n_taxa):
+    return n_taxa > DENSE_FLATTENING_MAX_TAXA
+
+
+def _sparse_table(alignment):
+    """Pattern table of an alignment of 17..64 taxa: uint64 keys up to 31 taxa, 128-bit keys (raw counts as values) above."""
+    n = _num_taxa(alignment)
+    if n <= engine.NARROW_MAX_TAXA:
+        return engine.count_patterns(_as_alignment(alignment, want_sm=True, want_planes=False))
+    if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
+        raise NotImplementedError(f"flattening scores of {n} taxa need the alignment as characters (dict, array or tensor): "
+                                  "the packed forms hold at most 32 taxa per site word")
+    chars, is_ascii, taxa = _chars(alignment)
+    wide, valid, n, N = engine.pack_wide(chars, is_ascii)
+    keys, counts = engine.count_patterns_wide(wide, valid, n, N).compact()
+    return engine.WidePatternTable(n, keys, (counts.to(torch.int64) & 0xFFFFFFFF).to(torch.float64), taxa)
 
 
 def _positions(splits, taxa):
@@ -136,6 +172,10 @@ class SplitScorer:
         # the call after a re-cut reallocates batch buffers, so two listed steps must be at least two calls apart)
         self.refit_steps = tuple(refit_steps)
         if method == Method.flattening and world > 1 and self.S:
+            n = len(self.idx_all[0][0]) + len(self.idx_all[0][1])
+            if uses_sparse_flattening(n):
+                raise NotImplementedError(f"score_splits(Method.flattening) on several GPUs: at most {DENSE_FLATTENING_MAX_TAXA} taxa "
+                                          f"(this split list covers {n}); above that score on one GPU")
             # contiguous runs of the class-ordered list, cut at equal modelled cost (distributed.partition_by_cost): most ranks
             # then score ONE size class in one batch instead of an eighth of every class
             self._n = len(self.idx_all[0][0]) + len(self.idx_all[0][1])
@@ -214,7 +254,12 @@ class SplitScorer:
         if refit:
             ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             ev0.record()
-        if self.method == Method.flattening:
+        if self.method == Method.flattening and uses_sparse_flattening(_num_taxa(alignment)):
+            with _span(t, "count"):
+                table = _sparse_table(alignment)
+            with _span(t, "sparse"):
+                out = engine.sparse_flattening_scores(table, self.idx_mine)
+        elif self.method == Method.flattening:
             with _span(t, "h2d+pack"):
                 aln = _as_alignment(alignment, want_sm=True, want_planes=False)
             with _span(t, "count"):

@@ -9,6 +9,7 @@
 // total is trace(G) = ||F||_F^2.
 #include "common.cuh"
 #include "jacobi.cuh"
+#include "sparse.cuh"
 #include <cstdlib>
 #include <cstring>
 #include <vector>
@@ -438,6 +439,21 @@ __global__ void krylov_start_rows_kernel(const GramView g, const int* __restrict
   for (int c = kHeavyStart; c < kKB; ++c) {
     // counter-based pseudo-random entry in (-1, 1): depends only on (vector, position), so the result is reproducible
     // and independent of the batch composition; SVQB normalises the block afterwards
+    const uint64_t hsh = mix64(((uint64_t)c << 40) ^ (uint64_t)pos ^ 0x9E3779B97F4A7C15ull);
+    Q[bt * strideQ + (int64_t)c * k + pos] = (double)(int64_t)(hsh >> 11) * (1.0 / 4503599627370496.0) - 1.0;
+  }
+}
+
+// Start block of the sparse operator (no entry of G can be read directly): unit vectors e_j of the kHeavyStart heaviest
+// rows, multiplied by G afterwards (krylov_cycle), plus the same pseudo-random vectors as krylov_start_rows_kernel.
+__global__ void krylov_start_sparse_kernel(const int* __restrict__ idx, double* Q, int64_t strideQ, int k) {
+  const int64_t bt = blockIdx.y;
+  const int pos = blockIdx.x * blockDim.x + threadIdx.x;
+  if (pos >= k) return;
+#pragma unroll
+  for (int c = 0; c < kHeavyStart; ++c) Q[bt * strideQ + (int64_t)c * k + pos] = idx[bt * kKB + c] == pos ? 1.0 : 0.0;
+#pragma unroll
+  for (int c = kHeavyStart; c < kKB; ++c) {
     const uint64_t hsh = mix64(((uint64_t)c << 40) ^ (uint64_t)pos ^ 0x9E3779B97F4A7C15ull);
     Q[bt * strideQ + (int64_t)c * k + pos] = (double)(int64_t)(hsh >> 11) * (1.0 / 4503599627370496.0) - 1.0;
   }
@@ -1181,6 +1197,7 @@ thread_local int g_last_unconverged = 0;  // spb_score_last_unconverged()
 struct KrylovWs {
   double *Q, *AQ, *C, *S, *U, *T, *Vtop, *theta, *res2, *info, *part, *idx, *diag, *Qt;
   int64_t sQ, sC, sS, sT, part_elems;
+  double *W, *sp_part;  // sparse operator only: F^T Q [ncols][8] and the segment partial sums (sparse.cu)
 };
 
 static int64_t krylov_layout(int64_t k, int64_t batch, double* base, KrylovWs* w) {
@@ -1207,6 +1224,25 @@ static int64_t krylov_layout(int64_t k, int64_t batch, double* base, KrylovWs* w
   w->part_elems = batch * ((k + kDotChunk - 1) / kDotChunk) * (int64_t)kKDim * kKDim;
   w->part = take(w->part_elems);
   return off;
+}
+
+// Sparse operator: W and the segment partials after the dense layout
+static int64_t sparse_layout(const SparseBatch& f, double* base, KrylovWs* w) {
+  const int64_t off = krylov_layout(f.k, f.batch, base, w);
+  const int64_t nw = (f.ncols * 8 + 1) / 2 * 2;
+  w->W = base ? base + off : nullptr;
+  w->sp_part = base ? base + off + nw : nullptr;
+  return off + nw + sparse_part_doubles(f);
+}
+
+// AQ = F (F^T Q) for one block of 8 vectors: Q transposed into Qt [batch * k][8] (krylov_transpose_kernel with no padding),
+// then the two segment products of sparse.cu
+static int sparse_apply(const SparseBatch& f, const double* Q, int64_t strideQ, double* AQ, double* Qt, double* W, double* part,
+                        cudaStream_t st) {
+  dim3 tg((f.k + 255) / 256, f.batch);
+  krylov_transpose_kernel<<<tg, 256, 0, st>>>(Q, strideQ, Qt, (int64_t)f.k * kKB, f.k, f.k);
+  SPB_LAUNCH_CHECK();
+  return sparse_product_launch(f, Qt, W, AQ, strideQ, part, st);
 }
 
 }  // namespace
@@ -1267,7 +1303,8 @@ static bool accept_matrix(const double* inf, int cycle) {
 
 // One Krylov cycle with `nb` blocks (dim = 8 nb).  first = 1 starts from the heaviest rows of G plus pseudo-random
 // vectors (krylov_start_rows_kernel), otherwise from the Ritz vectors the previous cycle left in Q_0.
-static int krylov_cycle(const GramView& gv, int k, int batch, int nb, bool first, const KrylovWs& w, cudaStream_t st) {
+static int krylov_cycle(const GramView& gv, int k, int batch, int nb, bool first, const KrylovWs& w, cudaStream_t st,
+                        const SparseBatch* sf = nullptr) {
   const int64_t ld = gv.ld;
   const int64_t blk = (int64_t)kKB * k;
   const int dim = nb * kKB;
@@ -1284,7 +1321,19 @@ static int krylov_cycle(const GramView& gv, int k, int batch, int nb, bool first
     }
     return SPB_OK;
   };
-  if (first) {
+  if (first && sf) {
+    dim3 grid((k + 255) / 256, batch);
+    if ((rc = sparse_diag_launch(*sf, w.diag, st))) return rc;
+    krylov_top8_kernel<<<batch, 256, 0, st>>>(w.diag, k, reinterpret_cast<int*>(w.idx));
+    SPB_LAUNCH_CHECK();
+    krylov_start_sparse_kernel<<<grid, 256, 0, st>>>(reinterpret_cast<const int*>(w.idx), w.Q, w.sQ, k);
+    SPB_LAUNCH_CHECK();
+    if ((rc = sparse_apply(*sf, w.Q, w.sQ, w.AQ, w.Qt, w.W, w.sp_part, st))) return rc;
+    dim3 cg((unsigned)((kHeavyStart * (int64_t)k + 255) / 256), batch);  // G e_j in place of e_j
+    copy_block_kernel<<<cg, 256, 0, st>>>(w.AQ, w.sQ, w.Q, w.sQ, kHeavyStart * (int64_t)k);
+    SPB_LAUNCH_CHECK();
+    if ((rc = ortho_block(w.Q, 2))) return rc;
+  } else if (first) {
     dim3 grid((k + 255) / 256, batch);
     gram_diag_kernel<<<grid, 256, 0, st>>>(gv, k, w.diag);
     SPB_LAUNCH_CHECK();
@@ -1306,7 +1355,9 @@ static int krylov_cycle(const GramView& gv, int k, int batch, int nb, bool first
   for (int j = 0; j < nb; ++j) {
     double* Qj = w.Q + (int64_t)j * blk;
     double* AQj = w.AQ + (int64_t)j * blk;
-    {
+    if (sf) {
+      if ((rc = sparse_apply(*sf, Qj, w.sQ, AQj, w.Qt, w.W, w.sp_part, st))) return rc;
+    } else {
       dim3 grid((k + kSymvRows - 1) / kSymvRows, batch);
       if (gv.Gf) symv_block_kernel<<<grid, 256, symv_smem, st>>>(gv.Gf, ld, ld * ld, Qj, w.sQ, AQj, k);
       else {
@@ -1367,14 +1418,15 @@ static int krylov_cycle(const GramView& gv, int k, int batch, int nb, bool first
 }
 
 static int score_gram_large(const GramView& gv, int64_t k64, int64_t batch64, double* d_scores, double* d_info, double* d_ws,
-                            void* stream, int max_cycles = 40) {
-  SPB_REQUIRE((gv.Gf || gv.Gi) && d_scores && d_ws && k64 > kJacobiMaxK && gv.ld >= k64 && batch64 >= 1 && k64 < (1 << 24) &&
+                            void* stream, int max_cycles = 40, const SparseBatch* sf = nullptr) {
+  SPB_REQUIRE((gv.Gf || gv.Gi || sf) && d_scores && d_ws && k64 > kJacobiMaxK && gv.ld >= k64 && batch64 >= 1 && k64 < (1 << 24) &&
                   batch64 <= 65535,
               "spb_score_gram_large: need k > %d and a workspace", kJacobiMaxK);
   const int k = (int)k64, batch = (int)batch64;
   cudaStream_t st = (cudaStream_t)stream;
   KrylovWs w;
-  krylov_layout(k, batch, d_ws, &w);
+  if (sf) sparse_layout(*sf, d_ws, &w);
+  else krylov_layout(k, batch, d_ws, &w);
   SPB_CUDA(cudaMemsetAsync(w.info, 0, (size_t)batch * kInfo * sizeof(double), st));
   static thread_local std::vector<double> h_info;
   static thread_local std::vector<double> h_flag;
@@ -1386,7 +1438,7 @@ static int score_gram_large(const GramView& gv, int64_t k64, int64_t batch64, do
   bool done = false;
   for (int cycle = 0; cycle < kMaxCycles && !done; ++cycle) {
     const int nb = cycle < 2 ? 2 : (cycle < 4 ? 4 : kKMaxBlocks);
-    if ((rc = krylov_cycle(gv, k, batch, nb, cycle == 0, w, st))) return rc;
+    if ((rc = krylov_cycle(gv, k, batch, nb, cycle == 0, w, st, sf))) return rc;
     krylov_finish_kernel<<<(batch + 127) / 128, 128, 0, st>>>(w.theta, w.res2, w.info, d_scores, batch);
     SPB_LAUNCH_CHECK();
     SPB_CUDA(cudaMemcpyAsync(h_info.data(), w.info, (size_t)batch * kInfo * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -1475,4 +1527,46 @@ extern "C" int spb_symv_i32(const int32_t* d_Gi, int64_t k64, int64_t ld, int64_
   }
   SPB_LAUNCH_CHECK();
   return SPB_OK;
+}
+
+// ---- sparse flattenings (sparse.cu): the same solver with G Q = F (F^T Q) ----
+static SparseBatch sparse_batch(const int64_t* row_off, const int32_t* row_col, const double* row_val, const int64_t* col_off,
+                                const int32_t* col_row, const double* col_val, int64_t ncols, int64_t nnz, int64_t k, int64_t batch) {
+  return SparseBatch{row_off, row_col, row_val, col_off, col_row, col_val, ncols, nnz, (int)k, (int)batch};
+}
+
+extern "C" int64_t spb_score_sparse_large_ws(int64_t k, int64_t batch, int64_t ncols, int64_t nnz) {
+  KrylovWs w;
+  return sparse_layout(sparse_batch(nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, ncols, nnz, k, batch), nullptr, &w);
+}
+
+extern "C" int spb_score_sparse_large_n(const int64_t* d_row_off, const int32_t* d_row_col, const double* d_row_val, const int64_t* d_col_off,
+                                        const int32_t* d_col_row, const double* d_col_val, int64_t ncols, int64_t nnz, int64_t k, int64_t batch,
+                                        double* d_scores, double* d_info, double* d_ws, int max_cycles, void* stream) {
+  SPB_REQUIRE(k > kJacobiMaxK && k < (1 << 24), "spb_score_sparse_large: need %d < k < 2^24 (got %lld)", kJacobiMaxK, (long long)k);
+  const SparseBatch f = sparse_batch(d_row_off, d_row_col, d_row_val, d_col_off, d_col_row, d_col_val, ncols, nnz, k, batch);
+  int rc = sparse_check(f);
+  if (rc) return rc;
+  GramView gv{nullptr, nullptr, k, nullptr, 0, nullptr, nullptr, nullptr};
+  return score_gram_large(gv, k, batch, d_scores, d_info, d_ws, stream, max_cycles, &f);
+}
+
+// Diagnostic entry: d_AQ = F (F^T d_Q) for a batch of sparse flattenings, launched exactly as the solver launches it.
+// d_Q, d_AQ: [batch][8][k]; d_ws: spb_sparse_product_ws(k, batch, ncols, nnz) doubles.
+extern "C" int64_t spb_sparse_product_ws(int64_t k, int64_t batch, int64_t ncols, int64_t nnz) {
+  const SparseBatch f = sparse_batch(nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, ncols, nnz, k, batch);
+  return batch * k * kKB + (ncols * 8 + 1) / 2 * 2 + sparse_part_doubles(f);
+}
+
+extern "C" int spb_sparse_product(const int64_t* d_row_off, const int32_t* d_row_col, const double* d_row_val, const int64_t* d_col_off,
+                                  const int32_t* d_col_row, const double* d_col_val, int64_t ncols, int64_t nnz, int64_t k, int64_t batch,
+                                  const double* d_Q, double* d_AQ, double* d_ws, void* stream) {
+  SPB_REQUIRE(d_Q && d_AQ && d_ws, "spb_sparse_product: bad arguments");
+  const SparseBatch f = sparse_batch(d_row_off, d_row_col, d_row_val, d_col_off, d_col_row, d_col_val, ncols, nnz, k, batch);
+  int rc = sparse_check(f);
+  if (rc) return rc;
+  double* Qt = d_ws;
+  double* W = Qt + batch * k * kKB;
+  double* part = W + (ncols * 8 + 1) / 2 * 2;
+  return sparse_apply(f, d_Q, (int64_t)kKB * k, d_AQ, Qt, W, part, (cudaStream_t)stream);
 }

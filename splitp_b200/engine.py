@@ -565,23 +565,25 @@ FIRST_CYCLES = 2   # cycles the WHOLE batch runs through (two blocks each); matr
 MIN_COMPACT = 16   # batches below this are not worth a second call
 
 
-def _solve_large(batch, scores, run, k):
+def _solve_large(batch, scores, run, k, ws=None):
     """Block-Krylov scores of a batch with straggler compaction.  The solver keeps every matrix of a batch in the cycle until the
     last one is accepted, and its cycles grow (2, 2, 4, 4, 12, ... blocks of 8 vectors = that many G Q products per matrix): with
     up to 512 matrices per batch one slow matrix would cost hundreds of products.  So the whole batch gets FIRST_CYCLES cycles;
     whatever reports converged = 0 after them is gathered into a batch of its own and solved with the full budget.
-    run(sel, scores, info, ws, budget): one solver call on the matrices `sel` (None = all).  Returns the info array [batch, 10]."""
+    run(sel, scores, info, ws, budget): one solver call on the matrices `sel` (None = all).  ws(k, batch): its workspace (default:
+    the dense solver's).  Returns the info array [batch, 10]."""
+    ws = _krylov_ws if ws is None else ws
     info = _empty((batch, SCORE_INFO), torch.float64)
     if batch < MIN_COMPACT:
-        run(None, scores, info, _krylov_ws(k, batch), 40)
+        run(None, scores, info, ws(k, batch), 40)
         return info
-    run(None, scores, info, _krylov_ws(k, batch), FIRST_CYCLES)
+    run(None, scores, info, ws(k, batch), FIRST_CYCLES)
     if int(lib.spb_score_last_unconverged()) == 0:
         return info
     sel = torch.nonzero(info[:, 8] == 0.0).flatten()
     m = int(sel.shape[0])
     sc2, inf2 = _empty(m, torch.float64), _empty((m, SCORE_INFO), torch.float64)
-    run(sel, sc2, inf2, _krylov_ws(k, m), 40)
+    run(sel, sc2, inf2, ws(k, m), 40)
     scores.index_copy_(0, sel, sc2)
     info.index_copy_(0, sel, inf2)
     return info
@@ -1008,6 +1010,217 @@ def score_splits_counts(table, splits_idx, reduced=False):
     out = scorer.score_many(splits_idx, reduced)
     scorer.check_hi()
     return out
+
+
+# --------------------------------------------------------------------------------------------
+# sparse flattenings (csrc/sparse.cu): flattening scores of any covering split of up to 64 taxa from the pattern list.
+# The flattening of such a split has exactly one non-zero per pattern, so its Gram matrix is applied as F (F^T Q) in
+# O(P) per block of 8 Krylov vectors, with memory linear in the number of patterns.
+# --------------------------------------------------------------------------------------------
+SPARSE_BATCH_BYTES = 16 << 30     # device memory of one batched sparse solver call (workspace + CSR / CSC arrays)
+SPARSE_K_ALIGN = 128              # Gram sides of a large batch are padded to a multiple of this with empty rows
+SPARSE_PLAN_CACHE_BYTES = 1 << 30  # plans kept between the sizing pass and the scoring pass of sparse_flattening_scores
+
+
+class SparsePlan:
+    """Dense ids of the row and column of every non-zero of a flattening.  g: ids on the Gram side (k distinct values),
+    o: ids on the other side (C >= k distinct values), vals: float64 values; all device tensors of one length.  The ids are
+    in no particular order: singular values do not depend on the order of rows or columns."""
+
+    def __init__(self, g, o, k, C, vals):
+        self.g, self.o, self.k, self.C, self.vals = g, o, int(k), int(C), vals
+
+    @property
+    def nnz(self):
+        return int(self.g.shape[0])
+
+
+def _dense_ids(x):
+    """(ids int64 [P], distinct count) of int64 [P] values or 128-bit keys int64 [P, 2]: equal values share an id."""
+    if x.shape[0] == 0:
+        return torch.zeros(0, dtype=torch.int64, device=x.device), 0
+    if x.dim() == 1:
+        u, inv = torch.unique(x, return_inverse=True)  # library sort (DESIGN.md section 7)
+        return inv, int(u.shape[0])
+    order = _wide_order(x)  # stable two-pass sort, then run boundaries, as marginalise
+    xs = x[order]
+    new = torch.ones(xs.shape[0], dtype=torch.int64, device=x.device)
+    new[1:] = (xs[1:] != xs[:-1]).any(dim=1).to(torch.int64)
+    run = torch.cumsum(new, 0) - 1
+    ids = torch.empty_like(run)
+    ids[order] = run
+    return ids, int(run[-1].item()) + 1
+
+
+def _side_keys(table, idx):
+    """Projection of every pattern onto the taxon positions idx (int64, or 128-bit keys above 31 positions)."""
+    if not idx:
+        return torch.zeros(table.num, dtype=torch.int64, device=table.keys.device)
+    if isinstance(table, WidePatternTable):
+        return project_keys(table, idx)
+    return flatten_coo(table, idx, [])[0]
+
+
+def _table_values(table):
+    """Values of the non-zeros: raw counts as fp64 (the score is scale-invariant) or the mapping's values."""
+    if table.counts is not None:
+        return (table.counts.to(torch.int64) & 0xFFFFFFFF).to(torch.float64)
+    return table.values
+
+
+def sparse_plan(table, idx_a, idx_b, vals=None):
+    """SparsePlan of the flattening of (idx_a | idx_b) of a PatternTable or WidePatternTable; the split must place every taxon on
+    exactly one side (ValueError otherwise).  The Gram side is the side with fewer distinct projections."""
+    if not covers_all(table.n, idx_a, idx_b):
+        raise ValueError("sparse flattening scores need a split that places every taxon on exactly one side")
+    if isinstance(table, WidePatternTable) or not idx_a or not idx_b:
+        ka, kb = _side_keys(table, list(idx_a)), _side_keys(table, list(idx_b))
+    else:
+        ka, kb = flatten_coo(table, idx_a, idx_b)
+    ra, R = _dense_ids(ka)
+    rb, Cc = _dense_ids(kb)
+    vals = _table_values(table) if vals is None else vals
+    return SparsePlan(ra, rb, R, Cc, vals) if R <= Cc else SparsePlan(rb, ra, Cc, R, vals)
+
+
+def sparse_batch_arrays(plans, k):
+    """CSR / CSC arrays of a batch of plans over global indices (layout of csrc/sparse.cuh): row b * k + g, column
+    base_b + o.  Both groupings come from stable sorts, so every sum of the kernels has a fixed order."""
+    dev = device()
+    B = len(plans)
+    rows, cols, vals, colbase = [], [], [], [0]
+    for b, p in enumerate(plans):
+        rows.append(p.g + b * k)
+        cols.append(p.o + colbase[-1])
+        vals.append(p.vals)
+        colbase.append(colbase[-1] + p.C)
+    rows = torch.cat(rows) if rows else torch.zeros(0, dtype=torch.int64, device=dev)
+    cols = torch.cat(cols) if cols else torch.zeros(0, dtype=torch.int64, device=dev)
+    vals = torch.cat(vals).to(torch.float64) if vals else torch.zeros(0, dtype=torch.float64, device=dev)
+    ncols = colbase[-1]
+    pr = torch.sort(rows, stable=True).indices  # library sorts (DESIGN.md section 7)
+    pc = torch.sort(cols, stable=True).indices
+    row_off = torch.zeros(B * k + 1, dtype=torch.int64, device=dev)
+    row_off[1:] = torch.cumsum(torch.bincount(rows, minlength=B * k), 0)
+    col_off = torch.zeros(ncols + 1, dtype=torch.int64, device=dev)
+    col_off[1:] = torch.cumsum(torch.bincount(cols, minlength=ncols), 0)
+    return {"row_off": row_off, "row_col": cols[pr].to(torch.int32), "row_val": vals[pr].contiguous(),
+            "col_off": col_off, "col_row": rows[pc].to(torch.int32), "col_val": vals[pc].contiguous(),
+            "ncols": ncols, "nnz": int(rows.shape[0]), "colbase": torch.tensor(colbase, dtype=torch.int64, device=dev)}
+
+
+def _array_bytes(ncols, nnz, rows):
+    """Device bytes of sparse_batch_arrays (+ the sort temporaries, about as much again)."""
+    return 2 * (8 * (rows + ncols + 2) + 2 * nnz * (4 + 8) + 3 * nnz * 8)
+
+
+def sparse_chunks(sizes, ws_bytes, cap, max_batch=65535):
+    """Cuts [(k, C, nnz), ...] (in the order given, normally ascending k) into consecutive batches whose device bytes
+    ws_bytes(kmax, batch, ncols, nnz, max_cols) stay within cap (a batch holds at least one matrix).  Returns index lists."""
+    out, cur = [], []
+    kmax = ncols = nnz = maxc = 0
+    for i, (k, Cc, z) in enumerate(sizes):
+        nk, nc, nz, nm = max(kmax, k), ncols + Cc, nnz + z, max(maxc, Cc)
+        if cur and (len(cur) >= max_batch or ws_bytes(nk, len(cur) + 1, nc, nz, nm) > cap):
+            out.append(cur)
+            cur, nk, nc, nz, nm = [], k, Cc, z, Cc
+        cur.append(i)
+        kmax, ncols, nnz, maxc = nk, nc, nz, nm
+    if cur:
+        out.append(cur)
+    return out
+
+
+def _pad_k(k):
+    return -(-k // SPARSE_K_ALIGN) * SPARSE_K_ALIGN
+
+
+def _small_bytes(k, batch, ncols, nnz, max_cols):
+    return 8 * (int(lib.spb_sparse_gram_small_ws(k, batch, max_cols)) + batch * k * k) + _array_bytes(ncols, nnz, batch * k)
+
+
+def _large_bytes(k, batch, ncols, nnz, max_cols):
+    kp = _pad_k(k)
+    return 8 * int(lib.spb_score_sparse_large_ws(kp, batch, ncols, nnz)) + _array_bytes(ncols, nnz, batch * kp)
+
+
+def _sparse_scores(sizes, make, timer=None):
+    """Scores of flattenings given as sizes [(k, C, nnz), ...] and make(i) -> SparsePlan: k <= 4 -> 0.0; 4 < k <= 128: exact Gram
+    from the CSC + the small-matrix scorer; above: the block-Krylov solver on F (F^T Q).  Splits are grouped by ascending k and
+    batched within SPARSE_BATCH_BYTES."""
+    out = _zeros(len(sizes), torch.float64)
+    cap = SPARSE_BATCH_BYTES
+    small = sorted((i for i, s in enumerate(sizes) if 4 < s[0] <= JACOBI_MAX_K), key=lambda i: sizes[i][0])
+    large = sorted((i for i, s in enumerate(sizes) if s[0] > JACOBI_MAX_K), key=lambda i: sizes[i][0])
+    for chunk in sparse_chunks([sizes[i] for i in small], _small_bytes, cap):
+        members = [small[j] for j in chunk]
+        k = max(sizes[i][0] for i in members)
+        with _span(timer, "plan", len(members)):
+            a = sparse_batch_arrays([make(i) for i in members], k)
+        with _span(timer, "solver", len(members)):
+            B, maxc = len(members), max(sizes[i][1] for i in members)
+            G = _empty((B, k, k), torch.float64)
+            ws = _empty(max(int(lib.spb_sparse_gram_small_ws(k, B, maxc)), 1), torch.float64)
+            call("spb_sparse_gram_small", _p(a["col_off"]), _p(a["col_row"]), _p(a["col_val"]), _p(a["colbase"]), k, B, maxc, _p(G),
+                 _p(ws), _st())
+            sc = _empty(B, torch.float64)
+            call("spb_score_gram_small", _p(G), k, k, B, _p(sc), None, _st())
+        out.index_copy_(0, torch.tensor(members, dtype=torch.int64, device=out.device), sc)
+    for chunk in sparse_chunks([sizes[i] for i in large], _large_bytes, cap):
+        members = [large[j] for j in chunk]
+        k = _pad_k(max(sizes[i][0] for i in members))
+
+        def run(sel, sc, inf, _ws, budget, members=members, k=k):
+            mine = members if sel is None else [members[j] for j in sel.tolist()]
+            with _span(timer, "plan", len(mine)):
+                a = sparse_batch_arrays([make(i) for i in mine], k)
+            ws = _empty(int(lib.spb_score_sparse_large_ws(k, len(mine), a["ncols"], a["nnz"])), torch.float64)
+            with _span(timer, "solver", len(mine)):
+                call("spb_score_sparse_large_n", _p(a["row_off"]), _p(a["row_col"]), _p(a["row_val"]), _p(a["col_off"]), _p(a["col_row"]),
+                     _p(a["col_val"]), a["ncols"], a["nnz"], k, len(mine), _p(sc), _p(inf), _p(ws), budget, _st())
+
+        sc = _empty(len(members), torch.float64)
+        _solve_large(len(members), sc, run, k, ws=lambda k, b: None)
+        _warn_unconverged()
+        out.index_copy_(0, torch.tensor(members, dtype=torch.int64, device=out.device), sc)
+    return out
+
+
+def sparse_flattening_scores(table, splits_idx, timer=None):
+    """Flattening scores (split_score of the flattening, phylogenetics.py:280-328) of many splits [(idx_a, idx_b), ...] of a
+    PatternTable (counts or values) or WidePatternTable, up to 64 taxa, without materialising any flattening.  Every split must
+    place every taxon on exactly one side (ValueError otherwise).  Returns a float64 device tensor, one score per split; a split
+    whose Gram side has at most 4 distinct rows scores 0.0."""
+    for ia, ib in splits_idx:
+        if not covers_all(table.n, ia, ib):
+            raise ValueError("sparse flattening scores need a split that places every taxon on exactly one side")
+    if table.num == 0:  # no non-zero: every Gram side is empty
+        return _zeros(len(splits_idx), torch.float64)
+    vals = _table_values(table)
+    cache, cached = {}, 0
+    sizes = []
+    with _span(timer, "plan", len(splits_idx)):
+        for i, (ia, ib) in enumerate(splits_idx):
+            p = sparse_plan(table, ia, ib, vals)
+            sizes.append((p.k, p.C, p.nnz))
+            if cached + 16 * p.nnz <= SPARSE_PLAN_CACHE_BYTES:
+                cache[i] = p
+                cached += 16 * p.nnz
+
+    def make(i):
+        p = cache.get(i)
+        return p if p is not None else sparse_plan(table, *splits_idx[i], vals)
+
+    return _sparse_scores(sizes, make, timer)
+
+
+def sparse_matrix_score(rows, cols, vals):
+    """Score of one sparse matrix given by the dense ids of its non-zeros (device int64 tensors; no repeated (row, col) pair)
+    and their values; float64 device tensor [1]."""
+    R = int(rows.max().item()) + 1 if rows.shape[0] else 0
+    Cc = int(cols.max().item()) + 1 if cols.shape[0] else 0
+    p = SparsePlan(rows, cols, R, Cc, vals) if R <= Cc else SparsePlan(cols, rows, Cc, R, vals)
+    return _sparse_scores([(p.k, p.C, p.nnz)], lambda i: p)
 
 
 # --------------------------------------------------------------------------------------------

@@ -19,6 +19,15 @@ from . import engine
 from .enums import Method
 
 
+# A flattening with more cells than this (1 GiB of fp64) is scored from its non-zeros (engine.sparse_flattening_scores /
+# engine.sparse_matrix_score) instead of as a dense matrix.
+SPARSE_MIN_CELLS = 2 ** 27
+
+
+def use_sparse_route(rows, cols):
+    return rows * cols > SPARSE_MIN_CELLS
+
+
 def is_sparse(matrix):
     return scipy.sparse.issparse(matrix)
 
@@ -37,6 +46,16 @@ def split_score(matrix, return_singular_values=False, force_frob_norm_on_dense=F
         ur, ri = np.unique(coo.row, return_inverse=True)
         uc, ci = np.unique(coo.col, return_inverse=True)
         dev = engine.device()
+        if use_sparse_route(len(ur), len(uc)):
+            if min(len(ur), len(uc)) <= 4:
+                return 0.0
+            coo = coo.copy()
+            coo.sum_duplicates()  # scipy adds repeated entries; the sparse route needs one non-zero per cell
+            _, ri = np.unique(coo.row, return_inverse=True)
+            _, ci = np.unique(coo.col, return_inverse=True)
+            ids = [torch.from_numpy(x.astype(np.int64)).to(dev) for x in (ri, ci)]
+            vals = torch.from_numpy(np.asarray(coo.data, dtype=np.float64)).to(dev)
+            return float(engine.sparse_matrix_score(ids[0], ids[1], vals)[0].item())
         dense = torch.zeros((len(ur), len(uc)), dtype=torch.float64, device=dev)
         if len(coo.data):
             dense[torch.from_numpy(ri).to(dev), torch.from_numpy(ci).to(dev)] = torch.from_numpy(
@@ -154,7 +173,8 @@ def erickson_SVD(alignment, taxa=None, method=Method.flattening, show_work=False
     n - 2 chosen splits as sorted 2-tuples of leaf tuples, like the reference.  The candidate splits of a step are
     scored as ONE batch on the device: the batched subflattening kernel for `Method.subflattening`; for
     `Method.flattening` (up to 12 taxa) the dense flattenings of a whole side-size class, one batched fp64 Gram and one
-    batched eigen-solver call; for `Method.mutual_information` the divergences are queued for all candidates and read back
+    batched eigen-solver call (above 12 taxa, candidates whose reduced flattening has more than SPARSE_MIN_CELLS cells are
+    scored from the pattern list in one batched sparse call per step); for `Method.mutual_information` the divergences are queued for all candidates and read back
     once per step.  `trace` (an optional list, not in the reference's signature) receives the candidate scores of every step.  `Method.mutual_information` scores a split by the rank-1 divergence of
     its flattening (phylogenetics.py:136-140, 364-373), computed straight from the pattern table.  `Method.distance`
     leaves every score at infinity, as the reference does.
@@ -191,10 +211,19 @@ def erickson_SVD(alignment, taxa=None, method=Method.flattening, show_work=False
             if table.n <= FLATTENING_DENSE_MAX_TAXA and all(engine.covers_all(table.n, ia, ib) for ia, ib in idx):
                 # one batch per side size: no per-split host synchronisation (ONE device -> host copy per step)
                 return [np.float64(v) for v in _flattening_scores_batched(table, idx).cpu().numpy()]
-            out = []
-            for ia, ib in idx:
+            out, big = [], []
+            for j, (ia, ib) in enumerate(idx):
+                if engine.covers_all(table.n, ia, ib):
+                    plan = engine.sparse_plan(table, ia, ib)
+                    if use_sparse_route(plan.k, plan.C):  # a dense reduced flattening of this size would not fit
+                        big.append(j)
+                        out.append(None)
+                        continue
                 F = engine.flatten_reduced(table, ia, ib)
                 out.append(np.float64(0.0) if min(F.shape) <= 4 else np.float64(engine.score_matrix(F)[0].item()))
+            if big:  # one batched call for the whole step
+                for j, v in zip(big, engine.sparse_flattening_scores(table, [idx[j] for j in big]).cpu().numpy()):
+                    out[j] = np.float64(v)
             return out
         if method == Method.mutual_information:
             # every divergence stays on the device until the whole step is queued: ONE device -> host copy per step
