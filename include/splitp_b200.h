@@ -199,6 +199,23 @@ int spb_flatten_u8_batch(const uint64_t* d_keys, const uint32_t* d_counts, int64
                          int32_t* d_hi_rc, uint32_t* d_hi_val, uint32_t* d_hi_num, int64_t hi_cap, void* stream);
 int spb_flatten_u8_clear_batch(const uint64_t* d_keys, int64_t num, const spb_split* h_splits, int nb, uint8_t* d_s0,
                                int64_t s0_stride, int64_t rows_pad, int64_t pitch, int layout, void* stream);
+/* Column ranks of a batch: only the columns some pattern projects to are non-zero, so S0 can hold column c at its rank among
+ * the occupied columns; S0 S0^T and the high-part correction are unchanged, and the Gram contracts over ncols instead of 4^b.
+ * spb_col_ranks_batch: for the nb <= SPB_MAX_BATCH splits h_splits (HOST array), d_colrank uint32 [nb][2 * words] with
+ * words = spb_col_rank_words(b) receives per split the occupancy bits of the 4^b columns followed by the exclusive prefix
+ * counts of those bit words; d_ncols int32 [nb] the number of occupied columns (at most min(4^b, num)).
+ * spb_flatten_u8_batch_cols / spb_flatten_u8_clear_batch_cols: spb_flatten_u8_batch / _clear_batch with every column mapped
+ * through those ranks (d_hi_rc holds ranked columns too); pitch >= min(4^b, num) suffices. */
+int64_t spb_col_rank_words(int b);
+int spb_col_ranks_batch(const uint64_t* d_keys, int64_t num, const spb_split* h_splits, int nb, uint32_t* d_colrank, int64_t words,
+                        int32_t* d_ncols, void* stream);
+int spb_flatten_u8_batch_cols(const uint64_t* d_keys, const uint32_t* d_counts, int64_t num, const spb_split* h_splits, int nb,
+                              const uint32_t* d_colrank, int64_t words, uint8_t* d_s0, int64_t s0_stride, int64_t rows_pad, int64_t pitch,
+                              int layout, int flags, int32_t* d_hi_rc, uint32_t* d_hi_val, uint32_t* d_hi_num, int64_t hi_cap,
+                              void* stream);
+int spb_flatten_u8_clear_batch_cols(const uint64_t* d_keys, int64_t num, const spb_split* h_splits, int nb, const uint32_t* d_colrank,
+                                    int64_t words, uint8_t* d_s0, int64_t s0_stride, int64_t rows_pad, int64_t pitch, int layout,
+                                    void* stream);
 
 /* ---- a11: subflattening (constructions.py:108-198) ---- */
 /* Raw pair statistics of sites [32*word_begin, 32*word_end) accumulated (atomicAdd) into d_raw
@@ -255,6 +272,11 @@ int spb_gram_u8(const uint8_t* d_s0, int64_t rows_pad, int64_t pitch, int layout
  * d_ws: uint64 [spb_gram_u8_ws(rows_pad, pitch, layout, nb)]. */
 int spb_gram_u8_batch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, int layout,
                       double* d_G, int64_t g_stride, uint64_t* d_ws, void* stream);
+/* spb_gram_u8_batch with K given per matrix: d_ncols int32 [nb] (device) = the columns of S0 entry b that may be non-zero
+ * (all beyond them are zero), as spb_col_ranks_batch returns them.  The launch is planned for K = pitch; each matrix runs
+ * only the K tiles (or dp4a words) that hold its columns.  NULL d_ncols is spb_gram_u8_batch. */
+int spb_gram_u8_batch_cols(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, int layout,
+                           const int32_t* d_ncols, double* d_G, int64_t g_stride, uint64_t* d_ws, void* stream);
 /* Same result from a plain SIMT loop, any layout and size: the on-device cross-check used by the tests. */
 int spb_gram_u8_simt(const uint8_t* d_s0, int64_t rows_pad, int64_t pitch, int layout, double* d_G, void* stream);
 /* Adds the terms of the sparse high part H (F = S0 + H): G += S0 H^T + H S0^T + H H^T, so that G = F F^T. */
@@ -300,6 +322,9 @@ int spb_score_gram_large_n(const double* d_G, int64_t k, int64_t ld, int64_t bat
  * product kernel reads it column-wise. */
 int spb_gram_u8_batch_i32(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, int32_t* d_Gi,
                           int64_t g_stride, void* stream);
+/* spb_gram_u8_batch_i32 with per-matrix K d_ncols int32 [nb] (see spb_gram_u8_batch_cols). */
+int spb_gram_u8_batch_i32_cols(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, const int32_t* d_ncols,
+                               int32_t* d_Gi, int64_t g_stride, void* stream);
 int spb_gram_hi_strip_batch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, int layout,
                             const int32_t* d_hi_rc, const uint32_t* d_hi_val, const uint32_t* d_hi_num, int64_t hi_cap,
                             double* d_Cs, int64_t cs_rows, int32_t* d_pos, int32_t* d_hr, int32_t* d_hm, void* stream);
@@ -313,6 +338,12 @@ int spb_gram_hi_strip_batch_table(const uint64_t* d_keys, const uint32_t* d_coun
                                   int64_t rows_pad, int64_t pitch, const int32_t* d_hi_rc, const uint32_t* d_hi_val,
                                   const uint32_t* d_hi_num, int64_t hi_cap, double* d_Cs, int64_t cs_rows, int32_t* d_pos, int32_t* d_hr,
                                   int32_t* d_hm, int32_t* d_ws, void* stream);
+/* The same for S0 / high lists scattered with column ranks (spb_flatten_u8_batch_cols): d_colrank, words as given there;
+ * pitch >= min(4^b, num) suffices.  NULL d_colrank is spb_gram_hi_strip_batch_table. */
+int spb_gram_hi_strip_batch_table_cols(const uint64_t* d_keys, const uint32_t* d_counts, int64_t num, const spb_split* h_splits, int nb,
+                                       int64_t rows_pad, int64_t pitch, const uint32_t* d_colrank, int64_t words, const int32_t* d_hi_rc,
+                                       const uint32_t* d_hi_val, const uint32_t* d_hi_num, int64_t hi_cap, double* d_Cs, int64_t cs_rows,
+                                       int32_t* d_pos, int32_t* d_hr, int32_t* d_hm, int32_t* d_ws, void* stream);
 int spb_score_gram_large_i32(const int32_t* d_Gi, int64_t k, int64_t ld, int64_t batch, const double* d_Cs, int64_t cs_rows,
                              const int32_t* d_pos, const int32_t* d_hr, const int32_t* d_hm, double* d_scores, double* d_info,
                              double* d_ws, void* stream);

@@ -122,6 +122,11 @@ PROTOTYPES = {
     "spb_gram_hi_correction_batch": (_i, [_p, _l, _i, _l, _l, _i, _p, _p, _p, _l, _p, _l, _p]),
     "spb_flatten_u8_batch": (_i, [_p, _p, _l, _sp, _i, _p, _l, _l, _l, _i, _i, _p, _p, _p, _l, _p]),
     "spb_flatten_u8_clear_batch": (_i, [_p, _l, _sp, _i, _p, _l, _l, _l, _i, _p]),
+    "spb_col_rank_words": (_l, [_i]),
+    "spb_col_ranks_batch": (_i, [_p, _l, _sp, _i, _p, _l, _p, _p]),
+    "spb_flatten_u8_batch_cols": (_i, [_p, _p, _l, _sp, _i, _p, _l, _p, _l, _l, _l, _i, _i, _p, _p, _p, _l, _p]),
+    "spb_flatten_u8_clear_batch_cols": (_i, [_p, _l, _sp, _i, _p, _l, _p, _l, _l, _l, _i, _p]),
+    "spb_gram_u8_batch_cols": (_i, [_p, _l, _i, _l, _l, _i, _p, _p, _l, _p, _p]),
     "spb_gram_u8": (_i, [_p, _l, _l, _i, _p, _p, _p]),
     "spb_gram_u8_simt": (_i, [_p, _l, _l, _i, _p, _p]),
     "spb_gram_hi_correction": (_i, [_p, _l, _l, _i, _p, _p, _p, _l, _p, _p]),
@@ -131,9 +136,11 @@ PROTOTYPES = {
     "spb_score_gram_large": (_i, [_p, _l, _l, _l, _p, _p, _p, _p]),
     "spb_score_gram_large_n": (_i, [_p, _l, _l, _l, _p, _p, _p, _i, _p]),
     "spb_gram_u8_batch_i32": (_i, [_p, _l, _i, _l, _l, _p, _l, _p]),
+    "spb_gram_u8_batch_i32_cols": (_i, [_p, _l, _i, _l, _l, _p, _p, _l, _p]),
     "spb_gram_hi_strip_batch": (_i, [_p, _l, _i, _l, _l, _i, _p, _p, _p, _l, _p, _l, _p, _p, _p, _p]),
     "spb_gram_hi_strip_table_ws": (_l, [_i, _l, _l]),
     "spb_gram_hi_strip_batch_table": (_i, [_p, _p, _l, _sp, _i, _l, _l, _p, _p, _p, _l, _p, _l, _p, _p, _p, _p, _p]),
+    "spb_gram_hi_strip_batch_table_cols": (_i, [_p, _p, _l, _sp, _i, _l, _l, _p, _l, _p, _p, _p, _l, _p, _l, _p, _p, _p, _p, _p]),
     "spb_score_gram_large_i32": (_i, [_p, _l, _l, _l, _p, _l, _p, _p, _p, _p, _p, _p, _p]),
     "spb_score_gram_large_i32_n": (_i, [_p, _l, _l, _l, _p, _l, _p, _p, _p, _p, _p, _p, _i, _p]),
     "spb_symv_i32_ws": (_l, [_l, _l]),

@@ -77,9 +77,10 @@ inline int make_split_dev(const spb_split* s, SplitDev* d, bool need_key64 = tru
   return SPB_OK;
 }
 
-// gram.cu: G0 = S0 S0^T (int32, both triangles) of nb tiled u8 matrices on the tensor cores; one K pass (pitch <= 32768)
-int gram_u8_i32_launch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, int32_t* d_Gi,
-                       int64_t g_stride, cudaStream_t st);
+// gram.cu: G0 = S0 S0^T (int32, both triangles) of nb tiled u8 matrices on the tensor cores; one K pass (pitch <= 32768).
+// d_ncols: NULL (K = pitch) or int32 [nb] occupied columns per matrix.
+int gram_u8_i32_launch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, const int32_t* d_ncols,
+                       int32_t* d_Gi, int64_t g_stride, cudaStream_t st);
 
 // pairs.cu: scores of `batch` symmetric k x k matrices (4 < k <= 64, leading dimension ld, stride ld * ld), one warp per matrix
 int score_gram_warp_launch(const double* d_G, int k, int64_t ld, int64_t batch, double* d_scores, cudaStream_t st);

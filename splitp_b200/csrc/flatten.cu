@@ -75,12 +75,74 @@ struct SplitBatch {  // passed by value as a kernel parameter (64 x 140 bytes; C
   SplitDev s[SPB_MAX_BATCH];
 };
 
+// ---------------------------------------------------------------------------------------------------
+// Column ranks of a batch of count flattenings.  Only the columns that some pattern projects to are non-zero, so the u8
+// scatter can store column c at its rank among the occupied columns: the Gram S0 S0^T, which contracts over the columns, is
+// unchanged, and its K shrinks from 4^b to the occupied count.  Per split, `words` = ceil(4^b / 32) words of occupancy bits
+// followed by `words` exclusive prefix counts of those bits (col_rank):
+//     rank(c) = pre[c >> 5] + popc(bits[c >> 5] & ((1 << (c & 31)) - 1)).
+// ---------------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t col_rank(const uint32_t* cr, int64_t words, uint64_t c) {
+  const uint32_t w = cr[c >> 5];
+  return cr[words + (int64_t)(c >> 5)] + (uint32_t)__popc(w & ((1u << (c & 31u)) - 1u));
+}
+
+__global__ void col_mark_kernel(const uint64_t* __restrict__ keys, int64_t num, const __grid_constant__ SplitBatch sb,
+                                uint32_t* __restrict__ cr_base, int64_t words) {
+  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= num) return;
+  const int b = blockIdx.y;
+  const SplitDev& sp = sb.s[b];
+  const uint64_t c = side_index(keys[i], sp.sh_b, sp.b);
+  uint32_t* w = cr_base + (size_t)b * 2 * words + (c >> 5);
+  const uint32_t m = 1u << (c & 31u);
+  if (!(*w & m)) atomicOr(w, m);  // most columns hold many patterns: skip the atomic once the bit is seen
+}
+
+// one block per split: exclusive prefix of the popcounts of its bit words; ncols[b] = occupied columns
+constexpr int kRankThreads = 1024;
+__global__ void __launch_bounds__(kRankThreads) col_prefix_kernel(uint32_t* __restrict__ cr_base, int64_t words, int32_t* __restrict__ ncols) {
+  __shared__ uint32_t s_warp[kRankThreads / 32];
+  uint32_t* bits = cr_base + (size_t)blockIdx.x * 2 * words;
+  uint32_t* pre = bits + words;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int64_t per = (words + kRankThreads - 1) / kRankThreads;  // contiguous words per thread
+  const int64_t w0 = tid * per, w1 = min(words, w0 + per);
+  uint32_t cnt = 0;
+  for (int64_t w = w0; w < w1; ++w) cnt += __popc(bits[w]);
+  uint32_t inc = cnt;  // inclusive scan over the block: warp shuffles, then the 32 warp totals
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    uint32_t v = __shfl_up_sync(0xffffffffu, inc, o);
+    if (lane >= o) inc += v;
+  }
+  if (lane == 31) s_warp[warp] = inc;
+  __syncthreads();
+  if (warp == 0) {
+    uint32_t t = s_warp[lane], x = t;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      uint32_t v = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += v;
+    }
+    s_warp[lane] = x - t;  // exclusive warp offsets
+  }
+  __syncthreads();
+  uint32_t run = s_warp[warp] + inc - cnt;
+  for (int64_t w = w0; w < w1; ++w) {
+    pre[w] = run;
+    run += __popc(bits[w]);
+  }
+  if (tid == kRankThreads - 1) ncols[blockIdx.x] = (int32_t)run;
+}
+
 // blockIdx.y = batch entry: split sb.s[b], S0 buffer s0 + b * s0_stride, high-part buffers offset by b * hi_cap.
 // counts == NULL: clear pass (writes zeros to the cells the scatter touched).
+// colrank != NULL: column c of batch entry b is stored at its rank (col_rank over colrank + b * 2 * cr_words)
 __global__ void u8_kernel(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ counts, int64_t num,
-                          const __grid_constant__ SplitBatch sb, const uint32_t* rank_r, const uint32_t* rank_c, uint8_t* s0_base,
-                          int64_t s0_stride, int64_t rows_pad, int64_t pitch, int layout, int32_t* hi_rc_base, uint32_t* hi_val_base,
-                          uint32_t* hi_num_base, int64_t hi_cap) {
+                          const __grid_constant__ SplitBatch sb, const uint32_t* rank_r, const uint32_t* rank_c,
+                          const uint32_t* __restrict__ colrank, int64_t cr_words, uint8_t* s0_base, int64_t s0_stride, int64_t rows_pad,
+                          int64_t pitch, int layout, int32_t* hi_rc_base, uint32_t* hi_val_base, uint32_t* hi_num_base, int64_t hi_cap) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= num) return;
   const int b = blockIdx.y;
@@ -90,6 +152,7 @@ __global__ void u8_kernel(const uint64_t* __restrict__ keys, const uint32_t* __r
   uint32_t cnt = counts ? counts[i] : 0u;
   uint64_t r = side_index(k, sp.sh_a, sp.a), c = side_index(k, sp.sh_b, sp.b);
   if (rank_r) { r = rank_r[r]; c = rank_c[c]; }
+  if (colrank) c = col_rank(colrank + (size_t)b * 2 * cr_words, cr_words, c);
   s0[s0_cell(layout, rows_pad, pitch, r, c)] = (uint8_t)(cnt & 255u);
   if (cnt >= 256u) {
     uint32_t slot = atomicAdd(hi_num_base + b, 1u);
@@ -218,7 +281,7 @@ extern "C" int spb_flatten_reduced_fill(const uint64_t* d_keys, const void* d_va
 }
 
 static int u8_check(const spb_split* split, SplitDev* sp, const uint32_t* d_rank_r, const uint32_t* d_rank_c, uint8_t* d_s0,
-                    int64_t rows_pad, int64_t pitch, int layout) {
+                    int64_t rows_pad, int64_t pitch, int layout, int64_t col_bound) {
   int rc = make_split_dev(split, sp);
   if (rc) return rc;
   SPB_REQUIRE(covers_all(split), "spb_flatten_u8: the split must cover all %d taxa", sp->n);
@@ -232,21 +295,27 @@ static int u8_check(const spb_split* split, SplitDev* sp, const uint32_t* d_rank
   SPB_REQUIRE((d_rank_r == nullptr) == (d_rank_c == nullptr), "spb_flatten_u8: give both rank arrays or neither");
   if (!d_rank_r) {
     SPB_REQUIRE(sp->a <= 15 && sp->b <= 15, "spb_flatten_u8: side too large without rank arrays");
-    SPB_REQUIRE(rows_pad >= (1ll << (2 * sp->a)) && pitch >= (1ll << (2 * sp->b)), "spb_flatten_u8: s0 too small");
+    const int64_t cols = col_bound >= 0 && col_bound < (1ll << (2 * sp->b)) ? col_bound : (1ll << (2 * sp->b));
+    SPB_REQUIRE(rows_pad >= (1ll << (2 * sp->a)) && pitch >= cols, "spb_flatten_u8: s0 too small");
   }
   return SPB_OK;
 }
 
 static int u8_batch_common(const uint64_t* d_keys, const uint32_t* d_counts, int64_t num, const spb_split* h_splits, int nb,
-                           const uint32_t* d_rank_r, const uint32_t* d_rank_c, uint8_t* d_s0, int64_t s0_stride, int64_t rows_pad,
-                           int64_t pitch, int layout, int flags, int32_t* d_hi_rc, uint32_t* d_hi_val, uint32_t* d_hi_num,
-                           int64_t hi_cap, bool clear, cudaStream_t st) {
+                           const uint32_t* d_rank_r, const uint32_t* d_rank_c, const uint32_t* d_colrank, int64_t cr_words,
+                           uint8_t* d_s0, int64_t s0_stride, int64_t rows_pad, int64_t pitch, int layout, int flags, int32_t* d_hi_rc,
+                           uint32_t* d_hi_val, uint32_t* d_hi_num, int64_t hi_cap, bool clear, cudaStream_t st) {
   SPB_REQUIRE(h_splits && nb >= 1 && nb <= SPB_MAX_BATCH, "spb_flatten_u8: batch size must be 1..%d (got %d)", SPB_MAX_BATCH, nb);
   SPB_REQUIRE(nb == 1 || (s0_stride >= rows_pad * pitch && !d_rank_r), "spb_flatten_u8: bad batch stride / rank arrays in a batch");
+  SPB_REQUIRE(!d_colrank || !d_rank_r, "spb_flatten_u8: column ranks and reduced-format rank arrays exclude each other");
   SplitBatch sb;
   for (int b = 0; b < nb; ++b) {
-    int rc = u8_check(h_splits + b, &sb.s[b], d_rank_r, d_rank_c, d_s0, rows_pad, pitch, layout);
+    // ranked columns: at most min(4^b, num) of them are occupied
+    int rc = u8_check(h_splits + b, &sb.s[b], d_rank_r, d_rank_c, d_s0, rows_pad, pitch, layout, d_colrank ? (num > 0 ? num : 0) : -1);
     if (rc) return rc;
+    if (d_colrank)
+      SPB_REQUIRE(cr_words == ((1ll << (2 * sb.s[b].b)) + 31) / 32, "spb_flatten_u8: column-rank words %lld do not match 4^%d columns",
+                  (long long)cr_words, sb.s[b].b);
   }
   if (!clear) {
     SPB_REQUIRE(d_hi_rc && d_hi_val && d_hi_num, "spb_flatten_u8: NULL high-part buffers");
@@ -258,8 +327,8 @@ static int u8_batch_common(const uint64_t* d_keys, const uint32_t* d_counts, int
   if (num <= 0) return SPB_OK;
   SPB_REQUIRE(d_keys && (clear || d_counts), "spb_flatten_u8: NULL pattern table");
   dim3 grid(nblk(num, 256), (unsigned)nb);
-  u8_kernel<<<grid, 256, 0, st>>>(d_keys, clear ? nullptr : d_counts, num, sb, d_rank_r, d_rank_c, d_s0, s0_stride, rows_pad, pitch,
-                                  layout, d_hi_rc, d_hi_val, d_hi_num, hi_cap);
+  u8_kernel<<<grid, 256, 0, st>>>(d_keys, clear ? nullptr : d_counts, num, sb, d_rank_r, d_rank_c, d_colrank, cr_words, d_s0, s0_stride,
+                                  rows_pad, pitch, layout, d_hi_rc, d_hi_val, d_hi_num, hi_cap);
   SPB_LAUNCH_CHECK();
   return SPB_OK;
 }
@@ -267,27 +336,68 @@ static int u8_batch_common(const uint64_t* d_keys, const uint32_t* d_counts, int
 extern "C" int spb_flatten_u8_batch(const uint64_t* d_keys, const uint32_t* d_counts, int64_t num, const spb_split* h_splits, int nb,
                                     uint8_t* d_s0, int64_t s0_stride, int64_t rows_pad, int64_t pitch, int layout, int flags,
                                     int32_t* d_hi_rc, uint32_t* d_hi_val, uint32_t* d_hi_num, int64_t hi_cap, void* stream) {
-  return u8_batch_common(d_keys, d_counts, num, h_splits, nb, nullptr, nullptr, d_s0, s0_stride, rows_pad, pitch, layout, flags,
-                         d_hi_rc, d_hi_val, d_hi_num, hi_cap, false, (cudaStream_t)stream);
+  return u8_batch_common(d_keys, d_counts, num, h_splits, nb, nullptr, nullptr, nullptr, 0, d_s0, s0_stride, rows_pad, pitch, layout,
+                         flags, d_hi_rc, d_hi_val, d_hi_num, hi_cap, false, (cudaStream_t)stream);
 }
 
 extern "C" int spb_flatten_u8_clear_batch(const uint64_t* d_keys, int64_t num, const spb_split* h_splits, int nb, uint8_t* d_s0,
                                           int64_t s0_stride, int64_t rows_pad, int64_t pitch, int layout, void* stream) {
-  return u8_batch_common(d_keys, nullptr, num, h_splits, nb, nullptr, nullptr, d_s0, s0_stride, rows_pad, pitch, layout, 0, nullptr,
-                         nullptr, nullptr, 0, true, (cudaStream_t)stream);
+  return u8_batch_common(d_keys, nullptr, num, h_splits, nb, nullptr, nullptr, nullptr, 0, d_s0, s0_stride, rows_pad, pitch, layout, 0,
+                         nullptr, nullptr, nullptr, 0, true, (cudaStream_t)stream);
 }
 
 extern "C" int spb_flatten_u8(const uint64_t* d_keys, const uint32_t* d_counts, int64_t num, const spb_split* split,
                               const uint32_t* d_rank_r, const uint32_t* d_rank_c, uint8_t* d_s0, int64_t rows_pad,
                               int64_t pitch, int layout, int flags, int32_t* d_hi_rc, uint32_t* d_hi_val, uint32_t* d_hi_num,
                               int64_t hi_cap, void* stream) {
-  return u8_batch_common(d_keys, d_counts, num, split, 1, d_rank_r, d_rank_c, d_s0, rows_pad * pitch, rows_pad, pitch, layout, flags,
-                         d_hi_rc, d_hi_val, d_hi_num, hi_cap, false, (cudaStream_t)stream);
+  return u8_batch_common(d_keys, d_counts, num, split, 1, d_rank_r, d_rank_c, nullptr, 0, d_s0, rows_pad * pitch, rows_pad, pitch, layout,
+                         flags, d_hi_rc, d_hi_val, d_hi_num, hi_cap, false, (cudaStream_t)stream);
 }
 
 extern "C" int spb_flatten_u8_clear(const uint64_t* d_keys, int64_t num, const spb_split* split, const uint32_t* d_rank_r,
                                     const uint32_t* d_rank_c, uint8_t* d_s0, int64_t rows_pad, int64_t pitch, int layout,
                                     void* stream) {
-  return u8_batch_common(d_keys, nullptr, num, split, 1, d_rank_r, d_rank_c, d_s0, rows_pad * pitch, rows_pad, pitch, layout, 0,
+  return u8_batch_common(d_keys, nullptr, num, split, 1, d_rank_r, d_rank_c, nullptr, 0, d_s0, rows_pad * pitch, rows_pad, pitch, layout,
+                         0, nullptr, nullptr, nullptr, 0, true, (cudaStream_t)stream);
+}
+
+extern "C" int64_t spb_col_rank_words(int b) { return ((1ll << (2 * b)) + 31) / 32; }
+
+extern "C" int spb_col_ranks_batch(const uint64_t* d_keys, int64_t num, const spb_split* h_splits, int nb, uint32_t* d_colrank,
+                                   int64_t words, int32_t* d_ncols, void* stream) {
+  SPB_REQUIRE(h_splits && nb >= 1 && nb <= SPB_MAX_BATCH, "spb_col_ranks: batch size must be 1..%d (got %d)", SPB_MAX_BATCH, nb);
+  SPB_REQUIRE(d_colrank && d_ncols && (num <= 0 || d_keys), "spb_col_ranks: NULL buffer");
+  SplitBatch sb;
+  for (int b = 0; b < nb; ++b) {
+    int rc = make_split_dev(h_splits + b, &sb.s[b]);
+    if (rc) return rc;
+    SPB_REQUIRE(sb.s[b].b <= 15 && words == spb_col_rank_words(sb.s[b].b), "spb_col_ranks: %lld words do not match 4^%d columns",
+                (long long)words, sb.s[b].b);
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  SPB_CUDA(cudaMemsetAsync(d_colrank, 0, (size_t)nb * 2 * words * sizeof(uint32_t), st));
+  if (num > 0) {
+    col_mark_kernel<<<dim3(nblk(num, 256), (unsigned)nb), 256, 0, st>>>(d_keys, num, sb, d_colrank, words);
+    SPB_LAUNCH_CHECK();
+  }
+  col_prefix_kernel<<<nb, kRankThreads, 0, st>>>(d_colrank, words, d_ncols);
+  SPB_LAUNCH_CHECK();
+  return SPB_OK;
+}
+
+extern "C" int spb_flatten_u8_batch_cols(const uint64_t* d_keys, const uint32_t* d_counts, int64_t num, const spb_split* h_splits, int nb,
+                                         const uint32_t* d_colrank, int64_t words, uint8_t* d_s0, int64_t s0_stride, int64_t rows_pad,
+                                         int64_t pitch, int layout, int flags, int32_t* d_hi_rc, uint32_t* d_hi_val, uint32_t* d_hi_num,
+                                         int64_t hi_cap, void* stream) {
+  SPB_REQUIRE(d_colrank, "spb_flatten_u8_batch_cols: NULL column ranks");
+  return u8_batch_common(d_keys, d_counts, num, h_splits, nb, nullptr, nullptr, d_colrank, words, d_s0, s0_stride, rows_pad, pitch, layout,
+                         flags, d_hi_rc, d_hi_val, d_hi_num, hi_cap, false, (cudaStream_t)stream);
+}
+
+extern "C" int spb_flatten_u8_clear_batch_cols(const uint64_t* d_keys, int64_t num, const spb_split* h_splits, int nb,
+                                               const uint32_t* d_colrank, int64_t words, uint8_t* d_s0, int64_t s0_stride,
+                                               int64_t rows_pad, int64_t pitch, int layout, void* stream) {
+  SPB_REQUIRE(d_colrank, "spb_flatten_u8_clear_batch_cols: NULL column ranks");
+  return u8_batch_common(d_keys, nullptr, num, h_splits, nb, nullptr, nullptr, d_colrank, words, d_s0, s0_stride, rows_pad, pitch, layout, 0,
                          nullptr, nullptr, nullptr, 0, true, (cudaStream_t)stream);
 }

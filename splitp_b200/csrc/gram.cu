@@ -88,6 +88,14 @@ __host__ __device__ constexpr uint32_t make_idesc_i8(int M, int N) {
   return (2u << 4) | (0u << 7) | (0u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
+// K tiles of matrix b: all KT of the allocation pitch, or (ncols != NULL) the tiles holding its ncols[b] occupied columns (the
+// columns beyond them are zero).  At least one tile, so every work item issues an MMA and writes its accumulator.
+__device__ __forceinline__ int k_tiles(const int32_t* ncols, int b, int KT) {
+  if (!ncols) return KT;
+  const int t = (ncols[b] + kTile - 1) / kTile;
+  return t < 1 ? 1 : (t > KT ? KT : t);
+}
+
 // ---------------------------------------------------------------------------------------------------
 // work decomposition shared by all roles.  Tiles: row tile i (128 rows) x column tile j (BN columns), computed
 // only if the tile's 256-block column index >= its 256-block row index.  Work item = (tile, k-split).
@@ -122,6 +130,17 @@ __device__ __forceinline__ bool get_work(int w, int T, int TN, int tiles, int ks
   return false;
 }
 
+// K-tile range [kt0, kt1) of a work item; false when it is empty (a K split of a matrix with fewer occupied tiles than the
+// split has parts: the work item is skipped by all three roles alike).  With column counts every matrix splits its own K tiles
+// into ksplit equal parts (at most kt_per_split each, as the host planned them for the full pitch).
+__device__ __forceinline__ bool k_range(const int32_t* ncols, const Work& wk, int KT, int ksplit, int kt_per_split, int* kt0, int* kt1) {
+  const int kb = k_tiles(ncols, wk.b, KT);
+  const int per = ncols ? (kb + ksplit - 1) / ksplit : kt_per_split;
+  *kt0 = wk.ks * per;
+  *kt1 = min(kb, *kt0 + per);
+  return *kt0 < *kt1;
+}
+
 template <int BN>
 int count_tiles(int T, int TN) {
   int c = 0;
@@ -139,7 +158,7 @@ int count_tiles(int T, int TN) {
 template <int BN>
 __global__ void __launch_bounds__(kUmmaThreads, 1)
 gram_u8_umma_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int T, int KT, int tiles, int ksplit, int kt_per_split,
-                    int num_work, int64_t ldg, double* __restrict__ G_base, int64_t g_stride,
+                    const int32_t* __restrict__ ncols, int num_work, int64_t ldg, double* __restrict__ G_base, int64_t g_stride,
                     unsigned long long* __restrict__ acc_base, int32_t* __restrict__ Gi_base) {
   constexpr int kStageBytes = kTileBytes + BN * kTile;  // A tile + B tile(s)
   constexpr uint32_t kTmemCols = 2 * BN;                 // two accumulator stages (power of two >= 32)
@@ -176,8 +195,8 @@ gram_u8_umma_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int 
       for (int w = blockIdx.x; w < num_work; w += gridDim.x) {
         Work wk;
         if (!get_work<BN>(w, T, TN, tiles, ksplit, &wk)) break;
-        const int kt0 = wk.ks * kt_per_split;
-        const int kt1 = min(KT, kt0 + kt_per_split);
+        int kt0, kt1;
+        if (!k_range(ncols, wk, KT, ksplit, kt_per_split, &kt0, &kt1)) continue;
         const uint8_t* s0t = s0_base + (size_t)wk.b * s0_stride;
         for (int kt = kt0; kt < kt1; ++kt) {
           mbar_wait(smem_u32(empty_bar + stage), phase ^ 1);
@@ -202,8 +221,8 @@ gram_u8_umma_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int 
       for (int w = blockIdx.x; w < num_work; w += gridDim.x) {
         Work wk;
         if (!get_work<BN>(w, T, TN, tiles, ksplit, &wk)) break;
-        const int kt0 = wk.ks * kt_per_split;
-        const int kt1 = min(KT, kt0 + kt_per_split);
+        int kt0, kt1;
+        if (!k_range(ncols, wk, KT, ksplit, kt_per_split, &kt0, &kt1)) continue;
         mbar_wait(smem_u32(tempty_bar + acc), acc_phase ^ 1);  // epilogue has drained this accumulator
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + acc * BN;
@@ -234,6 +253,8 @@ gram_u8_umma_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int 
     for (int w = blockIdx.x; w < num_work; w += gridDim.x) {
       Work wk;
       if (!get_work<BN>(w, T, TN, tiles, ksplit, &wk)) break;
+      int kt0, kt1;
+      if (!k_range(ncols, wk, KT, ksplit, kt_per_split, &kt0, &kt1)) continue;
       mbar_wait(smem_u32(tfull_bar + acc), acc_phase);
       tc_fence_after();
       const int row = wk.i * kTile + q * 32 + lane;
@@ -353,8 +374,8 @@ __device__ __forceinline__ void get_work2(int w, int B, int nblk, Work2* out) {
 }
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
-gram_u8_umma2_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int B, int KT, int nblk, int num_work, int64_t ldg,
-                     double* __restrict__ G_base, int64_t g_stride, int32_t* __restrict__ Gi_base) {
+gram_u8_umma2_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int B, int KT, const int32_t* __restrict__ ncols, int nblk,
+                     int num_work, int64_t ldg, double* __restrict__ G_base, int64_t g_stride, int32_t* __restrict__ Gi_base) {
   constexpr uint32_t kIdesc = make_idesc_i8(256, 256);
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* ring = smem + ((1024u - (smem_u32(smem) & 1023u)) & 1023u);  // same offset in both CTAs (same kernel, same layout)
@@ -396,7 +417,8 @@ gram_u8_umma2_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int
         const uint8_t* s0t = s0_base + (size_t)wk.b * s0_stride;
         const uint8_t* a_src = s0t + (size_t)(2 * wk.bi + (int)rank) * KT * kTileBytes;
         const uint8_t* b_src = s0t + (size_t)(2 * wk.bj + (int)rank) * KT * kTileBytes;
-        for (int kt = 0; kt < KT; ++kt) {
+        const int kb = k_tiles(ncols, wk.b, KT);
+        for (int kt = 0; kt < kb; ++kt) {
           mbar_wait(smem_u32(empty_bar + stage), phase ^ 1);
           const uint32_t fb = smem_u32(full_bar + stage);
           mbar_expect_tx(fb, (uint32_t)kStage2Bytes);
@@ -412,10 +434,11 @@ gram_u8_umma2_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int
       // ===== MMA issuer of the pair =====
       uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0;
       for (int w = pair; w < num_work; w += npairs) {
+        const int kb = k_tiles(ncols, w / nblk, KT);
         mbar_wait(smem_u32(tempty_bar + acc), acc_phase ^ 1);  // both epilogues have drained this accumulator
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + acc * 256;
-        for (int kt = 0; kt < KT; ++kt) {
+        for (int kt = 0; kt < kb; ++kt) {
           mbar_wait(smem_u32(full_bar + stage), phase);
           mbar_wait(smem_u32(peer_full_bar + stage), phase);
           tc_fence_after();
@@ -435,7 +458,8 @@ gram_u8_umma2_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int
       // ===== relay: "stage s of CTA 1 is full" -> leader =====
       uint32_t stage = 0, phase = 0;
       for (int w = pair; w < num_work; w += npairs) {
-        for (int kt = 0; kt < KT; ++kt) {
+        const int kb = k_tiles(ncols, w / nblk, KT);
+        for (int kt = 0; kt < kb; ++kt) {
           mbar_wait(smem_u32(full_bar + stage), phase);
           mbar_arrive_remote(map_to_cta(smem_u32(peer_full_bar + stage), 0));
           if (++stage == kStages2) { stage = 0; phase ^= 1; }
@@ -523,7 +547,8 @@ __global__ void gram_finalize_kernel(const unsigned long long* __restrict__ acc_
 constexpr int kSmallWords = 256;  // word columns (= 1024 k) per chunk
 
 __global__ void __launch_bounds__(256) gram_u8_small_kernel(const uint32_t* __restrict__ s0w_base, int64_t s0_stride_words, int Rp,
-                                                            int64_t words, unsigned long long* __restrict__ acc_base) {
+                                                            int64_t words, const int32_t* __restrict__ ncols,
+                                                            unsigned long long* __restrict__ acc_base) {
   extern __shared__ __align__(16) uint32_t s_chunk[];  // [kSmallWords][Rp]
   const uint32_t* s0w = s0w_base + (size_t)blockIdx.y * s0_stride_words;
   unsigned long long* acc64 = acc_base + (size_t)blockIdx.y * Rp * Rp;
@@ -537,6 +562,7 @@ __global__ void __launch_bounds__(256) gram_u8_small_kernel(const uint32_t* __re
   unsigned long long tot[16];
 #pragma unroll
   for (int e = 0; e < 16; ++e) tot[e] = 0ull;
+  if (ncols) words = min(words, ((int64_t)ncols[blockIdx.y] + 3) / 4);  // word columns holding the occupied columns
   const int64_t nchunks = (words + kSmallWords - 1) / kSmallWords;
   for (int64_t ch = blockIdx.x; ch < nchunks; ch += gridDim.x) {
     const int64_t w0 = ch * kSmallWords;
@@ -771,7 +797,8 @@ __global__ void __launch_bounds__(256) hi_join_kernel(const uint64_t* __restrict
                                                       const int32_t* __restrict__ hi_rc_base, const uint32_t* __restrict__ hi_val_base,
                                                       int64_t hi_cap, const int32_t* __restrict__ colmap_base,
                                                       const int32_t* __restrict__ next_base, const int32_t* __restrict__ pos_base,
-                                                      double* __restrict__ Cs_base, int64_t cs_rows) {
+                                                      double* __restrict__ Cs_base, int64_t cs_rows, const uint32_t* __restrict__ colrank,
+                                                      int64_t cr_words) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= num) return;
   const uint32_t s = counts[i] & 255u;
@@ -779,7 +806,13 @@ __global__ void __launch_bounds__(256) hi_join_kernel(const uint64_t* __restrict
   const int b = blockIdx.y;
   const SplitDev& sp = sb.s[b];
   const uint64_t k = keys[i];
-  const int64_t ri = (int64_t)side_index(k, sp.sh_a, sp.a), ci = (int64_t)side_index(k, sp.sh_b, sp.b);
+  const int64_t ri = (int64_t)side_index(k, sp.sh_a, sp.a);
+  int64_t ci = (int64_t)side_index(k, sp.sh_b, sp.b);
+  if (colrank) {  // the high list holds ranked columns (spb_flatten_u8_batch_cols): look the pattern's column up the same way
+    const uint32_t* cr = colrank + (size_t)b * 2 * cr_words;
+    const uint32_t w = cr[ci >> 5];
+    ci = (int64_t)cr[cr_words + (ci >> 5)] + __popc(w & ((1u << (ci & 31)) - 1u));
+  }
   int32_t e = colmap_base[(size_t)b * pitch + ci];
   if (e == 0) return;
   const int32_t* hi_rc = hi_rc_base + (size_t)b * 2 * hi_cap;
@@ -837,8 +870,8 @@ UmmaPlan plan_umma(int64_t rows_pad, int64_t pitch, int nb, bool single_pass = f
 }
 
 // Launches the CTA-pair kernel for nb matrices (no K split: one accumulation covers all of K, KT <= 256).
-int launch_umma2(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, double* d_G, int32_t* d_Gi,
-                 int64_t g_stride, cudaStream_t st) {
+int launch_umma2(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, const int32_t* d_ncols, double* d_G,
+                 int32_t* d_Gi, int64_t g_stride, cudaStream_t st) {
   const int B = (int)(rows_pad / 256), KT = (int)(pitch / kTile);
   const int nblk = B * (B + 1) / 2;
   const int num_work = nblk * nb;
@@ -859,7 +892,8 @@ int launch_umma2(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pa
     max_pairs = n;
   }
   const int pairs = num_work < max_pairs ? num_work : max_pairs;
-  gram_u8_umma2_kernel<<<2 * pairs, kUmmaThreads, smem, st>>>(d_s0, s0_stride, B, KT, nblk, num_work, rows_pad, d_G, g_stride, d_Gi);
+  gram_u8_umma2_kernel<<<2 * pairs, kUmmaThreads, smem, st>>>(d_s0, s0_stride, B, KT, d_ncols, nblk, num_work, rows_pad, d_G, g_stride,
+                                                             d_Gi);
   SPB_LAUNCH_CHECK();
   return SPB_OK;
 }
@@ -886,8 +920,10 @@ extern "C" int64_t spb_gram_u8_ws(int64_t rows_pad, int64_t pitch, int layout, i
   return p.ksplit > 1 ? nb * rows_pad * rows_pad : 0;
 }
 
-extern "C" int spb_gram_u8_batch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, int layout,
-                                 double* d_G, int64_t g_stride, uint64_t* d_ws, void* stream) {
+// d_ncols: NULL (K = pitch) or int32 [nb] occupied columns per matrix (K = ncols[b]; S0 is zero beyond it).  The launch is
+// planned for K = pitch; each matrix then runs only the K tiles that hold its columns.
+extern "C" int spb_gram_u8_batch_cols(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, int layout,
+                                      const int32_t* d_ncols, double* d_G, int64_t g_stride, uint64_t* d_ws, void* stream) {
   SPB_REQUIRE(d_s0 && d_G && rows_pad >= 1 && pitch >= 16 && pitch % 16 == 0 && nb >= 1 && nb <= 65535,
               "spb_gram_u8: bad arguments");
   SPB_REQUIRE(nb == 1 || (s0_stride >= rows_pad * pitch && s0_stride % 16 == 0 && g_stride >= rows_pad * rows_pad),
@@ -907,7 +943,7 @@ extern "C" int spb_gram_u8_batch(const uint8_t* d_s0, int64_t s0_stride, int nb,
     if (gx > nchunks) gx = nchunks;
     if (gx < 1) gx = 1;
     dim3 grid((unsigned)gx, (unsigned)nb);
-    gram_u8_small_kernel<<<grid, 256, smem, st>>>(reinterpret_cast<const uint32_t*>(d_s0), s0_stride / 4, R, words,
+    gram_u8_small_kernel<<<grid, 256, smem, st>>>(reinterpret_cast<const uint32_t*>(d_s0), s0_stride / 4, R, words, d_ncols,
                                                   (unsigned long long*)d_ws);
     SPB_LAUNCH_CHECK();
     dim3 fg((R * R + 255) / 256, (unsigned)nb);
@@ -928,15 +964,15 @@ extern "C" int spb_gram_u8_batch(const uint8_t* d_s0, int64_t s0_stride, int nb,
     SPB_CUDA(cudaMemsetAsync(acc, 0, (size_t)nb * rows_pad * rows_pad * 8, st));
   }
   if (p.BN == 256 && p.ksplit == 1 && p.KT <= 256 && use_pair_kernel())
-    return launch_umma2(d_s0, s0_stride, nb, rows_pad, pitch, d_G, nullptr, g_stride, st);
+    return launch_umma2(d_s0, s0_stride, nb, rows_pad, pitch, d_ncols, d_G, nullptr, g_stride, st);
   int grid = p.num_work < sm_count() ? p.num_work : sm_count();
   if (p.BN == 256) {
     SPB_CUDA(cudaFuncSetAttribute(gram_u8_umma_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
-    gram_u8_umma_kernel<256><<<grid, kUmmaThreads, p.smem, st>>>(d_s0, s0_stride, p.T, p.KT, p.tiles, p.ksplit, p.kt_per_split,
+    gram_u8_umma_kernel<256><<<grid, kUmmaThreads, p.smem, st>>>(d_s0, s0_stride, p.T, p.KT, p.tiles, p.ksplit, p.kt_per_split, d_ncols,
                                                                p.num_work, rows_pad, d_G, g_stride, acc, nullptr);
   } else {
     SPB_CUDA(cudaFuncSetAttribute(gram_u8_umma_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
-    gram_u8_umma_kernel<128><<<grid, kUmmaThreads, p.smem, st>>>(d_s0, s0_stride, p.T, p.KT, p.tiles, p.ksplit, p.kt_per_split,
+    gram_u8_umma_kernel<128><<<grid, kUmmaThreads, p.smem, st>>>(d_s0, s0_stride, p.T, p.KT, p.tiles, p.ksplit, p.kt_per_split, d_ncols,
                                                                p.num_work, rows_pad, d_G, g_stride, acc, nullptr);
   }
   SPB_LAUNCH_CHECK();
@@ -949,9 +985,14 @@ extern "C" int spb_gram_u8_batch(const uint8_t* d_s0, int64_t s0_stride, int nb,
   return SPB_OK;
 }
 
+extern "C" int spb_gram_u8_batch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, int layout,
+                                 double* d_G, int64_t g_stride, uint64_t* d_ws, void* stream) {
+  return spb_gram_u8_batch_cols(d_s0, s0_stride, nb, rows_pad, pitch, layout, nullptr, d_G, g_stride, d_ws, stream);
+}
+
 namespace spb {
-int gram_u8_i32_launch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, int32_t* d_Gi,
-                       int64_t g_stride, cudaStream_t st) {
+int gram_u8_i32_launch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, const int32_t* d_ncols,
+                       int32_t* d_Gi, int64_t g_stride, cudaStream_t st) {
   SPB_REQUIRE(d_s0 && d_Gi && nb >= 1 && nb <= 65535, "spb_gram_u8_batch_i32: bad arguments");
   SPB_REQUIRE(rows_pad % 256 == 0 && rows_pad >= 256 && rows_pad <= 32768 && pitch % kTile == 0 && pitch >= kTile,
               "spb_gram_u8_batch_i32: needs the tiled layout with rows_pad %% 256 == 0 and pitch %% 128 == 0 (got %lld, %lld)",
@@ -960,13 +1001,13 @@ int gram_u8_i32_launch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t r
               (long long)pitch, 256 * kTile);
   SPB_REQUIRE(nb == 1 || (s0_stride >= rows_pad * pitch && s0_stride % 16 == 0 && g_stride >= rows_pad * rows_pad),
               "spb_gram_u8_batch_i32: bad batch strides");
-  if (use_pair_kernel()) return launch_umma2(d_s0, s0_stride, nb, rows_pad, pitch, nullptr, d_Gi, g_stride, st);
+  if (use_pair_kernel()) return launch_umma2(d_s0, s0_stride, nb, rows_pad, pitch, d_ncols, nullptr, d_Gi, g_stride, st);
   UmmaPlan p = plan_umma(rows_pad, pitch, nb, true);
   if (p.ksplit != 1) { set_error("spb_gram_u8_batch_i32: internal: K split"); return SPB_ERR_ARG; }
   int grid = p.num_work < sm_count() ? p.num_work : sm_count();
   SPB_CUDA(cudaFuncSetAttribute(gram_u8_umma_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
-  gram_u8_umma_kernel<256><<<grid, kUmmaThreads, p.smem, st>>>(d_s0, s0_stride, p.T, p.KT, p.tiles, 1, p.kt_per_split, p.num_work, rows_pad,
-                                                             nullptr, g_stride, nullptr, d_Gi);
+  gram_u8_umma_kernel<256><<<grid, kUmmaThreads, p.smem, st>>>(d_s0, s0_stride, p.T, p.KT, p.tiles, 1, p.kt_per_split, d_ncols, p.num_work,
+                                                             rows_pad, nullptr, g_stride, nullptr, d_Gi);
   SPB_LAUNCH_CHECK();
   return SPB_OK;
 }
@@ -974,7 +1015,12 @@ int gram_u8_i32_launch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t r
 
 extern "C" int spb_gram_u8_batch_i32(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch,
                                      int32_t* d_Gi, int64_t g_stride, void* stream) {
-  return spb::gram_u8_i32_launch(d_s0, s0_stride, nb, rows_pad, pitch, d_Gi, g_stride, (cudaStream_t)stream);
+  return spb::gram_u8_i32_launch(d_s0, s0_stride, nb, rows_pad, pitch, nullptr, d_Gi, g_stride, (cudaStream_t)stream);
+}
+
+extern "C" int spb_gram_u8_batch_i32_cols(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch,
+                                          const int32_t* d_ncols, int32_t* d_Gi, int64_t g_stride, void* stream) {
+  return spb::gram_u8_i32_launch(d_s0, s0_stride, nb, rows_pad, pitch, d_ncols, d_Gi, g_stride, (cudaStream_t)stream);
 }
 
 extern "C" int spb_gram_hi_strip_batch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pad, int64_t pitch, int layout,
@@ -1002,10 +1048,12 @@ extern "C" int spb_gram_hi_strip_batch(const uint8_t* d_s0, int64_t s0_stride, i
 
 extern "C" int64_t spb_gram_hi_strip_table_ws(int nb, int64_t pitch, int64_t hi_cap) { return (int64_t)nb * (pitch + hi_cap); }
 
-extern "C" int spb_gram_hi_strip_batch_table(const uint64_t* d_keys, const uint32_t* d_counts, int64_t num, const spb_split* h_splits,
-                                             int nb, int64_t rows_pad, int64_t pitch, const int32_t* d_hi_rc, const uint32_t* d_hi_val,
-                                             const uint32_t* d_hi_num, int64_t hi_cap, double* d_Cs, int64_t cs_rows, int32_t* d_pos,
-                                             int32_t* d_hr, int32_t* d_hm, int32_t* d_ws, void* stream) {
+// d_colrank: NULL, or the column ranks the high list was scattered with (spb_col_ranks_batch, `words` per split)
+extern "C" int spb_gram_hi_strip_batch_table_cols(const uint64_t* d_keys, const uint32_t* d_counts, int64_t num, const spb_split* h_splits,
+                                                  int nb, int64_t rows_pad, int64_t pitch, const uint32_t* d_colrank, int64_t words,
+                                                  const int32_t* d_hi_rc, const uint32_t* d_hi_val, const uint32_t* d_hi_num, int64_t hi_cap,
+                                                  double* d_Cs, int64_t cs_rows, int32_t* d_pos, int32_t* d_hr, int32_t* d_hm, int32_t* d_ws,
+                                                  void* stream) {
   SPB_REQUIRE(h_splits && d_hi_rc && d_hi_val && d_hi_num && d_pos && d_hm && d_ws && hi_cap >= 0 && nb >= 1 && nb <= SPB_MAX_BATCH &&
                   cs_rows >= 0 && cs_rows <= 65535 && rows_pad % 2 == 0,
               "spb_gram_hi_strip_table: bad arguments");
@@ -1015,8 +1063,9 @@ extern "C" int spb_gram_hi_strip_batch_table(const uint64_t* d_keys, const uint3
   for (int b = 0; b < nb; ++b) {
     int rc = make_split_dev(h_splits + b, &sb.s[b]);
     if (rc) return rc;
+    const int64_t cols = d_colrank ? (num < (1ll << (2 * sb.s[b].b)) ? num : (1ll << (2 * sb.s[b].b))) : (1ll << (2 * sb.s[b].b));
     SPB_REQUIRE(sb.s[b].a + sb.s[b].b == sb.s[b].n && sb.s[b].a <= 15 && sb.s[b].b <= 15 && rows_pad >= (1ll << (2 * sb.s[b].a)) &&
-                    pitch >= (1ll << (2 * sb.s[b].b)),
+                    pitch >= cols && (!d_colrank || words == ((1ll << (2 * sb.s[b].b)) + 31) / 32),
                 "spb_gram_hi_strip_table: every split must cover all taxa and fit rows_pad x pitch");
   }
   cudaStream_t st = (cudaStream_t)stream;
@@ -1039,7 +1088,7 @@ extern "C" int spb_gram_hi_strip_batch_table(const uint64_t* d_keys, const uint3
   if (num > 0) {
     dim3 jg((unsigned)((num + 255) / 256), (unsigned)nb);
     hi_join_kernel<<<jg, 256, 0, st>>>(d_keys, d_counts, num, sb, rows_pad, pitch, d_hi_rc, d_hi_val, hi_cap, colmap, next, d_pos, d_Cs,
-                                       cs_rows);
+                                       cs_rows, d_colrank, words);
     SPB_LAUNCH_CHECK();
   }
   int64_t gx = (4 * (int64_t)sm_count() + nb - 1) / nb;
@@ -1047,6 +1096,14 @@ extern "C" int spb_gram_hi_strip_batch_table(const uint64_t* d_keys, const uint3
   hi_strip_self_kernel<<<sg, 256, 0, st>>>(d_hi_rc, d_hi_val, d_hi_num, hi_cap, rows_pad, d_pos, d_Cs, cs_rows);
   SPB_LAUNCH_CHECK();
   return SPB_OK;
+}
+
+extern "C" int spb_gram_hi_strip_batch_table(const uint64_t* d_keys, const uint32_t* d_counts, int64_t num, const spb_split* h_splits,
+                                             int nb, int64_t rows_pad, int64_t pitch, const int32_t* d_hi_rc, const uint32_t* d_hi_val,
+                                             const uint32_t* d_hi_num, int64_t hi_cap, double* d_Cs, int64_t cs_rows, int32_t* d_pos,
+                                             int32_t* d_hr, int32_t* d_hm, int32_t* d_ws, void* stream) {
+  return spb_gram_hi_strip_batch_table_cols(d_keys, d_counts, num, h_splits, nb, rows_pad, pitch, nullptr, 0, d_hi_rc, d_hi_val, d_hi_num,
+                                            hi_cap, d_Cs, cs_rows, d_pos, d_hr, d_hm, d_ws, stream);
 }
 
 extern "C" int spb_gram_u8(const uint8_t* d_s0, int64_t rows_pad, int64_t pitch, int layout, double* d_G, uint64_t* d_ws,

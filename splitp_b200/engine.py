@@ -638,6 +638,7 @@ class CountScorer:
         self._ws = {}
         self._batch_bytes = None
         self._hi_ws = {}
+        self._cr = {}          # (stream slot, words) -> column-rank buffers of one Gram batch, see _col_ranks
         self._plans = {}       # (id(split list), taxa, class) -> encoded splits + output positions, see _encoded_group
         self.strip_from_table = os.environ.get("SPB_STRIP_KERNEL", "table") != "scan"  # A/B switch: column scans of S0 (round 1)
         self.int32_gram = True  # large dense splits keep G as int32 + correction strip (half the eigen-stage traffic)
@@ -731,44 +732,73 @@ class CountScorer:
             ws = self._hi_ws[key] = _empty(need, torch.int32)
         return ws
 
-    def _scatter(self, arr, nb, s0, layout, rows_pad, pitch, clear=False):
-        """Scatter (or un-scatter) nb <= GNB splits into s0[0:nb], SPB_MAX_BATCH splits per launch."""
+    def _col_pitch(self, layout, pitch):
+        """S0 pitch of a batch scattered with column ranks: room for min(4^b, P) occupied columns.  P is rounded up to a power
+        of two so that tables of similar size share the cached S0 buffers."""
+        return min(int(pitch), 1 << max(7, (max(int(self.table.num), 1) - 1).bit_length()))
+
+    def _col_ranks(self, arr, nb):
+        """Column ranks of nb <= GNB splits of equal shape (spb_col_ranks_batch) into this stream slot's buffers:
+        (colrank, words, ncols); ncols [nb] = occupied columns of every split, the K of its Gram."""
         t = self.table
-        s0_stride, sz = rows_pad * pitch, C.sizeof(_lib.SpbSplit)
+        words = int(lib.spb_col_rank_words(int(arr[0].b)))
+        key = (self._slot, words)
+        if key not in self._cr:
+            self._cr[key] = (_empty(self.GNB * 2 * words, torch.int32), _empty(self.GNB, torch.int32))
+        cr, ncols = self._cr[key]
+        sz = C.sizeof(_lib.SpbSplit)
         for j in range(0, nb, self.NB):
             m = min(self.NB, nb - j)
             sub = (_lib.SpbSplit * m).from_buffer(arr, j * sz)
+            call("spb_col_ranks_batch", _p(t.keys), t.num, sub, m, _p(cr[j * 2 * words:]), words, _p(ncols[j:]), _st())
+        return cr, words, ncols
+
+    def _scatter(self, arr, nb, s0, layout, rows_pad, pitch, cr, clear=False):
+        """Scatter (or un-scatter) nb <= GNB splits into the S0 buffer s0 (entry b at byte b * rows_pad * pitch), columns
+        mapped through the ranks cr = (colrank, words), SPB_MAX_BATCH splits per launch."""
+        t = self.table
+        s0_stride, sz = rows_pad * pitch, C.sizeof(_lib.SpbSplit)
+        colrank, words = cr
+        flat = s0.view(-1)
+        for j in range(0, nb, self.NB):
+            m = min(self.NB, nb - j)
+            sub = (_lib.SpbSplit * m).from_buffer(arr, j * sz)
+            crj, s0j = _p(colrank[j * 2 * words:]), _p(flat[j * s0_stride:])
             if clear:
-                call("spb_flatten_u8_clear_batch", _p(t.keys), t.num, sub, m, _p(s0[j:]), s0_stride, rows_pad, pitch, layout, _st())
+                call("spb_flatten_u8_clear_batch_cols", _p(t.keys), t.num, sub, m, crj, words, s0j, s0_stride, rows_pad, pitch, layout,
+                     _st())
             else:
-                call("spb_flatten_u8_batch", _p(t.keys), _p(t.counts), t.num, sub, m, _p(s0[j:]), s0_stride, rows_pad, pitch, layout,
-                     SPB_U8_NO_MEMSET, _p(self.hi_rc[j:]), _p(self.hi_val[j:]), _p(self.hi_num[j:]), self.hi_cap, _st())
+                call("spb_flatten_u8_batch_cols", _p(t.keys), _p(t.counts), t.num, sub, m, crj, words, s0j, s0_stride, rows_pad, pitch,
+                     layout, SPB_U8_NO_MEMSET, _p(self.hi_rc[j:]), _p(self.hi_val[j:]), _p(self.hi_num[j:]), self.hi_cap, _st())
 
     def _gram_batch_i32(self, splits, s0, buf, b0, layout, rows_pad, pitch):
         """As _gram_batch, into the int32 Gram + strip buffers at batch offset b0."""
         nb = len(splits)
         arr = splits if isinstance(splits, C.Array) else (_lib.SpbSplit * nb)(*splits)
+        pitch = self._col_pitch(layout, pitch)
         s0_stride, g_stride = rows_pad * pitch, rows_pad * rows_pad
         cs_rows = int(buf["Cs"].shape[1])
         G, Cs, pos, hr, hm = buf["G"][b0:], buf["Cs"][b0:], buf["pos"][b0:], buf["hr"][b0:], buf["hm"][b0:]
         t = self.timer
         try:
             with _span(t, "scatter", nb):
-                self._scatter(arr, nb, s0, layout, rows_pad, pitch)
-            run = lambda: call("spb_gram_u8_batch_i32", _p(s0), s0_stride, nb, rows_pad, pitch, _p(G), g_stride, _st())  # noqa: E731
+                colrank, words, ncols = self._col_ranks(arr, nb)
+                self._scatter(arr, nb, s0, layout, rows_pad, pitch, (colrank, words))
+            run = lambda: call("spb_gram_u8_batch_i32_cols", _p(s0), s0_stride, nb, rows_pad, pitch, _p(ncols), _p(G), g_stride,  # noqa: E731
+                               _st())
             with _span(t, f"gram_i32_r{rows_pad}", nb):  # int32 tensor-core Gram, one span name per row count (bench.py roofline)
                 run() if self.gram_hook is None else self.gram_hook(run, nb)
             with _span(t, "correction", nb):
                 if self.strip_from_table and nb <= self.NB:
                     tb = self.table  # cross terms by a join of the pattern list with the high list (no column scans of S0)
-                    call("spb_gram_hi_strip_batch_table", _p(tb.keys), _p(tb.counts), tb.num, arr, nb, rows_pad, pitch, _p(self.hi_rc),
-                         _p(self.hi_val), _p(self.hi_num), self.hi_cap, _p(Cs), cs_rows, _p(pos), _p(hr), _p(hm),
+                    call("spb_gram_hi_strip_batch_table_cols", _p(tb.keys), _p(tb.counts), tb.num, arr, nb, rows_pad, pitch, _p(colrank),
+                         words, _p(self.hi_rc), _p(self.hi_val), _p(self.hi_num), self.hi_cap, _p(Cs), cs_rows, _p(pos), _p(hr), _p(hm),
                          _p(self._strip_ws(pitch)), _st())
                 else:
                     call("spb_gram_hi_strip_batch", _p(s0), s0_stride, nb, rows_pad, pitch, layout, _p(self.hi_rc), _p(self.hi_val),
                          _p(self.hi_num), self.hi_cap, _p(Cs), cs_rows, _p(pos), _p(hr), _p(hm), _st())
             with _span(t, "scatter", 0):
-                self._scatter(arr, nb, s0, layout, rows_pad, pitch, clear=True)
+                self._scatter(arr, nb, s0, layout, rows_pad, pitch, (colrank, words), clear=True)
         except BaseException:
             self._drop_s0()  # the cached S0 buffers are assumed all-zero between uses: never keep a dirty one
             raise
@@ -829,23 +859,29 @@ class CountScorer:
             raise
 
     def _gram_batch(self, splits, s0, G, ws, layout, rows_pad, pitch):
-        """nb <= GNB dense splits of equal shape: scatter, ONE Gram launch, ONE correction launch, un-scatter.
-        G: [nb, rows_pad, rows_pad] view."""
+        """nb <= GNB dense splits of equal shape: column ranks + scatter, ONE Gram launch, ONE correction launch, un-scatter.
+        G: [nb, rows_pad, rows_pad] view.  (layout, rows_pad, pitch) is the geometry of the split class; S0 holds the occupied
+        columns only (_col_pitch), so s0 needs nb * rows_pad * _col_pitch(layout, pitch) bytes, and the Gram of every matrix
+        contracts over its own occupied columns.  G is the Gram of the full flattening all the same: the columns left out are
+        zero."""
         nb = len(splits)
         arr = splits if isinstance(splits, C.Array) else (_lib.SpbSplit * nb)(*splits)
+        pitch = self._col_pitch(layout, pitch)
         s0_stride, g_stride = rows_pad * pitch, rows_pad * rows_pad
         t = self.timer
         try:
             with _span(t, "scatter", nb):
-                self._scatter(arr, nb, s0, layout, rows_pad, pitch)
-            run = lambda: call("spb_gram_u8_batch", _p(s0), s0_stride, nb, rows_pad, pitch, layout, _p(G), g_stride, _p(ws), _st())  # noqa: E731
+                colrank, words, ncols = self._col_ranks(arr, nb)
+                self._scatter(arr, nb, s0, layout, rows_pad, pitch, (colrank, words))
+            run = lambda: call("spb_gram_u8_batch_cols", _p(s0), s0_stride, nb, rows_pad, pitch, layout, _p(ncols), _p(G), g_stride,  # noqa: E731
+                               _p(ws), _st())
             with _span(t, "gram", nb):
                 run() if self.gram_hook is None else self.gram_hook(run, nb)
             with _span(t, "correction", nb):
                 call("spb_gram_hi_correction_batch", _p(s0), s0_stride, nb, rows_pad, pitch, layout, _p(self.hi_rc), _p(self.hi_val),
                      _p(self.hi_num), self.hi_cap, _p(G), g_stride, _st())
             with _span(t, "scatter", 0):
-                self._scatter(arr, nb, s0, layout, rows_pad, pitch, clear=True)
+                self._scatter(arr, nb, s0, layout, rows_pad, pitch, (colrank, words), clear=True)
         except BaseException:
             self._drop_s0()
             raise
@@ -976,11 +1012,11 @@ class CountScorer:
         per_matrix = rows_pad * rows_pad * 8 if not i32 else rows_pad * rows_pad * 4 + max(self.n_hi, 1) * rows_pad * 8
         B = int(max(1, min(len(members), max_batch, max_batch_bytes // per_matrix)))
         B = -(-len(members) // -(-len(members) // B))  # equal chunks: no small tail batch through the eigen-solver
-        if i32:
-            s0 = self._buffers(layout, rows_pad, pitch, 1)[0]
+        if i32:  # S0 sized for the occupied columns (_gram_batch); the route was chosen above on the full geometry
+            s0 = self._buffers(layout, rows_pad, self._col_pitch(layout, pitch), 1)[0]
             buf = self._buffers_i32(rows_pad, B)
         else:
-            s0, G, ws = self._buffers(layout, rows_pad, pitch, B)
+            s0, G, ws = self._buffers(layout, rows_pad, self._col_pitch(layout, pitch), B)
         for c0 in range(0, len(members), B):
             chunk = members[c0:c0 + B]
             gnb = self._gnb(rows_pad, pitch)
