@@ -239,8 +239,7 @@ int spb_subflatten(const double* d_T, const double* d_total, int n_taxa, const s
 /* Batched: scores of `num` splits given as bit masks over taxon positions (bit t set = taxon t on
  * side A; side B = d_masks_b[s] if non-NULL else the complement).  d_scores double [num].
  * Up to 21 taxa: one warp per split (Gram, Householder tridiagonalisation, the 4 largest eigenvalues by bisection,
- * score = sqrt((trace - top4) / trace)); above: one CTA per split with a shared-memory Jacobi solver.
- * SPB_SUBFLATTEN_WARP=0 in the environment forces the second kernel. */
+ * score = sqrt((trace - top4) / trace)); above: one CTA per split with a shared-memory Jacobi solver. */
 int spb_subflatten_score(const double* d_T, const double* d_total, int n_taxa, const uint64_t* d_masks_a,
                          const uint64_t* d_masks_b, int64_t num, double* d_scores, void* stream);
 
@@ -351,9 +350,10 @@ int spb_score_gram_large_i32_n(const int32_t* d_Gi, int64_t k, int64_t ld, int64
                                const int32_t* d_pos, const int32_t* d_hr, const int32_t* d_hm, double* d_scores, double* d_info,
                                double* d_ws, int max_cycles, void* stream);
 /* Diagnostic: d_AQ = G0 d_Q for `batch` int32 Gram matrices through ONE of the product kernels of the eigen-solver
- * (variant 0: column-owning FMA kernel; 1..6: fp64 tensor-core (DMMA) kernels), launched exactly as the solver launches
- * them.  d_Q, d_AQ: [batch][8][k] doubles; d_Qt: spb_symv_i32_ws(k, batch) doubles of scratch.  For tests and
- * scripts/symv_bench.py; the product path reaches these kernels through spb_score_gram_large_i32. */
+ * (variant 0: column-owning FMA kernel; 1: fp64 tensor-core (DMMA) kernel, needs k % 256 == 0 and ld % 4 == 0; any other
+ * value is SPB_ERR_ARG), launched exactly as the solver launches it.  d_Q, d_AQ: [batch][8][k] doubles; d_Qt:
+ * spb_symv_i32_ws(k, batch) doubles of scratch.  For tests and scripts/symv_bench.py; the product path reaches these
+ * kernels through spb_score_gram_large_i32. */
 int64_t spb_symv_i32_ws(int64_t k, int64_t batch);
 int spb_symv_i32(const int32_t* d_Gi, int64_t k, int64_t ld, int64_t batch, const double* d_Q, double* d_AQ, double* d_Qt, int variant,
                  void* stream);

@@ -1,5 +1,5 @@
 """One pattern-count launch (12 taxa x 10^8 sites, direct table) bracketed by cudaProfilerStart/Stop, for
-`ncu --profile-from-start off`; prints the CUDA-event time of the same launch.  SPB_COUNT_KERNEL selects the kernel."""
+`ncu --profile-from-start off`; prints the CUDA-event time of the same launch."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -30,5 +30,5 @@ torch.cuda.synchronize()
 torch.cuda.profiler.stop()
 cnt = table.to(torch.int64)
 consts = [int(cnt[c * 0x555555].item()) for c in range(4)]
-print(f"kernel={os.environ.get('SPB_COUNT_KERNEL', 'default')} N={N} ms={a.elapsed_time(b):.4f} distinct={int((cnt > 0).sum())} "
+print(f"N={N} ms={a.elapsed_time(b):.4f} distinct={int((cnt > 0).sum())} "
       f"constant-pattern share={sum(consts) / N:.4f} sum={int(cnt.sum())}")

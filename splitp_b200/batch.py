@@ -27,8 +27,6 @@ ranks takes 1.5 ms).
 """
 from __future__ import annotations
 
-import os
-
 import numpy as np
 import torch
 
@@ -190,7 +188,6 @@ class SplitScorer:
         self.scorer = None
         self.masks = None
         self.timer = None
-        self.refit_enabled = os.environ.get("SPB_PARTITION_REFIT", "1") != "0"
         self.rank_times_us = None
         if method == Method.subflattening:
             ma, mb = engine.masks_from_splits(self.idx_mine)
@@ -250,7 +247,7 @@ class SplitScorer:
         from . import distributed as spd
         t = self.timer
         self._steps += 1
-        refit = self._cls is not None and self._steps in self.refit_steps and self.refit_enabled
+        refit = self._cls is not None and self._steps in self.refit_steps
         if refit:
             ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             ev0.record()

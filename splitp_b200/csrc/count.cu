@@ -17,7 +17,6 @@
 //      in the warp and made the first two versions of this kernel issue-bound (profiles/r1_kernel_roofline_*).
 //   -> global sink: direct-indexed table (n <= 14, one RED per eviction) or open-addressing hash table.
 #include "common.cuh"
-#include <stdlib.h>
 #include <type_traits>
 
 using namespace spb;
@@ -499,19 +498,11 @@ int launch_class(const uint32_t* d_sm, const uint32_t* d_valid, int n, int64_t s
 // direct table, 12 taxa: cache kernel 1.47 ms, stream kernel 1.96 ms -- two thirds of the sites are ~260 single-mutation
 // patterns, and fire-and-forget REDs to so few addresses serialise in the L2 atomic units (3.4e10 RED/s in total);
 // hash table, 20 taxa: stream 3.39 ms, cache 3.59 ms; 31 taxa: 2.55 ms against 2.70 ms.  So: stream for hashed tables,
-// the classified kernel (stream + on-chip single-mutation classes) for direct tables.
-// SPB_COUNT_KERNEL=cache / stream / class in the environment forces one of them (A/B runs).
+// the classified kernel (stream + on-chip single-mutation classes) for direct tables.  The cache kernel is the route when
+// first-site indices are requested or the site stream is not 16-byte aligned.
 enum CountKernel { kCountCache = 0, kCountStream = 1, kCountClass = 2 };
 static CountKernel pick_count_kernel(const void* d_sm, const void* d_first, bool hashed) {
-  static int forced = -1;
-  if (forced < 0) {
-    const char* e = getenv("SPB_COUNT_KERNEL");
-    forced = !e ? 0 : (e[0] == 'c' && e[1] == 'a') ? 1 : (e[0] == 's') ? 2 : (e[0] == 'c' && e[1] == 'l') ? 3 : 0;
-  }
   if (d_first != nullptr || (reinterpret_cast<uintptr_t>(d_sm) & 15) != 0) return kCountCache;
-  if (forced == 1) return kCountCache;
-  if (forced == 2) return kCountStream;
-  if (forced == 3) return hashed ? kCountStream : kCountClass;
   return hashed ? kCountStream : kCountClass;
 }
 

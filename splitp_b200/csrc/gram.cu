@@ -24,7 +24,6 @@
 // Only tiles touching the upper triangle (in 256-wide blocks) are computed; the rest is mirrored.
 #include "common.cuh"
 #include "ptx.cuh"
-#include <stdlib.h>
 
 using namespace spb;
 
@@ -159,7 +158,7 @@ template <int BN>
 __global__ void __launch_bounds__(kUmmaThreads, 1)
 gram_u8_umma_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int T, int KT, int tiles, int ksplit, int kt_per_split,
                     const int32_t* __restrict__ ncols, int num_work, int64_t ldg, double* __restrict__ G_base, int64_t g_stride,
-                    unsigned long long* __restrict__ acc_base, int32_t* __restrict__ Gi_base) {
+                    unsigned long long* __restrict__ acc_base) {
   constexpr int kStageBytes = kTileBytes + BN * kTile;  // A tile + B tile(s)
   constexpr uint32_t kTmemCols = 2 * BN;                 // two accumulator stages (power of two >= 32)
   constexpr uint32_t kIdesc = make_idesc_i8(kTile, BN);
@@ -272,17 +271,6 @@ gram_u8_umma_kernel(const uint8_t* __restrict__ s0_base, int64_t s0_stride, int 
 #pragma unroll
           for (int e = 0; e < 32; ++e)
             if (v[e]) atomicAdd(dst + e, (unsigned long long)v[e]);
-        } else if (Gi_base) {
-          // 32-bit integer output (one K pass stays below 2^31): half the store traffic of the fp64 form
-          int32_t* Gi = Gi_base + (size_t)wk.b * g_stride;
-          int32_t* dst = Gi + (size_t)row * ldg + col0;
-#pragma unroll
-          for (int e = 0; e < 32; e += 4)
-            *reinterpret_cast<int4*>(dst + e) = make_int4((int)v[e], (int)v[e + 1], (int)v[e + 2], (int)v[e + 3]);
-          if ((col0 >> 8) > rb) {
-#pragma unroll
-            for (int e = 0; e < 32; ++e) Gi[(size_t)(col0 + e) * ldg + row] = (int)v[e];
-          }
         } else {
           double* dst = G + (size_t)row * ldg + col0;
 #pragma unroll
@@ -845,7 +833,7 @@ struct UmmaPlan {
   size_t smem;
 };
 
-UmmaPlan plan_umma(int64_t rows_pad, int64_t pitch, int nb, bool single_pass = false) {
+UmmaPlan plan_umma(int64_t rows_pad, int64_t pitch, int nb) {
   UmmaPlan p;
   p.BN = rows_pad >= 256 ? 256 : 128;
   p.T = (int)(rows_pad / kTile);
@@ -857,7 +845,7 @@ UmmaPlan plan_umma(int64_t rows_pad, int64_t pitch, int nb, bool single_pass = f
   int sms = sm_count();
   int total = p.tiles * nb;
   int ks = 1;
-  if (total < sms && !single_pass) ks = (sms + total - 1) / total;
+  if (total < sms) ks = (sms + total - 1) / total;
   if (ks > p.KT) ks = p.KT;
   int per = (p.KT + ks - 1) / ks;
   if (per > 256) per = 256;
@@ -896,16 +884,6 @@ int launch_umma2(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t rows_pa
                                                              d_Gi);
   SPB_LAUNCH_CHECK();
   return SPB_OK;
-}
-
-// SPB_GRAM_KERNEL=1cta in the environment selects the single-CTA kernel everywhere (A/B measurements)
-bool use_pair_kernel() {
-  static int forced = -1;
-  if (forced < 0) {
-    const char* e = getenv("SPB_GRAM_KERNEL");
-    forced = (e && e[0] == '1') ? 1 : 0;
-  }
-  return !forced;
 }
 
 }  // namespace
@@ -963,17 +941,17 @@ extern "C" int spb_gram_u8_batch_cols(const uint8_t* d_s0, int64_t s0_stride, in
     acc = (unsigned long long*)d_ws;
     SPB_CUDA(cudaMemsetAsync(acc, 0, (size_t)nb * rows_pad * rows_pad * 8, st));
   }
-  if (p.BN == 256 && p.ksplit == 1 && p.KT <= 256 && use_pair_kernel())
+  if (p.BN == 256 && p.ksplit == 1 && p.KT <= 256)
     return launch_umma2(d_s0, s0_stride, nb, rows_pad, pitch, d_ncols, d_G, nullptr, g_stride, st);
   int grid = p.num_work < sm_count() ? p.num_work : sm_count();
   if (p.BN == 256) {
     SPB_CUDA(cudaFuncSetAttribute(gram_u8_umma_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
     gram_u8_umma_kernel<256><<<grid, kUmmaThreads, p.smem, st>>>(d_s0, s0_stride, p.T, p.KT, p.tiles, p.ksplit, p.kt_per_split, d_ncols,
-                                                               p.num_work, rows_pad, d_G, g_stride, acc, nullptr);
+                                                               p.num_work, rows_pad, d_G, g_stride, acc);
   } else {
     SPB_CUDA(cudaFuncSetAttribute(gram_u8_umma_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
     gram_u8_umma_kernel<128><<<grid, kUmmaThreads, p.smem, st>>>(d_s0, s0_stride, p.T, p.KT, p.tiles, p.ksplit, p.kt_per_split, d_ncols,
-                                                               p.num_work, rows_pad, d_G, g_stride, acc, nullptr);
+                                                               p.num_work, rows_pad, d_G, g_stride, acc);
   }
   SPB_LAUNCH_CHECK();
   if (acc) {
@@ -1001,15 +979,7 @@ int gram_u8_i32_launch(const uint8_t* d_s0, int64_t s0_stride, int nb, int64_t r
               (long long)pitch, 256 * kTile);
   SPB_REQUIRE(nb == 1 || (s0_stride >= rows_pad * pitch && s0_stride % 16 == 0 && g_stride >= rows_pad * rows_pad),
               "spb_gram_u8_batch_i32: bad batch strides");
-  if (use_pair_kernel()) return launch_umma2(d_s0, s0_stride, nb, rows_pad, pitch, d_ncols, nullptr, d_Gi, g_stride, st);
-  UmmaPlan p = plan_umma(rows_pad, pitch, nb, true);
-  if (p.ksplit != 1) { set_error("spb_gram_u8_batch_i32: internal: K split"); return SPB_ERR_ARG; }
-  int grid = p.num_work < sm_count() ? p.num_work : sm_count();
-  SPB_CUDA(cudaFuncSetAttribute(gram_u8_umma_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
-  gram_u8_umma_kernel<256><<<grid, kUmmaThreads, p.smem, st>>>(d_s0, s0_stride, p.T, p.KT, p.tiles, 1, p.kt_per_split, d_ncols, p.num_work,
-                                                             rows_pad, nullptr, g_stride, nullptr, d_Gi);
-  SPB_LAUNCH_CHECK();
-  return SPB_OK;
+  return launch_umma2(d_s0, s0_stride, nb, rows_pad, pitch, d_ncols, nullptr, d_Gi, g_stride, st);
 }
 }  // namespace spb
 

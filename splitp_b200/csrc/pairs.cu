@@ -5,7 +5,6 @@
 // constructions.py:143-161.  So the alignment is read ONCE (pair_kernel: bit-plane AND + POPC), the
 // Hadamard-type basis change is n^2 batched 4x4x4 products (finalize / transform kernels) and each
 // split is a gather + a small Gram + Jacobi in shared memory (subflatten_score_kernel).
-#include <stdlib.h>
 #include "common.cuh"
 #include "jacobi.cuh"
 
@@ -788,13 +787,6 @@ inline size_t subflat_smem(int n, int* m_elems) {
   return ((size_t)*m_elems + (size_t)jacobi_dim(kmax) * jacobi_ld(kmax)) * sizeof(double);
 }
 
-// The warp-per-split scorer is the default up to 21 taxa; SPB_SUBFLATTEN_WARP=0 in the environment selects the
-// block-wide Jacobi kernel instead (A/B: scripts/ab_subflatten_warp.py).
-inline bool subflatten_warp_enabled() {
-  const char* e = getenv("SPB_SUBFLATTEN_WARP");
-  return !(e && e[0] == '0');
-}
-
 }  // namespace
 
 extern "C" int64_t spb_pair_raw_words(int n_taxa) { return (int64_t)n_taxa * n_taxa * 9 + (int64_t)n_taxa * 3 + 1; }
@@ -934,7 +926,7 @@ extern "C" int spb_subflatten_score(const double* d_T, const double* d_total, in
   SPB_REQUIRE(d_T && d_total && n_taxa >= 2 && n_taxa <= SPB_MAX_TAXA, "spb_subflatten_score: bad arguments");
   if (num <= 0) return SPB_OK;
   SPB_REQUIRE(d_masks_a && d_scores, "spb_subflatten_score: NULL buffer");
-  if (n_taxa <= kWarpMaxTaxa && subflatten_warp_enabled()) {
+  if (n_taxa <= kWarpMaxTaxa) {
     const size_t wsmem = (size_t)kWarpsPerCta * sizeof(WarpScratch);
     SPB_CUDA(cudaFuncSetAttribute(subflatten_score_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
     int wocc = 1;

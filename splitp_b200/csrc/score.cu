@@ -10,8 +10,6 @@
 #include "common.cuh"
 #include "jacobi.cuh"
 #include "sparse.cuh"
-#include <cstdlib>
-#include <cstring>
 #include <vector>
 
 using namespace spb;
@@ -272,8 +270,7 @@ static int choose_ksplit(int M, int N, int K, int batch) {
 // C (ldc, strideC) = A B^T for the tall-skinny Krylov operands; part must hold batch * ceil(k/128) * M * N doubles
 static int dot_product(const double* A, int64_t strideA, const double* B, int64_t strideB, int M, int N, int k, int batch,
                        double* C, int64_t ldc, int64_t strideC, double* part, cudaStream_t st) {
-  static const bool dmma_dots = [] { const char* e = getenv("SPB_DOT_KERNEL"); return !(e && !strcmp(e, "simt")); }();
-  if (dmma_dots && (M == 8 || M == 16) && (N == 8 || N == 16) && k % 128 == 0 && strideA % 2 == 0 && strideB % 2 == 0 &&
+  if ((M == 8 || M == 16) && (N == 8 || N == 16) && k % 128 == 0 && strideA % 2 == 0 && strideB % 2 == 0 &&
       reinterpret_cast<uintptr_t>(A) % 16 == 0 && reinterpret_cast<uintptr_t>(B) % 16 == 0) {
     if (M == 8 && N == 8) dot_dmma_kernel<1, 1><<<batch, 256, 0, st>>>(A, strideA, B, strideB, k, C, ldc, strideC);
     else if (M == 16 && N == 8) dot_dmma_kernel<2, 1><<<batch, 256, 0, st>>>(A, strideA, B, strideB, k, C, ldc, strideC);
@@ -668,7 +665,11 @@ __global__ void __launch_bounds__(32 * kColsWarps, kColsCtasPerSm) symv_cols_i32
 // So lane l ends up with vector v = l / 4 of the 8 adjacent columns c0 + 8 (l % 4) + {j, 4 + j}.  Against the column-owning
 // kernel above: 1 + 1 loads, 4 conversions and 4 MMAs per 128 matrix elements instead of 54 instructions, no shared memory in
 // the main loop, and half the registers -- twice the warps and four times the bytes in flight per SM.
-// CW = 32-column groups per warp (the A fragment is shared by them), U = row quads in flight per lane.
+// A CTA owns 32 kDmmaCW columns; every lane keeps kDmmaU row quads in flight, with an explicit register double buffer: the
+// loads of the NEXT batch are issued before the MMAs of this one (without it ptxas schedules for minimum registers: two loads in
+// flight per lane).  Measured per 4096^2 product inside a 48-matrix launch (scripts/symv_bench.py, B200): 11.4 us = 5.9 TB/s,
+// 0.90 of the HBM peak, against 17.3 us for the column-owning kernel, 12.3 us without the double buffer and 11.7-12.4 us with
+// 64 columns per CTA (those variants were deleted after measurement).
 // ---------------------------------------------------------------------------------------------------
 __device__ __forceinline__ int4 ldg_stream_v4(const int32_t* p) {
   int4 v;
@@ -676,70 +677,13 @@ __device__ __forceinline__ int4 ldg_stream_v4(const int32_t* p) {
   return v;
 }
 constexpr int kDmmaWarps = 8;
-template <int CW, int U>
-__global__ void __launch_bounds__(32 * kDmmaWarps) symv_dmma_i32_kernel(const int32_t* __restrict__ G, int64_t ld, int64_t strideG,
-                                                                       const double* __restrict__ Qt, int64_t strideQt,
-                                                                       double* __restrict__ AQ, int64_t strideQ, int k, int rows_per_warp) {
-  __shared__ double red[kDmmaWarps][kKB][32 * CW];
-  const int bt = blockIdx.y;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int kq = lane & 3, grp = lane >> 2;
-  const int col0 = blockIdx.x * 32 * CW;
-  const int32_t* Gl = G + (int64_t)bt * strideG + col0 + 4 * grp;
-  const double* Ql = Qt + (int64_t)bt * strideQt + grp;
-  double acc[CW][4][2];
-#pragma unroll
-  for (int w = 0; w < CW; ++w)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[w][j][0] = acc[w][j][1] = 0.0;
-  const int row_begin = warp * rows_per_warp;
-  const int row_end = min(k, row_begin + rows_per_warp);   // k and rows_per_warp are multiples of 4 U (checked by the launcher)
-#pragma unroll 1
-  for (int r = row_begin + kq; r < row_end; r += 4 * U) {
-    int4 g[U][CW];
-    double a[U];
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      const int32_t* p = Gl + (int64_t)(r + 4 * u) * ld;
-#pragma unroll
-      for (int w = 0; w < CW; ++w) g[u][w] = ldg_stream_v4(p + 32 * w);
-      a[u] = __ldg(Ql + (int64_t)(r + 4 * u) * kKB);
-    }
-#pragma unroll
-    for (int u = 0; u < U; ++u)
-#pragma unroll
-      for (int w = 0; w < CW; ++w) {
-        dmma884(acc[w][0][0], acc[w][0][1], a[u], u31_to_double(g[u][w].x));
-        dmma884(acc[w][1][0], acc[w][1][1], a[u], u31_to_double(g[u][w].y));
-        dmma884(acc[w][2][0], acc[w][2][1], a[u], u31_to_double(g[u][w].z));
-        dmma884(acc[w][3][0], acc[w][3][1], a[u], u31_to_double(g[u][w].w));
-      }
-  }
-#pragma unroll
-  for (int w = 0; w < CW; ++w)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      red[warp][grp][32 * w + 8 * kq + j] = acc[w][j][0];
-      red[warp][grp][32 * w + 8 * kq + 4 + j] = acc[w][j][1];
-    }
-  __syncthreads();
-  double* out = AQ + (int64_t)bt * strideQ;
-  for (int idx = threadIdx.x; idx < kKB * 32 * CW; idx += 32 * kDmmaWarps) {  // warps added in warp order: deterministic
-    const int c = idx / (32 * CW), jj = idx - c * (32 * CW);
-    double v = 0.0;
-#pragma unroll
-    for (int w = 0; w < kDmmaWarps; ++w) v += red[w][c][jj];
-    out[(int64_t)c * k + col0 + jj] = v;
-  }
-}
-
-// The same kernel with an explicit register double buffer: the loads of the NEXT batch of U row quads are issued before the
-// MMAs of this one (ptxas schedules the plain form above for minimum registers: two loads in flight per lane, 48 registers).
-template <int CW, int U>
+constexpr int kDmmaCW = 1;  // 32-column groups per warp (the A fragment is shared by them)
+constexpr int kDmmaU = 4;   // row quads in flight per lane
 __global__ void __launch_bounds__(32 * kDmmaWarps) symv_dmma_pipe_i32_kernel(const int32_t* __restrict__ G, int64_t ld, int64_t strideG,
                                                                             const double* __restrict__ Qt, int64_t strideQt,
                                                                             double* __restrict__ AQ, int64_t strideQ, int k,
                                                                             int rows_per_warp) {
+  constexpr int CW = kDmmaCW, U = kDmmaU;
   __shared__ double red[kDmmaWarps][kKB][32 * CW];
   const int bt = blockIdx.y;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -803,43 +747,14 @@ __global__ void __launch_bounds__(32 * kDmmaWarps) symv_dmma_pipe_i32_kernel(con
   }
 }
 
-// which G0 Q kernel: 0 = column-owning FMA kernel, 1..3 = DMMA kernel <CW, U> = <1, 8>, <2, 4>, <1, 4>,
-// 4..6 = pipelined DMMA kernel <1, 4>, <2, 2>, <2, 4>
-static int symv_variant() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("SPB_SYMV_KERNEL");
-    v = e ? atoi(e) : 4;  // measured per 4096^2 product inside a 48-matrix launch (scripts/symv_bench.py, B200): variant 0: 17.3 us,
-                          // 1: 15.6, 2: 14.0, 3: 12.3, 4: 11.4 (5.9 TB/s = 0.90 of the HBM peak), 5: 12.4, 6: 11.7
-    if (v < 0 || v > 6) v = 4;
-  }
-  return v;
-}
 inline bool symv_dmma_ok(int k, int64_t ld, const void* G) {
   return k % (kDmmaWarps * 32) == 0 && ld % 4 == 0 && reinterpret_cast<uintptr_t>(G) % 16 == 0;
 }
-static void launch_symv_dmma(int variant, const int32_t* G, int64_t ld, int64_t strideG, const double* Qt, int64_t strideQt, double* AQ,
+static void launch_symv_dmma(const int32_t* G, int64_t ld, int64_t strideG, const double* Qt, int64_t strideQt, double* AQ,
                              int64_t strideQ, int k, int batch, cudaStream_t st) {
-  const int rpw = k / kDmmaWarps;  // a multiple of 32 = 4 U for every U <= 8
-  if (variant == 4) {
-    dim3 grid(k / 32, batch);
-    symv_dmma_pipe_i32_kernel<1, 4><<<grid, 32 * kDmmaWarps, 0, st>>>(G, ld, strideG, Qt, strideQt, AQ, strideQ, k, rpw);
-  } else if (variant == 5) {
-    dim3 grid(k / 64, batch);
-    symv_dmma_pipe_i32_kernel<2, 2><<<grid, 32 * kDmmaWarps, 0, st>>>(G, ld, strideG, Qt, strideQt, AQ, strideQ, k, rpw);
-  } else if (variant == 6) {
-    dim3 grid(k / 64, batch);
-    symv_dmma_pipe_i32_kernel<2, 4><<<grid, 32 * kDmmaWarps, 0, st>>>(G, ld, strideG, Qt, strideQt, AQ, strideQ, k, rpw);
-  } else if (variant == 2) {
-    dim3 grid(k / 64, batch);
-    symv_dmma_i32_kernel<2, 4><<<grid, 32 * kDmmaWarps, 0, st>>>(G, ld, strideG, Qt, strideQt, AQ, strideQ, k, rpw);
-  } else if (variant == 3) {
-    dim3 grid(k / 32, batch);
-    symv_dmma_i32_kernel<1, 4><<<grid, 32 * kDmmaWarps, 0, st>>>(G, ld, strideG, Qt, strideQt, AQ, strideQ, k, rpw);
-  } else {
-    dim3 grid(k / 32, batch);
-    symv_dmma_i32_kernel<1, 8><<<grid, 32 * kDmmaWarps, 0, st>>>(G, ld, strideG, Qt, strideQt, AQ, strideQ, k, rpw);
-  }
+  const int rpw = k / kDmmaWarps;  // a multiple of 32 = 8 kDmmaU
+  dim3 grid(k / (32 * kDmmaCW), batch);
+  symv_dmma_pipe_i32_kernel<<<grid, 32 * kDmmaWarps, 0, st>>>(G, ld, strideG, Qt, strideQt, AQ, strideQ, k, rpw);
 }
 
 // AQ += C Q for the strip form of the correction (GramView).  Two deterministic passes, no atomics:
@@ -1266,8 +1181,7 @@ extern "C" int spb_score_gram_small(const double* d_G, int64_t k, int64_t ld, in
               "spb_score_gram_small: need 1 <= k <= %d (got %lld)", kJacobiMaxK, (long long)k);
   if (batch == 0) return SPB_OK;
   // Score only (no eigenvalue list), 4 < k <= 64: warp-per-matrix Householder + 9-section (pairs.cu) instead of the Jacobi sweep
-  static const bool jacobi_only = [] { const char* e = getenv("SPB_SMALL_EIG"); return e && !strcmp(e, "jacobi"); }();
-  if (!d_eig && k > 4 && k <= 64 && !jacobi_only) return score_gram_warp_launch(d_G, (int)k, ld, batch, d_scores, (cudaStream_t)stream);
+  if (!d_eig && k > 4 && k <= 64) return score_gram_warp_launch(d_G, (int)k, ld, batch, d_scores, (cudaStream_t)stream);
   size_t smem = (size_t)jacobi_dim((int)k) * jacobi_ld((int)k) * sizeof(double);
   SPB_CUDA(cudaFuncSetAttribute(score_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int threads = k <= 32 ? 128 : 256;
@@ -1365,14 +1279,14 @@ static int krylov_cycle(const GramView& gv, int k, int batch, int nb, bool first
         krylov_transpose_kernel<<<tg, 256, 0, st>>>(Qj, w.sQ, w.Qt, (int64_t)k_pad * kKB, k, k_pad);
         SPB_LAUNCH_CHECK();
         dim3 gi((k + kColsPerCta - 1) / kColsPerCta, batch);
-        if (symv_variant() > 0 && symv_dmma_ok(k, ld, gv.Gi))
-          launch_symv_dmma(symv_variant(), gv.Gi, ld, ld * ld, w.Qt, (int64_t)k_pad * kKB, AQj, w.sQ, k, batch, st);
+        if (symv_dmma_ok(k, ld, gv.Gi))
+          launch_symv_dmma(gv.Gi, ld, ld * ld, w.Qt, (int64_t)k_pad * kKB, AQj, w.sQ, k, batch, st);
         else if (cols_vec) symv_cols_i32_kernel<true><<<gi, 32 * kColsWarps, cols_smem, st>>>(gv.Gi, ld, ld * ld, w.Qt, (int64_t)k_pad * kKB, AQj, w.sQ, k, rpw);
         else symv_cols_i32_kernel<false><<<gi, 32 * kColsWarps, cols_smem, st>>>(gv.Gi, ld, ld * ld, w.Qt, (int64_t)k_pad * kKB, AQj, w.sQ, k, rpw);
       }
       SPB_LAUNCH_CHECK();
       if (!gv.Gf && gv.cs_rows) {
-        if (symv_variant() > 0 && k % 128 == 0 && ld % 2 == 0 && reinterpret_cast<uintptr_t>(gv.Cs) % 16 == 0 &&
+        if (k % 128 == 0 && ld % 2 == 0 && reinterpret_cast<uintptr_t>(gv.Cs) % 16 == 0 &&
             reinterpret_cast<uintptr_t>(Qj) % 16 == 0 && w.sQ % 2 == 0) {
           dim3 rg((unsigned)((gv.cs_rows + kStripDmmaRows - 1) / kStripDmmaRows), batch);
           strip_rows_dmma_kernel<<<rg, 256, 0, st>>>(gv, Qj, w.sQ, AQj, k);
@@ -1497,15 +1411,16 @@ extern "C" int spb_score_gram_large_i32(const int32_t* d_Gi, int64_t k, int64_t 
   return score_gram_large(gv, k, batch, d_scores, d_info, d_ws, stream);
 }
 
-// Diagnostic entry: AQ = G0 Q for a batch of int32 Gram matrices through one chosen kernel (0 = column-owning FMA kernel,
-// 1..3 = DMMA kernels), exactly as krylov_cycle launches them.  d_Q, d_AQ: [batch][8][k]; d_Qt: spb_symv_i32_ws(k, batch)
-// doubles of scratch.  Used by tests/test_gpu_parity_r2.py and scripts/symv_bench.py, not by the product path.
+// Diagnostic entry: AQ = G0 Q for a batch of int32 Gram matrices through one chosen kernel, launched exactly as krylov_cycle
+// launches it: variant 0 = column-owning FMA kernel, 1 = DMMA kernel (needs k % 256 == 0, ld % 4 == 0).  d_Q, d_AQ:
+// [batch][8][k]; d_Qt: spb_symv_i32_ws(k, batch) doubles of scratch.  Used by tests/test_gpu_parity_r2.py and
+// scripts/symv_bench.py, not by the product path.
 extern "C" int64_t spb_symv_i32_ws(int64_t k, int64_t batch) { return (int64_t)symv_k_pad((int)k) * kKB * batch; }
 
 extern "C" int spb_symv_i32(const int32_t* d_Gi, int64_t k64, int64_t ld, int64_t batch64, const double* d_Q, double* d_AQ, double* d_Qt,
                             int variant, void* stream) {
-  SPB_REQUIRE(d_Gi && d_Q && d_AQ && d_Qt && k64 > 0 && k64 <= (1 << 20) && ld >= k64 && batch64 > 0 && batch64 <= 65535,
-              "spb_symv_i32: bad arguments");
+  SPB_REQUIRE(d_Gi && d_Q && d_AQ && d_Qt && k64 > 0 && k64 <= (1 << 20) && ld >= k64 && batch64 > 0 && batch64 <= 65535 &&
+              (variant == 0 || variant == 1), "spb_symv_i32: bad arguments");
   cudaStream_t st = (cudaStream_t)stream;
   const int k = (int)k64, batch = (int)batch64;
   const int rpw = symv_rows_per_warp(k), k_pad = symv_k_pad(k);
@@ -1513,9 +1428,9 @@ extern "C" int spb_symv_i32(const int32_t* d_Gi, int64_t k64, int64_t ld, int64_
   dim3 tg((k_pad + 255) / 256, batch);
   krylov_transpose_kernel<<<tg, 256, 0, st>>>(d_Q, sQ, d_Qt, (int64_t)k_pad * kKB, k, k_pad);
   SPB_LAUNCH_CHECK();
-  if (variant > 0) {
-    SPB_REQUIRE(variant <= 6 && symv_dmma_ok(k, ld, d_Gi), "spb_symv_i32: the DMMA kernels need k % 256 == 0, ld % 4 == 0");
-    launch_symv_dmma(variant, d_Gi, ld, ld * ld, d_Qt, (int64_t)k_pad * kKB, d_AQ, sQ, k, batch, st);
+  if (variant == 1) {
+    SPB_REQUIRE(symv_dmma_ok(k, ld, d_Gi), "spb_symv_i32: the DMMA kernel needs k % 256 == 0, ld % 4 == 0");
+    launch_symv_dmma(d_Gi, ld, ld * ld, d_Qt, (int64_t)k_pad * kKB, d_AQ, sQ, k, batch, st);
   } else {
     const size_t cols_smem = (size_t)kColsWarps * 2 * kColsQRows * kKB * sizeof(double);
     SPB_CUDA(cudaFuncSetAttribute(symv_cols_i32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cols_smem));

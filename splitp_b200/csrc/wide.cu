@@ -554,15 +554,10 @@ extern "C" int spb_thin_gram_wide_filtered(const uint64_t* d_hkeys, const uint32
 
 extern "C" int64_t spb_thin_filter_words(int64_t cap) {
   int64_t w = 1;
-  // bits per bitmap: 8 x cap by default (false-positive rate of the column filter ~ patterns / bits: 1 in 16 at a half-full
-  // table; 2 x cap bits, the round-1 size, let one pattern in six through to its 4^a - 1 random table reads)
-  static int per_cap = 0;
-  if (!per_cap) {
-    const char* e = getenv("SPB_THIN_FILTER_BITS_PER_SLOT");
-    per_cap = e ? atoi(e) : 8;
-    if (per_cap < 1 || per_cap > 64) per_cap = 8;
-  }
-  while (w * 32 < cap * per_cap) w *= 2;
+  // bits per bitmap: 8 x cap (false-positive rate of the column filter ~ patterns / bits: 1 in 16 at a half-full table;
+  // 2 x cap bits, the round-1 size, let one pattern in six through to its 4^a - 1 random table reads)
+  constexpr int kBitsPerSlot = 8;
+  while (w * 32 < cap * kBitsPerSlot) w *= 2;
   return w;
 }
 

@@ -16,8 +16,6 @@ from __future__ import annotations
 
 import contextlib
 import ctypes as C
-import os
-import threading
 import warnings
 
 import numpy as np
@@ -624,13 +622,7 @@ class CountScorer:
             raise ValueError("CountScorer needs a PatternTable with integer counts")
         self._table = None
         self.hi_cap = int(hi_cap) if hi_cap is not None else 0
-        # Size classes can be scored on up to NSTREAMS CUDA streams at once (one host thread per stream; buffers that a class
-        # writes per launch exist once per stream slot).  Measured on B200 (12 taxa, 10^6 sites): 67.0 ms with two streams
-        # against 66.5 ms with one, at N = 1 and N = 2 alike -- the big kernels already fill the SMs -- so the default is 1.
-        self.nstreams = max(1, int(os.environ.get("SPB_SCORE_STREAMS", "1")))
-        self._tl = threading.local()
-        self._hi = {}
-        self._side = None
+        self.hi_rc = None
         self.table = table
         self._s0 = {}
         self._G = {}
@@ -638,9 +630,8 @@ class CountScorer:
         self._ws = {}
         self._batch_bytes = None
         self._hi_ws = {}
-        self._cr = {}          # (stream slot, words) -> column-rank buffers of one Gram batch, see _col_ranks
+        self._cr = {}          # words -> column-rank buffers of one Gram batch, see _col_ranks
         self._plans = {}       # (id(split list), taxa, class) -> encoded splits + output positions, see _encoded_group
-        self.strip_from_table = os.environ.get("SPB_STRIP_KERNEL", "table") != "scan"  # A/B switch: column scans of S0 (round 1)
         self.int32_gram = True  # large dense splits keep G as int32 + correction strip (half the eigen-stage traffic)
         self.gram_hook = None  # optional wrapper (fn, nb) around the Gram launch
         self.timer = None      # optional PhaseTimer: scatter / gram / correction / eigen spans (bench.py phase_ms)
@@ -655,26 +646,11 @@ class CountScorer:
         high-part buffers are sized once per table: no per-split overflow tracking is needed."""
         self._table = table
         self.n_hi = int((table.counts.to(torch.int64) & 0xFFFFFFFF).ge(256).sum().item()) if table.num else 0
-        if not self._hi or self.n_hi > self.hi_cap:
+        if self.hi_rc is None or self.n_hi > self.hi_cap:
             self.hi_cap = max(self.hi_cap, 1024, 2 * self.n_hi)
-            self._hi = {slot: (_empty((self.GNB, self.hi_cap, 2), torch.int32), _empty((self.GNB, self.hi_cap), torch.int32),
-                               _zeros(self.GNB, torch.int32)) for slot in range(self.nstreams)}
-
-    @property
-    def _slot(self):
-        return getattr(self._tl, "slot", 0)
-
-    @property
-    def hi_rc(self):
-        return self._hi[self._slot][0]
-
-    @property
-    def hi_val(self):
-        return self._hi[self._slot][1]
-
-    @property
-    def hi_num(self):
-        return self._hi[self._slot][2]
+            self.hi_rc = _empty((self.GNB, self.hi_cap, 2), torch.int32)
+            self.hi_val = _empty((self.GNB, self.hi_cap), torch.int32)
+            self.hi_num = _zeros(self.GNB, torch.int32)
 
     @staticmethod
     def geometry(rows, cols):
@@ -700,7 +676,7 @@ class CountScorer:
             self._ws[key] = _empty(self._gnb(rows_pad, pitch) * rows_pad * rows_pad, torch.int64) if n else None
         return self._s0[key], g, self._ws[key]
 
-    I32_MIN_ROWS = int(os.environ.get("SPB_I32_MIN_ROWS", "1024"))  # 1024: the 5|7 class of 12 taxa as well (round 1: 2048)
+    I32_MIN_ROWS = 1024  # 1024: the 5|7 class of 12 taxa as well (round 1: 2048)
     I32_MAX_HI = 4096  # strip rows: the correction strip costs n_hi * rows_pad * 8 bytes per matrix and O(n_hi^2) work
 
     def _use_i32(self, layout, rows_pad, pitch):
@@ -724,8 +700,8 @@ class CountScorer:
         return b
 
     def _strip_ws(self, pitch):
-        """int32 scratch of spb_gram_hi_strip_batch_table for this thread's stream slot."""
-        key = (getattr(self._tl, "slot", 0), int(pitch))
+        """int32 scratch of spb_gram_hi_strip_batch_table."""
+        key = int(pitch)
         ws = self._hi_ws.get(key)
         need = int(_lib.lib.spb_gram_hi_strip_table_ws(self.GNB, int(pitch), self.hi_cap))
         if ws is None or ws.numel() < need:
@@ -738,14 +714,13 @@ class CountScorer:
         return min(int(pitch), 1 << max(7, (max(int(self.table.num), 1) - 1).bit_length()))
 
     def _col_ranks(self, arr, nb):
-        """Column ranks of nb <= GNB splits of equal shape (spb_col_ranks_batch) into this stream slot's buffers:
+        """Column ranks of nb <= GNB splits of equal shape (spb_col_ranks_batch) into the scorer's buffers:
         (colrank, words, ncols); ncols [nb] = occupied columns of every split, the K of its Gram."""
         t = self.table
         words = int(lib.spb_col_rank_words(int(arr[0].b)))
-        key = (self._slot, words)
-        if key not in self._cr:
-            self._cr[key] = (_empty(self.GNB * 2 * words, torch.int32), _empty(self.GNB, torch.int32))
-        cr, ncols = self._cr[key]
+        if words not in self._cr:
+            self._cr[words] = (_empty(self.GNB * 2 * words, torch.int32), _empty(self.GNB, torch.int32))
+        cr, ncols = self._cr[words]
         sz = C.sizeof(_lib.SpbSplit)
         for j in range(0, nb, self.NB):
             m = min(self.NB, nb - j)
@@ -789,14 +764,10 @@ class CountScorer:
             with _span(t, f"gram_i32_r{rows_pad}", nb):  # int32 tensor-core Gram, one span name per row count (bench.py roofline)
                 run() if self.gram_hook is None else self.gram_hook(run, nb)
             with _span(t, "correction", nb):
-                if self.strip_from_table and nb <= self.NB:
-                    tb = self.table  # cross terms by a join of the pattern list with the high list (no column scans of S0)
-                    call("spb_gram_hi_strip_batch_table_cols", _p(tb.keys), _p(tb.counts), tb.num, arr, nb, rows_pad, pitch, _p(colrank),
-                         words, _p(self.hi_rc), _p(self.hi_val), _p(self.hi_num), self.hi_cap, _p(Cs), cs_rows, _p(pos), _p(hr), _p(hm),
-                         _p(self._strip_ws(pitch)), _st())
-                else:
-                    call("spb_gram_hi_strip_batch", _p(s0), s0_stride, nb, rows_pad, pitch, layout, _p(self.hi_rc), _p(self.hi_val),
-                         _p(self.hi_num), self.hi_cap, _p(Cs), cs_rows, _p(pos), _p(hr), _p(hm), _st())
+                tb = self.table  # cross terms by a join of the pattern list with the high list (no column scans of S0)
+                call("spb_gram_hi_strip_batch_table_cols", _p(tb.keys), _p(tb.counts), tb.num, arr, nb, rows_pad, pitch, _p(colrank),
+                     words, _p(self.hi_rc), _p(self.hi_val), _p(self.hi_num), self.hi_cap, _p(Cs), cs_rows, _p(pos), _p(hr), _p(hm),
+                     _p(self._strip_ws(pitch)), _st())
             with _span(t, "scatter", 0):
                 self._scatter(arr, nb, s0, layout, rows_pad, pitch, (colrank, words), clear=True)
         except BaseException:
@@ -929,43 +900,8 @@ class CountScorer:
                 groups.setdefault(min(len(ia), len(ib)), []).append(s)
             tasks = sorted(groups.items(), key=lambda g: -(4.0 ** (2 * g[0])) * 4.0 ** (n - g[0]) * len(g[1]))  # Gram work, descending
             self._plans[gkey] = (splits_idx, len(splits_idx), tasks)
-        if self.nstreams == 1 or len(tasks) == 1:
-            for a, members in tasks:
-                self._score_group(splits_idx, a, members, out, max_batch, max_batch_bytes)
-            return out
-        # two host threads, two streams: greedy split of the classes by Gram work (largest class alone on the caller's stream)
-        load, mine, theirs = [0.0, 0.0], [], []
         for a, members in tasks:
-            cost = (4.0 ** (2 * a)) * 4.0 ** (n - a) * len(members)
-            slot = 0 if load[0] <= load[1] else 1
-            load[slot] += cost
-            (mine if slot == 0 else theirs).append((a, members))
-        main = torch.cuda.current_stream()
-        if self._side is None:
-            self._side = torch.cuda.Stream(device=out.device)
-        side, dev_index, failure = self._side, out.device.index, []
-        side.wait_stream(main)  # the table and `out` were produced on the caller's stream
-
-        def worker():
-            try:
-                torch.cuda.set_device(dev_index)
-                self._tl.slot = 1
-                with torch.cuda.stream(side):
-                    for a, members in theirs:
-                        self._score_group(splits_idx, a, members, out, max_batch, max_batch_bytes)
-            except BaseException as exc:  # noqa: BLE001  (re-raised on the calling thread)
-                failure.append(exc)
-
-        th = threading.Thread(target=worker, name="splitp_b200-score-stream-1")
-        th.start()
-        try:
-            for a, members in mine:
-                self._score_group(splits_idx, a, members, out, max_batch, max_batch_bytes)
-        finally:
-            th.join()
-            main.wait_stream(side)
-        if failure:
-            raise failure[0]
+            self._score_group(splits_idx, a, members, out, max_batch, max_batch_bytes)
         return out
 
     def _encoded_group(self, splits_idx, a, members):
@@ -1330,13 +1266,13 @@ def subflatten_scores(pt, masks_a, masks_b=None):
         return torch.from_numpy(np.ascontiguousarray(m).view(np.int64)).to(device())
     ma, mb = up(masks_a), up(masks_b)
     out = _empty(int(ma.shape[0]), torch.float64)
-    if pt.n <= SUBFLATTEN_TABLES_MAX_TAXA and os.environ.get("SPB_SUBFLATTEN_KERNEL", "tables") == "tables":
+    if pt.n <= SUBFLATTEN_TABLES_MAX_TAXA:
         ready = pt.triples is not None
         if not ready:
             pt.triples = _empty(int(lib.spb_subflatten_tables_doubles(pt.n)), torch.float64)
         call("spb_subflatten_score_tables", _p(pt.T), _p(pt.total), pt.n, _p(ma), _p(mb), int(ma.shape[0]), _p(out), _p(pt.triples),
              int(ready), _st())
-    else:  # sides above 21 taxa (or SPB_SUBFLATTEN_KERNEL=staged for A/B runs): the kernels that stage the subflattening
+    else:  # sides above 21 taxa: the kernels that stage the subflattening
         call("spb_subflatten_score", _p(pt.T), _p(pt.total), pt.n, _p(ma), _p(mb), int(ma.shape[0]), _p(out), _st())
     return out
 

@@ -3,19 +3,15 @@ own occupied columns (spb_col_ranks_batch, spb_flatten_u8_batch_cols, spb_gram_u
 spb_gram_hi_strip_batch_table_cols).
 
   * the per-matrix-K Gram entry points against the full-K ones and an exact product, for every kernel: dp4a, umma<128>,
-    umma<256> with a K split, the CTA-pair kernel (fp64 and int32), and umma<256> without a K split in a process that
-    selects the single-CTA kernel;
-  * CountScorer batches of every class of 12 taxa (fp64 Gram and int32 Gram + strip, both strip modes) against the full-K
-    single-split Gram and a sparse numpy F F^T;
+    umma<256> with a K split and the CTA-pair kernel (fp64 and int32);
+  * CountScorer batches of every class of 12 taxa (fp64 Gram and int32 Gram + strip) against the full-K single-split Gram
+    and a sparse numpy F F^T;
   * edge tables: one occupied column, every column occupied, 128k and 128k + 1 occupied columns, high counts in sparse
     columns, more high counts than the int32 route takes;
   * score_many over all 2,035 splits of 12 taxa bit for bit against the same scorer building full-K Gram matrices.
 All integer work is compared bit for bit.
 """
 import ctypes as C
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -24,8 +20,6 @@ torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
 from tests.test_gpu_parity import _count_table  # noqa: E402
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope="module")
@@ -128,18 +122,6 @@ def test_gram_cols_matches_full_k(eng, case):
     direct_checks(eng, layout, rows, pitch, ncols, 100 + case, i32)
 
 
-def test_gram_cols_single_cta_kernel(eng):
-    """umma<256> without a K split: taken by the batches above when the single-CTA kernel is selected (SPB_GRAM_KERNEL=1cta is
-    read once per process, so these cases run in a child process)."""
-    code = ("import tests.test_gpu_gram_compaction as t, splitp_b200.engine as e\n"
-            "for c in (3, 4, 5): name, rows, pitch, ncols, i32 = t.DIRECT_CASES[c]; "
-            "t.direct_checks(e, e.SPB_S0_TILED, rows, pitch, ncols, 200 + c, i32)\n"
-            "print('ok')\n")
-    env = dict(os.environ, SPB_GRAM_KERNEL="1cta")
-    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and r.stdout.strip().endswith("ok"), r.stdout + r.stderr
-
-
 # ---------------------------------------------------------------------------------------------
 # the scorer's batches against full-K Gram matrices
 # ---------------------------------------------------------------------------------------------
@@ -203,7 +185,7 @@ def _numpy_gram(tab, ia, ib):
     return (F @ F.T).toarray()
 
 
-def _batch_grams(scorer, idx, mode=True):
+def _batch_grams(scorer, idx):
     """Gram matrices [nb, R, R] (fp64) of splits of one class through the scorer's batched route (int32 Gram + strip expanded)."""
     a = min(len(idx[0][0]), len(idx[0][1]))
     n = scorer.table.n
@@ -213,7 +195,6 @@ def _batch_grams(scorer, idx, mode=True):
     nb = len(plans)
     s0_pitch = scorer._col_pitch(layout, pitch)
     if scorer._use_i32(layout, rows_pad, pitch):
-        scorer.strip_from_table = mode
         s0 = scorer._buffers(layout, rows_pad, s0_pitch, 1)[0]
         buf = scorer._buffers_i32(rows_pad, nb)
         scorer._gram_batch_i32(plans, s0, buf, 0, layout, rows_pad, pitch)
@@ -250,9 +231,6 @@ def test_scorer_batches_every_class(sp, eng, c2_small, a):
         G, k = scorer.gram(ia, ib)  # single split: raw columns, full K
         assert np.array_equal(got[b], G[:k, :k].cpu().numpy()), b
     assert np.array_equal(got[0], _numpy_gram(tab, *idx[0]))
-    if i32:
-        other, _ = _batch_grams(scorer, idx, mode=False)  # correction strip by column scans of S0
-        assert np.array_equal(other, got)
 
 
 def _table(eng, n, keys, counts):
@@ -322,14 +300,11 @@ def test_edge_tables(eng, case):
     if n_hi > scorer.I32_MAX_HI:
         assert not scorer._use_i32(*scorer.geometry(4 ** a, 4 ** (n - a)))
     want = _numpy_gram(tab, ia, ib)
-    got, i32 = _batch_grams(scorer, [(ia, ib)] * 3)  # the same split three times in one batch
+    got, _ = _batch_grams(scorer, [(ia, ib)] * 3)  # the same split three times in one batch
     for b in range(3):
         assert np.array_equal(got[b], want), b
     G, k = scorer.gram(ia, ib)
     assert np.array_equal(G[:k, :k].cpu().numpy(), want)
-    if i32:
-        other, _ = _batch_grams(scorer, [(ia, ib)] * 3, mode=False)
-        assert np.array_equal(other, got)
 
 
 def test_score_many_all_splits_equals_full_k(sp, eng, c2_small):

@@ -20,6 +20,7 @@ import pytest
 torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
+from tests.test_gpu_gram_compaction import _full_k_scorer  # noqa: E402
 from tests.test_gpu_parity import _count_table, _tiled_from_rowmajor, assert_score, score_tol  # noqa: E402
 
 
@@ -303,9 +304,10 @@ def test_erickson_pick_order_matches_reference_trace(sp):
 
 
 @pytest.mark.parametrize("n,seed", [(20, 7), (22, 8), (44, 9)])
-def test_subflatten_score_staged_kernels_still_agree(sp, eng, oracle, monkeypatch, n, seed):
+def test_subflatten_score_staged_kernels_still_agree(sp, eng, oracle, n, seed):
     """The kernels that stage the subflattening (round 1: warp-per-split up to 21 taxa, block-wide Jacobi above) remain the
-    route for more than 43 taxa; SPB_SUBFLATTEN_KERNEL=staged forces them below that.  Both routes against the oracle."""
+    route for more than 43 taxa; below that they are called through their C entry point spb_subflatten_score.  Both routes
+    against the oracle."""
     N = 120_000
     tree = sp.trees.balanced_tree(n, 0.05)
     codes = sp.simulation.simulate_codes(tree, sp.simulation.GTR.JukesCantor(0.5), N, seed=seed)
@@ -318,9 +320,11 @@ def test_subflatten_score_staged_kernels_still_agree(sp, eng, oracle, monkeypatc
             side = sorted(rng.choice(n, size=a, replace=False).tolist())
             picks.append((side, [t for t in range(n) if t not in side]))
     ma, mb = eng.masks_from_splits(picks)
-    monkeypatch.setenv("SPB_SUBFLATTEN_KERNEL", "staged")
-    staged = eng.subflatten_scores(pt, ma, mb).cpu().numpy()
-    monkeypatch.delenv("SPB_SUBFLATTEN_KERNEL")
+    dev = torch.device("cuda")
+    da, db = (torch.from_numpy(m.view(np.int64)).to(dev) for m in (ma, mb))
+    staged = torch.empty(len(picks), dtype=torch.float64, device=dev)
+    eng.call("spb_subflatten_score", eng._p(pt.T), eng._p(pt.total), pt.n, eng._p(da), eng._p(db), len(picks), eng._p(staged), eng._st())
+    staged = staged.cpu().numpy()
     default = eng.subflatten_scores(pt, ma, mb).cpu().numpy()
     assert (pt.triples is not None) == (n <= eng.SUBFLATTEN_TABLES_MAX_TAXA)
     for s, (ia, ib) in enumerate(picks):
@@ -330,13 +334,13 @@ def test_subflatten_score_staged_kernels_still_agree(sp, eng, oracle, monkeypatc
 
 
 # ---------------------------------------------------------------------------------------------
-# G0 Q product kernels of the eigen-solver (column-owning FMA kernel and the fp64 tensor-core kernels)
+# G0 Q product kernels of the eigen-solver (column-owning FMA kernel and the fp64 tensor-core kernel)
 # ---------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("k,nb", [(256, 3), (1024, 5), (4096, 2)])
-@pytest.mark.parametrize("variant", [0, 1, 2, 3, 4, 5, 6])
+@pytest.mark.parametrize("variant", [0, 1])
 def test_symv_i32_kernels_against_fp64_matmul(eng, k, nb, variant):
-    """AQ[c][j] = sum_i G0[i][j] Q[c][i] with G0 entries up to 2^31 - 1: every variant within 64 eps of the fp64 product
-    (the kernels differ only in summation order); integer-valued Q gives a bit-exact answer."""
+    """AQ[c][j] = sum_i G0[i][j] Q[c][i] with G0 entries up to 2^31 - 1: the column-owning kernel (0) and the DMMA kernel (1)
+    within 64 eps of the fp64 product (the kernels differ only in summation order); integer-valued Q gives a bit-exact answer."""
     import ctypes as C
     dev = torch.device("cuda:0")
     g = torch.Generator(device=dev).manual_seed(100 + k + variant)
@@ -366,16 +370,15 @@ def test_symv_i32_kernels_against_fp64_matmul(eng, k, nb, variant):
 # ---------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("a", [5, 6])
 def test_correction_strip_from_table_equals_column_scan(sp, eng, a):
-    """spb_gram_hi_strip_batch_table against spb_gram_hi_strip_batch on the same scattered splits (12 taxa, 10^6 sites):
-    pos, hr, hm and the strip rows in use agree bit for bit (integer-valued fp64 sums)."""
+    """The scorer's strip (spb_gram_hi_strip_batch_table_cols on ranked columns) against spb_gram_hi_strip_batch (column
+    scans of S0, as the full-K reference scorer builds it) on the same splits (12 taxa, 10^6 sites): pos, hr, hm, G and the
+    strip rows in use agree bit for bit (integer-valued fp64 sums)."""
     n, N = 12, 1_000_000
     tree, codes, tab = _count_table(sp, eng, n, N, 2)
     splits = [s for s in sp.all_splits(tree) if len(s[0]) == a][::37][:9]
     idx = [eng.split_positions(s, tree.taxa) for s in splits]
     got = {}
-    for mode in (True, False):
-        scorer = eng.CountScorer(tab)
-        scorer.strip_from_table = mode
+    for route, scorer in (("table", eng.CountScorer(tab)), ("scan", _full_k_scorer(eng, tab))):
         R, Ccols = 4 ** a, 4 ** (n - a)
         layout, rows_pad, pitch = scorer.geometry(R, Ccols)
         assert scorer._use_i32(layout, rows_pad, pitch)
@@ -384,14 +387,14 @@ def test_correction_strip_from_table_equals_column_scan(sp, eng, a):
         buf["Cs"].fill_(float("nan"))  # rows >= hm are never written by the table form and never read
         scorer._gram_batch_i32([scorer._plan(ia, ib, False)[0] for ia, ib in idx], s0, buf, 0, layout, rows_pad, pitch)
         torch.cuda.synchronize()
-        got[mode] = {k: v[: len(idx)].clone() for k, v in buf.items()}
+        got[route] = {k: v[: len(idx)].clone() for k, v in buf.items()}
     for key in ("pos", "hm", "G"):
-        assert torch.equal(got[True][key], got[False][key]), key
+        assert torch.equal(got["table"][key], got["scan"][key]), key
     for b in range(len(idx)):
-        m = int(got[True]["hm"][b].item())
+        m = int(got["table"]["hm"][b].item())
         assert m > 0
-        assert torch.equal(got[True]["hr"][b, :m], got[False]["hr"][b, :m])
-        assert torch.equal(got[True]["Cs"][b, :m], got[False]["Cs"][b, :m])
+        assert torch.equal(got["table"]["hr"][b, :m], got["scan"]["hr"][b, :m])
+        assert torch.equal(got["table"]["Cs"][b, :m], got["scan"]["Cs"][b, :m])
 
 
 # ---------------------------------------------------------------------------------------------

@@ -50,6 +50,21 @@ def test_no_cpu_fallback_in_product():
                 assert "import oracle" not in src and "from oracle" not in src, f
 
 
+def test_product_reads_no_tuning_variable():
+    """The input alone chooses every kernel and route: the CUDA sources read no environment variable, and the Python package
+    reads no SPB_* variable (NVCC, RANK, WORLD_SIZE and LOCAL_RANK are not tuning switches)."""
+    csrc = os.path.join(ROOT, "splitp_b200", "csrc")
+    for f in sorted(os.listdir(csrc)):
+        if f.endswith((".cu", ".cuh")):
+            assert "getenv(" not in open(os.path.join(csrc, f)).read(), f
+    spb_read = re.compile(r"""(?:environ\s*(?:\.get\s*\(|\[)|getenv\s*\()\s*[rbf]?["']SPB_""")
+    for dirpath, _, files in os.walk(os.path.join(ROOT, "splitp_b200")):
+        for f in files:
+            if f.endswith(".py"):
+                src = open(os.path.join(dirpath, f)).read()
+                assert not spb_read.search(src), (f, spb_read.search(src))
+
+
 def test_all_splits_matches_golden(golden_small):
     from splitp_b200.splits import all_splits
 
