@@ -414,6 +414,26 @@ int spb_mi_table(const uint64_t* d_keys, const void* d_vals, int val_kind, doubl
                  const double* d_colsum, const uint64_t* d_ckeys, int64_t ccap, double* d_partials, double* d_out,
                  void* stream);
 
+/* ---- batched rank-1 divergence of many covering splits of one pattern list (mi_batch.cu; replaces the per-split loop
+ * over phylogenetics.py:136-140 / 364-373 that spb_table_marginals + spb_mi_table serve one split at a time) ----
+ * Keys: key_words = 1 (uint64 keys, <= 31 taxa) or 2 (128-bit keys {lo, hi}, 16-byte aligned, 32..64 taxa).  A split is
+ * given by the digit masks of its two sides inside the key: the side key of a pattern is key AND mask.  Both sides must be
+ * non-empty (a masked key then never is all ones, the EMPTY marker).  Every side owns an open-addressing table of cap
+ * slots (a power of two >= 2 x its distinct side keys: spb_mi_side_cap) starting at slot `slot` of the workspace.
+ * d_ws: spb_mi_scores_ws(num, key_words, slots, n_splits) uint64 words, slots = the slots of all tables of the call.
+ * d_out[s] = sum over non-zero patterns of v log(v / (r c)), r / c = the side sums of v; counts (SPB_VAL_U32) are summed
+ * as exact uint64 integers and, with divisor > 0, divided by it as spb_mi_table does.  Each score is summed in an order
+ * fixed by num alone: for count tables it is bitwise the same whichever other splits share the call. */
+typedef struct {
+  uint64_t mask[2][2]; /* digit mask {lo, hi} of side 0 and side 1 (hi = 0 for one-word keys) */
+  int64_t slot[2];     /* first slot of each side's table */
+  int64_t cap[2];      /* slots of each side's table */
+} spb_mi_split;
+int64_t spb_mi_side_cap(int64_t num, int side_len);
+int64_t spb_mi_scores_ws(int64_t num, int key_words, int64_t slots, int64_t n_splits);
+int spb_mi_scores(const uint64_t* d_keys, int key_words, const void* d_vals, int val_kind, double divisor, int64_t num,
+                  const spb_mi_split* d_splits, int64_t n_splits, int64_t slots, uint64_t* d_ws, double* d_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -158,6 +158,9 @@ PROTOTYPES = {
     "spb_flatten_coo_banned": (_i, [_p, _l, _sp, _i, _i, _p, _p, _p, _p]),
     "spb_table_marginals": (_i, [_p, _p, _i, _l, _sp, _i, _i, _p, _p, _l, _p, _p, _l, _p, _p]),
     "spb_mi_table": (_i, [_p, _p, _i, _d, _l, _sp, _p, _p, _l, _p, _p, _l, _p, _p, _p]),
+    "spb_mi_side_cap": (_l, [_l, _i]),
+    "spb_mi_scores_ws": (_l, [_l, _i, _l, _l]),
+    "spb_mi_scores": (_i, [_p, _i, _p, _i, _d, _l, _p, _l, _l, _p, _p, _p]),
 }
 
 for _name, (_res, _args) in PROTOTYPES.items():

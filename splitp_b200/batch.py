@@ -14,9 +14,12 @@ and the inner loop of `erickson_SVD` (phylogenetics.py:126-140).  `score_splits`
                           sparse flattening (dropping all-zero rows and columns does not change the singular values)
                           (up to 16 taxa; 17..64 taxa: pattern count -> engine.sparse_flattening_scores, csrc/sparse.cu)
     Method.subflattening  pack -> pair tables -> H N H^T -> per split: gather + Gram + eigenvalues (kernel 3)
+    Method.mutual_information  pattern count (uint64 keys up to 31 taxa; 32..64 taxa: pack_wide + count_patterns_wide) ->
+                          engine.rank1_divergence_scores (csrc/mi_batch.cu): the rank-1 divergence of every split's flattening
+                          of the pattern probabilities (count / usable sites), batches of splits per launch
 
 Under `torch.distributed` (one process per GPU) the splits are dealt to the ranks for scoring (flattening scores: contiguous
-runs of the size-class-ordered list cut at equal modelled cost; subflattening scores: round-robin) and every rank receives
+runs of the size-class-ordered list cut at equal modelled cost; subflattening and divergence scores: round-robin) and every rank receives
 the scores of all splits.  The counting stage has two forms: `sites="shard"` -- every rank passes ITS contiguous site
 shard (distributed.shard_range) and the pattern tables are merged -- or `sites="replicated"` -- every rank passes the
 WHOLE alignment and counts it itself, with no exchange at all.  The second form wins while counting the whole alignment
@@ -193,8 +196,8 @@ class SplitScorer:
             ma, mb = engine.masks_from_splits(self.idx_mine)
             dev = engine.device()
             self.masks = (torch.from_numpy(ma.view(np.int64)).to(dev), torch.from_numpy(mb.view(np.int64)).to(dev))
-        elif method != Method.flattening:
-            raise NotImplementedError("score_splits: Method.flattening or Method.subflattening")
+        elif method not in (Method.flattening, Method.mutual_information):
+            raise NotImplementedError("score_splits: Method.flattening, Method.subflattening or Method.mutual_information")
 
     REFIT_DAMPING = 0.5
 
@@ -257,20 +260,16 @@ class SplitScorer:
             with _span(t, "sparse"):
                 out = engine.sparse_flattening_scores(table, self.idx_mine)
         elif self.method == Method.flattening:
-            with _span(t, "h2d+pack"):
-                aln = _as_alignment(alignment, want_sm=True, want_planes=False)
-            with _span(t, "count"):
-                if aln.n <= engine.DIRECT_MAX_TAXA:
-                    table = engine.count_patterns(aln, gather_fn=self._timed_gather if self.gather_fn else None)
-                elif self.count_world > 1:  # hashed tables: gather + hash merge on every rank
-                    table = spd.count_patterns_sharded(aln, self.rank, self.world, self.group, local=True)
-                else:
-                    table = engine.count_patterns(aln)
+            table = self._count(alignment)
             if self.scorer is None:
                 self.scorer = engine.CountScorer(table)
             self.scorer.table = table
             self.scorer.timer = t
             out = self.scorer.score_many(self.idx_mine, big_hook=gram_hook)
+        elif self.method == Method.mutual_information:
+            table = self._count(alignment) if _num_taxa(alignment) <= engine.NARROW_MAX_TAXA else self._count_wide(alignment)
+            with _span(t, "mi"):
+                out = engine.rank1_divergence_scores(table, self.idx_mine)
         else:
             with _span(t, "h2d+pack"):
                 aln = _as_alignment(alignment, want_sm=False, want_planes=True)
@@ -296,6 +295,33 @@ class SplitScorer:
             self._refit(ev0.elapsed_time(ev1) * 1e3)
         return res
 
+    def _count(self, alignment):
+        """Pattern table (uint64 keys, up to 31 taxa) of the whole alignment from this rank's part of it."""
+        from . import distributed as spd
+        t = self.timer
+        with _span(t, "h2d+pack"):
+            aln = _as_alignment(alignment, want_sm=True, want_planes=False)
+        with _span(t, "count"):
+            if aln.n <= engine.DIRECT_MAX_TAXA:
+                return engine.count_patterns(aln, gather_fn=self._timed_gather if self.gather_fn else None)
+            if self.count_world > 1:  # hashed tables: gather + hash merge on every rank
+                return spd.count_patterns_sharded(aln, self.rank, self.world, self.group, local=True)
+            return engine.count_patterns(aln)
+
+    def _count_wide(self, alignment):
+        """engine.WideTable (128-bit keys, 32..64 taxa; divisor = usable sites) of the whole alignment from this rank's part."""
+        from . import distributed as spd
+        if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
+            raise NotImplementedError(f"scores of {alignment.n} taxa need the alignment as characters (dict, array or tensor): "
+                                      "the packed forms hold at most 32 taxa per site word")
+        with _span(self.timer, "h2d+pack"):
+            chars, is_ascii, taxa = _chars(alignment)
+            wide, valid, n, N = engine.pack_wide(chars, is_ascii)
+        with _span(self.timer, "count"):
+            if self.count_world > 1:
+                return spd.count_patterns_wide_sharded(wide, valid, n, N, self.rank, self.world, self.group, local=True)
+            return engine.count_patterns_wide(wide, valid, n, N, taxa=taxa)
+
     def _timed_gather(self, keys, counts):
         with _span(self.timer, "exchange"):
             return self.gather_fn(keys, counts)
@@ -310,8 +336,11 @@ def score_splits(alignment, splits, method=Method.flattening, taxa=None):
     alignment  {taxon: sequence} dict, uint8 [n_taxa, n_sites] matrix of ASCII bytes or codes 0..3 (host or device),
                `HostPlanes`, or `engine.DeviceAlignment`
     splits     pairs (left, right) of taxon labels (with `taxa`, or the dict's key order) or of taxon positions
-    method     Method.flattening (scores of the flattening, constructions.py:7-102 + phylogenetics.py:280-300) or
-               Method.subflattening (constructions.py:108-198)
+    method     Method.flattening (scores of the flattening, constructions.py:7-102 + phylogenetics.py:280-300),
+               Method.subflattening (constructions.py:108-198) or Method.mutual_information (rank-1 divergence of the
+               flattening of the pattern probabilities, count / usable sites, phylogenetics.py:136-140 + 364-373: what
+               erickson_SVD(..., method=Method.mutual_information) scores per candidate; 2..64 taxa, every split must place
+               every taxon on exactly one side, a split with an empty side scores 0.0)
     """
     if taxa is None and isinstance(alignment, dict):
         taxa = list(alignment.keys())

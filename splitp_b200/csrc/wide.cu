@@ -18,42 +18,11 @@
 //                        column indices (sides of <= 31 taxa) and the keys of a sub-alignment
 //   spb_pair_tables_wide joint 4x4 tables of every taxon pair of a weighted pattern list ({pattern: value} mappings),
 //                        N = E^T diag(v) E on the fp64 tensor cores; deterministic, exact for integer values
-#include "common.cuh"
+#include "key128.cuh"
 
 using namespace spb;
 
 namespace {
-
-constexpr unsigned long long kAll = 0xFFFFFFFFFFFFFFFFull;
-
-struct Key128 {
-  unsigned long long lo, hi;
-};
-
-__device__ __forceinline__ bool is_empty(Key128 k) { return k.lo == kAll && k.hi == kAll; }
-__device__ __forceinline__ bool same(Key128 a, Key128 b) { return a.lo == b.lo && a.hi == b.hi; }
-
-// plain 16-byte read: only used by kernels that run after all insertions have completed
-__device__ __forceinline__ Key128 load_key(const unsigned long long* keys, uint64_t slot) {
-  const ulonglong2 v = *reinterpret_cast<const ulonglong2*>(keys + 2 * slot);
-  return Key128{v.x, v.y};
-}
-
-__device__ __forceinline__ Key128 cas128(unsigned long long* ptr, Key128 cmp, Key128 val) {
-  Key128 old;
-  asm volatile(
-      "{\n\t.reg .b128 c, v, o;\n\t"
-      "mov.b128 c, {%2, %3};\n\t"
-      "mov.b128 v, {%4, %5};\n\t"
-      "atom.global.cas.b128 o, [%6], c, v;\n\t"
-      "mov.b128 {%0, %1}, o;\n\t}"
-      : "=l"(old.lo), "=l"(old.hi)
-      : "l"(cmp.lo), "l"(cmp.hi), "l"(val.lo), "l"(val.hi), "l"(ptr)
-      : "memory");
-  return old;
-}
-
-__device__ __forceinline__ uint64_t hash128(Key128 k) { return mix64(k.lo ^ mix64(k.hi + 0x9E3779B97F4A7C15ull)); }
 
 struct WideTable {
   unsigned long long* keys;  // [cap][2] = {lo, hi}, EMPTY = all ones

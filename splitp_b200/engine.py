@@ -1381,6 +1381,79 @@ def rank1_divergence_table(table, idx_a, idx_b):
     return out
 
 
+MI_BATCH_BYTES = 4 << 30  # device workspace of one batched divergence call (side tables + per-chunk partials)
+MI_MAX_SPLITS = 65535 * 8  # splits per spb_mi_scores call
+
+
+def side_mask(n, idx):
+    """Digit mask of the taxon positions idx inside the key of an n-taxon pattern, as (lo, hi) uint64 words: uint64 keys
+    and 128-bit keys {lo, hi} both hold the digit of taxon t at bits 2 (n - 1 - t) of one base-4 number."""
+    m = 0
+    for t in idx:
+        m |= 3 << (2 * (n - 1 - t))
+    return m & 0xFFFFFFFFFFFFFFFF, m >> 64
+
+
+def mi_batches(split_slots, num, key_words, cap=None):
+    """Cuts splits needing split_slots[i] table slots into consecutive batches whose spb_mi_scores workspace stays within
+    `cap` bytes (default MI_BATCH_BYTES; a batch holds at least one split).  Returns [begin, end) ranges."""
+    cap = MI_BATCH_BYTES if cap is None else cap
+    out, b, slots = [], 0, 0
+    for i, s in enumerate(split_slots):
+        if i > b and (i - b >= MI_MAX_SPLITS or 8 * int(lib.spb_mi_scores_ws(num, key_words, slots + s, i - b + 1)) > cap):
+            out.append((b, i))
+            b, slots = i, 0
+        slots += s
+    if b < len(split_slots):
+        out.append((b, len(split_slots)))
+    return out
+
+
+def rank1_divergence_scores(table, splits_idx, timer=None):
+    """Rank-1 divergences (phylogenetics.py:364-373) of many splits [(idx_a, idx_b), ...] of one table, batched on the device
+    (csrc/mi_batch.cu): the values rank1_divergence_table gives one split at a time, up to the summation order.  `table`: a
+    PatternTable (counts with their divisor, or values), a WidePatternTable, or the WideTable of count_patterns_wide (counts
+    divided by its usable sites).  Every split must place every taxon on exactly one side (ValueError otherwise); a split
+    with an empty side scores 0.0.  Returns a float64 device tensor, one score per split."""
+    if isinstance(table, WideTable):
+        keys, vals = table.compact()  # sorted: the pattern order, and with it every summation order, is the table's own
+        kind, div = SPB_VAL_U32, table.divisor
+    else:
+        keys = table.keys.contiguous()
+        vals, kind, div = (table.counts, SPB_VAL_U32, table.divisor) if table.counts is not None else (table.values, SPB_VAL_F64, 0.0)
+    vals, n = vals.contiguous(), table.n
+    for ia, ib in splits_idx:
+        if not covers_all(n, ia, ib):
+            raise ValueError("rank-1 divergence scores need a split that places every taxon on exactly one side")
+    out = _zeros(len(splits_idx), torch.float64)
+    live = [i for i, (ia, ib) in enumerate(splits_idx) if len(ia) and len(ib)]
+    num = int(keys.shape[0])
+    if num == 0 or not live:
+        return out
+    W = 2 if keys.dim() == 2 else 1
+    caps = [(int(lib.spb_mi_side_cap(num, len(splits_idx[i][0]))), int(lib.spb_mi_side_cap(num, len(splits_idx[i][1])))) for i in live]
+    batches = mi_batches([ca + cb for ca, cb in caps], num, W)
+    desc = np.zeros((len(live), 8), dtype=np.uint64)  # spb_mi_split: mask[2][2], slot[2], cap[2]
+    for b0, b1 in batches:
+        slot = 0
+        for j in range(b0, b1):
+            ia, ib = splits_idx[live[j]]
+            desc[j, 0:2], desc[j, 2:4] = side_mask(n, ia), side_mask(n, ib)
+            desc[j, 4], desc[j, 5] = slot, slot + caps[j][0]
+            desc[j, 6:8] = caps[j]
+            slot += caps[j][0] + caps[j][1]
+    with _span(timer, "mi", len(live)):
+        desc_d = torch.from_numpy(desc.view(np.int64)).to(device())
+        ws = _empty(max(int(lib.spb_mi_scores_ws(num, W, sum(a + b for a, b in caps[b0:b1]), b1 - b0)) for b0, b1 in batches), torch.int64)
+        res = _empty(len(live), torch.float64)
+        for b0, b1 in batches:
+            slots = sum(a + b for a, b in caps[b0:b1])
+            call("spb_mi_scores", _p(keys), W, _p(vals), kind, float(div), num, _p(desc_d[b0:b1]), b1 - b0, slots, _p(ws), _p(res[b0:b1]),
+                 _st())
+        out.index_copy_(0, torch.tensor(live, dtype=torch.int64, device=out.device), res)
+    return out
+
+
 def marginals_dense(F):
     """(row sums, column sums) of a device matrix."""
     F = F.contiguous()
