@@ -434,6 +434,25 @@ int64_t spb_mi_scores_ws(int64_t num, int key_words, int64_t slots, int64_t n_sp
 int spb_mi_scores(const uint64_t* d_keys, int key_words, const void* d_vals, int val_kind, double divisor, int64_t num,
                   const spb_mi_split* d_splits, int64_t n_splits, int64_t slots, uint64_t* d_ws, double* d_out, void* stream);
 
+/* ---- nonparametric bootstrap of a pattern table (bootstrap.cu) ----
+ * Replicate b draws N sites with replacement, i.e. N patterns with probability count / N.  Draw s of replicate b:
+ *   u = fmix(seed + 0x9E3779B97F4A7C15 (b 2^40 + s + 1))  (SplitMix64 finaliser, all mod 2^64)
+ *   j = high word of the 128-bit product u N;  pattern p with d_prefix[p] <= j < d_prefix[p + 1]
+ * d_prefix: uint32 [P], exclusive cumulative counts in table order (d_prefix[0] = 0), 16-byte aligned; N = the total count
+ * (1 .. 2^32 - 1).  d_counts: uint32 [reps][P], row r = the counts of replicate rep_first + r (overwritten).  Replicate
+ * indices stay below 2^24.  The counts depend on (prefix, N, seed, replicate index) only: any split of the replicates into
+ * calls gives the same rows. */
+int spb_bootstrap_counts(const uint32_t* d_prefix, int64_t P, int64_t N, uint64_t seed, int64_t rep_first, int64_t reps,
+                         uint32_t* d_counts, void* stream);
+/* Per replicate (row of d_counts), the patterns with a non-zero count in table order: keys (key_words uint64 each, as
+ * d_keys [P][key_words]) to d_out_keys, counts to d_out_counts, replicate r at [d_offsets[r], d_offsets[r + 1]) (int64
+ * [reps + 1]).  cap: entries of the outputs (reps x min(P, N) always suffices; entries past it are dropped).  reps <= 65535.
+ * d_ws: spb_bootstrap_compact_ws(P, reps) int64 words. */
+int64_t spb_bootstrap_compact_ws(int64_t P, int64_t reps);
+int spb_bootstrap_compact(const uint32_t* d_counts, const uint64_t* d_keys, int key_words, int64_t P, int64_t reps,
+                          uint64_t* d_out_keys, uint32_t* d_out_counts, int64_t cap, int64_t* d_offsets, int64_t* d_ws,
+                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -349,3 +349,51 @@ def score_splits(alignment, splits, method=Method.flattening, taxa=None):
     if dist.is_available() and dist.is_initialized():
         rank, world = dist.get_rank(), dist.get_world_size()
     return SplitScorer(splits, taxa, method, rank or 0, world or 1)(alignment)
+
+
+def bootstrap_scores(alignment, splits, method=Method.flattening, replicates=100, seed=0, taxa=None):
+    """Nonparametric bootstrap of split scores: numpy float64 [replicates, len(splits)], row b = the scores `score_splits`
+    gives for bootstrap replicate b of the alignment.
+
+    A replicate draws N sites with replacement from the N usable sites; as sites with the same pattern are exchangeable it
+    is drawn on the device as N patterns of the pattern table, each with probability count / N (engine.bootstrap_tables,
+    csrc/bootstrap.cu).  Row b depends on the alignment, `seed` and b only: two calls with the same arguments return equal
+    arrays.  `alignment`, `splits`, `method` and `taxa` have the meaning they have in `score_splits` (2..64 taxa).
+
+    The alignment is counted once; every replicate's table then goes through the scorer `score_splits` uses:
+      Method.flattening     up to 16 taxa: one engine.CountScorer for all replicates; above: engine.sparse_flattening_scores
+      Method.subflattening  pair tables of the replicate's counts (engine.pair_tables_from_table) + engine.subflatten_scores
+      Method.mutual_information  engine.rank1_divergence_scores (counts / N)
+    The scores stay on the device until the last replicate is scored."""
+    if isinstance(replicates, bool) or not isinstance(replicates, (int, np.integer)) or replicates < 1:
+        raise ValueError(f"bootstrap_scores: replicates must be an integer >= 1 (got {replicates!r})")
+    if replicates > engine.BOOTSTRAP_MAX_REPLICATES:
+        raise ValueError(f"bootstrap_scores: at most {engine.BOOTSTRAP_MAX_REPLICATES} replicates")
+    seed = engine.bootstrap_seed(seed)
+    import torch.distributed as dist
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        raise NotImplementedError("bootstrap_scores runs on one GPU: call it outside a torch.distributed group of several processes")
+    if taxa is None and isinstance(alignment, dict):
+        taxa = list(alignment.keys())
+    # one process: the SplitScorer holds the split positions, the subflattening masks and the counting stage of score_splits
+    ss = SplitScorer(splits, taxa, method)
+    idx, n = ss.idx_all, _num_taxa(alignment)
+    table = ss._count(alignment) if n <= engine.NARROW_MAX_TAXA else ss._count_wide(alignment)
+    out = engine._empty((int(replicates), len(idx)), torch.float64)
+    scorer = None
+    for b, tb in enumerate(engine.bootstrap_tables(table, replicates, seed)):
+        if not idx:
+            continue
+        if method == Method.flattening and uses_sparse_flattening(n):
+            out[b] = engine.sparse_flattening_scores(tb, idx)
+        elif method == Method.flattening:
+            if scorer is None:
+                scorer = engine.CountScorer(tb)
+            else:
+                scorer.table = tb
+            out[b] = scorer.score_many(idx)
+        elif method == Method.subflattening:
+            out[b] = engine.subflatten_scores(engine.pair_tables_from_table(tb, as_counts=True), *ss.masks)
+        else:
+            out[b] = engine.rank1_divergence_scores(tb, idx)
+    return out.cpu().numpy()

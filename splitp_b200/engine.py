@@ -1646,3 +1646,100 @@ def thin_split_scores(table, thin_sides, filtered=True):
         Gs = G[idx][:, :R * R].reshape(len(members), R, R).contiguous()
         out.index_copy_(0, idx, score_gram(Gs, R))
     return out
+
+
+# --------------------------------------------------------------------------------------------
+# nonparametric bootstrap of a pattern table (csrc/bootstrap.cu)
+# --------------------------------------------------------------------------------------------
+BOOTSTRAP_BATCH_BYTES = 2 << 30  # device memory of the replicates generated in one pass (count rows + compacted tables)
+BOOTSTRAP_MAX_REPLICATES = 1 << 24  # replicate indices b stay below 2^24, so the draw counters b 2^40 + s never collide
+
+
+def bootstrap_seed(seed):
+    """The seed as a Python int in [0, 2^64) (ValueError otherwise)."""
+    if isinstance(seed, bool) or not isinstance(seed, (int, np.integer)) or not 0 <= int(seed) < 1 << 64:
+        raise ValueError(f"bootstrap seed must be an integer in [0, 2^64) (got {seed!r})")
+    return int(seed)
+
+
+def _counted(table):
+    """(keys, counts) of a table of pattern counts in its sorted key order: a PatternTable from count_patterns or the
+    WideTable of count_patterns_wide (compacted, sorted)."""
+    if isinstance(table, WideTable):
+        keys, counts = table.compact()
+    elif isinstance(table, PatternTable) and table.counts is not None:
+        keys, counts = table.keys, table.counts
+    else:
+        raise ValueError("bootstrap replicates need a table of pattern counts (count_patterns or count_patterns_wide)")
+    return keys.contiguous(), counts.contiguous()
+
+
+def _bootstrap_prefix(counts):
+    """(exclusive cumulative counts as uint32 bits in an int32 tensor, total count N)."""
+    c = counts.to(torch.int64) & 0xFFFFFFFF
+    N = int(c.sum().item()) if c.shape[0] else 0
+    if N == 0:
+        raise ValueError("bootstrap replicates need an alignment with at least one usable site")
+    if N >= 1 << 32:
+        raise ValueError(f"bootstrap replicates need fewer than 2^32 usable sites (got {N})")
+    pre = torch.cumsum(c, 0) - c
+    return torch.where(pre >= 1 << 31, pre - (1 << 32), pre).to(torch.int32), N
+
+
+def _check_replicates(first, count):
+    if first < 0 or count < 0 or first + count > BOOTSTRAP_MAX_REPLICATES:
+        raise ValueError(f"bootstrap replicates [{first}, {first + count}) outside [0, 2^24)")
+
+
+def bootstrap_counts(table, first, count, seed):
+    """Counts of bootstrap replicates first .. first + count - 1 of a table of pattern counts (see _counted): int32 tensor
+    [count, P] holding uint32 counts, column p = pattern p of the table's sorted key order.  Every row sums to N, the usable
+    sites of the table.  Row r depends on the table, `seed` and the replicate index first + r only (csrc/bootstrap.cu)."""
+    seed = bootstrap_seed(seed)
+    first, count = int(first), int(count)
+    _check_replicates(first, count)
+    _, counts = _counted(table)
+    prefix, N = _bootstrap_prefix(counts)
+    out = _empty((count, int(counts.shape[0])), torch.int32)
+    call("spb_bootstrap_counts", _p(prefix), int(counts.shape[0]), N, seed, first, count, _p(out), _st())
+    return out
+
+
+def bootstrap_tables(table, replicates, seed):
+    """Yields the pattern table of bootstrap replicates 0 .. replicates - 1 of a table of pattern counts (see _counted), in
+    order: the patterns with a non-zero count in the table's sorted key order, so each is the table count_patterns /
+    count_patterns_wide gives for the alignment that repeats every pattern as often as the replicate drew it.
+      up to 31 taxa: PatternTable with uint32 counts and divisor N (the parent's usable sites);
+      32..64 taxa:   WidePatternTable with values count / N (one correctly rounded division per pattern) that also carries the
+                     uint32 counts and divisor N, so the scorers that take counts (exact integer sums) read those.
+    Replicates are generated in passes of at most BOOTSTRAP_BATCH_BYTES; a table depends on the input, `seed` and its index
+    only."""
+    seed = bootstrap_seed(seed)
+    replicates = int(replicates)
+    _check_replicates(0, replicates)
+    keys, counts = _counted(table)
+    prefix, N = _bootstrap_prefix(counts)
+    P, W = int(counts.shape[0]), (2 if keys.dim() == 2 else 1)
+    cap1 = min(P, N)  # non-zeros of one replicate at most
+    per_rep = 4 * P + (8 * W + 4 + 8) * cap1 + 8 * int(lib.spb_bootstrap_compact_ws(P, 1))
+    chunk = max(1, min(replicates, 65535, BOOTSTRAP_BATCH_BYTES // per_rep))
+    for first in range(0, replicates, chunk):
+        c = min(chunk, replicates - first)
+        rows = _empty((c, P), torch.int32)
+        call("spb_bootstrap_counts", _p(prefix), P, N, seed, first, c, _p(rows), _st())
+        ok = _empty((c * cap1, 2) if W == 2 else (c * cap1,), torch.int64)
+        oc, off = _empty(c * cap1, torch.int32), _empty(c + 1, torch.int64)
+        ws = _empty(int(lib.spb_bootstrap_compact_ws(P, c)), torch.int64)
+        call("spb_bootstrap_compact", _p(rows), _p(keys), W, P, c, _p(ok), _p(oc), c * cap1, _p(off), _p(ws), _st())
+        del rows, ws
+        off = off.cpu().tolist()  # one synchronisation per pass
+        for r in range(c):
+            # own storage per replicate: every table starts at an allocation boundary, as count_patterns' tables do
+            k, cnt = ok[off[r]:off[r + 1]].clone(), oc[off[r]:off[r + 1]].clone()
+            if W == 1:
+                yield PatternTable(table.n, k, counts=cnt, divisor=float(N), taxa=table.taxa)
+                continue
+            v = (cnt.to(torch.int64) & 0xFFFFFFFF).to(torch.float64)
+            t = WidePatternTable(table.n, k, torch.div(v, torch.full_like(v, float(N))), taxa=table.taxa)
+            t.counts, t.divisor = cnt, float(N)
+            yield t
