@@ -252,6 +252,15 @@ int64_t spb_subflatten_tables_doubles(int n_taxa);
 int spb_subflatten_score_tables(const double* d_T, const double* d_total, int n_taxa, const uint64_t* d_masks_a,
                                 const uint64_t* d_masks_b, int64_t num, double* d_scores, double* d_tables, int tables_ready,
                                 void* stream);
+/* Many tables in one launch: split s (masks as above) is scored against table s / per_table, with the arithmetic of the
+ * single-table kernels (bitwise equal scores).  _tables_multi (n <= 43): d_tables holds the triple tables of every table
+ * one after the other, spb_subflatten_tables_doubles(n) doubles each (as spb_subflatten_score_tables leaves them);
+ * _multi (22 <= n <= 64, the staged kernel of spb_subflatten_score): d_T holds the tables T [n][n][4][4] one after the other.
+ * d_totals: double [tables], the total of each table. */
+int spb_subflatten_score_tables_multi(const double* d_tables, const double* d_totals, int n_taxa, const uint64_t* d_masks_a,
+                                      const uint64_t* d_masks_b, int64_t num, int64_t per_table, double* d_scores, void* stream);
+int spb_subflatten_score_multi(const double* d_T, const double* d_totals, int n_taxa, const uint64_t* d_masks_a,
+                               const uint64_t* d_masks_b, int64_t num, int64_t per_table, double* d_scores, void* stream);
 
 /* ---- a12-a14: split_score (phylogenetics.py:280-328), K = 4 hard-coded ---- */
 /* G = A A^T for row-major double A [batch][R][C] (lda = C): d_G double [batch][R][R].
@@ -452,6 +461,20 @@ int64_t spb_bootstrap_compact_ws(int64_t P, int64_t reps);
 int spb_bootstrap_compact(const uint32_t* d_counts, const uint64_t* d_keys, int key_words, int64_t P, int64_t reps,
                           uint64_t* d_out_keys, uint32_t* d_out_counts, int64_t cap, int64_t* d_offsets, int64_t* d_ws,
                           void* stream);
+
+/* ---- lockstep agglomeration of erickson_SVD for many replicates (agglomerate.cu), 3 <= n <= 64 ----
+ * Cluster ids: leaves 0 .. n-1, the cluster merged at step t is n + t.  A candidate joins two current clusters against all
+ * other taxa and is written as uint64 masks (d_ma, d_mb) oriented so that side A holds taxon first_taxon.
+ * _init writes the C(n, 2) step-0 candidates of every replicate (replicate r at [r C(n, 2), (r + 1) C(n, 2))) and resets
+ * the state in d_ws (spb_agglomerate_ws_bytes(n, reps) bytes, 16-byte aligned).  _step(step) takes the scores of the
+ * step's candidates (d_scores: double, replicate r at [r P, (r + 1) P), P = C(n, 2) at step 0 and n - step - 1 after),
+ * picks the first minimum over all current pairs in combinations order (NaN ordered as +inf), writes the joined side's
+ * mask and score to d_chosen / d_chosen_scores [reps][n - 2] at column `step`, merges, and unless step = n - 3 writes the
+ * next step's n - step - 2 candidates per replicate to d_ma / d_mb. */
+int64_t spb_agglomerate_ws_bytes(int n_taxa, int64_t reps);
+int spb_agglomerate_init(int n_taxa, int64_t reps, int first_taxon, uint64_t* d_ma, uint64_t* d_mb, void* d_ws, void* stream);
+int spb_agglomerate_step(int n_taxa, int64_t reps, int step, int first_taxon, const double* d_scores, uint64_t* d_ma,
+                         uint64_t* d_mb, void* d_ws, uint64_t* d_chosen, double* d_chosen_scores, void* stream);
 
 #ifdef __cplusplus
 }

@@ -164,6 +164,11 @@ PROTOTYPES = {
     "spb_bootstrap_counts": (_i, [_p, _l, _l, C.c_uint64, _l, _l, _p, _p]),
     "spb_bootstrap_compact_ws": (_l, [_l, _l]),
     "spb_bootstrap_compact": (_i, [_p, _p, _i, _l, _l, _p, _p, _l, _p, _p, _p]),
+    "spb_subflatten_score_tables_multi": (_i, [_p, _p, _i, _p, _p, _l, _l, _p, _p]),
+    "spb_subflatten_score_multi": (_i, [_p, _p, _i, _p, _p, _l, _l, _p, _p]),
+    "spb_agglomerate_ws_bytes": (_l, [_i, _l]),
+    "spb_agglomerate_init": (_i, [_i, _l, _i, _p, _p, _p, _p]),
+    "spb_agglomerate_step": (_i, [_i, _l, _i, _i, _p, _p, _p, _p, _p, _p, _p]),
 }
 
 for _name, (_res, _args) in PROTOTYPES.items():

@@ -30,6 +30,8 @@ ranks takes 1.5 ms).
 """
 from __future__ import annotations
 
+from collections import namedtuple
+
 import numpy as np
 import torch
 
@@ -351,6 +353,19 @@ def score_splits(alignment, splits, method=Method.flattening, taxa=None):
     return SplitScorer(splits, taxa, method, rank or 0, world or 1)(alignment)
 
 
+def _bootstrap_checks(name, replicates, seed):
+    """The replicate count and seed checks of the bootstrap entry points and their one-process rule; returns the seed."""
+    if isinstance(replicates, bool) or not isinstance(replicates, (int, np.integer)) or replicates < 1:
+        raise ValueError(f"{name}: replicates must be an integer >= 1 (got {replicates!r})")
+    if replicates > engine.BOOTSTRAP_MAX_REPLICATES:
+        raise ValueError(f"{name}: at most {engine.BOOTSTRAP_MAX_REPLICATES} replicates")
+    seed = engine.bootstrap_seed(seed)
+    import torch.distributed as dist
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        raise NotImplementedError(f"{name} runs on one GPU: call it outside a torch.distributed group of several processes")
+    return seed
+
+
 def bootstrap_scores(alignment, splits, method=Method.flattening, replicates=100, seed=0, taxa=None):
     """Nonparametric bootstrap of split scores: numpy float64 [replicates, len(splits)], row b = the scores `score_splits`
     gives for bootstrap replicate b of the alignment.
@@ -365,14 +380,7 @@ def bootstrap_scores(alignment, splits, method=Method.flattening, replicates=100
       Method.subflattening  pair tables of the replicate's counts (engine.pair_tables_from_table) + engine.subflatten_scores
       Method.mutual_information  engine.rank1_divergence_scores (counts / N)
     The scores stay on the device until the last replicate is scored."""
-    if isinstance(replicates, bool) or not isinstance(replicates, (int, np.integer)) or replicates < 1:
-        raise ValueError(f"bootstrap_scores: replicates must be an integer >= 1 (got {replicates!r})")
-    if replicates > engine.BOOTSTRAP_MAX_REPLICATES:
-        raise ValueError(f"bootstrap_scores: at most {engine.BOOTSTRAP_MAX_REPLICATES} replicates")
-    seed = engine.bootstrap_seed(seed)
-    import torch.distributed as dist
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        raise NotImplementedError("bootstrap_scores runs on one GPU: call it outside a torch.distributed group of several processes")
+    seed = _bootstrap_checks("bootstrap_scores", replicates, seed)
     if taxa is None and isinstance(alignment, dict):
         taxa = list(alignment.keys())
     # one process: the SplitScorer holds the split positions, the subflattening masks and the counting stage of score_splits
@@ -397,3 +405,83 @@ def bootstrap_scores(alignment, splits, method=Method.flattening, replicates=100
         else:
             out[b] = engine.rank1_divergence_scores(tb, idx)
     return out.cpu().numpy()
+
+
+BootstrapTrees = namedtuple("BootstrapTrees", "tree support replicate_trees")
+
+
+def _default_taxa(n):
+    """erickson_SVD's leaf names of an alignment without names, in row order."""
+    return [str(np.base_repr(i, base=max(i + 1, 2))) if n <= 36 else f"t{i}" for i in range(n)]
+
+
+def _side_mask(side, index, n):
+    m = 0
+    for name in side:
+        if name not in index:
+            raise ValueError(f"bootstrap_trees: unknown leaf {name!r} in a split")
+        m |= 1 << index[name]
+    return m
+
+
+def bootstrap_trees(alignment, replicates=100, seed=0, taxa=None, method=Method.subflattening, splits=None):
+    """Bootstrap support of the splits of an erickson_SVD tree.  Returns BootstrapTrees(tree, support, replicate_trees):
+
+      tree             the n - 2 splits erickson_SVD(Method.subflattening) chooses for the alignment, in its format (a sorted
+                       2-tuple of sorted leaf-name tuples per step)
+      replicate_trees  the same for every bootstrap replicate; replicate b is the table engine.bootstrap_tables yields at
+                       index b, so also row b of bootstrap_scores with the same seed
+      support          numpy float64: entry i is the fraction of replicate trees that contain split i as a bipartition
+                       (orientation ignored); split i is splits[i] (a pair of leaf-name sequences) or, by default, tree[i]
+
+    Each tree is what erickson_SVD(Alignment(mapping, taxa), taxa=taxa, method=Method.subflattening) computes on its table:
+    candidates in combinations order over the current clusters (merged cluster appended), the first minimum wins, and every
+    bipartition is scored in the orientation score_canonical gives it (the side with the smallest leaf name first).  Scores
+    come from pair tables of the table's integer counts, so the result is bit-reproducible.  Every replicate is agglomerated
+    on the device at once (engine.bootstrap_tree_masks, csrc/agglomerate.cu): about three launches per step and no host
+    synchronisation until the trees are read back.
+
+    `alignment`, `replicates`, `seed` and `taxa` are as in bootstrap_scores; 2..64 taxa.  Leaf names are the dict's keys or
+    `taxa`, else erickson_SVD's default names in row order.  Only Method.subflattening is supported."""
+    if method in (Method.flattening, Method.mutual_information):
+        raise NotImplementedError(f"bootstrap_trees supports Method.subflattening only: the {method} scorers take one pattern "
+                                  "table per launch, so the replicates cannot be agglomerated in lockstep")
+    if method != Method.subflattening:
+        raise NotImplementedError("bootstrap_trees supports Method.subflattening only")
+    seed = _bootstrap_checks("bootstrap_trees", replicates, seed)
+    n = _num_taxa(alignment)
+    if not 2 <= n <= engine._lib.SPB_MAX_TAXA:
+        raise ValueError(f"bootstrap_trees: 2 to {engine._lib.SPB_MAX_TAXA} taxa (got {n})")
+    if taxa is None:
+        taxa = list(alignment.keys()) if isinstance(alignment, dict) else _default_taxa(n)
+    taxa = list(taxa)
+    if len(taxa) != n or len(set(taxa)) != n:
+        raise ValueError(f"bootstrap_trees: taxa must be {n} distinct names, one per row")
+    index = {t: i for i, t in enumerate(taxa)}
+    full = (1 << n) - 1
+    if splits is not None:
+        wanted = []
+        for side_a, side_b in splits:
+            ma, mb = _side_mask(side_a, index, n), _side_mask(side_b, index, n)
+            if ma & mb or ma | mb != full or len(side_a) + len(side_b) != n:
+                raise ValueError("bootstrap_trees: every split must place every taxon on exactly one side")
+            wanted.append(ma)
+    first = min(range(n), key=lambda i: taxa[i])
+    ss = SplitScorer([], taxa, Method.subflattening)  # the counting stage of bootstrap_scores: the same replicate tables
+    table = ss._count(alignment) if n <= engine.NARROW_MAX_TAXA else ss._count_wide(alignment)
+    masks, _ = engine.bootstrap_tree_masks(table, int(replicates), seed, first)
+
+    def split_of(m):
+        m = int(m)
+        joined = tuple(sorted(taxa[i] for i in range(n) if m >> i & 1))
+        rest = tuple(sorted(taxa[i] for i in range(n) if not m >> i & 1))
+        return tuple(sorted((joined, rest)))
+
+    trees = [[split_of(m) for m in row] for row in masks]
+    if splits is None:
+        wanted = [int(m) for m in masks[0]]
+    # a bipartition as the mask of the side without taxon 0: orientation-free
+    canon = lambda m: m if not m & 1 else full & ~m  # noqa: E731
+    have = [{canon(int(m)) for m in row} for row in masks[1:]]
+    support = np.array([sum(canon(w) in h for h in have) / len(have) for w in wanted], dtype=np.float64)
+    return BootstrapTrees(trees[0], support, trees[1:])

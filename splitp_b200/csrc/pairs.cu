@@ -220,6 +220,54 @@ __global__ void subflatten_kernel(const double* __restrict__ T, const double* __
 
 constexpr int kSThreads = 128;
 
+// Score of split s of the mask lists against the pair tables T / total, by the whole CTA (staged matrix + Jacobi): the
+// per-split body of subflatten_score_kernel and subflatten_score_multi_kernel.
+__device__ __forceinline__ void staged_split_score(const double* __restrict__ T, double tot, int n, const uint64_t* __restrict__ masks_a,
+                                                   const uint64_t* __restrict__ masks_b, int64_t s, double* M, double* G,
+                                                   double* scores) {
+  __shared__ JacobiScratchT<3 * (SPB_MAX_TAXA / 2) + 2> js;  // k = min(3a, 3b) + 1 <= 97
+  __shared__ double lam[kJacobiMaxK], tmp[kJacobiMaxK];
+  __shared__ uint8_t la[SPB_MAX_TAXA], lb[SPB_MAX_TAXA];
+  __shared__ int s_a, s_b;
+  const int tid = threadIdx.x;
+  const uint64_t full = (n == 64) ? ~0ull : ((1ull << n) - 1ull);
+  __syncthreads();
+  if (tid == 0) {
+    uint64_t ma = masks_a[s] & full;
+    uint64_t mb = masks_b ? (masks_b[s] & full & ~ma) : (full & ~ma);
+    int a = 0, b = 0;
+    while (ma) { la[a++] = (uint8_t)(__ffsll((long long)ma) - 1); ma &= ma - 1; }
+    while (mb) { lb[b++] = (uint8_t)(__ffsll((long long)mb) - 1); mb &= mb - 1; }
+    s_a = a; s_b = b;
+  }
+  __syncthreads();
+  const int a = s_a, b = s_b;
+  const int rows = 3 * a + 1, cols = 3 * b + 1;
+  const bool tr = rows > cols;          // orient so that k = smaller dimension
+  const int k = tr ? cols : rows, L = tr ? rows : cols;
+  const int ldm = (L + 1) | 1, ldg = jacobi_ld(k);  // odd strides: rows of M / G start on different banks
+  for (int idx = tid; idx < k * L; idx += kSThreads) {
+    int r = idx / L, c = idx - r * L;
+    M[r * ldm + c] = tr ? subflat_entry(T, tot, n, la, a, lb, b, c, r) : subflat_entry(T, tot, n, la, a, lb, b, r, c);
+  }
+  __syncthreads();
+  for (int idx = tid; idx < k * k; idx += kSThreads) {
+    int r1 = idx / k, r2 = idx - r1 * k;
+    if (r2 < r1) continue;
+    const double* x = M + r1 * ldm;
+    const double* y = M + r2 * ldm;
+    double acc = 0.0;
+    for (int c = 0; c < L; ++c) acc = fma(x[c], y[c], acc);
+    G[r1 * ldg + r2] = acc;
+    G[r2 * ldg + r1] = acc;
+  }
+  if ((k & 1) && tid <= k) { G[k * ldg + tid] = 0.0; G[tid * ldg + k] = 0.0; }  // zero padding of the odd dimension
+  __syncthreads();
+  jacobi_eig_smem(G, ldg, k, nullptr, 0, &js);
+  sort_diag_desc(G, ldg, k, tmp, lam);
+  if (tid == 0) scores[s] = (k <= 4) ? 0.0 : score_from_sorted(lam, k);
+}
+
 __global__ void __launch_bounds__(kSThreads) subflatten_score_kernel(const double* __restrict__ T, const double* __restrict__ total,
                                                                      int n, const uint64_t* __restrict__ masks_a,
                                                                      const uint64_t* __restrict__ masks_b, int64_t num,
@@ -227,49 +275,21 @@ __global__ void __launch_bounds__(kSThreads) subflatten_score_kernel(const doubl
   extern __shared__ __align__(16) double s_d[];
   double* M = s_d;                 // k x (L+1)
   double* G = M + m_elems;         // k x (k|1)
-  __shared__ JacobiScratchT<3 * (SPB_MAX_TAXA / 2) + 2> js;  // k = min(3a, 3b) + 1 <= 97
-  __shared__ double lam[kJacobiMaxK], tmp[kJacobiMaxK];
-  __shared__ uint8_t la[SPB_MAX_TAXA], lb[SPB_MAX_TAXA];
-  __shared__ int s_a, s_b;
-  const int tid = threadIdx.x;
-  const uint64_t full = (n == 64) ? ~0ull : ((1ull << n) - 1ull);
   const double tot = *total;
+  for (int64_t s = blockIdx.x; s < num; s += gridDim.x) staged_split_score(T, tot, n, masks_a, masks_b, s, M, G, scores);
+}
+
+// Split s against the pair tables T + (s / per_table) n^2 16, totals[s / per_table]: many tables in one launch.
+__global__ void __launch_bounds__(kSThreads) subflatten_score_multi_kernel(const double* __restrict__ T, const double* __restrict__ totals,
+                                                                           int n, const uint64_t* __restrict__ masks_a,
+                                                                           const uint64_t* __restrict__ masks_b, int64_t num,
+                                                                           int64_t per_table, double* scores, int m_elems) {
+  extern __shared__ __align__(16) double s_d[];
+  double* M = s_d;
+  double* G = M + m_elems;
   for (int64_t s = blockIdx.x; s < num; s += gridDim.x) {
-    __syncthreads();
-    if (tid == 0) {
-      uint64_t ma = masks_a[s] & full;
-      uint64_t mb = masks_b ? (masks_b[s] & full & ~ma) : (full & ~ma);
-      int a = 0, b = 0;
-      while (ma) { la[a++] = (uint8_t)(__ffsll((long long)ma) - 1); ma &= ma - 1; }
-      while (mb) { lb[b++] = (uint8_t)(__ffsll((long long)mb) - 1); mb &= mb - 1; }
-      s_a = a; s_b = b;
-    }
-    __syncthreads();
-    const int a = s_a, b = s_b;
-    const int rows = 3 * a + 1, cols = 3 * b + 1;
-    const bool tr = rows > cols;          // orient so that k = smaller dimension
-    const int k = tr ? cols : rows, L = tr ? rows : cols;
-    const int ldm = (L + 1) | 1, ldg = jacobi_ld(k);  // odd strides: rows of M / G start on different banks
-    for (int idx = tid; idx < k * L; idx += kSThreads) {
-      int r = idx / L, c = idx - r * L;
-      M[r * ldm + c] = tr ? subflat_entry(T, tot, n, la, a, lb, b, c, r) : subflat_entry(T, tot, n, la, a, lb, b, r, c);
-    }
-    __syncthreads();
-    for (int idx = tid; idx < k * k; idx += kSThreads) {
-      int r1 = idx / k, r2 = idx - r1 * k;
-      if (r2 < r1) continue;
-      const double* x = M + r1 * ldm;
-      const double* y = M + r2 * ldm;
-      double acc = 0.0;
-      for (int c = 0; c < L; ++c) acc = fma(x[c], y[c], acc);
-      G[r1 * ldg + r2] = acc;
-      G[r2 * ldg + r1] = acc;
-    }
-    if ((k & 1) && tid <= k) { G[k * ldg + tid] = 0.0; G[tid * ldg + k] = 0.0; }  // zero padding of the odd dimension
-    __syncthreads();
-    jacobi_eig_smem(G, ldg, k, nullptr, 0, &js);
-    sort_diag_desc(G, ldg, k, tmp, lam);
-    if (tid == 0) scores[s] = (k <= 4) ? 0.0 : score_from_sorted(lam, k);
+    const int64_t t = s / per_table;
+    staged_split_score(T + t * n * n * 16, totals[t], n, masks_a, masks_b, s, M, G, scores);
   }
 }
 
@@ -644,12 +664,11 @@ __device__ __forceinline__ double warp2_top4(double* G, int ldg, int k, double* 
   return ((fmax(l0, 0.0) + fmax(l1, 0.0)) + fmax(l2, 0.0)) + fmax(l3, 0.0);
 }
 
-__global__ void __launch_bounds__(32 * kW2WarpsPerCta) subflatten_score_warp2_kernel(const TripleTables tt, const double* __restrict__ total,
-                                                                                    const uint64_t* __restrict__ masks_a,
-                                                                                    const uint64_t* __restrict__ masks_b, int64_t num,
-                                                                                    double* scores, int kcap, int warp_doubles) {
-  extern __shared__ __align__(16) double s_w2[];
-  double* base = s_w2 + (size_t)(threadIdx.x >> 5) * warp_doubles;
+// Score of split s of the mask lists against one set of triple tables, by one warp (its shared-memory tile at `base`): the
+// per-split body of subflatten_score_warp2_kernel and subflatten_score_warp2_multi_kernel.
+__device__ __forceinline__ void warp2_split_score(const TripleTables& tt, double tot, const uint64_t* __restrict__ masks_a,
+                                                  const uint64_t* __restrict__ masks_b, int64_t s, double* scores, int kcap,
+                                                  uint64_t full, double* base, int lane) {
   const int ldg = kcap | 1;
   double* G = base;                       // [kcap][ldg]
   double* sv = G + (size_t)kcap * ldg;    // 4 x 64
@@ -658,13 +677,8 @@ __global__ void __launch_bounds__(32 * kW2WarpsPerCta) subflatten_score_warp2_ke
   double* se = sd + 64;
   uint8_t* la = reinterpret_cast<uint8_t*>(se + 64);  // row-side taxa (<= 21), then column-side taxa (<= 64)
   uint8_t* lb = la + 32;
-  const int lane = threadIdx.x & 31;
   const int n = tt.n;
-  const uint64_t full = (n == 64) ? ~0ull : ((1ull << n) - 1ull);
-  const double tot = *total;
-  const int64_t nwarps = (int64_t)gridDim.x * kW2WarpsPerCta;
-  for (int64_t s = (int64_t)blockIdx.x * kW2WarpsPerCta + (threadIdx.x >> 5); s < num; s += nwarps) {
-    __syncwarp();
+  {
     uint64_t ma = masks_a[s] & full;
     uint64_t mb = masks_b ? (masks_b[s] & full & ~ma) : (full & ~ma);
     if (__popcll(ma) > __popcll(mb)) { const uint64_t t = ma; ma = mb; mb = t; }  // rows = the smaller side (S S^T and S^T S share
@@ -672,11 +686,11 @@ __global__ void __launch_bounds__(32 * kW2WarpsPerCta) subflatten_score_warp2_ke
     const int k = 3 * a + 1;
     if (k <= 4 || b == 0) {  // at most 4 singular values: the score vanishes (phylogenetics.py:293-300)
       if (lane == 0) scores[s] = 0.0;
-      continue;
+      return;
     }
     if (k > kcap) {  // not reachable through spb_subflatten_score_tables (the host routes such batches elsewhere)
       if (lane == 0) scores[s] = nan("");
-      continue;
+      return;
     }
     for (int t = lane; t < 64; t += 32) {  // position lists in ascending taxon order
       const uint64_t below = (1ull << t) - 1ull;
@@ -735,6 +749,46 @@ __global__ void __launch_bounds__(32 * kW2WarpsPerCta) subflatten_score_warp2_ke
     const double trace = warp_sum_all(part);
     const double top = (k <= 32) ? warp2_top4<1>(G, ldg, k, sv, sq, sd, se, lane) : warp2_top4<2>(G, ldg, k, sv, sq, sd, se, lane);
     if (lane == 0) scores[s] = trace > 0.0 ? sqrt(fmax(trace - top, 0.0) / trace) : nan("");
+  }
+}
+
+__global__ void __launch_bounds__(32 * kW2WarpsPerCta) subflatten_score_warp2_kernel(const TripleTables tt, const double* __restrict__ total,
+                                                                                    const uint64_t* __restrict__ masks_a,
+                                                                                    const uint64_t* __restrict__ masks_b, int64_t num,
+                                                                                    double* scores, int kcap, int warp_doubles) {
+  extern __shared__ __align__(16) double s_w2[];
+  double* base = s_w2 + (size_t)(threadIdx.x >> 5) * warp_doubles;
+  const int lane = threadIdx.x & 31;
+  const uint64_t full = (tt.n == 64) ? ~0ull : ((1ull << tt.n) - 1ull);
+  const double tot = *total;
+  const int64_t nwarps = (int64_t)gridDim.x * kW2WarpsPerCta;
+  for (int64_t s = (int64_t)blockIdx.x * kW2WarpsPerCta + (threadIdx.x >> 5); s < num; s += nwarps) {
+    __syncwarp();
+    warp2_split_score(tt, tot, masks_a, masks_b, s, scores, kcap, full, base, lane);
+  }
+}
+
+// Split s against the triple tables at tables + (s / per_table) table_doubles (layout of spb_subflatten_score_tables) and
+// totals[s / per_table]: many tables in one launch.  No __launch_bounds__: with it ptxas holds the kernel to 64 registers and
+// spills 4 bytes; without it it takes 66 registers, which still fit 7 CTAs of 4 warps on an SM.
+__global__ void subflatten_score_warp2_multi_kernel(
+    const double* __restrict__ tables, int64_t table_doubles, const double* __restrict__ totals, int n,
+    const uint64_t* __restrict__ masks_a, const uint64_t* __restrict__ masks_b, int64_t num, int64_t per_table, double* scores,
+    int kcap, int warp_doubles) {
+  extern __shared__ __align__(16) double s_w2[];
+  double* base = s_w2 + (size_t)(threadIdx.x >> 5) * warp_doubles;
+  const int lane = threadIdx.x & 31;
+  const int64_t nn = n;
+  const uint64_t full = (n == 64) ? ~0ull : ((1ull << n) - 1ull);
+  const int64_t nwarps = (int64_t)gridDim.x * kW2WarpsPerCta;
+  for (int64_t s = (int64_t)blockIdx.x * kW2WarpsPerCta + (threadIdx.x >> 5); s < num; s += nwarps) {
+    const int64_t t = s / per_table;
+    const double* P = tables + t * table_doubles;
+    const double* R = P + nn * nn * nn * 9;
+    const double* D = R + nn * nn * 3;
+    const TripleTables tt{P, R, D, D + nn, n};
+    __syncwarp();
+    warp2_split_score(tt, totals[t], masks_a, masks_b, s, scores, kcap, full, base, lane);
   }
 }
 
@@ -904,6 +958,32 @@ extern "C" int spb_subflatten_score_tables(const double* d_T, const double* d_to
   return SPB_OK;
 }
 
+// Many tables per launch through the triple-table warp kernel (header: spb_subflatten_score_tables_multi).
+extern "C" int spb_subflatten_score_tables_multi(const double* d_tables, const double* d_totals, int n_taxa, const uint64_t* d_masks_a,
+                                                 const uint64_t* d_masks_b, int64_t num, int64_t per_table, double* d_scores,
+                                                 void* stream) {
+  SPB_REQUIRE(n_taxa >= 2 && n_taxa <= SPB_MAX_TAXA && per_table >= 1, "spb_subflatten_score_tables_multi: bad arguments");
+  const int kcap = 3 * (n_taxa / 2) + 1;
+  SPB_REQUIRE(kcap <= kW2MaxK, "spb_subflatten_score_tables_multi: handles up to %d taxa; use spb_subflatten_score_multi",
+              2 * ((kW2MaxK - 1) / 3) + 1);
+  if (num <= 0) return SPB_OK;
+  SPB_REQUIRE(d_tables && d_totals && d_masks_a && d_scores, "spb_subflatten_score_tables_multi: NULL buffer");
+  const int ldg = kcap | 1;
+  const int warp_doubles = kcap * ldg + 4 * 64 + 16;
+  const size_t smem = (size_t)kW2WarpsPerCta * warp_doubles * sizeof(double);
+  SPB_CUDA(cudaFuncSetAttribute(subflatten_score_warp2_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int occ = 1;
+  SPB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, subflatten_score_warp2_multi_kernel, 32 * kW2WarpsPerCta, smem));
+  if (occ < 1) occ = 1;
+  int64_t grid = (int64_t)sm_count() * occ;
+  const int64_t need = (num + kW2WarpsPerCta - 1) / kW2WarpsPerCta;
+  if (grid > need) grid = need;
+  subflatten_score_warp2_multi_kernel<<<(unsigned)grid, 32 * kW2WarpsPerCta, smem, (cudaStream_t)stream>>>(
+      d_tables, spb_subflatten_tables_doubles(n_taxa), d_totals, n_taxa, d_masks_a, d_masks_b, num, per_table, d_scores, kcap, warp_doubles);
+  SPB_LAUNCH_CHECK();
+  return SPB_OK;
+}
+
 namespace spb {
 int score_gram_warp_launch(const double* d_G, int k, int64_t ld, int64_t batch, double* d_scores, cudaStream_t st) {
   const int warp_doubles = k * (k | 1) + 4 * 64;
@@ -950,6 +1030,26 @@ extern "C" int spb_subflatten_score(const double* d_T, const double* d_total, in
   if (grid > num) grid = num;
   subflatten_score_kernel<<<(unsigned)grid, kSThreads, smem, (cudaStream_t)stream>>>(d_T, d_total, n_taxa, d_masks_a, d_masks_b,
                                                                                     num, d_scores, m_elems);
+  SPB_LAUNCH_CHECK();
+  return SPB_OK;
+}
+
+// Many tables per launch through the staged CTA kernel (header: spb_subflatten_score_multi).
+extern "C" int spb_subflatten_score_multi(const double* d_T, const double* d_totals, int n_taxa, const uint64_t* d_masks_a,
+                                          const uint64_t* d_masks_b, int64_t num, int64_t per_table, double* d_scores, void* stream) {
+  SPB_REQUIRE(n_taxa > kWarpMaxTaxa && n_taxa <= SPB_MAX_TAXA && per_table >= 1, "spb_subflatten_score_multi: bad arguments");
+  if (num <= 0) return SPB_OK;
+  SPB_REQUIRE(d_T && d_totals && d_masks_a && d_scores, "spb_subflatten_score_multi: NULL buffer");
+  int m_elems = 0;
+  size_t smem = subflat_smem(n_taxa, &m_elems);
+  SPB_CUDA(cudaFuncSetAttribute(subflatten_score_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int occ = 1;
+  SPB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, subflatten_score_multi_kernel, kSThreads, smem));
+  if (occ < 1) occ = 1;
+  int64_t grid = (int64_t)sm_count() * occ;
+  if (grid > num) grid = num;
+  subflatten_score_multi_kernel<<<(unsigned)grid, kSThreads, smem, (cudaStream_t)stream>>>(d_T, d_totals, n_taxa, d_masks_a, d_masks_b,
+                                                                                          num, per_table, d_scores, m_elems);
   SPB_LAUNCH_CHECK();
   return SPB_OK;
 }

@@ -1226,7 +1226,9 @@ def pair_tables_from_alignment(aln, as_counts=False):
     return pair_finalize(raw, aln.n, usable)
 
 
-def pair_tables_from_table(table, as_counts=False):
+def pair_tables_from_table(table, as_counts=False, T=None, total=None):
+    """Pair tables of a pattern table (values, or its counts when as_counts and it has them).  T (float64 [n, n, 4, 4]) and
+    total (float64 [1]), when given, receive the result: slices of a buffer that stacks the tables of several patterns."""
     n = table.n
     vals = table.counts.to(torch.float64) if (as_counts and table.counts is not None) else table.values_f64()
     if isinstance(table, WidePatternTable):  # deterministic fp64 tensor-core product (csrc/wide.cu)
@@ -1236,7 +1238,8 @@ def pair_tables_from_table(table, as_counts=False):
     else:
         N_tab = _zeros((n, n, 4, 4), torch.float64)
         call("spb_pair_tables_weighted", _p(table.keys), _p(vals.contiguous()), table.num, n, _p(N_tab), _st())
-    T, total = _empty((n, n, 4, 4), torch.float64), _empty(1, torch.float64)
+    T = _empty((n, n, 4, 4), torch.float64) if T is None else T
+    total = _empty(1, torch.float64) if total is None else total
     call("spb_pair_transform", _p(N_tab), n, _p(T), _p(total), _st())
     return PairTables(n, N_tab, T, total)
 
@@ -1275,6 +1278,67 @@ def subflatten_scores(pt, masks_a, masks_b=None):
     else:  # sides above 21 taxa: the kernels that stage the subflattening
         call("spb_subflatten_score", _p(pt.T), _p(pt.total), pt.n, _p(ma), _p(mb), int(ma.shape[0]), _p(out), _st())
     return out
+
+
+class SubflattenTables:
+    """The subflattening scoring tables of several pattern tables, stacked for subflatten_scores_multi: up to 43 taxa the
+    triple tables (spb_subflatten_tables_doubles(n) doubles each), from 44 taxa the tables T [n][n][4][4] of the staged
+    kernel; `total` holds one total per table.  add(i, table) fills slot i from the pair tables of the table's counts."""
+
+    def __init__(self, n, count):
+        self.n = n
+        per = int(lib.spb_subflatten_tables_doubles(n)) if n <= SUBFLATTEN_TABLES_MAX_TAXA else 16 * n * n
+        self.data = _empty((count, per), torch.float64)
+        self.total = _empty(count, torch.float64)
+
+    @staticmethod
+    def bytes_per_table(n):
+        return 8 * (int(lib.spb_subflatten_tables_doubles(n)) if n <= SUBFLATTEN_TABLES_MAX_TAXA else 16 * n * n) + 8
+
+    def add(self, i, table):
+        n, total = self.n, self.total[i:i + 1]
+        if n > SUBFLATTEN_TABLES_MAX_TAXA:
+            pair_tables_from_table(table, as_counts=True, T=self.data[i].view(n, n, 4, 4), total=total)
+            return
+        pt = pair_tables_from_table(table, as_counts=True, total=total)
+        # no splits: the call only tabulates the triple tables of pt into slot i
+        call("spb_subflatten_score_tables", _p(pt.T), _p(pt.total), n, None, None, 0, None, _p(self.data[i]), 0, _st())
+
+
+def subflatten_scores_multi(tables, masks_a, masks_b, per_table):
+    """Subflattening scores of splits against several tables (SubflattenTables): split s is scored against table
+    s // per_table.  masks: int64 device tensors holding uint64 bit masks, as subflatten_scores takes them.  Each score is
+    bitwise the one subflatten_scores gives for that split against the pair tables of that table alone."""
+    out = _empty(int(masks_a.shape[0]), torch.float64)
+    entry = "spb_subflatten_score_tables_multi" if tables.n <= SUBFLATTEN_TABLES_MAX_TAXA else "spb_subflatten_score_multi"
+    call(entry, _p(tables.data), _p(tables.total), tables.n, _p(masks_a), _p(masks_b), int(masks_a.shape[0]), int(per_table),
+         _p(out), _st())
+    return out
+
+
+def erickson_lockstep(n, reps, first_taxon, score_fn, timer=None):
+    """erickson_SVD's agglomeration of `reps` replicates at once on the device (csrc/agglomerate.cu).  At every step
+    score_fn(masks_a, masks_b, per_table) returns the float64 scores of the step's candidate splits (replicate r's at
+    [r per_table, (r + 1) per_table)); candidates are int64 tensors of uint64 masks oriented so that side A holds taxon
+    `first_taxon`.  Returns (joined-side masks, scores), both [reps, n - 2] on the device: the masks as uint64 bits in an
+    int64 tensor, column t = the split chosen at step t.  The pick is the first minimum over the current cluster pairs in
+    combinations order, clusters kept in erickson_SVD's list order; NaN counts as +inf.  `timer` (PhaseTimer) gets the
+    spans "score" (score_fn) and "step" (the step kernel)."""
+    steps = max(n - 2, 0)
+    chosen, scores = _empty((reps, steps), torch.int64), _empty((reps, steps), torch.float64)
+    if steps == 0 or reps == 0:
+        return chosen, scores
+    p0 = n * (n - 1) // 2
+    ma, mb = _empty(reps * p0, torch.int64), _empty(reps * p0, torch.int64)
+    ws = _empty(int(lib.spb_agglomerate_ws_bytes(n, reps)), torch.uint8)
+    call("spb_agglomerate_init", n, reps, first_taxon, _p(ma), _p(mb), _p(ws), _st())
+    for t in range(steps):
+        per = p0 if t == 0 else n - t - 1
+        with _span(timer, "score"):
+            sc = score_fn(ma[:reps * per], mb[:reps * per], per)
+        with _span(timer, "step"):
+            call("spb_agglomerate_step", n, reps, t, first_taxon, _p(sc), _p(ma), _p(mb), _p(ws), _p(chosen), _p(scores), _st())
+    return chosen, scores
 
 
 # --------------------------------------------------------------------------------------------
@@ -1735,11 +1799,58 @@ def bootstrap_tables(table, replicates, seed):
         off = off.cpu().tolist()  # one synchronisation per pass
         for r in range(c):
             # own storage per replicate: every table starts at an allocation boundary, as count_patterns' tables do
-            k, cnt = ok[off[r]:off[r + 1]].clone(), oc[off[r]:off[r + 1]].clone()
-            if W == 1:
-                yield PatternTable(table.n, k, counts=cnt, divisor=float(N), taxa=table.taxa)
-                continue
-            v = (cnt.to(torch.int64) & 0xFFFFFFFF).to(torch.float64)
-            t = WidePatternTable(table.n, k, torch.div(v, torch.full_like(v, float(N))), taxa=table.taxa)
-            t.counts, t.divisor = cnt, float(N)
-            yield t
+            yield _table_of_counts(table, ok[off[r]:off[r + 1]].clone(), oc[off[r]:off[r + 1]].clone(), N)
+
+
+def _table_of_counts(table, keys, counts, N):
+    """The pattern table of `keys` with uint32 `counts` and divisor N, in the form bootstrap_tables yields (see there)."""
+    if keys.dim() == 1:
+        return PatternTable(table.n, keys, counts=counts, divisor=float(N), taxa=table.taxa)
+    v = (counts.to(torch.int64) & 0xFFFFFFFF).to(torch.float64)
+    t = WidePatternTable(table.n, keys, torch.div(v, torch.full_like(v, float(N))), taxa=table.taxa)
+    t.counts, t.divisor = counts, float(N)
+    return t
+
+
+# --------------------------------------------------------------------------------------------
+# bootstrap trees: erickson_SVD(Method.subflattening) of every replicate in lockstep (csrc/agglomerate.cu)
+# --------------------------------------------------------------------------------------------
+BOOTSTRAP_TREES_BATCH_BYTES = 4 << 30  # device memory of one lockstep group: stacked scoring tables, candidates, state
+
+
+def bootstrap_tree_masks(table, replicates, seed, first_taxon, timer=None):
+    """erickson_SVD(Method.subflattening) agglomerations of a table of pattern counts (see _counted) and of its bootstrap
+    replicates: (joined-side masks as numpy uint64, scores as numpy float64), both [replicates + 1, n - 2].  Row 0 is the
+    table itself, row b + 1 replicate b as bootstrap_tables yields it.  Every table is scored from the pair tables of its
+    integer counts (SubflattenTables) with candidates oriented towards `first_taxon` (erickson_lockstep).  The tables run in
+    lockstep groups of at most BOOTSTRAP_TREES_BATCH_BYTES of device memory; a row depends on its table only.  `timer`
+    (PhaseTimer) gets the spans "resample", "tables", "score" and "step"."""
+    import itertools
+    seed, n = bootstrap_seed(seed), table.n
+    replicates = int(replicates)
+    _check_replicates(0, replicates)
+    keys, counts = _counted(table)
+    _, N = _bootstrap_prefix(counts)
+    count, steps = replicates + 1, max(n - 2, 0)
+    if steps == 0:
+        return np.zeros((count, 0), np.uint64), np.zeros((count, 0), np.float64)
+    tables = itertools.chain([_table_of_counts(table, keys, counts, N)], bootstrap_tables(table, replicates, seed))
+    p0 = n * (n - 1) // 2
+    per = SubflattenTables.bytes_per_table(n) + int(lib.spb_agglomerate_ws_bytes(n, 1)) + 24 * p0 + 16 * steps
+    group = max(1, min(count, BOOTSTRAP_TREES_BATCH_BYTES // per))
+    masks, scores = [], []
+    for g0 in range(0, count, group):
+        g = min(group, count - g0)
+        stack = SubflattenTables(n, g)
+        for i in range(g):
+            with _span(timer, "resample"):
+                tb = next(tables)
+            with _span(timer, "tables"):
+                stack.add(i, tb)
+            del tb
+        m, sc = erickson_lockstep(n, g, first_taxon, lambda ma, mb, per_table: subflatten_scores_multi(stack, ma, mb, per_table),
+                                  timer)
+        masks.append(m)
+        scores.append(sc)
+        del stack
+    return torch.cat(masks).cpu().numpy().view(np.uint64), torch.cat(scores).cpu().numpy()
