@@ -229,6 +229,17 @@ int spb_pair_tables(const uint32_t* d_planes, const uint32_t* d_valid, int n_tax
  * d_raw (fasta.py:66-70) without a host round trip; divisor == 0 keeps counts.  d_total (double) = sum of all values. */
 int spb_pair_finalize(const uint64_t* d_raw, int n_taxa, double divisor, double* d_N, double* d_T,
                       double* d_total, void* stream);
+/* Raw pair statistics of S consecutive site segments [bounds[s], bounds[s+1]) in one pass over the planes, accumulated
+ * into d_raw uint64 [S][spb_pair_raw_words(n)] (zeroed by the caller).  d_bounds: int64 [S + 1] on the device, ascending,
+ * bounds[S] <= 32 * plane_words; empty segments allowed.  Row s equals what spb_pair_tables gives for an alignment made
+ * of exactly those sites. */
+int spb_pair_tables_segments(const uint32_t* d_planes, const uint32_t* d_valid, int n_taxa, int64_t plane_words,
+                             const int64_t* d_bounds, int64_t n_segments, uint64_t* d_raw, void* stream);
+/* spb_pair_finalize of `rows` raw rows in one launch: row r reads d_raw + r * spb_pair_raw_words(n) and writes
+ * d_N / d_T + r * n * n * 16 and d_total[r] (d_N, d_total optional), bitwise what spb_pair_finalize gives for that row.
+ * With divisor < 0 each row is divided by its own usable sites. */
+int spb_pair_finalize_rows(const uint64_t* d_raw, int64_t rows, int n_taxa, double divisor, double* d_N, double* d_T,
+                           double* d_total, void* stream);
 /* Same tables from a weighted pattern list (dict inputs): d_N must be zeroed by the caller. */
 int spb_pair_tables_weighted(const uint64_t* d_keys, const double* d_vals, int64_t num, int n_taxa,
                              double* d_N, void* stream);

@@ -108,6 +108,8 @@ PROTOTYPES = {
     "spb_pair_raw_words": (_l, [_i]),
     "spb_pair_tables": (_i, [_p, _p, _i, _l, _l, _l, _p, _p]),
     "spb_pair_finalize": (_i, [_p, _i, _d, _p, _p, _p, _p]),
+    "spb_pair_tables_segments": (_i, [_p, _p, _i, _l, _p, _l, _p, _p]),
+    "spb_pair_finalize_rows": (_i, [_p, _l, _i, _d, _p, _p, _p, _p]),
     "spb_pair_tables_weighted": (_i, [_p, _p, _l, _i, _p, _p]),
     "spb_pair_transform": (_i, [_p, _i, _p, _p, _p]),
     "spb_subflatten": (_i, [_p, _p, _i, _sp, _p, _p]),

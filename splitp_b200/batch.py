@@ -360,10 +360,15 @@ def _bootstrap_checks(name, replicates, seed):
     if replicates > engine.BOOTSTRAP_MAX_REPLICATES:
         raise ValueError(f"{name}: at most {engine.BOOTSTRAP_MAX_REPLICATES} replicates")
     seed = engine.bootstrap_seed(seed)
+    _one_process(name)
+    return seed
+
+
+def _one_process(name):
+    """NotImplementedError inside a torch.distributed group of several processes: `name` runs on one GPU."""
     import torch.distributed as dist
     if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
         raise NotImplementedError(f"{name} runs on one GPU: call it outside a torch.distributed group of several processes")
-    return seed
 
 
 def bootstrap_scores(alignment, splits, method=Method.flattening, replicates=100, seed=0, taxa=None):
@@ -424,6 +429,14 @@ def _side_mask(side, index, n):
     return m
 
 
+def _split_of_mask(m, taxa):
+    """erickson_SVD's form of the bipartition whose joined side is the bit mask m over the rows of `taxa`."""
+    m, n = int(m), len(taxa)
+    joined = tuple(sorted(taxa[i] for i in range(n) if m >> i & 1))
+    rest = tuple(sorted(taxa[i] for i in range(n) if not m >> i & 1))
+    return tuple(sorted((joined, rest)))
+
+
 def bootstrap_trees(alignment, replicates=100, seed=0, taxa=None, method=Method.subflattening, splits=None):
     """Bootstrap support of the splits of an erickson_SVD tree.  Returns BootstrapTrees(tree, support, replicate_trees):
 
@@ -471,13 +484,7 @@ def bootstrap_trees(alignment, replicates=100, seed=0, taxa=None, method=Method.
     table = ss._count(alignment) if n <= engine.NARROW_MAX_TAXA else ss._count_wide(alignment)
     masks, _ = engine.bootstrap_tree_masks(table, int(replicates), seed, first)
 
-    def split_of(m):
-        m = int(m)
-        joined = tuple(sorted(taxa[i] for i in range(n) if m >> i & 1))
-        rest = tuple(sorted(taxa[i] for i in range(n) if not m >> i & 1))
-        return tuple(sorted((joined, rest)))
-
-    trees = [[split_of(m) for m in row] for row in masks]
+    trees = [[_split_of_mask(m, taxa) for m in row] for row in masks]
     if splits is None:
         wanted = [int(m) for m in masks[0]]
     # a bipartition as the mask of the side without taxon 0: orientation-free
@@ -485,3 +492,143 @@ def bootstrap_trees(alignment, replicates=100, seed=0, taxa=None, method=Method.
     have = [{canon(int(m)) for m in row} for row in masks[1:]]
     support = np.array([sum(canon(w) in h for h in have) / len(have) for w in wanted], dtype=np.float64)
     return BootstrapTrees(trees[0], support, trees[1:])
+
+
+# --------------------------------------------------------------------------------------------
+# site windows
+# --------------------------------------------------------------------------------------------
+def sliding_windows(n_sites, width, step=None):
+    """Every full window [k step, k step + width) of an alignment of n_sites sites, in order: int64 numpy [W, 2] (W = 0 when
+    width > n_sites).  `step` defaults to `width` (adjacent windows)."""
+    step = width if step is None else step
+    for name, v, least in (("n_sites", n_sites, 0), ("width", width, 1), ("step", step, 1)):
+        if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or v < least:
+            raise ValueError(f"sliding_windows: {name} must be an integer >= {least} (got {v!r})")
+    if width > n_sites:
+        return np.zeros((0, 2), np.int64)
+    k = np.arange((int(n_sites) - int(width)) // int(step) + 1, dtype=np.int64) * int(step)
+    return np.stack([k, k + int(width)], axis=1)
+
+
+def _num_sites(alignment):
+    if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
+        return alignment.N
+    if isinstance(alignment, dict):
+        return len(next(iter(alignment.values()))) if alignment else 0
+    return int(alignment.shape[1]) if hasattr(alignment, "shape") else len(alignment[0])
+
+
+def _check_windows(name, windows, n_sites):
+    """`windows` as int64 numpy [W, 2]; ValueError unless it is an integer [W, 2] array-like with 0 <= begin < end <= n_sites."""
+    try:
+        arr = np.asarray(windows)
+    except ValueError as e:  # ragged nested sequences
+        raise ValueError(f"{name}: windows must be an integer [W, 2] array ({e})") from None
+    if arr.size == 0 and (arr.ndim == 1 or (arr.ndim == 2 and arr.shape[1] == 2)):
+        return np.zeros((0, 2), np.int64)
+    if arr.dtype.kind not in "iu":
+        raise ValueError(f"{name}: windows must hold integers (got dtype {arr.dtype})")
+    if arr.ndim != 2 or arr.shape[1] != 2:
+        raise ValueError(f"{name}: windows must have shape [W, 2] (got {list(arr.shape)})")
+    if arr.dtype.kind == "u" and (arr > np.iinfo(np.int64).max).any():
+        raise ValueError(f"{name}: every window needs 0 <= begin < end <= {n_sites}")
+    arr = arr.astype(np.int64)
+    if ((arr[:, 0] < 0) | (arr[:, 1] > n_sites) | (arr[:, 0] >= arr[:, 1])).any():
+        raise ValueError(f"{name}: every window needs 0 <= begin < end <= {n_sites}")
+    return arr
+
+
+def _window_inputs(name, alignment, windows):
+    """(n_taxa, windows as int64 numpy [W, 2]) after the checks both window entry points share."""
+    _one_process(name)
+    n = _num_taxa(alignment)
+    if not 2 <= n <= engine._lib.SPB_MAX_TAXA:
+        raise ValueError(f"{name}: 2 to {engine._lib.SPB_MAX_TAXA} taxa (got {n})")
+    return n, _check_windows(name, windows, _num_sites(alignment))
+
+
+def window_scores(alignment, splits, windows, method=Method.flattening, taxa=None):
+    """Split scores along site windows: numpy float64 [len(windows), len(splits)], row w = the scores `score_splits` gives
+    for the alignment restricted to the sites [windows[w][0], windows[w][1]).
+
+    windows    integer [W, 2] array-like of (begin, end) with 0 <= begin < end <= n_sites, in any order (windows may overlap
+               or repeat; sliding_windows builds the usual scan); anything else raises ValueError before any device work
+    alignment, splits, method, taxa   as in score_splits (2..64 taxa; above 31 taxa Method.flattening and
+               Method.mutual_information need the alignment as characters)
+
+    Method.subflattening packs the alignment once and reads it once: one segment pass cuts it at every window end
+    (spb_pair_tables_segments), each window's pair tables are exact integer sums of its segments (engine.window_tables) and
+    every window is scored by the multi-table scorer; the scores are bitwise those of score_splits on each slice.
+    Method.flattening and Method.mutual_information pack once and count each window's patterns from the packed sites
+    (count_patterns / count_patterns_wide with a site range), then score each table with the scorer score_splits uses.
+
+    A window without usable sites scores what score_splits gives for such a slice: subflattening NaN for splits whose sides
+    both hold at least two taxa and 0.0 for the others (all-zero pair tables); flattening up to 16 taxa the same (empty count
+    flattening), above 16 taxa 0.0; mutual information 0.0.
+    Runs on one GPU: inside a torch.distributed group of several processes it raises NotImplementedError."""
+    n, wins = _window_inputs("window_scores", alignment, windows)
+    if taxa is None and isinstance(alignment, dict):
+        taxa = list(alignment.keys())
+    ss = SplitScorer(splits, taxa, method)  # split positions and subflattening masks, as score_splits builds them
+    idx, W = ss.idx_all, int(wins.shape[0])
+    if W == 0 or not idx:
+        return np.zeros((W, len(idx)), np.float64)
+    if method == Method.subflattening:
+        aln = _as_alignment(alignment, want_sm=False, want_planes=True)
+        return engine.window_subflatten_scores(aln, wins, *ss.masks).cpu().numpy()
+    if n <= engine.NARROW_MAX_TAXA:
+        aln = _as_alignment(alignment, want_sm=True, want_planes=False)
+
+        def table_of(b, e):
+            return engine.count_patterns(aln, b, e)
+    else:
+        if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
+            raise NotImplementedError(f"scores of {n} taxa need the alignment as characters (dict, array or tensor): "
+                                      "the packed forms hold at most 32 taxa per site word")
+        chars, is_ascii, names = _chars(alignment)
+        wide, valid, _, N = engine.pack_wide(chars, is_ascii)
+
+        def table_of(b, e):
+            return engine.count_patterns_wide(wide, valid, n, N, b, e, taxa=names)
+    out = engine._empty((W, len(idx)), torch.float64)
+    scorer = None
+    for w, (b, e) in enumerate(wins.tolist()):
+        tb = table_of(b, e)
+        if method == Method.flattening and uses_sparse_flattening(n):
+            if isinstance(tb, engine.WideTable):  # the table _sparse_table builds above 31 taxa
+                keys, counts = tb.compact()
+                tb = engine.WidePatternTable(n, keys, (counts.to(torch.int64) & 0xFFFFFFFF).to(torch.float64), names)
+            out[w] = engine.sparse_flattening_scores(tb, idx)
+        elif method == Method.flattening:
+            if scorer is None:
+                scorer = engine.CountScorer(tb)
+            else:
+                scorer.table = tb
+            out[w] = scorer.score_many(idx)
+        else:
+            out[w] = engine.rank1_divergence_scores(tb, idx)
+    return out.cpu().numpy()
+
+
+def window_trees(alignment, windows, taxa=None):
+    """erickson_SVD trees along site windows: tree w is the list of n - 2 splits erickson_SVD(..., method=
+    Method.subflattening) chooses for the alignment restricted to the sites [windows[w][0], windows[w][1]), in its format
+    (a sorted 2-tuple of sorted leaf-name tuples per step).
+
+    Every window is agglomerated on the device at once (engine.window_tree_masks): the tables are those of window_scores
+    (Method.subflattening), so every score the agglomeration compares equals the window_scores entry of that split bit for
+    bit, and the candidates are oriented as bootstrap_trees orients them.  `windows` and `alignment` are as in
+    window_scores; leaf names are the dict's keys or `taxa`, else erickson_SVD's default names in row order.  Runs on one
+    GPU: inside a torch.distributed group of several processes it raises NotImplementedError."""
+    n, wins = _window_inputs("window_trees", alignment, windows)
+    if taxa is None:
+        taxa = list(alignment.keys()) if isinstance(alignment, dict) else _default_taxa(n)
+    taxa = list(taxa)
+    if len(taxa) != n or len(set(taxa)) != n:
+        raise ValueError(f"window_trees: taxa must be {n} distinct names, one per row")
+    if wins.shape[0] == 0:
+        return []
+    first = min(range(n), key=lambda i: taxa[i])
+    aln = _as_alignment(alignment, want_sm=False, want_planes=True)
+    masks, _ = engine.window_tree_masks(aln, wins, first)
+    return [[_split_of_mask(m, taxa) for m in row] for row in masks]

@@ -17,94 +17,167 @@ __constant__ int c_H[16] = {1, -1, -1, 1, 1, 1, -1, -1, 1, -1, 1, -1, 1, 1, 1, 1
 constexpr int kPThreads = 256;
 constexpr int kPW = 64;  // plane words per tile (2048 sites)
 
+// The tile body and the flush of pair_kernel, shared with pair_segments_kernel.  They are macros rather than device functions:
+// inlining a function reorders what NVVM hoists out of the tile loop, and pair_kernel's SASS must not change (it is the c3
+// benchmark path).  Both expect in scope: tid, n, npairs, Wpad, planes, valid, Wp, s_mask, s_valid, s_ij, cnt, marg, total.
+//
+// SPB_PAIR_TILE(CUT): one 64-word tile at word wbase, words outside [word_begin, word_end) read as empty; CUT is a statement that
+// may narrow the tile word's valid bits v (of word gw) further.  Per-state masks go to shared memory, then the POPC loop adds
+// the thread's pairs, marginals and usable sites to its counters.
+#define SPB_PAIR_TILE(CUT)                                                                                               \
+  {                                                                                                                      \
+    for (int idx = tid; idx < n * kPW; idx += kPThreads) {                                                               \
+      int j = idx / kPW, w = idx - j * kPW;                                                                              \
+      int64_t gw = wbase + w;                                                                                            \
+      uint32_t lo = 0, hi = 0, v = 0;                                                                                    \
+      if (gw >= word_begin && gw < word_end) {                                                                           \
+        v = __ldg(valid + gw);                                                                                           \
+        CUT                                                                                                              \
+        lo = __ldg(planes + ((int64_t)j * 2) * Wp + gw);                                                                 \
+        hi = __ldg(planes + ((int64_t)j * 2 + 1) * Wp + gw);                                                             \
+      }                                                                                                                  \
+      s_mask[(j * 3 + 0) * Wpad + w] = ~hi & ~lo & v;                                                                    \
+      s_mask[(j * 3 + 1) * Wpad + w] = ~hi & lo & v;                                                                     \
+      s_mask[(j * 3 + 2) * Wpad + w] = hi & ~lo & v;                                                                     \
+      if (j == 0) s_valid[w] = v;                                                                                        \
+    }                                                                                                                    \
+    __syncthreads();                                                                                                     \
+    if (tid < n * 3) {                                                                                                   \
+      const uint32_t* m = s_mask + tid * Wpad;                                                                           \
+      _Pragma("unroll 8") for (int w = 0; w < kPW; ++w) marg += __popc(m[w]);                                            \
+    } else if (tid == kPThreads - 1) {                                                                                   \
+      _Pragma("unroll 8") for (int w = 0; w < kPW; ++w) total += __popc(s_valid[w]);                                     \
+    }                                                                                                                    \
+    _Pragma("unroll") for (int q = 0; q < PPT; ++q) {                                                                    \
+      int p = tid + q * kPThreads;                                                                                       \
+      if (p < npairs) {                                                                                                  \
+        const uint32_t* mi = s_mask + (int)s_ij[2 * p] * 3 * Wpad;                                                       \
+        const uint32_t* mj = s_mask + (int)s_ij[2 * p + 1] * 3 * Wpad;                                                   \
+        _Pragma("unroll 4") for (int w = 0; w < kPW; ++w) {                                                              \
+          uint32_t a0 = mi[w], a1 = mi[Wpad + w], a2 = mi[2 * Wpad + w];                                                 \
+          uint32_t b0 = mj[w], b1 = mj[Wpad + w], b2 = mj[2 * Wpad + w];                                                 \
+          cnt[q][0] += __popc(a0 & b0); cnt[q][1] += __popc(a0 & b1); cnt[q][2] += __popc(a0 & b2);                     \
+          cnt[q][3] += __popc(a1 & b0); cnt[q][4] += __popc(a1 & b1); cnt[q][5] += __popc(a1 & b2);                     \
+          cnt[q][6] += __popc(a2 & b0); cnt[q][7] += __popc(a2 & b1); cnt[q][8] += __popc(a2 & b2);                     \
+        }                                                                                                                \
+      }                                                                                                                  \
+    }                                                                                                                    \
+  }
+
+// SPB_PAIR_FLUSH(RAW): the thread's counters added to the raw row RAW, one 64-bit atomic per non-zero counter.
+#define SPB_PAIR_FLUSH(RAW)                                                                                              \
+  do {                                                                                                                   \
+    _Pragma("unroll") for (int q = 0; q < PPT; ++q) {                                                                    \
+      int p = tid + q * kPThreads;                                                                                       \
+      if (p < npairs) {                                                                                                  \
+        int i = s_ij[2 * p], j = s_ij[2 * p + 1];                                                                        \
+        _Pragma("unroll") for (int e = 0; e < 9; ++e)                                                                    \
+          if (cnt[q][e]) atomicAdd((RAW) + ((int64_t)i * n + j) * 9 + e, (unsigned long long)cnt[q][e]);               \
+      }                                                                                                                  \
+    }                                                                                                                    \
+    if (tid < n * 3 && marg) atomicAdd((RAW) + (int64_t)n * n * 9 + tid, (unsigned long long)marg);                      \
+    if (tid == kPThreads - 1 && total) atomicAdd((RAW) + (int64_t)n * n * 9 + n * 3, (unsigned long long)total);         \
+  } while (0)
+
+// Shared memory of both pair kernels: the per-state masks, the valid words and the (i, j) list of the thread's pairs.
+#define SPB_PAIR_SMEM()                                                                                                  \
+  extern __shared__ uint32_t s_mem[];                                                                                    \
+  const int Wpad = kPW + 1;                                                                                              \
+  uint32_t* s_mask = s_mem;                       /* [n*3][Wpad] */                                                      \
+  uint32_t* s_valid = s_mask + n * 3 * Wpad;      /* [kPW] */                                                            \
+  uint8_t* s_ij = reinterpret_cast<uint8_t*>(s_valid + kPW);  /* [npairs][2] */                                          \
+  const int tid = threadIdx.x;                                                                                           \
+  const int npairs = n * (n - 1) / 2;                                                                                    \
+  for (int p = tid; p < npairs; p += kPThreads) {                                                                        \
+    /* invert p = i*(2n-i-1)/2 + (j-i-1) */                                                                              \
+    int i = 0, rem = p;                                                                                                  \
+    while (rem >= n - 1 - i) { rem -= n - 1 - i; ++i; }                                                                  \
+    s_ij[2 * p] = (uint8_t)i;                                                                                            \
+    s_ij[2 * p + 1] = (uint8_t)(i + 1 + rem);                                                                            \
+  }                                                                                                                      \
+  uint32_t cnt[PPT][9];                                                                                                  \
+  _Pragma("unroll") for (int q = 0; q < PPT; ++q)                                                                        \
+    _Pragma("unroll") for (int e = 0; e < 9; ++e) cnt[q][e] = 0
+
 template <int PPT>
 __global__ void __launch_bounds__(kPThreads) pair_kernel(const uint32_t* __restrict__ planes, const uint32_t* __restrict__ valid,
                                                          int n, int64_t Wp, int64_t word_begin, int64_t word_end,
                                                          unsigned long long* raw) {
-  extern __shared__ uint32_t s_mem[];
-  const int Wpad = kPW + 1;
-  uint32_t* s_mask = s_mem;                       // [n*3][Wpad]
-  uint32_t* s_valid = s_mask + n * 3 * Wpad;      // [kPW]
-  uint8_t* s_ij = reinterpret_cast<uint8_t*>(s_valid + kPW);  // [npairs][2]
-  const int tid = threadIdx.x;
-  const int npairs = n * (n - 1) / 2;
-  for (int p = tid; p < npairs; p += kPThreads) {
-    // invert p = i*(2n-i-1)/2 + (j-i-1)
-    int i = 0, rem = p;
-    while (rem >= n - 1 - i) { rem -= n - 1 - i; ++i; }
-    s_ij[2 * p] = (uint8_t)i;
-    s_ij[2 * p + 1] = (uint8_t)(i + 1 + rem);
-  }
-  uint32_t cnt[PPT][9];
-#pragma unroll
-  for (int q = 0; q < PPT; ++q)
-#pragma unroll
-    for (int e = 0; e < 9; ++e) cnt[q][e] = 0;
+  SPB_PAIR_SMEM();
   uint32_t marg = 0, total = 0;
   const int64_t tile0 = word_begin / kPW, tile1 = (word_end + kPW - 1) / kPW;
   for (int64_t tile = tile0 + blockIdx.x; tile < tile1; tile += gridDim.x) {
     __syncthreads();
     const int64_t wbase = tile * kPW;
-    for (int idx = tid; idx < n * kPW; idx += kPThreads) {
-      int j = idx / kPW, w = idx - j * kPW;
-      int64_t gw = wbase + w;
-      uint32_t lo = 0, hi = 0, v = 0;
-      if (gw >= word_begin && gw < word_end) {
-        v = __ldg(valid + gw);
-        lo = __ldg(planes + ((int64_t)j * 2) * Wp + gw);
-        hi = __ldg(planes + ((int64_t)j * 2 + 1) * Wp + gw);
-      }
-      s_mask[(j * 3 + 0) * Wpad + w] = ~hi & ~lo & v;
-      s_mask[(j * 3 + 1) * Wpad + w] = ~hi & lo & v;
-      s_mask[(j * 3 + 2) * Wpad + w] = hi & ~lo & v;
-      if (j == 0) s_valid[w] = v;
-    }
-    __syncthreads();
-    if (tid < n * 3) {
-      const uint32_t* m = s_mask + tid * Wpad;
-#pragma unroll 8
-      for (int w = 0; w < kPW; ++w) marg += __popc(m[w]);
-    } else if (tid == kPThreads - 1) {
-#pragma unroll 8
-      for (int w = 0; w < kPW; ++w) total += __popc(s_valid[w]);
-    }
-#pragma unroll
-    for (int q = 0; q < PPT; ++q) {
-      int p = tid + q * kPThreads;
-      if (p < npairs) {
-        const uint32_t* mi = s_mask + (int)s_ij[2 * p] * 3 * Wpad;
-        const uint32_t* mj = s_mask + (int)s_ij[2 * p + 1] * 3 * Wpad;
-#pragma unroll 4
-        for (int w = 0; w < kPW; ++w) {
-          uint32_t a0 = mi[w], a1 = mi[Wpad + w], a2 = mi[2 * Wpad + w];
-          uint32_t b0 = mj[w], b1 = mj[Wpad + w], b2 = mj[2 * Wpad + w];
-          cnt[q][0] += __popc(a0 & b0); cnt[q][1] += __popc(a0 & b1); cnt[q][2] += __popc(a0 & b2);
-          cnt[q][3] += __popc(a1 & b0); cnt[q][4] += __popc(a1 & b1); cnt[q][5] += __popc(a1 & b2);
-          cnt[q][6] += __popc(a2 & b0); cnt[q][7] += __popc(a2 & b1); cnt[q][8] += __popc(a2 & b2);
-        }
-      }
-    }
+    SPB_PAIR_TILE()
   }
-  // flush: one 64-bit atomic per counter per CTA
-#pragma unroll
-  for (int q = 0; q < PPT; ++q) {
-    int p = tid + q * kPThreads;
-    if (p < npairs) {
-      int i = s_ij[2 * p], j = s_ij[2 * p + 1];
-#pragma unroll
-      for (int e = 0; e < 9; ++e)
-        if (cnt[q][e]) atomicAdd(raw + ((int64_t)i * n + j) * 9 + e, (unsigned long long)cnt[q][e]);
-    }
-  }
-  if (tid < n * 3 && marg) atomicAdd(raw + (int64_t)n * n * 9 + tid, (unsigned long long)marg);
-  if (tid == kPThreads - 1 && total) atomicAdd(raw + (int64_t)n * n * 9 + n * 3, (unsigned long long)total);
+  SPB_PAIR_FLUSH(raw);  // one 64-bit atomic per counter per CTA
 }
 
+// Pair statistics of the site segments [bounds[s], bounds[s+1]), s < S, into raw rows s (stride raw_words).  The work items
+// are the (segment, tile) pieces of the sites [bounds[0], bounds[S]) in site order; CTA c takes those of a contiguous run of
+// tiles, keeps its counters in registers while a segment lasts and flushes them to the segment's row when it ends (and
+// after its last tile), so a segment costs one flush per CTA it touches.  A tile holding k segment ends is read k + 1 times
+// from shared memory.
+template <int PPT>
+__global__ void __launch_bounds__(kPThreads) pair_segments_kernel(const uint32_t* __restrict__ planes, const uint32_t* __restrict__ valid,
+                                                                  int n, int64_t Wp, const int64_t* __restrict__ bounds, int64_t S,
+                                                                  int64_t raw_words, unsigned long long* raw) {
+  __shared__ int64_t s_seg;
+  SPB_PAIR_SMEM();
+  uint32_t marg = 0, total = 0;
+  const int64_t site0 = bounds[0], site1 = bounds[S];
+  if (site1 <= site0) return;
+  const int64_t tile0 = (site0 >> 5) / kPW, tile1 = (((site1 + 31) >> 5) + kPW - 1) / kPW;
+  const int64_t per = (tile1 - tile0 + gridDim.x - 1) / gridDim.x;
+  const int64_t t_lo = tile0 + (int64_t)blockIdx.x * per;
+  const int64_t t_hi = t_lo + per < tile1 ? t_lo + per : tile1;
+  if (t_lo >= t_hi) return;
+  if (tid == 0) {  // the segment holding the CTA's first site: the smallest s with bounds[s + 1] > that site
+    const int64_t x = t_lo * kPW * 32 > site0 ? t_lo * kPW * 32 : site0;
+    int64_t lo = 0, hi = S - 1;
+    while (lo < hi) {
+      const int64_t mid = (lo + hi) >> 1;
+      if (bounds[mid + 1] > x) hi = mid; else lo = mid + 1;
+    }
+    s_seg = lo;
+  }
+  int64_t seg = -1;
+  for (int64_t tile = t_lo; tile < t_hi; ++tile) {
+    const int64_t wbase = tile * kPW, f0 = wbase * 32, f1 = f0 + kPW * 32;
+    __syncthreads();
+    if (seg < 0) seg = s_seg;
+    while (seg < S) {
+      const int64_t sb = bounds[seg], se = bounds[seg + 1];
+      const int64_t site_begin = sb > f0 ? sb : f0, site_end = se < f1 ? se : f1;
+      if (site_begin < site_end) {
+        const int64_t word_begin = site_begin >> 5, word_end = (site_end + 31) >> 5;
+        SPB_PAIR_TILE({
+          const int64_t f = gw * 32;  // site 32 gw + i is bit i of word gw
+          if (site_begin > f) v &= ~0u << (int)(site_begin - f);
+          if (site_end < f + 32) v &= (1u << (int)(site_end - f)) - 1u;
+        })
+      }
+      if (se > f1) break;  // the segment goes on into the next tile
+      SPB_PAIR_FLUSH(raw + seg * raw_words);
+      _Pragma("unroll") for (int q = 0; q < PPT; ++q)
+        _Pragma("unroll") for (int e = 0; e < 9; ++e) cnt[q][e] = 0;
+      marg = 0;
+      total = 0;
+      ++seg;
+      __syncthreads();  // the next segment's tile overwrites the masks
+    }
+  }
+  if (seg < S) SPB_PAIR_FLUSH(raw + seg * raw_words);
+}
+
+#undef SPB_PAIR_SMEM
+#undef SPB_PAIR_FLUSH
+#undef SPB_PAIR_TILE
+
 // raw pair statistics -> full joint tables N[i][j][4][4] and T = H N H^T, one thread per ordered (i, j)
-__global__ void finalize_kernel(const unsigned long long* __restrict__ raw, int n, double divisor, double* Nout, double* Tout,
-                                double* total_out) {
-  int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= n * n) return;
+__device__ __forceinline__ void finalize_pair(const unsigned long long* __restrict__ raw, int n, double divisor, double* Nout, double* Tout,
+                                              double* total_out, int idx) {
   int i = idx / n, j = idx - i * n;
   const unsigned long long* marg = raw + (int64_t)n * n * 9;
   long long tot = (long long)marg[n * 3];
@@ -151,6 +224,23 @@ __global__ void finalize_kernel(const unsigned long long* __restrict__ raw, int 
     }
   }
   if (idx == 0 && total_out) *total_out = divisor > 0.0 ? (double)tot / divisor : (double)tot;
+}
+
+__global__ void finalize_kernel(const unsigned long long* __restrict__ raw, int n, double divisor, double* Nout, double* Tout,
+                                double* total_out) {
+  int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n * n) return;
+  finalize_pair(raw, n, divisor, Nout, Tout, total_out, idx);
+}
+
+// finalize_kernel of raw row blockIdx.y (stride raw_words) into T / N row blockIdx.y (n^2 16 doubles) and total_out[blockIdx.y].
+__global__ void finalize_rows_kernel(const unsigned long long* __restrict__ raw, int64_t raw_words, int n, double divisor, double* Nout,
+                                     double* Tout, double* total_out) {
+  int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n * n) return;
+  const int64_t r = blockIdx.y, cells = (int64_t)n * n * 16;
+  finalize_pair(raw + r * raw_words, n, divisor, Nout ? Nout + r * cells : nullptr, Tout + r * cells, total_out ? total_out + r : nullptr,
+                idx);
 }
 
 __global__ void weighted_kernel(const uint64_t* __restrict__ keys, const double* __restrict__ vals, int64_t num, int n,
@@ -879,6 +969,52 @@ extern "C" int spb_pair_finalize(const uint64_t* d_raw, int n_taxa, double divis
   finalize_kernel<<<(nn + 127) / 128, 128, 0, (cudaStream_t)stream>>>((const unsigned long long*)d_raw, n_taxa, divisor, d_N, d_T,
                                                                      d_total);
   SPB_LAUNCH_CHECK();
+  return SPB_OK;
+}
+
+extern "C" int spb_pair_tables_segments(const uint32_t* d_planes, const uint32_t* d_valid, int n_taxa, int64_t plane_words,
+                                        const int64_t* d_bounds, int64_t n_segments, uint64_t* d_raw, void* stream) {
+  SPB_REQUIRE(d_planes && d_valid && d_bounds && d_raw, "spb_pair_tables_segments: NULL buffer");
+  SPB_REQUIRE(n_taxa >= 1 && n_taxa <= SPB_MAX_TAXA, "spb_pair_tables_segments: n_taxa out of range");
+  SPB_REQUIRE(plane_words >= 0 && n_segments >= 0, "spb_pair_tables_segments: bad sizes");
+  if (n_segments == 0 || plane_words == 0) return SPB_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  int npairs = n_taxa * (n_taxa - 1) / 2;
+  size_t smem = ((size_t)n_taxa * 3 * (kPW + 1) + kPW) * 4 + (size_t)(npairs > 0 ? npairs : 1) * 2 + 16;
+  int64_t grid = (int64_t)sm_count() * 2;  // as spb_pair_tables; the CTAs split the tiles of [bounds[0], bounds[S]) into runs
+  const int64_t tiles = (plane_words + kPW - 1) / kPW;
+  if (grid > tiles) grid = tiles;
+  const int64_t raw_words = spb_pair_raw_words(n_taxa);
+#define SPB_SEG_LAUNCH(PPT)                                                                                            \
+  do {                                                                                                                 \
+    SPB_CUDA(cudaFuncSetAttribute(pair_segments_kernel<PPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    pair_segments_kernel<PPT><<<(unsigned)grid, kPThreads, smem, st>>>(d_planes, d_valid, n_taxa, plane_words, d_bounds,  \
+                                                                       n_segments, raw_words, (unsigned long long*)d_raw); \
+  } while (0)
+  if (npairs <= kPThreads) SPB_SEG_LAUNCH(1);
+  else if (npairs <= 2 * kPThreads) SPB_SEG_LAUNCH(2);
+  else if (npairs <= 4 * kPThreads) SPB_SEG_LAUNCH(4);
+  else SPB_SEG_LAUNCH(8);
+#undef SPB_SEG_LAUNCH
+  SPB_LAUNCH_CHECK();
+  return SPB_OK;
+}
+
+extern "C" int spb_pair_finalize_rows(const uint64_t* d_raw, int64_t rows, int n_taxa, double divisor, double* d_N, double* d_T,
+                                      double* d_total, void* stream) {
+  SPB_REQUIRE(n_taxa >= 1 && n_taxa <= SPB_MAX_TAXA && rows >= 0, "spb_pair_finalize_rows: bad arguments");
+  if (rows == 0) return SPB_OK;
+  SPB_REQUIRE(d_raw && d_T, "spb_pair_finalize_rows: NULL buffer");
+  const int nn = n_taxa * n_taxa;
+  const int64_t raw_words = spb_pair_raw_words(n_taxa), cells = (int64_t)nn * 16;
+  for (int64_t r0 = 0; r0 < rows; r0 += 65535) {  // gridDim.y <= 65535
+    const int64_t r = rows - r0 < 65535 ? rows - r0 : 65535;
+    dim3 grid((nn + 127) / 128, (unsigned)r);
+    finalize_rows_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>((const unsigned long long*)d_raw + r0 * raw_words, raw_words, n_taxa,
+                                                                 divisor, d_N ? d_N + r0 * cells : nullptr, d_T + r0 * cells,
+                                                                 d_total ? d_total + r0 : nullptr);
+    SPB_LAUNCH_CHECK();
+  }
   return SPB_OK;
 }
 

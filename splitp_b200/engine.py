@@ -1220,6 +1220,29 @@ def pair_finalize(raw, n, divisor=0.0):
     return PairTables(n, N_tab, T, total)
 
 
+def pair_raw_segments(aln, bounds):
+    """Raw pair statistics of the site segments [bounds[s], bounds[s + 1]) in one pass over the planes
+    (spb_pair_tables_segments): int64 [S, spb_pair_raw_words(n)], row s bitwise pair_raw of an alignment made of exactly those
+    sites.  bounds: S + 1 ascending site indices in [0, N]; empty segments are allowed."""
+    if aln.planes is None:
+        raise ValueError("pair tables need the taxon-major bit planes (pack(want_planes=True))")
+    b = np.asarray(bounds, dtype=np.int64).reshape(-1)
+    if b.shape[0] < 1 or b[0] < 0 or b[-1] > aln.N or (np.diff(b) < 0).any():
+        raise ValueError(f"pair_raw_segments: bounds must be ascending site indices in [0, {aln.N}]")
+    S = b.shape[0] - 1
+    raw = _zeros((S, int(lib.spb_pair_raw_words(aln.n))), torch.int64)
+    if S:
+        d_b = torch.from_numpy(b).to(device())
+        call("spb_pair_tables_segments", _p(aln.planes), _p(aln.valid), aln.n, aln.plane_words, _p(d_b), S, _p(raw), _st())
+    return raw
+
+
+def pair_finalize_rows(raw, n, divisor, T, total):
+    """spb_pair_finalize of every row of raw (int64 [R, words]) into T (float64, R n^2 16 contiguous) and total (float64 [R])
+    in one launch; divisor < 0 divides each row by its own usable sites."""
+    call("spb_pair_finalize_rows", _p(raw), int(raw.shape[0]), n, float(divisor), None, _p(T), _p(total), _st())
+
+
 def pair_tables_from_alignment(aln, as_counts=False):
     raw = pair_raw(aln)
     usable = 0.0 if as_counts else float(int(raw[-1].item()))
@@ -1303,6 +1326,17 @@ class SubflattenTables:
         pt = pair_tables_from_table(table, as_counts=True, total=total)
         # no splits: the call only tabulates the triple tables of pt into slot i
         call("spb_subflatten_score_tables", _p(pt.T), _p(pt.total), n, None, None, 0, None, _p(self.data[i]), 0, _st())
+
+    def add_pair_tables(self, i, T, total):
+        """Fills slot i from finalized pair tables: T float64 [n, n, 4, 4] and total float64 [1] on the device."""
+        n, slot = self.n, self.total[i:i + 1]
+        if total.data_ptr() != slot.data_ptr():
+            slot.copy_(total)
+        if n > SUBFLATTEN_TABLES_MAX_TAXA:
+            if T.data_ptr() != self.data[i].data_ptr():
+                self.data[i].view(n, n, 4, 4).copy_(T)
+            return
+        call("spb_subflatten_score_tables", _p(T), _p(total), n, None, None, 0, None, _p(self.data[i]), 0, _st())
 
 
 def subflatten_scores_multi(tables, masks_a, masks_b, per_table):
@@ -1854,3 +1888,90 @@ def bootstrap_tree_masks(table, replicates, seed, first_taxon, timer=None):
         scores.append(sc)
         del stack
     return torch.cat(masks).cpu().numpy().view(np.uint64), torch.cat(scores).cpu().numpy()
+
+
+# --------------------------------------------------------------------------------------------
+# site windows: pair tables of many windows from one segment pass (spb_pair_tables_segments)
+# --------------------------------------------------------------------------------------------
+WINDOW_BATCH_BYTES = 2 << 30  # device memory of one window group: segment rows and prefix sums, stacked tables, scores
+
+
+def _window_bytes(n, extra):
+    """Device bytes of one window in a group: two segment rows and their prefix sums, the window's raw row, its pair
+    tables (staged separately below 44 taxa), its slot of SubflattenTables, plus `extra`."""
+    words = int(lib.spb_pair_raw_words(n))
+    staged = 0 if n > SUBFLATTEN_TABLES_MAX_TAXA else 128 * n * n
+    return 8 * words * 5 + staged + SubflattenTables.bytes_per_table(n) + extra
+
+
+def _window_groups(windows, per_window):
+    """Row indices of `windows` (int64 [W, 2]) in (begin, end) order, cut into groups of at most WINDOW_BATCH_BYTES: the
+    windows of a group span few sites, so their segment pass reads little more than the sites they cover."""
+    order = np.lexsort((windows[:, 1], windows[:, 0]))
+    g = max(1, min(len(order), WINDOW_BATCH_BYTES // per_window))
+    for k in range(0, len(order), g):
+        yield order[k:k + g]
+
+
+def window_tables(aln, windows):
+    """SubflattenTables of the windows (int64 numpy [g, 2], 0 <= begin < end <= N): slot w holds the pair tables of sites
+    [begin_w, end_w) divided by that window's own usable sites (divisor -1), bitwise the tables score_splits builds for the
+    alignment restricted to those sites.  The alignment is cut at every distinct window end (one segment pass); a window's
+    raw statistics are the exact int64 difference of two prefix sums over the segments."""
+    n, g = aln.n, int(windows.shape[0])
+    ends = np.unique(windows.reshape(-1))
+    raw = pair_raw_segments(aln, ends)
+    prefix = torch.cat([_zeros((1, raw.shape[1]), torch.int64), torch.cumsum(raw, 0)])
+    del raw
+    lo = torch.from_numpy(np.searchsorted(ends, windows[:, 0])).to(device())
+    hi = torch.from_numpy(np.searchsorted(ends, windows[:, 1])).to(device())
+    wraw = (prefix[hi] - prefix[lo]).contiguous()
+    del prefix
+    stack = SubflattenTables(n, g)
+    staged = n <= SUBFLATTEN_TABLES_MAX_TAXA  # the triple tables are formed from T
+    T = _empty((g, 16 * n * n), torch.float64) if staged else stack.data
+    pair_finalize_rows(wraw, n, -1.0, T, stack.total)
+    if staged:
+        for w in range(g):
+            stack.add_pair_tables(w, T[w].view(n, n, 4, 4), stack.total[w:w + 1])
+    return stack
+
+
+def window_subflatten_scores(aln, windows, masks_a, masks_b):
+    """Subflattening scores of every split in every window: float64 [W, S] on the device, row w bitwise
+    subflatten_scores(pair_finalize(pair_raw(alignment of sites [begin_w, end_w)), n, -1), masks).  masks: int64 device
+    tensors of uint64 bit masks, as subflatten_scores takes them.  Windows run in groups (WINDOW_BATCH_BYTES)."""
+    S = int(masks_a.shape[0])
+    out = _empty((int(windows.shape[0]), S), torch.float64)
+    if S == 0:
+        return out
+    for rows in _window_groups(windows, _window_bytes(aln.n, 24 * S)):
+        g = len(rows)
+        stack = window_tables(aln, windows[rows])
+        sc = subflatten_scores_multi(stack, masks_a.repeat(g), masks_b.repeat(g), S)
+        out[torch.from_numpy(rows).to(device())] = sc.view(g, S)
+        del stack
+    return out
+
+
+def window_tree_masks(aln, windows, first_taxon, timer=None):
+    """erickson_SVD(Method.subflattening) agglomerations of the windows (int64 numpy [W, 2]) in lockstep: (joined-side
+    masks as numpy uint64, scores as numpy float64), both [W, n - 2].  Window w is scored against the tables of
+    window_tables, so every score equals window_subflatten_scores for that split; candidates are oriented towards
+    `first_taxon` (erickson_lockstep).  `timer` (PhaseTimer) gets the spans "tables", "score" and "step"."""
+    n, W = aln.n, int(windows.shape[0])
+    steps = max(n - 2, 0)
+    if steps == 0 or W == 0:
+        return np.zeros((W, steps), np.uint64), np.zeros((W, steps), np.float64)
+    p0 = n * (n - 1) // 2
+    masks, scores = _empty((W, steps), torch.int64), _empty((W, steps), torch.float64)
+    per = _window_bytes(n, int(lib.spb_agglomerate_ws_bytes(n, 1)) + 24 * p0 + 16 * steps)
+    for rows in _window_groups(windows, per):
+        with _span(timer, "tables"):
+            stack = window_tables(aln, windows[rows])
+        m, sc = erickson_lockstep(n, len(rows), first_taxon,
+                                  lambda ma, mb, per_table: subflatten_scores_multi(stack, ma, mb, per_table), timer)
+        idx = torch.from_numpy(rows).to(device())
+        masks[idx], scores[idx] = m, sc
+        del stack
+    return masks.cpu().numpy().view(np.uint64), scores.cpu().numpy()
