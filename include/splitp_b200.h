@@ -243,6 +243,13 @@ int spb_pair_finalize_rows(const uint64_t* d_raw, int64_t rows, int n_taxa, doub
 /* Same tables from a weighted pattern list (dict inputs): d_N must be zeroed by the caller. */
 int spb_pair_tables_weighted(const uint64_t* d_keys, const double* d_vals, int64_t num, int n_taxa,
                              double* d_N, void* stream);
+/* Same tables for `rows` count rows over one sorted pattern list, in one launch (pair_rows.cu): d_N double
+ * [rows][n][n][4][4] (written in full), row r bitwise what spb_pair_tables_weighted (n <= 31) / spb_pair_tables_wide
+ * (n >= 32) give for the keys with values (double) d_counts[r][p].  d_keys: uint64 [num] up to 31 taxa, {lo, hi} [num][2]
+ * (16-byte aligned) above; d_counts: uint32 [rows][num], as spb_bootstrap_counts writes them, zeros allowed.  Every row
+ * must sum to less than 2^32: the sums are then exact integers and do not depend on scheduling.  n_taxa 2..64. */
+int spb_pair_tables_count_rows(const uint64_t* d_keys, const uint32_t* d_counts, int64_t rows, int64_t num, int n_taxa,
+                               double* d_N, void* stream);
 int spb_pair_transform(const double* d_N, int n_taxa, double* d_T, double* d_total, void* stream);
 /* One subflattening matrix, row-major double [(3a+1)][(3b+1)]. */
 int spb_subflatten(const double* d_T, const double* d_total, int n_taxa, const spb_split* split, double* d_out,

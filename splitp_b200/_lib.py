@@ -111,6 +111,7 @@ PROTOTYPES = {
     "spb_pair_tables_segments": (_i, [_p, _p, _i, _l, _p, _l, _p, _p]),
     "spb_pair_finalize_rows": (_i, [_p, _l, _i, _d, _p, _p, _p, _p]),
     "spb_pair_tables_weighted": (_i, [_p, _p, _l, _i, _p, _p]),
+    "spb_pair_tables_count_rows": (_i, [_p, _p, _l, _l, _i, _p, _p]),
     "spb_pair_transform": (_i, [_p, _i, _p, _p, _p]),
     "spb_subflatten": (_i, [_p, _p, _i, _sp, _p, _p]),
     "spb_subflatten_score": (_i, [_p, _p, _i, _p, _p, _l, _p, _p]),

@@ -420,13 +420,34 @@ def _default_taxa(n):
     return [str(np.base_repr(i, base=max(i + 1, 2))) if n <= 36 else f"t{i}" for i in range(n)]
 
 
-def _side_mask(side, index, n):
+def _side_mask(side, index, fn):
     m = 0
     for name in side:
         if name not in index:
-            raise ValueError(f"bootstrap_trees: unknown leaf {name!r} in a split")
+            raise ValueError(f"{fn}: unknown leaf {name!r} in a split")
         m |= 1 << index[name]
     return m
+
+
+def _tree_taxa(fn, alignment, n, taxa, splits):
+    """(leaf names, joined-side masks of `splits` or None) after the taxa and splits checks of the bootstrap tree entry
+    points; `fn` names the entry point in the messages."""
+    if taxa is None:
+        taxa = list(alignment.keys()) if isinstance(alignment, dict) else _default_taxa(n)
+    taxa = list(taxa)
+    if len(taxa) != n or len(set(taxa)) != n:
+        raise ValueError(f"{fn}: taxa must be {n} distinct names, one per row")
+    if splits is None:
+        return taxa, None
+    index = {t: i for i, t in enumerate(taxa)}
+    full = (1 << n) - 1
+    wanted = []
+    for side_a, side_b in splits:
+        ma, mb = _side_mask(side_a, index, fn), _side_mask(side_b, index, fn)
+        if ma & mb or ma | mb != full or len(side_a) + len(side_b) != n:
+            raise ValueError(f"{fn}: every split must place every taxon on exactly one side")
+        wanted.append(ma)
+    return taxa, wanted
 
 
 def _split_of_mask(m, taxa):
@@ -435,6 +456,30 @@ def _split_of_mask(m, taxa):
     joined = tuple(sorted(taxa[i] for i in range(n) if m >> i & 1))
     rest = tuple(sorted(taxa[i] for i in range(n) if not m >> i & 1))
     return tuple(sorted((joined, rest)))
+
+
+def _trees_of_masks(masks, taxa):
+    """erickson_SVD's format of every row of joined-side masks (numpy uint64 [..., n - 2]): nested lists of splits.  Each
+    distinct mask is converted once: replicate trees share most of their splits."""
+    memo = {}
+
+    def split(m):
+        s = memo.get(m)
+        if s is None:
+            s = memo[m] = _split_of_mask(m, taxa)
+        return s
+    return [[split(m) for m in row] for row in masks.reshape(int(np.prod(masks.shape[:-1])), masks.shape[-1]).tolist()]
+
+
+def _support(masks, wanted, n):
+    """Fraction of the trees masks[1:] (numpy uint64 [B + 1, n - 2] joined-side masks) that contain each bipartition of
+    `wanted` (masks; default: the splits of tree 0), orientation ignored: numpy float64."""
+    full = np.uint64((1 << n) - 1)
+    canon = lambda m: np.where(m & np.uint64(1), full & ~m, m)  # noqa: E731  the side without taxon 0: orientation-free
+    want = canon(masks[0] if wanted is None else np.array(wanted, dtype=np.uint64))
+    have = canon(masks[1:])
+    hits = (have[:, :, None] == want[None, None, :]).any(axis=1).sum(axis=0)
+    return hits / have.shape[0]
 
 
 def bootstrap_trees(alignment, replicates=100, seed=0, taxa=None, method=Method.subflattening, splits=None):
@@ -465,33 +510,13 @@ def bootstrap_trees(alignment, replicates=100, seed=0, taxa=None, method=Method.
     n = _num_taxa(alignment)
     if not 2 <= n <= engine._lib.SPB_MAX_TAXA:
         raise ValueError(f"bootstrap_trees: 2 to {engine._lib.SPB_MAX_TAXA} taxa (got {n})")
-    if taxa is None:
-        taxa = list(alignment.keys()) if isinstance(alignment, dict) else _default_taxa(n)
-    taxa = list(taxa)
-    if len(taxa) != n or len(set(taxa)) != n:
-        raise ValueError(f"bootstrap_trees: taxa must be {n} distinct names, one per row")
-    index = {t: i for i, t in enumerate(taxa)}
-    full = (1 << n) - 1
-    if splits is not None:
-        wanted = []
-        for side_a, side_b in splits:
-            ma, mb = _side_mask(side_a, index, n), _side_mask(side_b, index, n)
-            if ma & mb or ma | mb != full or len(side_a) + len(side_b) != n:
-                raise ValueError("bootstrap_trees: every split must place every taxon on exactly one side")
-            wanted.append(ma)
+    taxa, wanted = _tree_taxa("bootstrap_trees", alignment, n, taxa, splits)
     first = min(range(n), key=lambda i: taxa[i])
     ss = SplitScorer([], taxa, Method.subflattening)  # the counting stage of bootstrap_scores: the same replicate tables
     table = ss._count(alignment) if n <= engine.NARROW_MAX_TAXA else ss._count_wide(alignment)
     masks, _ = engine.bootstrap_tree_masks(table, int(replicates), seed, first)
-
-    trees = [[_split_of_mask(m, taxa) for m in row] for row in masks]
-    if splits is None:
-        wanted = [int(m) for m in masks[0]]
-    # a bipartition as the mask of the side without taxon 0: orientation-free
-    canon = lambda m: m if not m & 1 else full & ~m  # noqa: E731
-    have = [{canon(int(m)) for m in row} for row in masks[1:]]
-    support = np.array([sum(canon(w) in h for h in have) / len(have) for w in wanted], dtype=np.float64)
-    return BootstrapTrees(trees[0], support, trees[1:])
+    trees = _trees_of_masks(masks, taxa)
+    return BootstrapTrees(trees[0], _support(masks, wanted, n), trees[1:])
 
 
 # --------------------------------------------------------------------------------------------
@@ -632,3 +657,57 @@ def window_trees(alignment, windows, taxa=None):
     aln = _as_alignment(alignment, want_sm=False, want_planes=True)
     masks, _ = engine.window_tree_masks(aln, wins, first)
     return [[_split_of_mask(m, taxa) for m in row] for row in masks]
+
+
+def window_bootstrap_trees(alignment, windows, replicates=100, seed=0, taxa=None, splits=None):
+    """Bootstrap support of erickson_SVD trees along site windows (a bootscan): a list with one BootstrapTrees(tree,
+    support, replicate_trees) per window, in the order of `windows`.  Entry w equals
+
+        bootstrap_trees(<alignment restricted to the sites [b_w, e_w)>, replicates,
+                        seed=engine.window_bootstrap_seed(seed, b_w, e_w), taxa=taxa, splits=splits)
+
+    exactly (trees, replicate trees and support): a window's replicates depend on `seed` and its bounds only, so a
+    repeated window gives equal entries and a window's entry does not depend on the other windows.
+
+    The alignment is packed once (as window_scores packs it for flattening) and every window is counted from the packed
+    sites.  All windows then go to engine.bootstrap_tree_masks_multi: each window's own counts and its replicates' counts
+    become pair tables, in one launch per window up to engine.COUNT_ROWS_MAX_TAXA taxa (spb_pair_tables_count_rows) and
+    through spb_pair_tables_wide per compacted row above, and every tree of every window is agglomerated in lockstep.
+    Support is computed from the split masks.
+
+    `windows` is as in window_scores; `alignment`, `replicates`, `seed`, `taxa` and `splits` as in bootstrap_trees (2..64
+    taxa; above 31 taxa the alignment must be given as characters).  A window without a usable site raises ValueError.
+    Runs on one GPU: inside a torch.distributed group of several processes it raises NotImplementedError."""
+    fn = "window_bootstrap_trees"
+    n, wins = _window_inputs(fn, alignment, windows)
+    seed = _bootstrap_checks(fn, replicates, seed)
+    taxa, wanted = _tree_taxa(fn, alignment, n, taxa, splits)
+    if wins.shape[0] == 0:
+        return []
+    if n <= engine.NARROW_MAX_TAXA:
+        aln = _as_alignment(alignment, want_sm=True, want_planes=False)
+
+        def table_of(b, e):
+            return engine.count_patterns(aln, b, e)
+    else:
+        if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
+            raise NotImplementedError(f"{fn} of {n} taxa needs the alignment as characters (dict, array or tensor): "
+                                      "the packed forms hold at most 32 taxa per site word")
+        chars, is_ascii, names = _chars(alignment)
+        wide, valid, _, N = engine.pack_wide(chars, is_ascii)
+
+        def table_of(b, e):
+            return engine.count_patterns_wide(wide, valid, n, N, b, e, taxa=names)
+    tables = []
+    for w, (b, e) in enumerate(wins.tolist()):
+        tables.append(table_of(b, e))
+        if tables[-1].divisor == 0:
+            raise ValueError(f"{fn}: window {w} [{b}, {e}) has no usable site")
+    seeds = [engine.window_bootstrap_seed(seed, b, e) for b, e in wins.tolist()]
+    first = min(range(n), key=lambda i: taxa[i])
+    masks, _ = engine.bootstrap_tree_masks_multi(tables, int(replicates), seeds, first)
+    del tables
+    trees = _trees_of_masks(masks, taxa)
+    per = masks.shape[1]
+    return [BootstrapTrees(trees[w * per], _support(masks[w], wanted, n), trees[w * per + 1:(w + 1) * per])
+            for w in range(masks.shape[0])]

@@ -1852,42 +1852,178 @@ def _table_of_counts(table, keys, counts, N):
 BOOTSTRAP_TREES_BATCH_BYTES = 4 << 30  # device memory of one lockstep group: stacked scoring tables, candidates, state
 
 
+# Taxon counts up to which bootstrap_group_tables builds pair tables with spb_pair_tables_count_rows; above, each row is
+# compacted and goes through the DMMA spb_pair_tables_wide.  profiles/r9_window_bootstrap_timing.json ("routes_by_taxa":
+# 101 count rows of 10^5 simulated sites, NVIDIA B200 at a 1,000 W power limit): the count-row kernel takes 4.9 / 8.5 /
+# 12.2 ms at 32 / 40 / 48 taxa against 18.0 / 18.4 / 18.7 ms for the DMMA launches alone, and 18.8 / 19.6 ms at 56 / 64
+# taxa against 18.6 / 19.2 ms.  With 21 rows at 64 taxa it takes 5.4 ms against 4.0 ms ("t64_b20", window 0).
+COUNT_ROWS_MAX_TAXA = 48
+
+
+def pair_tables_count_rows(keys, rows, n):
+    """Joint pair tables of count rows over one sorted pattern list (spb_pair_tables_count_rows): float64 [R, n, n, 4, 4],
+    row r bitwise the N of pair_tables_from_table for the keys with values rows[r] (uint32 counts in an int32 [R, P]
+    tensor; each row sums to less than 2^32)."""
+    R, P = int(rows.shape[0]), int(rows.shape[1])
+    N_tab = _empty((R, n, n, 4, 4), torch.float64)
+    call("spb_pair_tables_count_rows", _p(keys), _p(rows), R, P, n, _p(N_tab), _st())
+    return N_tab
+
+
+def _pair_tables_compacted_rows(keys, rows, n):
+    """pair_tables_count_rows through spb_pair_tables_wide on each row's non-zero patterns (spb_bootstrap_compact), as
+    pair_tables_from_table builds them for a bootstrap_tables table: bitwise the same tables, for 32..64 taxa."""
+    R, P = int(rows.shape[0]), int(rows.shape[1])
+    cap = R * P
+    ok, oc, off = _empty((max(cap, 1), 2), torch.int64), _empty(max(cap, 1), torch.int32), _empty(R + 1, torch.int64)
+    ws = _empty(int(lib.spb_bootstrap_compact_ws(P, R)), torch.int64)
+    call("spb_bootstrap_compact", _p(rows), _p(keys), 2, P, R, _p(ok), _p(oc), cap, _p(off), _p(ws), _st())
+    del ws
+    off = off.cpu().tolist()
+    N_tab = _empty((R, n, n, 4, 4), torch.float64)
+    for r in range(R):
+        num = off[r + 1] - off[r]
+        vals = (oc[off[r]:off[r + 1]].to(torch.int64) & 0xFFFFFFFF).to(torch.float64)
+        ws = _empty(max(int(lib.spb_pair_tables_wide_ws(num, n)), 1), torch.float64)
+        call("spb_pair_tables_wide", _p(ok[off[r]:off[r + 1]]), _p(vals), num, n, _p(N_tab[r]), _p(ws), _st())
+    return N_tab
+
+
+def bootstrap_sources(tables, seeds):
+    """(keys, counts, prefix, N, seed) of every table of pattern counts (see _counted) with its seed: what
+    bootstrap_group_tables reads.  ValueError for a table without usable sites."""
+    if len(seeds) != len(tables):
+        raise ValueError("bootstrap_sources: one seed per table")
+    srcs = []
+    for t, seed in zip(tables, seeds):
+        keys, counts = _counted(t)
+        prefix, N = _bootstrap_prefix(counts)
+        srcs.append((keys, counts, prefix, N, bootstrap_seed(seed)))
+    return srcs
+
+
+def _bootstrap_rows(src, b0, b1):
+    """Count rows b0 .. b1 - 1 of a bootstrap source (bootstrap_sources): row 0 is the source's own counts, row b + 1
+    replicate b (int32 [b1 - b0, P] holding uint32 counts)."""
+    keys, counts, prefix, N, seed = src
+    P = int(counts.shape[0])
+    rows = _empty((b1 - b0, P), torch.int32)
+    r0 = 0
+    if b0 == 0:
+        rows[0].copy_(counts)
+        r0 = 1
+    first, c = b0 + r0 - 1, b1 - b0 - r0
+    if c:
+        call("spb_bootstrap_counts", _p(prefix), P, N, seed, first, c, _p(rows[r0:]), _st())
+    return rows
+
+
+def bootstrap_group_tables(srcs, count, f0, f1, n, timer=None):
+    """SubflattenTables of the rows f0 .. f1 - 1 of the sources (bootstrap_sources), `count` rows per source: row
+    s count + b is source s's own counts (b = 0) or its replicate b - 1.  Slot i holds what SubflattenTables.add gives
+    for that table (bootstrap_tables' replicate table), bit for bit.  Up to COUNT_ROWS_MAX_TAXA taxa a source's count rows
+    go through spb_pair_tables_count_rows in one launch, above through spb_pair_tables_wide per compacted row; then
+    spb_pair_transform and the triple tables per row."""
+    staged = n <= SUBFLATTEN_TABLES_MAX_TAXA  # the triple tables are formed from T
+    stack = SubflattenTables(n, f1 - f0)
+    for s in range(f0 // count, (f1 - 1) // count + 1):
+        b0, b1 = max(f0, s * count) - s * count, min(f1, (s + 1) * count) - s * count
+        slot0 = s * count + b0 - f0
+        with _span(timer, "resample"):
+            rows = _bootstrap_rows(srcs[s], b0, b1)
+        with _span(timer, "tables"):
+            with _span(timer, "pair tables"):
+                if n <= COUNT_ROWS_MAX_TAXA:
+                    N_tab = pair_tables_count_rows(srcs[s][0], rows, n)
+                else:
+                    N_tab = _pair_tables_compacted_rows(srcs[s][0], rows, n)
+            del rows
+            with _span(timer, "triple tables"):
+                T = _empty((n, n, 4, 4), torch.float64) if staged else None
+                for r in range(b1 - b0):
+                    i = slot0 + r
+                    out = T if staged else stack.data[i]
+                    call("spb_pair_transform", _p(N_tab[r]), n, _p(out), _p(stack.total[i:i + 1]), _st())
+                    if staged:  # no splits: the call only tabulates the triple tables of T into slot i
+                        call("spb_subflatten_score_tables", _p(T), _p(stack.total[i:i + 1]), n, None, None, 0, None,
+                             _p(stack.data[i]), 0, _st())
+            del N_tab, T
+    return stack
+
+
+def bootstrap_row_bytes(n, P_max):
+    """Device bytes of one row of a lockstep group of bootstrap_tree_masks_multi, for sources of at most P_max patterns:
+    its scoring tables, agglomeration state and candidates, its pair tables N and T, its count row and (above
+    COUNT_ROWS_MAX_TAXA taxa) its compacted keys and counts."""
+    p0, steps = n * (n - 1) // 2, max(n - 2, 0)
+    return (SubflattenTables.bytes_per_table(n) + int(lib.spb_agglomerate_ws_bytes(n, 1)) + 24 * p0 + 16 * steps
+            + 256 * n * n + 4 * P_max + (20 * P_max if n > COUNT_ROWS_MAX_TAXA else 0))
+
+
+def bootstrap_tree_masks_multi(tables, replicates, seeds, first_taxon, timer=None):
+    """erickson_SVD(Method.subflattening) agglomerations of several tables of pattern counts (see _counted; all of n taxa)
+    and of their bootstrap replicates, in lockstep: (joined-side masks as numpy uint64, scores as numpy float64), both
+    [len(tables), replicates + 1, n - 2].  Row [s, 0] is table s itself, row [s, b + 1] its replicate b with seed
+    seeds[s] (the replicate bootstrap_counts / bootstrap_tables give).
+
+    Every table is scored from the pair tables of its integer counts (bootstrap_group_tables) with candidates oriented
+    towards `first_taxon` (erickson_lockstep).  Rows run in lockstep groups of at most BOOTSTRAP_TREES_BATCH_BYTES of device
+    memory; a row depends on its table, its seed and its replicate index only, never on grouping.  `timer` (PhaseTimer)
+    gets the spans "resample" (replicate counts), "pair tables" (pair tables N), "triple tables" (transform +
+    triple tables), "tables" (both of those), "score" and "step"."""
+    seeds = [bootstrap_seed(s) for s in seeds]
+    replicates = int(replicates)
+    _check_replicates(0, replicates)
+    srcs = bootstrap_sources(tables, seeds)
+    S = len(srcs)
+    n = tables[0].n if S else 2
+    count, steps = replicates + 1, max(n - 2, 0)
+    if steps == 0 or S == 0:
+        return np.zeros((S, count, steps), np.uint64), np.zeros((S, count, steps), np.float64)
+    per = bootstrap_row_bytes(n, max(int(s[1].shape[0]) for s in srcs))
+    total = S * count
+    group = max(1, min(total, BOOTSTRAP_TREES_BATCH_BYTES // per))
+    masks, scores = _empty((total, steps), torch.int64), _empty((total, steps), torch.float64)
+    for f0 in range(0, total, group):
+        f1 = min(total, f0 + group)
+        stack = bootstrap_group_tables(srcs, count, f0, f1, n, timer)
+        m, sc = erickson_lockstep(n, f1 - f0, first_taxon,
+                                  lambda ma, mb, per_table: subflatten_scores_multi(stack, ma, mb, per_table), timer)
+        masks[f0:f1], scores[f0:f1] = m, sc
+        del stack
+    return (masks.cpu().numpy().view(np.uint64).reshape(S, count, steps), scores.cpu().numpy().reshape(S, count, steps))
+
+
 def bootstrap_tree_masks(table, replicates, seed, first_taxon, timer=None):
     """erickson_SVD(Method.subflattening) agglomerations of a table of pattern counts (see _counted) and of its bootstrap
     replicates: (joined-side masks as numpy uint64, scores as numpy float64), both [replicates + 1, n - 2].  Row 0 is the
-    table itself, row b + 1 replicate b as bootstrap_tables yields it.  Every table is scored from the pair tables of its
-    integer counts (SubflattenTables) with candidates oriented towards `first_taxon` (erickson_lockstep).  The tables run in
-    lockstep groups of at most BOOTSTRAP_TREES_BATCH_BYTES of device memory; a row depends on its table only.  `timer`
-    (PhaseTimer) gets the spans "resample", "tables", "score" and "step"."""
-    import itertools
-    seed, n = bootstrap_seed(seed), table.n
-    replicates = int(replicates)
-    _check_replicates(0, replicates)
-    keys, counts = _counted(table)
-    _, N = _bootstrap_prefix(counts)
-    count, steps = replicates + 1, max(n - 2, 0)
-    if steps == 0:
-        return np.zeros((count, 0), np.uint64), np.zeros((count, 0), np.float64)
-    tables = itertools.chain([_table_of_counts(table, keys, counts, N)], bootstrap_tables(table, replicates, seed))
-    p0 = n * (n - 1) // 2
-    per = SubflattenTables.bytes_per_table(n) + int(lib.spb_agglomerate_ws_bytes(n, 1)) + 24 * p0 + 16 * steps
-    group = max(1, min(count, BOOTSTRAP_TREES_BATCH_BYTES // per))
-    masks, scores = [], []
-    for g0 in range(0, count, group):
-        g = min(group, count - g0)
-        stack = SubflattenTables(n, g)
-        for i in range(g):
-            with _span(timer, "resample"):
-                tb = next(tables)
-            with _span(timer, "tables"):
-                stack.add(i, tb)
-            del tb
-        m, sc = erickson_lockstep(n, g, first_taxon, lambda ma, mb, per_table: subflatten_scores_multi(stack, ma, mb, per_table),
-                                  timer)
-        masks.append(m)
-        scores.append(sc)
-        del stack
-    return torch.cat(masks).cpu().numpy().view(np.uint64), torch.cat(scores).cpu().numpy()
+    table itself, row b + 1 replicate b as bootstrap_tables yields it.  bootstrap_tree_masks_multi with one table (see
+    there for the tables, the grouping and the spans `timer` gets)."""
+    masks, scores = bootstrap_tree_masks_multi([table], replicates, [seed], first_taxon, timer)
+    return masks[0], scores[0]
+
+
+def window_bootstrap_seed(seed, begin, end):
+    """The bootstrap seed of the site window [begin, end) under `seed`, in [0, 2^64): with
+    fmix(z) = SplitMix64's finaliser (z ^= z >> 30; z *= 0xBF58476D1CE4E5B9; z ^= z >> 27; z *= 0x94D049BB133111EB;
+    z ^= z >> 31) and gamma = 0x9E3779B97F4A7C15, all mod 2^64,
+        h = fmix(seed + gamma);  h = fmix(h + begin + gamma);  h = fmix(h + end + gamma);  return h
+    i.e. three SplitMix64 steps, each absorbing one value.  A window's replicates so depend on `seed` and its bounds only,
+    not on its position in a list of windows."""
+    seed = bootstrap_seed(seed)
+    M, G = (1 << 64) - 1, 0x9E3779B97F4A7C15
+
+    def fmix(z):
+        z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & M
+        z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & M
+        return z ^ (z >> 31)
+
+    h = fmix((seed + G) & M)
+    for v in (int(begin), int(end)):
+        if not 0 <= v < 1 << 64:
+            raise ValueError(f"window_bootstrap_seed: window bounds must be in [0, 2^64) (got {v})")
+        h = fmix((h + v + G) & M)
+    return h
 
 
 # --------------------------------------------------------------------------------------------
