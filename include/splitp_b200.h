@@ -460,6 +460,23 @@ int64_t spb_mi_side_cap(int64_t num, int side_len);
 int64_t spb_mi_scores_ws(int64_t num, int key_words, int64_t slots, int64_t n_splits);
 int spb_mi_scores(const uint64_t* d_keys, int key_words, const void* d_vals, int val_kind, double divisor, int64_t num,
                   const spb_mi_split* d_splits, int64_t n_splits, int64_t slots, uint64_t* d_ws, double* d_out, void* stream);
+/* The same divergences for many count rows over one pattern list (bootstrap replicates: uint32 d_counts [rows][num], as
+ * spb_bootstrap_counts writes them).  The side-table layout depends on the keys only, so it is built once:
+ *   spb_mi_row_slots   inserts the num keys into the side tables of every split (d_tkeys: slots x key_words uint64,
+ *                      16-byte aligned, slots = the slots of all tables of the call) and writes the slot of every (split,
+ *                      side, pattern), relative to the side's first slot, to d_slot_of: uint32 [n_splits][2][num].
+ *   spb_mi_row_scores  per (row, split): the row's counts added into its side sums at those slots (exact uint64 integers),
+ *                      then the terms of the row's non-zero patterns in table order, which d_index (uint64 pattern indices)
+ *                      lists at [d_offsets[r], d_offsets[r + 1]) (spb_bootstrap_compact with key_words = 0).  d_out [rows]
+ *                      [n_splits]: bitwise what spb_mi_scores gives for the table of the row's non-zero patterns with its
+ *                      counts (SPB_VAL_U32) and `divisor`, whichever other rows and splits share the call.  rows <= 65535;
+ *                      d_ws: spb_mi_rows_ws(num, rows, slots, n_splits) uint64 words. */
+int spb_mi_row_slots(const uint64_t* d_keys, int key_words, int64_t num, const spb_mi_split* d_splits, int64_t n_splits,
+                     int64_t slots, uint64_t* d_tkeys, uint32_t* d_slot_of, void* stream);
+int64_t spb_mi_rows_ws(int64_t num, int64_t rows, int64_t slots, int64_t n_splits);
+int spb_mi_row_scores(const uint32_t* d_counts, int64_t num, const uint64_t* d_index, const int64_t* d_offsets, int64_t rows,
+                      double divisor, const spb_mi_split* d_splits, int64_t n_splits, int64_t slots, const uint32_t* d_slot_of,
+                      uint64_t* d_ws, double* d_out, void* stream);
 
 /* ---- nonparametric bootstrap of a pattern table (bootstrap.cu) ----
  * Replicate b draws N sites with replacement, i.e. N patterns with probability count / N.  Draw s of replicate b:
@@ -472,7 +489,8 @@ int spb_mi_scores(const uint64_t* d_keys, int key_words, const void* d_vals, int
 int spb_bootstrap_counts(const uint32_t* d_prefix, int64_t P, int64_t N, uint64_t seed, int64_t rep_first, int64_t reps,
                          uint32_t* d_counts, void* stream);
 /* Per replicate (row of d_counts), the patterns with a non-zero count in table order: keys (key_words uint64 each, as
- * d_keys [P][key_words]) to d_out_keys, counts to d_out_counts, replicate r at [d_offsets[r], d_offsets[r + 1]) (int64
+ * d_keys [P][key_words]; key_words = 0: the pattern's index p as one uint64, d_keys unused) to d_out_keys, counts to
+ * d_out_counts, replicate r at [d_offsets[r], d_offsets[r + 1]) (int64
  * [reps + 1]).  cap: entries of the outputs (reps x min(P, N) always suffices; entries past it are dropped).  reps <= 65535.
  * d_ws: spb_bootstrap_compact_ws(P, reps) int64 words. */
 int64_t spb_bootstrap_compact_ws(int64_t P, int64_t reps);

@@ -164,6 +164,9 @@ PROTOTYPES = {
     "spb_mi_side_cap": (_l, [_l, _i]),
     "spb_mi_scores_ws": (_l, [_l, _i, _l, _l]),
     "spb_mi_scores": (_i, [_p, _i, _p, _i, _d, _l, _p, _l, _l, _p, _p, _p]),
+    "spb_mi_row_slots": (_i, [_p, _i, _l, _p, _l, _l, _p, _p, _p]),
+    "spb_mi_rows_ws": (_l, [_l, _l, _l, _l]),
+    "spb_mi_row_scores": (_i, [_p, _l, _p, _p, _l, _d, _p, _l, _l, _p, _p, _p, _p]),
     "spb_bootstrap_counts": (_i, [_p, _l, _l, C.c_uint64, _l, _l, _p, _p]),
     "spb_bootstrap_compact_ws": (_l, [_l, _l]),
     "spb_bootstrap_compact": (_i, [_p, _p, _i, _l, _l, _p, _p, _l, _p, _p, _p]),

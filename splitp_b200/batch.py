@@ -380,36 +380,24 @@ def bootstrap_scores(alignment, splits, method=Method.flattening, replicates=100
     csrc/bootstrap.cu).  Row b depends on the alignment, `seed` and b only: two calls with the same arguments return equal
     arrays.  `alignment`, `splits`, `method` and `taxa` have the meaning they have in `score_splits` (2..64 taxa).
 
-    The alignment is counted once; every replicate's table then goes through the scorer `score_splits` uses:
+    The alignment is counted once; engine.bootstrap_scores_multi then scores every replicate with the scorer
+    `score_splits` uses, bitwise what that scorer gives for the replicate's table:
       Method.flattening     up to 16 taxa: one engine.CountScorer for all replicates; above: engine.sparse_flattening_scores
-      Method.subflattening  pair tables of the replicate's counts (engine.pair_tables_from_table) + engine.subflatten_scores
-      Method.mutual_information  engine.rank1_divergence_scores (counts / N)
+      Method.subflattening  pair tables of every replicate's count row (spb_pair_tables_count_rows, one launch per group
+                            of replicates; above engine.COUNT_ROWS_MAX_TAXA taxa spb_pair_tables_wide per replicate) +
+                            the multi-table subflattening scorer
+      Method.mutual_information  side tables of every split built once from the pattern list, then every replicate's
+                            count row scored in a few launches (engine.rank1_divergence_count_rows, counts / N)
     The scores stay on the device until the last replicate is scored."""
     seed = _bootstrap_checks("bootstrap_scores", replicates, seed)
     if taxa is None and isinstance(alignment, dict):
         taxa = list(alignment.keys())
     # one process: the SplitScorer holds the split positions, the subflattening masks and the counting stage of score_splits
     ss = SplitScorer(splits, taxa, method)
-    idx, n = ss.idx_all, _num_taxa(alignment)
+    n = _num_taxa(alignment)
     table = ss._count(alignment) if n <= engine.NARROW_MAX_TAXA else ss._count_wide(alignment)
-    out = engine._empty((int(replicates), len(idx)), torch.float64)
-    scorer = None
-    for b, tb in enumerate(engine.bootstrap_tables(table, replicates, seed)):
-        if not idx:
-            continue
-        if method == Method.flattening and uses_sparse_flattening(n):
-            out[b] = engine.sparse_flattening_scores(tb, idx)
-        elif method == Method.flattening:
-            if scorer is None:
-                scorer = engine.CountScorer(tb)
-            else:
-                scorer.table = tb
-            out[b] = scorer.score_many(idx)
-        elif method == Method.subflattening:
-            out[b] = engine.subflatten_scores(engine.pair_tables_from_table(tb, as_counts=True), *ss.masks)
-        else:
-            out[b] = engine.rank1_divergence_scores(tb, idx)
-    return out.cpu().numpy()
+    out = engine.bootstrap_scores_multi([table], int(replicates), [seed], method, ss.idx_all, ss.masks)
+    return out[0].cpu().numpy()
 
 
 BootstrapTrees = namedtuple("BootstrapTrees", "tree support replicate_trees")
@@ -684,6 +672,20 @@ def window_bootstrap_trees(alignment, windows, replicates=100, seed=0, taxa=None
     taxa, wanted = _tree_taxa(fn, alignment, n, taxa, splits)
     if wins.shape[0] == 0:
         return []
+    tables, seeds = _window_sources(fn, alignment, n, wins, seed)
+    first = min(range(n), key=lambda i: taxa[i])
+    masks, _ = engine.bootstrap_tree_masks_multi(tables, int(replicates), seeds, first)
+    del tables
+    trees = _trees_of_masks(masks, taxa)
+    per = masks.shape[1]
+    return [BootstrapTrees(trees[w * per], _support(masks[w], wanted, n), trees[w * per + 1:(w + 1) * per])
+            for w in range(masks.shape[0])]
+
+
+def _window_sources(fn, alignment, n, wins, seed):
+    """(pattern count table of every window, its bootstrap seed engine.window_bootstrap_seed(seed, b_w, e_w)): the
+    alignment is packed once and every window is counted from the packed sites.  ValueError naming the first window
+    without a usable site; above 31 taxa the packed forms raise NotImplementedError."""
     if n <= engine.NARROW_MAX_TAXA:
         aln = _as_alignment(alignment, want_sm=True, want_planes=False)
 
@@ -703,11 +705,36 @@ def window_bootstrap_trees(alignment, windows, replicates=100, seed=0, taxa=None
         tables.append(table_of(b, e))
         if tables[-1].divisor == 0:
             raise ValueError(f"{fn}: window {w} [{b}, {e}) has no usable site")
-    seeds = [engine.window_bootstrap_seed(seed, b, e) for b, e in wins.tolist()]
-    first = min(range(n), key=lambda i: taxa[i])
-    masks, _ = engine.bootstrap_tree_masks_multi(tables, int(replicates), seeds, first)
+    return tables, [engine.window_bootstrap_seed(seed, b, e) for b, e in wins.tolist()]
+
+
+def window_bootstrap_scores(alignment, splits, windows, method=Method.flattening, replicates=100, seed=0, taxa=None):
+    """Bootstrap split scores along site windows: numpy float64 [len(windows), replicates, len(splits)].  Entry [w] equals
+
+        bootstrap_scores(<alignment restricted to the sites [b_w, e_w)>, splits, method, replicates,
+                         seed=engine.window_bootstrap_seed(seed, b_w, e_w), taxa=taxa)
+
+    bit for bit: a window's replicates depend on `seed` and its bounds only, so a repeated window gives equal entries and a
+    window's entry does not depend on the other windows.  This is the confidence band of a split score along the genome.
+
+    The alignment is packed once and every window is counted from the packed sites (as window_bootstrap_trees counts
+    them); all windows then go to engine.bootstrap_scores_multi (see bootstrap_scores for the scorer of each method):
+    subflattening builds the pair tables of the replicates of several windows per launch, mutual information builds each
+    split's side tables once per window and scores all its replicates in a few launches.
+
+    `windows` is as in window_scores; `alignment`, `splits`, `method`, `replicates`, `seed` and `taxa` as in
+    bootstrap_scores (2..64 taxa; above 31 taxa the alignment must be given as characters).  A window without a usable
+    site raises ValueError.  Runs on one GPU: inside a torch.distributed group of several processes it raises
+    NotImplementedError."""
+    fn = "window_bootstrap_scores"
+    n, wins = _window_inputs(fn, alignment, windows)
+    seed = _bootstrap_checks(fn, replicates, seed)
+    if taxa is None and isinstance(alignment, dict):
+        taxa = list(alignment.keys())
+    ss = SplitScorer(splits, taxa, method)  # split positions and subflattening masks, as score_splits builds them
+    if wins.shape[0] == 0:
+        return np.zeros((0, int(replicates), ss.S), np.float64)
+    tables, seeds = _window_sources(fn, alignment, n, wins, seed)
+    out = engine.bootstrap_scores_multi(tables, int(replicates), seeds, method, ss.idx_all, ss.masks)
     del tables
-    trees = _trees_of_masks(masks, taxa)
-    per = masks.shape[1]
-    return [BootstrapTrees(trees[w * per], _support(masks[w], wanted, n), trees[w * per + 1:(w + 1) * per])
-            for w in range(masks.shape[0])]
+    return out.cpu().numpy()

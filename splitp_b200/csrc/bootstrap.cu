@@ -13,7 +13,8 @@
 //                             added by one integer atomic (__match_any_sync): constant sites hold a large share of the draws
 //                             and same-address atomics serialise in one L2 slice.  Integer sums make the counts exact.
 //   compaction                three passes over tiles of kTile patterns: non-zeros per (replicate, tile); one exclusive scan
-//                             of all of them in (replicate, tile) order; ordered write of keys, counts and replicate offsets.
+//                             of all of them in (replicate, tile) order; ordered write of keys (or pattern indices), counts
+//                             and replicate offsets.
 #include "common.cuh"
 
 namespace spb {
@@ -177,6 +178,7 @@ __global__ void __launch_bounds__(kThreads) compact_write_kernel(const uint32_t*
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     if (v[i] != 0u && pos < cap) {
+      if (W == 0) out_keys[pos] = (uint64_t)(q + i);  // the pattern's index instead of its key
 #pragma unroll
       for (int t = 0; t < W; ++t) out_keys[pos * W + t] = keys[(q + i) * W + t];
       out_counts[pos] = v[i];
@@ -222,7 +224,7 @@ extern "C" int64_t spb_bootstrap_compact_ws(int64_t P, int64_t reps) {
 extern "C" int spb_bootstrap_compact(const uint32_t* d_counts, const uint64_t* d_keys, int key_words, int64_t P, int64_t reps,
                                      uint64_t* d_out_keys, uint32_t* d_out_counts, int64_t cap, int64_t* d_offsets, int64_t* d_ws,
                                      void* stream) {
-  SPB_REQUIRE(key_words == 1 || key_words == 2, "spb_bootstrap_compact: key_words must be 1 or 2 (got %d)", key_words);
+  SPB_REQUIRE(key_words >= 0 && key_words <= 2, "spb_bootstrap_compact: key_words must be 0, 1 or 2 (got %d)", key_words);
   SPB_REQUIRE(P >= 1 && reps >= 0 && cap >= 0, "spb_bootstrap_compact: bad sizes P=%lld reps=%lld cap=%lld", (long long)P,
               (long long)reps, (long long)cap);
   SPB_REQUIRE(reps <= 65535, "spb_bootstrap_compact: at most 65535 replicates per call");
@@ -232,7 +234,7 @@ extern "C" int spb_bootstrap_compact(const uint32_t* d_counts, const uint64_t* d
     SPB_CUDA(cudaMemsetAsync(d_offsets, 0, sizeof(int64_t), st));
     return SPB_OK;
   }
-  SPB_REQUIRE(d_counts && d_keys && d_out_keys && d_out_counts && d_ws, "spb_bootstrap_compact: NULL buffer");
+  SPB_REQUIRE(d_counts && (d_keys || key_words == 0) && d_out_keys && d_out_counts && d_ws, "spb_bootstrap_compact: NULL buffer");
   const int64_t tiles = (P + kTile - 1) / kTile;
   SPB_REQUIRE(tiles <= 0x7FFFFFFF, "spb_bootstrap_compact: too many patterns");
   const dim3 grid((unsigned)tiles, (unsigned)reps);
@@ -240,7 +242,9 @@ extern "C" int spb_bootstrap_compact(const uint32_t* d_counts, const uint64_t* d
   SPB_LAUNCH_CHECK();
   compact_scan_kernel<<<1, kScanThreads, 0, st>>>(d_ws, tiles * reps, tiles, reps, d_offsets);
   SPB_LAUNCH_CHECK();
-  if (key_words == 1)
+  if (key_words == 0)
+    compact_write_kernel<0><<<grid, kThreads, 0, st>>>(d_counts, d_keys, P, d_ws, cap, d_out_keys, d_out_counts);
+  else if (key_words == 1)
     compact_write_kernel<1><<<grid, kThreads, 0, st>>>(d_counts, d_keys, P, d_ws, cap, d_out_keys, d_out_counts);
   else
     compact_write_kernel<2><<<grid, kThreads, 0, st>>>(d_counts, d_keys, P, d_ws, cap, d_out_keys, d_out_counts);

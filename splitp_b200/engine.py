@@ -23,6 +23,7 @@ import torch
 
 from . import _lib
 from ._lib import SPB_S0_K4MAJOR, SPB_S0_ROWMAJOR, SPB_S0_TILED, SPB_U8_NO_MEMSET, SPB_VAL_F64, SPB_VAL_U32, call, lib, make_split
+from .enums import Method
 
 STATES = "ACGT"
 _UPPER_LUT = np.full(256, 255, dtype=np.uint8)
@@ -1507,6 +1508,21 @@ def mi_batches(split_slots, num, key_words, cap=None):
     return out
 
 
+def _mi_split_desc(n, splits_idx, caps, batches):
+    """spb_mi_split records (numpy uint64 [len(splits_idx), 8]: mask[2][2], slot[2], cap[2]) of splits whose sides get
+    tables of caps[j] slots; the tables of every batch [b0, b1) are laid out from slot 0 in split order."""
+    desc = np.zeros((len(splits_idx), 8), dtype=np.uint64)
+    for b0, b1 in batches:
+        slot = 0
+        for j in range(b0, b1):
+            ia, ib = splits_idx[j]
+            desc[j, 0:2], desc[j, 2:4] = side_mask(n, ia), side_mask(n, ib)
+            desc[j, 4], desc[j, 5] = slot, slot + caps[j][0]
+            desc[j, 6:8] = caps[j]
+            slot += caps[j][0] + caps[j][1]
+    return desc
+
+
 def rank1_divergence_scores(table, splits_idx, timer=None):
     """Rank-1 divergences (phylogenetics.py:364-373) of many splits [(idx_a, idx_b), ...] of one table, batched on the device
     (csrc/mi_batch.cu): the values rank1_divergence_table gives one split at a time, up to the summation order.  `table`: a
@@ -1531,15 +1547,7 @@ def rank1_divergence_scores(table, splits_idx, timer=None):
     W = 2 if keys.dim() == 2 else 1
     caps = [(int(lib.spb_mi_side_cap(num, len(splits_idx[i][0]))), int(lib.spb_mi_side_cap(num, len(splits_idx[i][1])))) for i in live]
     batches = mi_batches([ca + cb for ca, cb in caps], num, W)
-    desc = np.zeros((len(live), 8), dtype=np.uint64)  # spb_mi_split: mask[2][2], slot[2], cap[2]
-    for b0, b1 in batches:
-        slot = 0
-        for j in range(b0, b1):
-            ia, ib = splits_idx[live[j]]
-            desc[j, 0:2], desc[j, 2:4] = side_mask(n, ia), side_mask(n, ib)
-            desc[j, 4], desc[j, 5] = slot, slot + caps[j][0]
-            desc[j, 6:8] = caps[j]
-            slot += caps[j][0] + caps[j][1]
+    desc = _mi_split_desc(n, [splits_idx[i] for i in live], caps, batches)
     with _span(timer, "mi", len(live)):
         desc_d = torch.from_numpy(desc.view(np.int64)).to(device())
         ws = _empty(max(int(lib.spb_mi_scores_ws(num, W, sum(a + b for a, b in caps[b0:b1]), b1 - b0)) for b0, b1 in batches), torch.int64)
@@ -1902,25 +1910,26 @@ def bootstrap_sources(tables, seeds):
     return srcs
 
 
-def _bootstrap_rows(src, b0, b1):
-    """Count rows b0 .. b1 - 1 of a bootstrap source (bootstrap_sources): row 0 is the source's own counts, row b + 1
-    replicate b (int32 [b1 - b0, P] holding uint32 counts)."""
+def _bootstrap_rows(src, b0, b1, own=True):
+    """Count rows b0 .. b1 - 1 of a bootstrap source (bootstrap_sources) as int32 [b1 - b0, P] holding uint32 counts.  With
+    `own`, row 0 is the source's own counts and row b + 1 replicate b; without, row b is replicate b."""
     keys, counts, prefix, N, seed = src
     P = int(counts.shape[0])
     rows = _empty((b1 - b0, P), torch.int32)
     r0 = 0
-    if b0 == 0:
+    if own and b0 == 0:
         rows[0].copy_(counts)
         r0 = 1
-    first, c = b0 + r0 - 1, b1 - b0 - r0
+    first, c = b0 + r0 - int(own), b1 - b0 - r0
     if c:
         call("spb_bootstrap_counts", _p(prefix), P, N, seed, first, c, _p(rows[r0:]), _st())
     return rows
 
 
-def bootstrap_group_tables(srcs, count, f0, f1, n, timer=None):
+def bootstrap_group_tables(srcs, count, f0, f1, n, timer=None, own=True):
     """SubflattenTables of the rows f0 .. f1 - 1 of the sources (bootstrap_sources), `count` rows per source: row
-    s count + b is source s's own counts (b = 0) or its replicate b - 1.  Slot i holds what SubflattenTables.add gives
+    s count + b is source s's own counts (b = 0) or its replicate b - 1; without `own`, replicate b.  Slot i holds what
+    SubflattenTables.add gives
     for that table (bootstrap_tables' replicate table), bit for bit.  Up to COUNT_ROWS_MAX_TAXA taxa a source's count rows
     go through spb_pair_tables_count_rows in one launch, above through spb_pair_tables_wide per compacted row; then
     spb_pair_transform and the triple tables per row."""
@@ -1930,7 +1939,7 @@ def bootstrap_group_tables(srcs, count, f0, f1, n, timer=None):
         b0, b1 = max(f0, s * count) - s * count, min(f1, (s + 1) * count) - s * count
         slot0 = s * count + b0 - f0
         with _span(timer, "resample"):
-            rows = _bootstrap_rows(srcs[s], b0, b1)
+            rows = _bootstrap_rows(srcs[s], b0, b1, own)
         with _span(timer, "tables"):
             with _span(timer, "pair tables"):
                 if n <= COUNT_ROWS_MAX_TAXA:
@@ -2001,6 +2010,145 @@ def bootstrap_tree_masks(table, replicates, seed, first_taxon, timer=None):
     there for the tables, the grouping and the spans `timer` gets)."""
     masks, scores = bootstrap_tree_masks_multi([table], replicates, [seed], first_taxon, timer)
     return masks[0], scores[0]
+
+
+# --------------------------------------------------------------------------------------------
+# bootstrap split scores of several tables of pattern counts (bootstrap_scores, window_bootstrap_scores)
+# --------------------------------------------------------------------------------------------
+BOOTSTRAP_SCORES_BATCH_BYTES = 2 << 30  # device memory of one group of replicate rows scored by subflattening
+
+
+def _nonzero_rows(rows, row_cap):
+    """(rows, uint64 indices of every row's non-zero patterns in table order as an int64 tensor, int64 offsets [R + 1]:
+    row r's at [offsets[r], offsets[r + 1])), by spb_bootstrap_compact with key_words 0.  row_cap: non-zeros of a row at
+    most."""
+    rows = rows.contiguous()
+    R, P = int(rows.shape[0]), int(rows.shape[1])
+    cap = R * row_cap
+    index, nz, offsets = _empty(max(cap, 1), torch.int64), _empty(max(cap, 1), torch.int32), _empty(R + 1, torch.int64)
+    ws = _empty(int(lib.spb_bootstrap_compact_ws(P, R)), torch.int64)
+    call("spb_bootstrap_compact", _p(rows), None, 0, P, R, _p(index), _p(nz), cap, _p(offsets), _p(ws), _st())
+    return rows, index, offsets
+
+
+def rank1_divergence_count_rows(keys, rows_of, R, n, divisor, splits_idx, row_cap=None, timer=None):
+    """Rank-1 divergences of many splits [(idx_a, idx_b), ...] for R count rows over one sorted pattern list: float64 device
+    tensor [R, len(splits_idx)], entry [r, s] bitwise rank1_divergence_scores of the table of row r's non-zero patterns
+    (keys and uint32 counts in table order, with `divisor`), as bootstrap_tables yields it for a replicate.
+
+    keys: uint64 [P] (up to 31 taxa) or int64 [P, 2] 128-bit keys; rows_of(r0, r1) returns rows r0 .. r1 - 1 as int32 [r1 -
+    r0, P] holding uint32 counts (zeros allowed); row_cap: non-zeros of a row at most (default P).  The side tables of each
+    batch of splits are built once from the keys (spb_mi_row_slots); rows then go through spb_mi_row_scores in groups.
+    Batches and groups keep their workspace within MI_BATCH_BYTES; no score depends on them.  Split checks as in
+    rank1_divergence_scores.  `timer` gets the spans "slots", "rows" and "score"."""
+    for ia, ib in splits_idx:
+        if not covers_all(n, ia, ib):
+            raise ValueError("rank-1 divergence scores need a split that places every taxon on exactly one side")
+    P, W = int(keys.shape[0]), (2 if keys.dim() == 2 else 1)
+    out = _zeros((R, len(splits_idx)), torch.float64)
+    live = [i for i, (ia, ib) in enumerate(splits_idx) if len(ia) and len(ib)]
+    if R == 0 or P == 0 or not live:
+        return out
+    cap1 = P if row_cap is None else max(1, min(P, int(row_cap)))
+    cmax = int(lib.spb_mi_rows_ws(P, 1, 0, 1))  # partials per (row, split)
+    caps = [(int(lib.spb_mi_side_cap(P, len(splits_idx[i][0]))), int(lib.spb_mi_side_cap(P, len(splits_idx[i][1])))) for i in live]
+    row_bytes = 4 * P + 12 * cap1 + 8 * int(lib.spb_bootstrap_compact_ws(P, 1))  # count row, compacted indices and counts
+
+    def fixed(slots, k):  # side tables of the slot pass and the slots of every (split, side, pattern)
+        return 8 * W * slots + 8 * k * P
+
+    def per_row(slots, k):  # side sums, partials and scores of one row
+        return 8 * (slots + k * cmax + k) + row_bytes
+    batches, b0, slots = [], 0, 0
+    for i, (ca, cb) in enumerate(caps):
+        grown = slots + ca + cb
+        if i > b0 and (i - b0 >= MI_MAX_SPLITS or fixed(grown, i - b0 + 1) + per_row(grown, i - b0 + 1) > MI_BATCH_BYTES):
+            batches.append((b0, i))
+            b0, grown = i, ca + cb
+        slots = grown
+    batches.append((b0, len(caps)))
+    slots = [sum(ca + cb for ca, cb in caps[b0:b1]) for b0, b1 in batches]
+    worst = max(fixed(s, b1 - b0) for s, (b0, b1) in zip(slots, batches))
+    g = max(1, min(R, 65535, (MI_BATCH_BYTES - worst) // max(per_row(s, b1 - b0) for s, (b0, b1) in zip(slots, batches))))
+    groups = [(r0, min(R, r0 + g)) for r0 in range(0, R, g)]
+    desc_d = torch.from_numpy(_mi_split_desc(n, [splits_idx[i] for i in live], caps, batches).view(np.int64)).to(device())
+    live_d = torch.tensor(live, dtype=torch.int64, device=device())
+    held = None  # the compacted rows of the last group: one group serves every batch
+    for (b0, b1), sl in zip(batches, slots):
+        k = b1 - b0
+        with _span(timer, "slots"):
+            tkeys, slot_of = _empty(sl * W, torch.int64), _empty(2 * k * P, torch.int32)
+            call("spb_mi_row_slots", _p(keys), W, P, _p(desc_d[b0:b1]), k, sl, _p(tkeys), _p(slot_of), _st())
+            del tkeys
+        for r0, r1 in groups:
+            if held is None or held[0] != r0:
+                held = None
+                with _span(timer, "rows"):
+                    held = (r0, *_nonzero_rows(rows_of(r0, r1), cap1))
+            _, rows, index, offsets = held
+            with _span(timer, "score"):
+                ws, res = _empty(int(lib.spb_mi_rows_ws(P, r1 - r0, sl, k)), torch.int64), _empty((r1 - r0, k), torch.float64)
+                call("spb_mi_row_scores", _p(rows), P, _p(index), _p(offsets), r1 - r0, float(divisor), _p(desc_d[b0:b1]), k, sl,
+                     _p(slot_of), _p(ws), _p(res), _st())
+                out[r0:r1].index_copy_(1, live_d[b0:b1], res)
+        del slot_of
+    return out
+
+
+def bootstrap_scores_multi(tables, replicates, seeds, method, splits_idx, masks=None, timer=None):
+    """Bootstrap split scores of several tables of pattern counts (see _counted; all of n taxa): float64 device tensor
+    [len(tables), replicates, len(splits_idx)].  Entry [s, b] holds the scores of replicate b of table s with seed
+    seeds[s], the table bootstrap_tables yields at index b, bitwise what the scorer of score_splits gives for it:
+      Method.subflattening       pair tables of the replicates' count rows (bootstrap_group_tables without the tables' own
+                                 counts) + subflatten_scores_multi; masks = (masks_a, masks_b) of splits_idx as device
+                                 tensors (SplitScorer.masks); rows in groups of at most BOOTSTRAP_SCORES_BATCH_BYTES
+      Method.mutual_information  rank1_divergence_count_rows of every table's replicate count rows, divisor N
+      Method.flattening          every replicate table through CountScorer up to 16 taxa, sparse_flattening_scores above
+    A score depends on its table, seed, replicate index and split only, never on the grouping.  ValueError for a table
+    without usable sites."""
+    seeds = [bootstrap_seed(s) for s in seeds]
+    B = int(replicates)
+    _check_replicates(0, B)
+    srcs = bootstrap_sources(tables, seeds)
+    S, K = len(srcs), len(splits_idx)
+    out = _zeros((S, B, K), torch.float64)
+    if S == 0 or K == 0 or B == 0:
+        return out
+    n = tables[0].n
+    if method == Method.subflattening:
+        masks_a, masks_b = masks
+        P_max = max(int(src[1].shape[0]) for src in srcs)
+        per = (SubflattenTables.bytes_per_table(n) + 256 * n * n + 4 * P_max + (20 * P_max if n > COUNT_ROWS_MAX_TAXA else 0)
+               + 24 * K)
+        total, flat = S * B, out.view(S * B, K)
+        group = max(1, min(total, BOOTSTRAP_SCORES_BATCH_BYTES // per))
+        for f0 in range(0, total, group):
+            f1 = min(total, f0 + group)
+            stack = bootstrap_group_tables(srcs, B, f0, f1, n, timer, own=False)
+            with _span(timer, "score"):
+                flat[f0:f1] = subflatten_scores_multi(stack, masks_a.repeat(f1 - f0), masks_b.repeat(f1 - f0), K).view(f1 - f0, K)
+            del stack
+    elif method == Method.mutual_information:
+        for s, src in enumerate(srcs):
+            keys, counts, _, N, _ = src
+            out[s] = rank1_divergence_count_rows(keys, lambda r0, r1, src=src: _bootstrap_rows(src, r0, r1, own=False), B, n,
+                                                 float(N), splits_idx, row_cap=min(int(counts.shape[0]), N), timer=timer)
+    elif method == Method.flattening:
+        from .batch import uses_sparse_flattening
+        scorer = None
+        for s, t in enumerate(tables):
+            for b, tb in enumerate(bootstrap_tables(t, B, seeds[s])):
+                if uses_sparse_flattening(n):
+                    out[s, b] = sparse_flattening_scores(tb, splits_idx)
+                    continue
+                if scorer is None:
+                    scorer = CountScorer(tb)
+                else:
+                    scorer.table = tb
+                out[s, b] = scorer.score_many(splits_idx)
+    else:
+        raise NotImplementedError("bootstrap scores: Method.flattening, Method.subflattening or Method.mutual_information")
+    return out
 
 
 def window_bootstrap_seed(seed, begin, end):
