@@ -12,7 +12,8 @@ and the inner loop of `erickson_SVD` (phylogenetics.py:126-140).  `score_splits`
     Method.flattening     pack -> pattern count (kernel 1) -> per split: u8 scatter (kernel 2) -> exact integer Gram on the
                           tensor cores (kernel 4) -> eigen-solver (kernel 5); scores equal those of the reduced / dense /
                           sparse flattening (dropping all-zero rows and columns does not change the singular values)
-                          (up to 16 taxa; 17..64 taxa: pattern count -> engine.sparse_flattening_scores, csrc/sparse.cu)
+                          (up to 16 taxa, shorter side up to 6 taxa; 7|7 .. 8|8 splits and 17..64 taxa: pattern count ->
+                          engine.sparse_flattening_scores, csrc/sparse.cu)
     Method.subflattening  pack -> pair tables -> H N H^T -> per split: gather + Gram + eigenvalues (kernel 3)
     Method.mutual_information  pattern count (uint64 keys up to 31 taxa; 32..64 taxa: pack_wide + count_patterns_wide) ->
                           engine.rank1_divergence_scores (csrc/mi_batch.cu): the rank-1 divergence of every split's flattening

@@ -612,11 +612,22 @@ class CountScorer:
     (tcgen05 kind::i8) or dp4a for <= 64 rows -> sparse high-part correction -> eigen-solver.
     Buffers are allocated once and reused across splits; up to SPB_MAX_BATCH splits share one launch of
     every stage (the scatter / correction kernels are a few microseconds each, so batching them is what
-    keeps the GPU busy)."""
+    keeps the GPU busy).  score_many sends the size classes whose Gram side has SPARSE_MIN_ROWS rows or more (7|7 .. 8|8 of
+    14..16 taxa) to sparse_flattening_scores instead."""
 
     NB = _lib.SPB_MAX_BATCH   # splits per scatter / clear launch (kernel-parameter limit); 16 in round 1: 266 launches per c2 step
     GNB = 64                  # matrices per Gram / correction launch: 20 tiles x 16 matrices leave the 148 persistent CTAs
                               # with 2 or 3 tiles each (72 % efficiency at 5|7 of 12 taxa), 64 matrices level that out
+    # Dense Gram sides of 4^8 rows exceed the tensor-core Gram (rows_pad <= 32768) and, above 32,768 patterns, would need a
+    # split-K workspace of 16 x 65536^2 int64; 4^7-row sides are slower dense than sparse.  NVIDIA B200, 1,000 W power limit,
+    # 4 splits per call (profiles/r11_dense_flattening_limits_timing.json): 7|8 of 15 taxa 9.5 ms dense / 2.8 ms sparse at
+    # 12,013 patterns and 44.2 / 3.1 ms at 38,459; 6|9 1.2 / 2.7 ms and 2.1 / 2.7 ms.
+    SPARSE_MIN_ROWS = 4 ** 7
+
+    @classmethod
+    def sparse_class(cls, a):
+        """True when score_many scores the splits whose shorter side has `a` taxa with sparse_flattening_scores."""
+        return 4 ** a >= cls.SPARSE_MIN_ROWS
 
     def __init__(self, table, hi_cap=None):
         if table.counts is None:
@@ -902,7 +913,13 @@ class CountScorer:
             tasks = sorted(groups.items(), key=lambda g: -(4.0 ** (2 * g[0])) * 4.0 ** (n - g[0]) * len(g[1]))  # Gram work, descending
             self._plans[gkey] = (splits_idx, len(splits_idx), tasks)
         for a, members in tasks:
-            self._score_group(splits_idx, a, members, out, max_batch, max_batch_bytes)
+            if not self.sparse_class(a):
+                self._score_group(splits_idx, a, members, out, max_batch, max_batch_bytes)
+            elif self.table.num == 0:  # what the dense route gives for an all-zero flattening
+                out[members] = float("nan")
+            else:
+                sc = sparse_flattening_scores(self.table, [splits_idx[s] for s in members], self.timer)
+                out.index_copy_(0, torch.tensor(members, dtype=torch.int64, device=out.device), sc)
         return out
 
     def _encoded_group(self, splits_idx, a, members):

@@ -400,7 +400,7 @@ def test_correction_strip_from_table_equals_column_scan(sp, eng, a):
 # ---------------------------------------------------------------------------------------------
 # small Gram matrices: warp-per-matrix Householder + 9-section against the Jacobi kernel and LAPACK
 # ---------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("k", [5, 16, 31, 33, 64])
+@pytest.mark.parametrize("k", [5, 16, 31, 32, 33, 34, 63, 64])
 def test_score_gram_small_warp_path_against_lapack(eng, k):
     """engine.score_gram without the eigenvalue list takes the warp-per-matrix kernel (k <= 64); with it, the Jacobi kernel.
     Both against LAPACK singular values of integer count flattenings with planted rank-4 structure (small scores)."""

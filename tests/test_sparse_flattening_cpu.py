@@ -26,6 +26,15 @@ def test_route_choice_taxon_bound(sp):
     assert batch.uses_sparse_flattening(64)
 
 
+def test_route_choice_dense_size_classes(sp):
+    """CountScorer keeps the dense route for Gram sides up to 4^6 rows (every class of 12 taxa) and scores 7|7 .. 8|8 from
+    the pattern list."""
+    from splitp_b200 import engine
+    assert engine.CountScorer.SPARSE_MIN_ROWS == 4 ** 7
+    assert not any(engine.CountScorer.sparse_class(a) for a in range(1, 7))
+    assert engine.CountScorer.sparse_class(7) and engine.CountScorer.sparse_class(8)
+
+
 def test_route_choice_cell_bound(sp):
     from splitp_b200 import phylogenetics
     assert phylogenetics.SPARSE_MIN_CELLS == 2 ** 27
