@@ -498,6 +498,24 @@ int spb_bootstrap_compact(const uint32_t* d_counts, const uint64_t* d_keys, int 
                           uint64_t* d_out_keys, uint32_t* d_out_counts, int64_t cap, int64_t* d_offsets, int64_t* d_ws,
                           void* stream);
 
+/* ---- quartet split scores (quartets.cu; replaces the per-quartet loop Alignment.sub_alignment([a, b, c, d]) ->
+ * flattening(split, sub, FlatFormat.reduced) -> split_score over the three 2|2 splits of every quartet) ----
+ * d_quartets: uint8 [num][4] taxon positions (a, b, c, d); a quartet with a position >= n_taxa is skipped (its table stays
+ * as it was).  Pairing p of a quartet: 0 = {a,b}|{c,d}, 1 = {a,c}|{b,d}, 2 = {a,d}|{b,c}.
+ * spb_quartet_tables: the exact joint counts of the 256 states (x_a, x_b, x_c, x_d) over the usable sites of
+ *   [32 word_begin, 32 word_end), ADDED (64-bit atomics) into d_tables uint64 [num][256] (zeroed by the caller) at cell
+ *   64 x_a + 16 x_b + 4 x_c + x_d (the key convention: first taxon most significant).  n_taxa 4..64.
+ * spb_quartet_flattening_scores: d_scores double [num][3] = split_score of the reduced count flattening of each pairing (rows
+ *   = the side holding a): the 16 x 16 fp64 Gram scored by spb_score_gram_small; 0.0 when the flattening has at most 4
+ *   non-empty rows or columns, NaN when the table is all zero.  d_ws: spb_quartet_flattening_ws(num) doubles.
+ * spb_quartet_mi_scores: d_scores double [num][3] = the rank-1 divergence of each pairing's flattening of the probabilities
+ *   count / (sum of the table); 0.0 for an all-zero table.  Each score depends on its table only. */
+int spb_quartet_tables(const uint32_t* d_planes, const uint32_t* d_valid, int n_taxa, int64_t plane_words, int64_t word_begin,
+                       int64_t word_end, const uint8_t* d_quartets, int64_t num, uint64_t* d_tables, void* stream);
+int64_t spb_quartet_flattening_ws(int64_t num);
+int spb_quartet_flattening_scores(const uint64_t* d_tables, int64_t num, double* d_ws, double* d_scores, void* stream);
+int spb_quartet_mi_scores(const uint64_t* d_tables, int64_t num, double* d_scores, void* stream);
+
 /* ---- lockstep agglomeration of erickson_SVD for many replicates (agglomerate.cu), 3 <= n <= 64 ----
  * Cluster ids: leaves 0 .. n-1, the cluster merged at step t is n + t.  A candidate joins two current clusters against all
  * other taxa and is written as uint64 masks (d_ma, d_mb) oriented so that side A holds taxon first_taxon.

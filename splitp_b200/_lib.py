@@ -172,6 +172,10 @@ PROTOTYPES = {
     "spb_bootstrap_compact": (_i, [_p, _p, _i, _l, _l, _p, _p, _l, _p, _p, _p]),
     "spb_subflatten_score_tables_multi": (_i, [_p, _p, _i, _p, _p, _l, _l, _p, _p]),
     "spb_subflatten_score_multi": (_i, [_p, _p, _i, _p, _p, _l, _l, _p, _p]),
+    "spb_quartet_tables": (_i, [_p, _p, _i, _l, _l, _l, _p, _l, _p, _p]),
+    "spb_quartet_flattening_ws": (_l, [_l]),
+    "spb_quartet_flattening_scores": (_i, [_p, _l, _p, _p, _p]),
+    "spb_quartet_mi_scores": (_i, [_p, _l, _p, _p]),
     "spb_agglomerate_ws_bytes": (_l, [_i, _l]),
     "spb_agglomerate_init": (_i, [_i, _l, _i, _p, _p, _p, _p]),
     "spb_agglomerate_step": (_i, [_i, _l, _i, _i, _p, _p, _p, _p, _p, _p, _p]),

@@ -739,3 +739,81 @@ def window_bootstrap_scores(alignment, splits, windows, method=Method.flattening
     out = engine.bootstrap_scores_multi(tables, int(replicates), seeds, method, ss.idx_all, ss.masks)
     del tables
     return out.cpu().numpy()
+
+
+# --------------------------------------------------------------------------------------------
+# quartets
+# --------------------------------------------------------------------------------------------
+def _quartet_positions(quartets, n, taxa):
+    """int64 numpy [Q, 4] of taxon positions from 4-tuples of positions or of labels (resolved with `taxa`); ValueError for
+    a malformed argument, an unknown label or a position out of range (engine.check_quartets then checks range and
+    distinctness of every row)."""
+    if isinstance(quartets, (str, bytes, dict)):
+        raise ValueError("quartet_scores: quartets must be a sequence of 4-tuples of taxon labels or positions")
+    if isinstance(quartets, (np.ndarray, torch.Tensor)):
+        arr = quartets.cpu().numpy() if isinstance(quartets, torch.Tensor) else quartets
+        if arr.dtype.kind in "iu":  # positions: engine.check_quartets checks shape, range and distinctness at once
+            return arr
+    try:
+        items = list(quartets)
+    except TypeError:
+        raise ValueError("quartet_scores: quartets must be a sequence of 4-tuples of taxon labels or positions") from None
+    index = {t: i for i, t in enumerate(taxa)} if taxa is not None else None
+    out = np.empty((len(items), 4), np.int64)
+    for r, quartet in enumerate(items):
+        if isinstance(quartet, (str, bytes, dict)) or not hasattr(quartet, "__len__") or len(quartet) != 4:
+            raise ValueError(f"quartet_scores: quartet {r} is not a 4-tuple of taxon labels or positions ({quartet!r})")
+        for c, t in enumerate(quartet):
+            if isinstance(t, (bool, np.bool_)):
+                raise ValueError(f"quartet_scores: quartet {r} holds a boolean ({quartet!r})")
+            if isinstance(t, (int, np.integer)):
+                if not 0 <= t < n:
+                    raise ValueError(f"quartet_scores: position {t} of quartet {r} is out of range [0, {n})")
+                out[r, c] = t
+            elif index is not None and t in index:
+                out[r, c] = index[t]
+            else:
+                raise ValueError(f"quartet_scores: unknown taxon {t!r} in quartet {r}"
+                                 + ("" if index is not None else " (labels need `taxa` or a dict alignment)"))
+    return out
+
+
+def quartet_scores(alignment, quartets=None, method=Method.flattening, taxa=None):
+    """Scores of the three 2|2 splits of every quartet: numpy float64 [Q, 3].  For the quartet written (a, b, c, d), column 0
+    scores {a,b}|{c,d}, column 1 {a,c}|{b,d} and column 2 {a,d}|{b,c}; the lowest score is the supported quartet topology.
+
+    alignment  any form score_splits takes (dict, uint8 matrix of ASCII bytes or codes on the host or the device, HostPlanes,
+               engine.DeviceAlignment), 4 to 64 taxa
+    quartets   4-tuples of taxon labels (resolved with `taxa` or the dict's key order) or positions; None = every quartet in
+               itertools.combinations(range(n), 4) order
+    method     Method.flattening: split_score(flattening(split, sub, FlatFormat.reduced)) with sub =
+               Alignment(<pattern counts of the whole alignment>, taxa).sub_alignment([a, b, c, d]): the usable sites are those
+               of the whole alignment; at most 4 non-empty rows or columns score 0.0, no usable site NaN.
+               Method.mutual_information: the rank-1 divergence of the same flattening of count / usable sites (0.0 without a
+               usable site).  Method.subflattening: bitwise score_splits(alignment, splits, Method.subflattening) of the three
+               splits written with the quartet's smallest position first.
+
+    The 256-cell joint count table of every quartet is counted from the bit planes in one pass per group of quartets
+    (engine.quartet_scores, csrc/quartets.cu) and its three flattenings are scored on the device.  A bipartition gets the same
+    float however its quartet is written: each quartet is scored in sorted form and the columns are mapped back.  Checks raise
+    ValueError before any device work; Method.distance raises NotImplementedError.  Runs on one GPU: inside a
+    torch.distributed group of several processes it raises NotImplementedError."""
+    if method not in (Method.flattening, Method.subflattening, Method.mutual_information):
+        raise NotImplementedError("quartet_scores: Method.flattening, Method.subflattening or Method.mutual_information")
+    _one_process("quartet_scores")
+    n = _num_taxa(alignment)
+    if not 4 <= n <= engine._lib.SPB_MAX_TAXA:
+        raise ValueError(f"quartet_scores: 4 to {engine._lib.SPB_MAX_TAXA} taxa (got {n})")
+    if taxa is None and isinstance(alignment, dict):
+        taxa = list(alignment.keys())
+    if quartets is None:
+        q = engine.all_quartets(n)
+    else:
+        try:
+            q = engine.check_quartets(_quartet_positions(quartets, n, taxa), n)
+        except ValueError as e:
+            raise ValueError(str(e) if str(e).startswith("quartet_scores") else f"quartet_scores: {e}") from None
+    if q.shape[0] == 0:
+        return np.zeros((0, 3), np.float64)
+    aln = _as_alignment(alignment, want_sm=False, want_planes=True)
+    return engine.quartet_scores(aln, q, method).cpu().numpy()

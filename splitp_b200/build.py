@@ -20,7 +20,7 @@ INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB = os.path.join(HERE, "libsplitp_b200.so")
 OBJ = os.path.join(HERE, "build")
 SOURCES = ["pack.cu", "count.cu", "wide.cu", "flatten.cu", "pairs.cu", "gram.cu", "score.cu", "sparse.cu", "marginals.cu", "mi_batch.cu",
-           "bootstrap.cu", "agglomerate.cu", "pair_rows.cu"]
+           "bootstrap.cu", "agglomerate.cu", "pair_rows.cu", "quartets.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
               "-I", INCLUDE]
 

@@ -2276,3 +2276,138 @@ def window_tree_masks(aln, windows, first_taxon, timer=None):
         masks[idx], scores[idx] = m, sc
         del stack
     return masks.cpu().numpy().view(np.uint64), scores.cpu().numpy()
+
+
+# --------------------------------------------------------------------------------------------
+# quartet split scores: joint tables of every quartet from the bit planes (csrc/quartets.cu)
+# --------------------------------------------------------------------------------------------
+QUARTET_BATCH_BYTES = 1 << 30  # device memory of one quartet group: quartet list, tables, Grams, scores
+# device bytes per quartet of a group: uint8 positions, uint64 [256] table, flattening workspace, sorted and mapped scores
+_QUARTET_BYTES = 4 + 8 * 256 + 8 * (3 * 256 + 2) + 2 * 24 + 24
+
+
+def all_quartets(n):
+    """Every quartet of n taxa as int64 numpy [C(n, 4), 4], in itertools.combinations(range(n), 4) order.  Built a column at a
+    time: each row is followed by every larger position, in ascending order, so the rows stay in lexicographic order."""
+    X = np.arange(max(int(n), 0), dtype=np.int64)[:, None]
+    for _ in range(3):
+        last = X[:, -1]
+        cnt = n - 1 - last
+        start = np.repeat(np.cumsum(cnt) - cnt, cnt)
+        new = np.repeat(last + 1, cnt) + (np.arange(int(cnt.sum()), dtype=np.int64) - start)
+        X = np.concatenate([np.repeat(X, cnt, axis=0), new[:, None]], axis=1)
+    return X
+
+
+def check_quartets(quartets, n):
+    """int64 numpy [Q, 4] of taxon positions; ValueError unless every row holds four distinct positions in [0, n)."""
+    q = np.asarray(quartets)
+    if q.size == 0:
+        return np.zeros((0, 4), np.int64)
+    if q.dtype.kind not in "iu" or q.ndim != 2 or q.shape[1] != 4:
+        raise ValueError(f"quartets must be an integer [Q, 4] array of taxon positions (got {q.dtype} {list(q.shape)})")
+    if (q >= n).any() or (q < 0).any():
+        raise ValueError(f"quartet positions must lie in [0, {n})")
+    q = q.astype(np.int64)
+    if (np.diff(np.sort(q, axis=1), axis=1) == 0).any():
+        raise ValueError("every quartet needs four distinct taxa")
+    return q
+
+
+def _quartet_column_lut():
+    """[64][3]: for a quartet whose positions have the ranks (r0, r1, r2, r3) (code 16 r0 + 4 r1 + r2), the column of the
+    sorted quartet that holds the bipartition of column j = {q0, q_(j+1)} | the other two."""
+    import itertools
+    lut = np.zeros((64, 3), np.int64)
+    for rank in itertools.permutations(range(4)):
+        for j in range(3):
+            pair = (0, j + 1) if 0 in (rank[0], rank[j + 1]) else tuple(i for i in (1, 2, 3) if i != j + 1)
+            partner = pair[1] if rank[pair[0]] == 0 else pair[0]
+            lut[16 * rank[0] + 4 * rank[1] + rank[2], j] = rank[partner] - 1
+    return lut
+
+
+_QUARTET_LUT = _quartet_column_lut()
+
+
+def quartet_column_map(quartets):
+    """(quartets sorted by position, int64 [Q, 3] column map): column j of quartet q as written is column map[q, j] of its
+    sorted form.  Scoring the sorted form and gathering makes a bipartition's score independent of how a quartet is written."""
+    q = np.asarray(quartets, dtype=np.int64).reshape(-1, 4)
+    rank = np.argsort(np.argsort(q, axis=1, kind="stable"), axis=1, kind="stable")
+    return np.sort(q, axis=1), _QUARTET_LUT[16 * rank[:, 0] + 4 * rank[:, 1] + rank[:, 2]]
+
+
+def _planes_of(aln, what):
+    if aln.planes is None:
+        raise ValueError(f"{what} need the taxon-major bit planes (pack(want_planes=True))")
+    if not 4 <= aln.n <= _lib.SPB_MAX_TAXA:
+        raise ValueError(f"{what}: 4 to {_lib.SPB_MAX_TAXA} taxa (got {aln.n})")
+
+
+def _quartet_tables(aln, d_q):
+    """uint64 tables (int64 [Q, 256]) of the quartets d_q (uint8 [Q, 4] on the device) over all sites."""
+    Q = int(d_q.shape[0])
+    tables = _zeros((Q, 256), torch.int64)
+    call("spb_quartet_tables", _p(aln.planes), _p(aln.valid), aln.n, aln.plane_words, 0, (aln.N + 31) // 32, _p(d_q), Q, _p(tables),
+         _st())
+    return tables
+
+
+def quartet_tables(aln, quartets):
+    """Joint counts of the 256 states of every quartet (int64 [Q, 256] on the device, uint64 values) over the usable sites of
+    the DeviceAlignment: cell 64 x_a + 16 x_b + 4 x_c + x_d for the quartet (a, b, c, d) as written."""
+    _planes_of(aln, "quartet tables")
+    q = check_quartets(quartets, aln.n)
+    if q.shape[0] == 0:
+        return _zeros((0, 256), torch.int64)
+    return _quartet_tables(aln, torch.from_numpy(q.astype(np.uint8)).to(device()))
+
+
+def quartet_scores(aln, quartets, method=Method.flattening, timer=None):
+    """Scores of the three 2|2 splits of every quartet: float64 [Q, 3] on the device, column 0 = {a,b}|{c,d}, 1 = {a,c}|{b,d},
+    2 = {a,d}|{b,c} for the quartet (a, b, c, d) as written.  Every quartet is scored in its sorted form and the columns are
+    mapped back, so a bipartition gets the same float however its quartet is written.
+      Method.flattening          split_score of the reduced count flattening (spb_quartet_flattening_scores)
+      Method.mutual_information  rank-1 divergence of the flattening of count / usable sites (spb_quartet_mi_scores)
+      Method.subflattening       the masks of the three splits through subflatten_scores, bitwise score_splits
+    Quartets run in groups of at most QUARTET_BATCH_BYTES; a score does not depend on the grouping.  `timer` (PhaseTimer)
+    gets the spans "tables" and "score"."""
+    if method not in (Method.flattening, Method.subflattening, Method.mutual_information):
+        raise NotImplementedError("quartet_scores: Method.flattening, Method.subflattening or Method.mutual_information")
+    _planes_of(aln, "quartet scores")
+    q = check_quartets(quartets, aln.n)
+    Q = int(q.shape[0])
+    out = _empty((Q, 3), torch.float64)
+    if Q == 0:
+        return out
+    srt, cmap = quartet_column_map(q)
+    pt = None
+    if method == Method.subflattening:
+        with _span(timer, "tables"):
+            pt = pair_finalize(pair_raw(aln), aln.n, -1.0)  # the tables score_splits scores against
+    g = max(1, QUARTET_BATCH_BYTES // _QUARTET_BYTES)
+    for q0 in range(0, Q, g):
+        part = srt[q0:q0 + g]
+        k = int(part.shape[0])
+        if method == Method.subflattening:
+            bit = np.left_shift(np.uint64(1), part.astype(np.uint64))
+            ma = np.stack([bit[:, 0] | bit[:, 1], bit[:, 0] | bit[:, 2], bit[:, 0] | bit[:, 3]], axis=1).reshape(-1)
+            mb = np.stack([bit[:, 2] | bit[:, 3], bit[:, 1] | bit[:, 3], bit[:, 1] | bit[:, 2]], axis=1).reshape(-1)
+            with _span(timer, "score"):
+                sc = subflatten_scores(pt, ma, mb)
+        else:
+            with _span(timer, "tables"):
+                tables = _quartet_tables(aln, torch.from_numpy(part.astype(np.uint8)).to(device()))
+            sc = _empty(3 * k, torch.float64)
+            with _span(timer, "score"):
+                if method == Method.flattening:
+                    ws = _empty(int(lib.spb_quartet_flattening_ws(k)), torch.float64)
+                    call("spb_quartet_flattening_scores", _p(tables), k, _p(ws), _p(sc), _st())
+                    del ws
+                else:
+                    call("spb_quartet_mi_scores", _p(tables), k, _p(sc), _st())
+            del tables
+        cols = torch.from_numpy(cmap[q0:q0 + g]).to(device())
+        out[q0:q0 + k] = torch.gather(sc.view(k, 3), 1, cols)
+    return out
