@@ -123,8 +123,7 @@ def windows_case(n, B, host_windows, S=16):
 def parent_route(codes, splits, method, B, seed):
     """bootstrap_scores as the parent commit computed it: the same counting, then one scorer call per replicate table."""
     ss = batch.SplitScorer(splits, None, method)
-    n = codes.shape[0]
-    table = ss._count(codes) if n <= eng.NARROW_MAX_TAXA else ss._count_wide(codes)
+    table = ss._count(codes)
     out = eng._empty((B, len(splits)), torch.float64)
     for b, tb in enumerate(eng.bootstrap_tables(table, B, seed)):
         if method == Method.subflattening:

@@ -37,7 +37,8 @@ import numpy as np
 import torch
 
 from . import engine
-from .engine import PhaseTimer, _span  # noqa: F401  (PhaseTimer is re-exported: bench.py's `phase_ms`)
+# re-exported: PhaseTimer for bench.py's `phase_ms`, the flattening route for callers of score_splits
+from .engine import DENSE_FLATTENING_MAX_TAXA, PhaseTimer, _span, uses_sparse_flattening  # noqa: F401
 from .enums import Method
 
 
@@ -113,27 +114,29 @@ def _num_taxa(alignment):
     return int(alignment.shape[0]) if hasattr(alignment, "shape") else len(alignment)
 
 
-# Flattening scores of alignments with more taxa than this go through engine.sparse_flattening_scores: the dense count
-# flattenings of CountScorer (4^a x 4^b bytes per split, at least 16 per launch) stop fitting in memory at 17 taxa.
-DENSE_FLATTENING_MAX_TAXA = 16
+class _Counter:
+    """An alignment (any form _as_alignment takes) packed once for pattern counting.  Calling it counts the sites
+    [site_begin, site_end): up to 31 taxa engine.count_patterns of the packed alignment `aln` (a PatternTable, uint64 keys),
+    from 32 to 64 taxa engine.count_patterns_wide of `wide` = pack_wide's (wide, valid, n, N) (a WideTable, 128-bit keys,
+    divisor = usable sites).  The packed forms hold 32 taxa per site word, so above 31 taxa they raise
+    NotImplementedError; `fn` names the entry point in its message."""
 
+    def __init__(self, fn, alignment):
+        n = _num_taxa(alignment)
+        self.aln = self.wide = self.taxa = None
+        if n <= engine.NARROW_MAX_TAXA:
+            self.aln = _as_alignment(alignment, want_sm=True, want_planes=False)
+            return
+        if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
+            raise NotImplementedError(f"{fn} of {n} taxa needs the alignment as characters (dict, array or tensor): "
+                                      "the packed forms hold at most 32 taxa per site word")
+        chars, is_ascii, self.taxa = _chars(alignment)
+        self.wide = engine.pack_wide(chars, is_ascii)
 
-def uses_sparse_flattening(n_taxa):
-    return n_taxa > DENSE_FLATTENING_MAX_TAXA
-
-
-def _sparse_table(alignment):
-    """Pattern table of an alignment of 17..64 taxa: uint64 keys up to 31 taxa, 128-bit keys (raw counts as values) above."""
-    n = _num_taxa(alignment)
-    if n <= engine.NARROW_MAX_TAXA:
-        return engine.count_patterns(_as_alignment(alignment, want_sm=True, want_planes=False))
-    if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
-        raise NotImplementedError(f"flattening scores of {n} taxa need the alignment as characters (dict, array or tensor): "
-                                  "the packed forms hold at most 32 taxa per site word")
-    chars, is_ascii, taxa = _chars(alignment)
-    wide, valid, n, N = engine.pack_wide(chars, is_ascii)
-    keys, counts = engine.count_patterns_wide(wide, valid, n, N).compact()
-    return engine.WidePatternTable(n, keys, (counts.to(torch.int64) & 0xFFFFFFFF).to(torch.float64), taxa)
+    def __call__(self, site_begin=0, site_end=None):
+        if self.aln is not None:
+            return engine.count_patterns(self.aln, site_begin, site_end)
+        return engine.count_patterns_wide(*self.wide, site_begin, site_end, taxa=self.taxa)
 
 
 def _positions(splits, taxa):
@@ -199,7 +202,9 @@ class SplitScorer:
             ma, mb = engine.masks_from_splits(self.idx_mine)
             dev = engine.device()
             self.masks = (torch.from_numpy(ma.view(np.int64)).to(dev), torch.from_numpy(mb.view(np.int64)).to(dev))
-        elif method not in (Method.flattening, Method.mutual_information):
+        elif method in (Method.flattening, Method.mutual_information):
+            self.scorer = engine.TableScorer(self.idx_mine, method)
+        else:
             raise NotImplementedError("score_splits: Method.flattening, Method.subflattening or Method.mutual_information")
 
     REFIT_DAMPING = 0.5
@@ -245,7 +250,7 @@ class SplitScorer:
         self._fixed = {a: self._fixed[a] + d * (fixed[a] - self._fixed[a]) for a in fixed}
         self._cut()
 
-    def device_scores(self, alignment, gram_hook=None):
+    def device_scores(self, alignment):
         """Scores of ALL splits as a device tensor.  `alignment`: this rank's site shard, or the whole alignment when the
         scorer was built with sites="replicated" (any form _as_alignment takes)."""
         import torch.distributed as dist
@@ -257,22 +262,10 @@ class SplitScorer:
         if refit:
             ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             ev0.record()
-        if self.method == Method.flattening and uses_sparse_flattening(_num_taxa(alignment)):
-            with _span(t, "count"):
-                table = _sparse_table(alignment)
-            with _span(t, "sparse"):
-                out = engine.sparse_flattening_scores(table, self.idx_mine)
-        elif self.method == Method.flattening:
+        if self.scorer is not None:  # flattening, mutual information: the pattern table of the whole alignment
             table = self._count(alignment)
-            if self.scorer is None:
-                self.scorer = engine.CountScorer(table)
-            self.scorer.table = table
-            self.scorer.timer = t
-            out = self.scorer.score_many(self.idx_mine, big_hook=gram_hook)
-        elif self.method == Method.mutual_information:
-            table = self._count(alignment) if _num_taxa(alignment) <= engine.NARROW_MAX_TAXA else self._count_wide(alignment)
-            with _span(t, "mi"):
-                out = engine.rank1_divergence_scores(table, self.idx_mine)
+            self.scorer.splits_idx, self.scorer.timer = self.idx_mine, t  # a re-cut of the partition replaces idx_mine
+            out = self.scorer(table)
         else:
             with _span(t, "h2d+pack"):
                 aln = _as_alignment(alignment, want_sm=False, want_planes=True)
@@ -299,31 +292,21 @@ class SplitScorer:
         return res
 
     def _count(self, alignment):
-        """Pattern table (uint64 keys, up to 31 taxa) of the whole alignment from this rank's part of it."""
+        """Pattern table of the whole alignment from this rank's part of it (see _Counter): a PatternTable up to 31 taxa,
+        a WideTable from 32 to 64 taxa."""
         from . import distributed as spd
         t = self.timer
         with _span(t, "h2d+pack"):
-            aln = _as_alignment(alignment, want_sm=True, want_planes=False)
+            count = _Counter("score_splits", alignment)
         with _span(t, "count"):
-            if aln.n <= engine.DIRECT_MAX_TAXA:
-                return engine.count_patterns(aln, gather_fn=self._timed_gather if self.gather_fn else None)
-            if self.count_world > 1:  # hashed tables: gather + hash merge on every rank
-                return spd.count_patterns_sharded(aln, self.rank, self.world, self.group, local=True)
-            return engine.count_patterns(aln)
-
-    def _count_wide(self, alignment):
-        """engine.WideTable (128-bit keys, 32..64 taxa; divisor = usable sites) of the whole alignment from this rank's part."""
-        from . import distributed as spd
-        if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
-            raise NotImplementedError(f"scores of {alignment.n} taxa need the alignment as characters (dict, array or tensor): "
-                                      "the packed forms hold at most 32 taxa per site word")
-        with _span(self.timer, "h2d+pack"):
-            chars, is_ascii, taxa = _chars(alignment)
-            wide, valid, n, N = engine.pack_wide(chars, is_ascii)
-        with _span(self.timer, "count"):
-            if self.count_world > 1:
-                return spd.count_patterns_wide_sharded(wide, valid, n, N, self.rank, self.world, self.group, local=True)
-            return engine.count_patterns_wide(wide, valid, n, N, taxa=taxa)
+            if self.count_world == 1:
+                return count()
+            if count.wide is not None:
+                return spd.count_patterns_wide_sharded(*count.wide, self.rank, self.world, self.group, local=True)
+            if count.aln.n <= engine.DIRECT_MAX_TAXA:  # direct tables: the ranks exchange their compacted lists
+                return engine.count_patterns(count.aln, gather_fn=self._timed_gather)
+            # hashed tables: gather + hash merge on every rank
+            return spd.count_patterns_sharded(count.aln, self.rank, self.world, self.group, local=True)
 
     def _timed_gather(self, keys, counts):
         with _span(self.timer, "exchange"):
@@ -393,10 +376,8 @@ def bootstrap_scores(alignment, splits, method=Method.flattening, replicates=100
     seed = _bootstrap_checks("bootstrap_scores", replicates, seed)
     if taxa is None and isinstance(alignment, dict):
         taxa = list(alignment.keys())
-    # one process: the SplitScorer holds the split positions, the subflattening masks and the counting stage of score_splits
-    ss = SplitScorer(splits, taxa, method)
-    n = _num_taxa(alignment)
-    table = ss._count(alignment) if n <= engine.NARROW_MAX_TAXA else ss._count_wide(alignment)
+    ss = SplitScorer(splits, taxa, method)  # split positions and subflattening masks, as score_splits builds them
+    table = _Counter("bootstrap_scores", alignment)()
     out = engine.bootstrap_scores_multi([table], int(replicates), [seed], method, ss.idx_all, ss.masks)
     return out[0].cpu().numpy()
 
@@ -501,8 +482,7 @@ def bootstrap_trees(alignment, replicates=100, seed=0, taxa=None, method=Method.
         raise ValueError(f"bootstrap_trees: 2 to {engine._lib.SPB_MAX_TAXA} taxa (got {n})")
     taxa, wanted = _tree_taxa("bootstrap_trees", alignment, n, taxa, splits)
     first = min(range(n), key=lambda i: taxa[i])
-    ss = SplitScorer([], taxa, Method.subflattening)  # the counting stage of bootstrap_scores: the same replicate tables
-    table = ss._count(alignment) if n <= engine.NARROW_MAX_TAXA else ss._count_wide(alignment)
+    table = _Counter("bootstrap_trees", alignment)()  # the counting of bootstrap_scores: the same replicate tables
     masks, _ = engine.bootstrap_tree_masks(table, int(replicates), seed, first)
     trees = _trees_of_masks(masks, taxa)
     return BootstrapTrees(trees[0], _support(masks, wanted, n), trees[1:])
@@ -580,7 +560,7 @@ def window_scores(alignment, splits, windows, method=Method.flattening, taxa=Non
     both hold at least two taxa and 0.0 for the others (all-zero pair tables); flattening up to 16 taxa the same (empty count
     flattening), above 16 taxa 0.0; mutual information 0.0.
     Runs on one GPU: inside a torch.distributed group of several processes it raises NotImplementedError."""
-    n, wins = _window_inputs("window_scores", alignment, windows)
+    _, wins = _window_inputs("window_scores", alignment, windows)
     if taxa is None and isinstance(alignment, dict):
         taxa = list(alignment.keys())
     ss = SplitScorer(splits, taxa, method)  # split positions and subflattening masks, as score_splits builds them
@@ -590,37 +570,10 @@ def window_scores(alignment, splits, windows, method=Method.flattening, taxa=Non
     if method == Method.subflattening:
         aln = _as_alignment(alignment, want_sm=False, want_planes=True)
         return engine.window_subflatten_scores(aln, wins, *ss.masks).cpu().numpy()
-    if n <= engine.NARROW_MAX_TAXA:
-        aln = _as_alignment(alignment, want_sm=True, want_planes=False)
-
-        def table_of(b, e):
-            return engine.count_patterns(aln, b, e)
-    else:
-        if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
-            raise NotImplementedError(f"scores of {n} taxa need the alignment as characters (dict, array or tensor): "
-                                      "the packed forms hold at most 32 taxa per site word")
-        chars, is_ascii, names = _chars(alignment)
-        wide, valid, _, N = engine.pack_wide(chars, is_ascii)
-
-        def table_of(b, e):
-            return engine.count_patterns_wide(wide, valid, n, N, b, e, taxa=names)
+    count, scorer = _Counter("window_scores", alignment), engine.TableScorer(idx, method)
     out = engine._empty((W, len(idx)), torch.float64)
-    scorer = None
     for w, (b, e) in enumerate(wins.tolist()):
-        tb = table_of(b, e)
-        if method == Method.flattening and uses_sparse_flattening(n):
-            if isinstance(tb, engine.WideTable):  # the table _sparse_table builds above 31 taxa
-                keys, counts = tb.compact()
-                tb = engine.WidePatternTable(n, keys, (counts.to(torch.int64) & 0xFFFFFFFF).to(torch.float64), names)
-            out[w] = engine.sparse_flattening_scores(tb, idx)
-        elif method == Method.flattening:
-            if scorer is None:
-                scorer = engine.CountScorer(tb)
-            else:
-                scorer.table = tb
-            out[w] = scorer.score_many(idx)
-        else:
-            out[w] = engine.rank1_divergence_scores(tb, idx)
+        out[w] = scorer(count(b, e))
     return out.cpu().numpy()
 
 
@@ -635,11 +588,7 @@ def window_trees(alignment, windows, taxa=None):
     window_scores; leaf names are the dict's keys or `taxa`, else erickson_SVD's default names in row order.  Runs on one
     GPU: inside a torch.distributed group of several processes it raises NotImplementedError."""
     n, wins = _window_inputs("window_trees", alignment, windows)
-    if taxa is None:
-        taxa = list(alignment.keys()) if isinstance(alignment, dict) else _default_taxa(n)
-    taxa = list(taxa)
-    if len(taxa) != n or len(set(taxa)) != n:
-        raise ValueError(f"window_trees: taxa must be {n} distinct names, one per row")
+    taxa, _ = _tree_taxa("window_trees", alignment, n, taxa, None)
     if wins.shape[0] == 0:
         return []
     first = min(range(n), key=lambda i: taxa[i])
@@ -673,7 +622,7 @@ def window_bootstrap_trees(alignment, windows, replicates=100, seed=0, taxa=None
     taxa, wanted = _tree_taxa(fn, alignment, n, taxa, splits)
     if wins.shape[0] == 0:
         return []
-    tables, seeds = _window_sources(fn, alignment, n, wins, seed)
+    tables, seeds = _window_counts(fn, alignment, wins, seed)
     first = min(range(n), key=lambda i: taxa[i])
     masks, _ = engine.bootstrap_tree_masks_multi(tables, int(replicates), seeds, first)
     del tables
@@ -683,27 +632,14 @@ def window_bootstrap_trees(alignment, windows, replicates=100, seed=0, taxa=None
             for w in range(masks.shape[0])]
 
 
-def _window_sources(fn, alignment, n, wins, seed):
+def _window_counts(fn, alignment, wins, seed):
     """(pattern count table of every window, its bootstrap seed engine.window_bootstrap_seed(seed, b_w, e_w)): the
-    alignment is packed once and every window is counted from the packed sites.  ValueError naming the first window
-    without a usable site; above 31 taxa the packed forms raise NotImplementedError."""
-    if n <= engine.NARROW_MAX_TAXA:
-        aln = _as_alignment(alignment, want_sm=True, want_planes=False)
-
-        def table_of(b, e):
-            return engine.count_patterns(aln, b, e)
-    else:
-        if isinstance(alignment, (engine.DeviceAlignment, HostPlanes)):
-            raise NotImplementedError(f"{fn} of {n} taxa needs the alignment as characters (dict, array or tensor): "
-                                      "the packed forms hold at most 32 taxa per site word")
-        chars, is_ascii, names = _chars(alignment)
-        wide, valid, _, N = engine.pack_wide(chars, is_ascii)
-
-        def table_of(b, e):
-            return engine.count_patterns_wide(wide, valid, n, N, b, e, taxa=names)
+    alignment is packed once and every window is counted from the packed sites (_Counter).  ValueError naming the first
+    window without a usable site."""
+    count = _Counter(fn, alignment)
     tables = []
     for w, (b, e) in enumerate(wins.tolist()):
-        tables.append(table_of(b, e))
+        tables.append(count(b, e))
         if tables[-1].divisor == 0:
             raise ValueError(f"{fn}: window {w} [{b}, {e}) has no usable site")
     return tables, [engine.window_bootstrap_seed(seed, b, e) for b, e in wins.tolist()]
@@ -728,14 +664,14 @@ def window_bootstrap_scores(alignment, splits, windows, method=Method.flattening
     site raises ValueError.  Runs on one GPU: inside a torch.distributed group of several processes it raises
     NotImplementedError."""
     fn = "window_bootstrap_scores"
-    n, wins = _window_inputs(fn, alignment, windows)
+    _, wins = _window_inputs(fn, alignment, windows)
     seed = _bootstrap_checks(fn, replicates, seed)
     if taxa is None and isinstance(alignment, dict):
         taxa = list(alignment.keys())
     ss = SplitScorer(splits, taxa, method)  # split positions and subflattening masks, as score_splits builds them
     if wins.shape[0] == 0:
         return np.zeros((0, int(replicates), ss.S), np.float64)
-    tables, seeds = _window_sources(fn, alignment, n, wins, seed)
+    tables, seeds = _window_counts(fn, alignment, wins, seed)
     out = engine.bootstrap_scores_multi(tables, int(replicates), seeds, method, ss.idx_all, ss.masks)
     del tables
     return out.cpu().numpy()

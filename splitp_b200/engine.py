@@ -884,7 +884,7 @@ class CountScorer:
             return torch.full((1,), float("nan"), dtype=torch.float64, device=G.device)
         return score_gram(G, k)
 
-    def score_many(self, splits_idx, reduced=False, max_batch=512, max_batch_bytes=None, big_hook=None):
+    def score_many(self, splits_idx, reduced=False, max_batch=512, max_batch_bytes=None):
         """Scores of many splits.  Dense count flattenings of equal shape are batched: their Gram matrices are
         built up to 64 at a time into G[b] and ONE batched eigen-solver call scores up to `max_batch` of them
         (the Jacobi / Krylov kernels are latency-bound per matrix, so batching is what keeps all SMs busy)."""
@@ -1051,10 +1051,15 @@ def _side_keys(table, idx):
     return flatten_coo(table, idx, [])[0]
 
 
+def _u32_f64(counts):
+    """uint32 counts held in an int32 tensor, as float64."""
+    return (counts.to(torch.int64) & 0xFFFFFFFF).to(torch.float64)
+
+
 def _table_values(table):
     """Values of the non-zeros: raw counts as fp64 (the score is scale-invariant) or the mapping's values."""
     if table.counts is not None:
-        return (table.counts.to(torch.int64) & 0xFFFFFFFF).to(torch.float64)
+        return _u32_f64(table.counts)
     return table.values
 
 
@@ -1178,9 +1183,11 @@ def _sparse_scores(sizes, make, timer=None):
 
 def sparse_flattening_scores(table, splits_idx, timer=None):
     """Flattening scores (split_score of the flattening, phylogenetics.py:280-328) of many splits [(idx_a, idx_b), ...] of a
-    PatternTable (counts or values) or WidePatternTable, up to 64 taxa, without materialising any flattening.  Every split must
-    place every taxon on exactly one side (ValueError otherwise).  Returns a float64 device tensor, one score per split; a split
-    whose Gram side has at most 4 distinct rows scores 0.0."""
+    PatternTable (counts or values), WidePatternTable or the WideTable of count_patterns_wide, up to 64 taxa, without
+    materialising any flattening.  Every split must place every taxon on exactly one side (ValueError otherwise).  Returns a
+    float64 device tensor, one score per split; a split whose Gram side has at most 4 distinct rows scores 0.0."""
+    if isinstance(table, WideTable):
+        table = _table_of_counts(table, *table.compact(), table.divisor)  # _table_values reads its raw counts
     for ia, ib in splits_idx:
         if not covers_all(table.n, ia, ib):
             raise ValueError("sparse flattening scores need a split that places every taxon on exactly one side")
@@ -1211,6 +1218,43 @@ def sparse_matrix_score(rows, cols, vals):
     Cc = int(cols.max().item()) + 1 if cols.shape[0] else 0
     p = SparsePlan(rows, cols, R, Cc, vals) if R <= Cc else SparsePlan(cols, rows, Cc, R, vals)
     return _sparse_scores([(p.k, p.C, p.nnz)], lambda i: p)
+
+
+# Flattening scores of tables with more taxa than this go through sparse_flattening_scores: the dense count flattenings of
+# CountScorer (4^a x 4^b bytes per split, at least 16 per launch) stop fitting in memory at 17 taxa.
+DENSE_FLATTENING_MAX_TAXA = 16
+
+
+def uses_sparse_flattening(n_taxa):
+    return n_taxa > DENSE_FLATTENING_MAX_TAXA
+
+
+class TableScorer:
+    """Scores of one split list [(idx_a, idx_b), ...] for one count table at a time (a PatternTable of count_patterns or
+    bootstrap_tables, a WideTable, or a WidePatternTable of bootstrap_tables), with the scorer score_splits uses:
+      Method.flattening          CountScorer up to DENSE_FLATTENING_MAX_TAXA taxa, kept between tables so that its buffers
+                                 and encoded splits are reused; sparse_flattening_scores above
+      Method.mutual_information  rank1_divergence_scores
+    `timer` (PhaseTimer) gets the CountScorer's spans, "sparse" or "mi"."""
+
+    def __init__(self, splits_idx, method):
+        self.splits_idx, self.method = splits_idx, method
+        self.timer = None
+        self.dense = None  # the CountScorer, built for the first table it scores
+
+    def __call__(self, table):
+        if self.method == Method.mutual_information:
+            with _span(self.timer, "mi"):
+                return rank1_divergence_scores(table, self.splits_idx)
+        if uses_sparse_flattening(table.n):
+            with _span(self.timer, "sparse"):
+                return sparse_flattening_scores(table, self.splits_idx)
+        if self.dense is None:
+            self.dense = CountScorer(table)
+        else:
+            self.dense.table = table
+        self.dense.timer = self.timer
+        return self.dense.score_many(self.splits_idx)
 
 
 # --------------------------------------------------------------------------------------------
@@ -1267,9 +1311,8 @@ def pair_tables_from_alignment(aln, as_counts=False):
     return pair_finalize(raw, aln.n, usable)
 
 
-def pair_tables_from_table(table, as_counts=False, T=None, total=None):
-    """Pair tables of a pattern table (values, or its counts when as_counts and it has them).  T (float64 [n, n, 4, 4]) and
-    total (float64 [1]), when given, receive the result: slices of a buffer that stacks the tables of several patterns."""
+def pair_tables_from_table(table, as_counts=False):
+    """Pair tables of a pattern table (values, or its counts when as_counts and it has them)."""
     n = table.n
     vals = table.counts.to(torch.float64) if (as_counts and table.counts is not None) else table.values_f64()
     if isinstance(table, WidePatternTable):  # deterministic fp64 tensor-core product (csrc/wide.cu)
@@ -1279,8 +1322,7 @@ def pair_tables_from_table(table, as_counts=False, T=None, total=None):
     else:
         N_tab = _zeros((n, n, 4, 4), torch.float64)
         call("spb_pair_tables_weighted", _p(table.keys), _p(vals.contiguous()), table.num, n, _p(N_tab), _st())
-    T = _empty((n, n, 4, 4), torch.float64) if T is None else T
-    total = _empty(1, torch.float64) if total is None else total
+    T, total = _empty((n, n, 4, 4), torch.float64), _empty(1, torch.float64)
     call("spb_pair_transform", _p(N_tab), n, _p(T), _p(total), _st())
     return PairTables(n, N_tab, T, total)
 
@@ -1324,29 +1366,41 @@ def subflatten_scores(pt, masks_a, masks_b=None):
 class SubflattenTables:
     """The subflattening scoring tables of several pattern tables, stacked for subflatten_scores_multi: up to 43 taxa the
     triple tables (spb_subflatten_tables_doubles(n) doubles each), from 44 taxa the tables T [n][n][4][4] of the staged
-    kernel; `total` holds one total per table.  add(i, table) fills slot i from the pair tables of the table's counts."""
+    kernel; `total` holds one total per table.  A slot is filled from its pair tables T (add_pair_tables), from its joint
+    pair tables N (add_joint_tables) or from a pattern table's counts (add)."""
 
     def __init__(self, n, count):
         self.n = n
         per = int(lib.spb_subflatten_tables_doubles(n)) if n <= SUBFLATTEN_TABLES_MAX_TAXA else 16 * n * n
         self.data = _empty((count, per), torch.float64)
         self.total = _empty(count, torch.float64)
+        self._T = None  # T of add_joint_tables up to 43 taxa, where the slots hold triple tables
 
     @staticmethod
     def bytes_per_table(n):
         return 8 * (int(lib.spb_subflatten_tables_doubles(n)) if n <= SUBFLATTEN_TABLES_MAX_TAXA else 16 * n * n) + 8
 
     def add(self, i, table):
-        n, total = self.n, self.total[i:i + 1]
+        """Fills slot i from the pair tables of the table's counts."""
+        pt = pair_tables_from_table(table, as_counts=True)
+        self.add_pair_tables(i, pt.T, pt.total)
+
+    def add_joint_tables(self, i, N_tab):
+        """Fills slot i from joint pair tables N float64 [n, n, 4, 4] on the device: spb_pair_transform, then
+        add_pair_tables."""
+        n = self.n
         if n > SUBFLATTEN_TABLES_MAX_TAXA:
-            pair_tables_from_table(table, as_counts=True, T=self.data[i].view(n, n, 4, 4), total=total)
-            return
-        pt = pair_tables_from_table(table, as_counts=True, total=total)
-        # no splits: the call only tabulates the triple tables of pt into slot i
-        call("spb_subflatten_score_tables", _p(pt.T), _p(pt.total), n, None, None, 0, None, _p(self.data[i]), 0, _st())
+            T = self.data[i].view(n, n, 4, 4)
+        else:
+            if self._T is None:
+                self._T = _empty((n, n, 4, 4), torch.float64)
+            T = self._T
+        call("spb_pair_transform", _p(N_tab), n, _p(T), _p(self.total[i:i + 1]), _st())
+        self.add_pair_tables(i, T, self.total[i:i + 1])
 
     def add_pair_tables(self, i, T, total):
-        """Fills slot i from finalized pair tables: T float64 [n, n, 4, 4] and total float64 [1] on the device."""
+        """Fills slot i from finalized pair tables: T float64 [n, n, 4, 4] and total float64 [1] on the device (either may
+        be the slot's own storage)."""
         n, slot = self.n, self.total[i:i + 1]
         if total.data_ptr() != slot.data_ptr():
             slot.copy_(total)
@@ -1354,6 +1408,7 @@ class SubflattenTables:
             if T.data_ptr() != self.data[i].data_ptr():
                 self.data[i].view(n, n, 4, 4).copy_(T)
             return
+        # no splits: the call only tabulates the triple tables of T into slot i
         call("spb_subflatten_score_tables", _p(T), _p(total), n, None, None, 0, None, _p(self.data[i]), 0, _st())
 
 
@@ -1546,12 +1601,10 @@ def rank1_divergence_scores(table, splits_idx, timer=None):
     PatternTable (counts with their divisor, or values), a WidePatternTable, or the WideTable of count_patterns_wide (counts
     divided by its usable sites).  Every split must place every taxon on exactly one side (ValueError otherwise); a split
     with an empty side scores 0.0.  Returns a float64 device tensor, one score per split."""
-    if isinstance(table, WideTable):
-        keys, vals = table.compact()  # sorted: the pattern order, and with it every summation order, is the table's own
-        kind, div = SPB_VAL_U32, table.divisor
-    else:
-        keys = table.keys.contiguous()
-        vals, kind, div = (table.counts, SPB_VAL_U32, table.divisor) if table.counts is not None else (table.values, SPB_VAL_F64, 0.0)
+    if isinstance(table, WideTable):  # sorted: the pattern order, and with it every summation order, is the table's own
+        table = _table_of_counts(table, *table.compact(), table.divisor)
+    keys = table.keys.contiguous()
+    vals, kind, div = (table.counts, SPB_VAL_U32, table.divisor) if table.counts is not None else (table.values, SPB_VAL_F64, 0.0)
     vals, n = vals.contiguous(), table.n
     for ia, ib in splits_idx:
         if not covers_all(n, ia, ib):
@@ -1862,10 +1915,11 @@ def bootstrap_tables(table, replicates, seed):
 
 
 def _table_of_counts(table, keys, counts, N):
-    """The pattern table of `keys` with uint32 `counts` and divisor N, in the form bootstrap_tables yields (see there)."""
+    """The pattern table of `keys` with uint32 `counts` and divisor N, in the form bootstrap_tables yields (see there); with
+    the compacted keys and counts of a WideTable and its divisor, the WidePatternTable the scorers read it as."""
     if keys.dim() == 1:
         return PatternTable(table.n, keys, counts=counts, divisor=float(N), taxa=table.taxa)
-    v = (counts.to(torch.int64) & 0xFFFFFFFF).to(torch.float64)
+    v = _u32_f64(counts)
     t = WidePatternTable(table.n, keys, torch.div(v, torch.full_like(v, float(N))), taxa=table.taxa)
     t.counts, t.divisor = counts, float(N)
     return t
@@ -1908,7 +1962,7 @@ def _pair_tables_compacted_rows(keys, rows, n):
     N_tab = _empty((R, n, n, 4, 4), torch.float64)
     for r in range(R):
         num = off[r + 1] - off[r]
-        vals = (oc[off[r]:off[r + 1]].to(torch.int64) & 0xFFFFFFFF).to(torch.float64)
+        vals = _u32_f64(oc[off[r]:off[r + 1]])
         ws = _empty(max(int(lib.spb_pair_tables_wide_ws(num, n)), 1), torch.float64)
         call("spb_pair_tables_wide", _p(ok[off[r]:off[r + 1]]), _p(vals), num, n, _p(N_tab[r]), _p(ws), _st())
     return N_tab
@@ -1948,9 +2002,8 @@ def bootstrap_group_tables(srcs, count, f0, f1, n, timer=None, own=True):
     s count + b is source s's own counts (b = 0) or its replicate b - 1; without `own`, replicate b.  Slot i holds what
     SubflattenTables.add gives
     for that table (bootstrap_tables' replicate table), bit for bit.  Up to COUNT_ROWS_MAX_TAXA taxa a source's count rows
-    go through spb_pair_tables_count_rows in one launch, above through spb_pair_tables_wide per compacted row; then
-    spb_pair_transform and the triple tables per row."""
-    staged = n <= SUBFLATTEN_TABLES_MAX_TAXA  # the triple tables are formed from T
+    go through spb_pair_tables_count_rows in one launch, above through spb_pair_tables_wide per compacted row; then each
+    row's joint tables fill its slot (SubflattenTables.add_joint_tables)."""
     stack = SubflattenTables(n, f1 - f0)
     for s in range(f0 // count, (f1 - 1) // count + 1):
         b0, b1 = max(f0, s * count) - s * count, min(f1, (s + 1) * count) - s * count
@@ -1965,15 +2018,9 @@ def bootstrap_group_tables(srcs, count, f0, f1, n, timer=None, own=True):
                     N_tab = _pair_tables_compacted_rows(srcs[s][0], rows, n)
             del rows
             with _span(timer, "triple tables"):
-                T = _empty((n, n, 4, 4), torch.float64) if staged else None
                 for r in range(b1 - b0):
-                    i = slot0 + r
-                    out = T if staged else stack.data[i]
-                    call("spb_pair_transform", _p(N_tab[r]), n, _p(out), _p(stack.total[i:i + 1]), _st())
-                    if staged:  # no splits: the call only tabulates the triple tables of T into slot i
-                        call("spb_subflatten_score_tables", _p(T), _p(stack.total[i:i + 1]), n, None, None, 0, None,
-                             _p(stack.data[i]), 0, _st())
-            del N_tab, T
+                    stack.add_joint_tables(slot0 + r, N_tab[r])
+            del N_tab
     return stack
 
 
@@ -2120,7 +2167,7 @@ def bootstrap_scores_multi(tables, replicates, seeds, method, splits_idx, masks=
                                  counts) + subflatten_scores_multi; masks = (masks_a, masks_b) of splits_idx as device
                                  tensors (SplitScorer.masks); rows in groups of at most BOOTSTRAP_SCORES_BATCH_BYTES
       Method.mutual_information  rank1_divergence_count_rows of every table's replicate count rows, divisor N
-      Method.flattening          every replicate table through CountScorer up to 16 taxa, sparse_flattening_scores above
+      Method.flattening          every replicate table through one TableScorer
     A score depends on its table, seed, replicate index and split only, never on the grouping.  ValueError for a table
     without usable sites."""
     seeds = [bootstrap_seed(s) for s in seeds]
@@ -2151,18 +2198,10 @@ def bootstrap_scores_multi(tables, replicates, seeds, method, splits_idx, masks=
             out[s] = rank1_divergence_count_rows(keys, lambda r0, r1, src=src: _bootstrap_rows(src, r0, r1, own=False), B, n,
                                                  float(N), splits_idx, row_cap=min(int(counts.shape[0]), N), timer=timer)
     elif method == Method.flattening:
-        from .batch import uses_sparse_flattening
-        scorer = None
+        scorer = TableScorer(splits_idx, method)
         for s, t in enumerate(tables):
             for b, tb in enumerate(bootstrap_tables(t, B, seeds[s])):
-                if uses_sparse_flattening(n):
-                    out[s, b] = sparse_flattening_scores(tb, splits_idx)
-                    continue
-                if scorer is None:
-                    scorer = CountScorer(tb)
-                else:
-                    scorer.table = tb
-                out[s, b] = scorer.score_many(splits_idx)
+                out[s, b] = scorer(tb)
     else:
         raise NotImplementedError("bootstrap scores: Method.flattening, Method.subflattening or Method.mutual_information")
     return out
@@ -2229,12 +2268,11 @@ def window_tables(aln, windows):
     wraw = (prefix[hi] - prefix[lo]).contiguous()
     del prefix
     stack = SubflattenTables(n, g)
-    staged = n <= SUBFLATTEN_TABLES_MAX_TAXA  # the triple tables are formed from T
-    T = _empty((g, 16 * n * n), torch.float64) if staged else stack.data
+    # from 44 taxa the slots hold T itself: the tables are finalized in place
+    T = stack.data if n > SUBFLATTEN_TABLES_MAX_TAXA else _empty((g, 16 * n * n), torch.float64)
     pair_finalize_rows(wraw, n, -1.0, T, stack.total)
-    if staged:
-        for w in range(g):
-            stack.add_pair_tables(w, T[w].view(n, n, 4, 4), stack.total[w:w + 1])
+    for w in range(g):
+        stack.add_pair_tables(w, T[w].view(n, n, 4, 4), stack.total[w:w + 1])
     return stack
 
 
